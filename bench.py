@@ -4,6 +4,7 @@
   python bench.py --gpus N --steps K --warmup W            (ours; one rank per GPU under torchrun for N>1)
   python bench.py --impl reference --steps K --warmup W    (CPU arm: the oracle port on all host threads)
   python bench.py --workload config2|config3|config3r|config4|config5 ...
+  python bench.py ... --dump-outputs DIR                   (also write what the last timed step computed, as .npy)
 
 A step = one pass of the hot path over one synthetic genome set (BASELINE.json configs):
   value : pairs/s with sketches already resident in HBM (prescreen + ANI/AF + edge gather), device-timed
@@ -46,7 +47,7 @@ SKDER_ANI, SKDER_AF = 99.5, 50.0           # skDER's default cutoffs (bin/skder:
 CPU_SAMPLE_CLADES, CPU_SAMPLE_PER_CLADE = 80, 5
 SEARCH_BATCH_MAX = int(os.environ.get("SKB_SEARCH_BATCH", "64"))  # queries searched per call at most (1 = strictly one by one)
 SEARCH_WORKLOADS = ("config4", "tiny4")  # low_mem_greedy: the `skani sketch` + `skani search` path
-REF_BUDGET_S = float(os.environ.get("SKB_REF_BUDGET_S", "240"))  # wall budget of the reference arm's timed steps
+DUMP_MAX_BYTES = 64 << 20  # --dump-outputs writes at most this much
 
 
 def cfg(name):
@@ -255,20 +256,15 @@ def run_reference(args):
         sample = cpu_triangle_components(args.workload, min(nc, CPU_SAMPLE_CLADES), CPU_SAMPLE_PER_CLADE, threads, GREEDY_SCREEN,
                                          GREEDY_MIN_AF)
     x_value, x_t = cpu_extrapolate(sample, n_full, pairs_full, surv_full, with_sketch=True)
-    # timed: FULL passes over the workload itself, as many of the requested steps as fit the wall budget (>= 1)
-    comps, t_begin = [], time.perf_counter()
-    for it in range(args.steps):
-        comps.append(cpu_triangle_components(args.workload, nc, per, threads, GREEDY_SCREEN, GREEDY_MIN_AF))
-        per_step_wall = (time.perf_counter() - t_begin) / len(comps)
-        if time.perf_counter() - t_begin + per_step_wall > REF_BUDGET_S:
-            break
+    # timed: --steps FULL passes over the workload itself
+    comps = [cpu_triangle_components(args.workload, nc, per, threads, GREEDY_SCREEN, GREEDY_MIN_AF) for _ in range(args.steps)]
     t_steps = [c["t_sketch"] + c["t_screen"] + c["t_ani"] for c in comps]
     t_full = float(np.mean(t_steps))
     value = pairs_full / t_full
     c0 = comps[-1]
-    sample_txt = ("the full workload, %d of the %d requested steps (wall budget %.0f s): %d genomes, %d pairs, %d survive the screen, "
+    sample_txt = ("the full workload, %d steps: %d genomes, %d pairs, %d survive the screen, "
                   "%d edges; per step: sketch %.2f s, inverted-index prescreen %.2f s, ANI/AF %.2f s on %d threads (genome generation "
-                  "not timed)" % (len(comps), args.steps, REF_BUDGET_S, c0["n"], c0["pairs"], c0["survivors"], c0["edges"],
+                  "not timed)" % (len(comps), c0["n"], c0["pairs"], c0["survivors"], c0["edges"],
                                   float(np.mean([c["t_sketch"] for c in comps])), float(np.mean([c["t_screen"] for c in comps])),
                                   float(np.mean([c["t_ani"] for c in comps])), threads))
     line = {
@@ -291,23 +287,25 @@ def run_reference(args):
 def run_reference_search(args, threads):
     nc, per, L = workload_shape(args.workload)
     s_clades = min(nc, int(os.environ.get("SKB_REF_SEARCH_CLADES", "20")))
-    r = None
-    for _ in range(max(1, min(args.warmup, 1)) + 1):
-        r = cpu_search_loop(args.workload, threads, s_clades, per)
+    for _ in range(args.warmup):
+        cpu_search_loop(args.workload, threads, s_clades, per)
+    runs = [cpu_search_loop(args.workload, threads, s_clades, per) for _ in range(args.steps)]
+    r = runs[-1]
+    t_sketch, t_loop = float(np.mean([x["t_sketch"] for x in runs])), float(np.mean([x["t_loop"] for x in runs]))
     # searches scale with representatives x database size: R ~ clades, each search touches N genomes' markers and
     # ~per same-clade survivors
     n_full = nc * per
-    t_search = r["t_loop"] / r["reps"]
-    t_full = r["t_sketch"] / r["n"] * n_full + (r["reps"] / s_clades * nc) * t_search * (n_full / r["n"])
+    t_search = t_loop / r["reps"]
+    t_full = t_sketch / r["n"] * n_full + (r["reps"] / s_clades * nc) * t_search * (n_full / r["n"])
     pairs = (r["reps"] / s_clades * nc) * n_full
     line = {
         "impl": "reference", "metric": "genome pairs/sec ANI+AF (search path)", "value": pairs / t_full, "unit": "pairs/s",
-        "n_gpus": args.gpus, "steps": 1, "steps_requested": args.steps, "warmup": args.warmup, "ms_per_step": t_full * 1e3,
+        "n_gpus": args.gpus, "steps": len(runs), "steps_requested": args.steps, "warmup": args.warmup, "ms_per_step": t_full * 1e3,
         "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "u64/int32 + f64", "data": "synthetic",
         "config": {"workload": workload_name(args.workload),
                    "note": "oracle-CPU, NOT skani; EXTRAPOLATED from %d clades x %d (%d genomes, %d searches, %.2f s sketch + "
-                           "%.2f s loop): sketching scales with genomes, the loop with representatives x database size"
-                           % (s_clades, per, r["n"], r["reps"], r["t_sketch"], r["t_loop"])},
+                           "%.2f s loop per step): sketching scales with genomes, the loop with representatives x database size"
+                           % (s_clades, per, r["n"], r["reps"], t_sketch, t_loop)},
         "cpu_baseline": {"value": pairs / t_full, "unit": "pairs/s", "cores": threads, "kind": "port",
                          "sample": "%d clades x %d of %s, extrapolated" % (s_clades, per, args.workload)},
         "e2e": {"value": pairs / t_full, "unit": "pairs/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
@@ -342,18 +340,37 @@ def pinned_views(packed, torch):
     return pin, views, keep, total * 8
 
 
-def canonical_edges(edges, canon):
-    """Edge records -> sorted text rows keyed by workload-wide genome numbers (clade * per + member), whatever order
-    the ranks ingested them in; sha256 of that text is the same for every N if the results are."""
+def canonical_table(edges, canon):
+    """Edge records -> columns keyed by workload-wide genome numbers (clade * per + member), the lower number in `a`
+    (AFs swapped with it), rows sorted by (a, b): the same whatever order the ranks ingested the genomes in."""
     a, b = canon[edges["a"]], canon[edges["b"]]
     sw = a > b
     lo, hi = np.where(sw, b, a), np.where(sw, a, b)
     af_lo, af_hi = np.where(sw, edges["af_b"], edges["af_a"]), np.where(sw, edges["af_a"], edges["af_b"])
     order = np.lexsort((hi, lo))
+    return {"a": lo[order], "b": hi[order], "ani": edges["ani"][order], "af_a": af_lo[order], "af_b": af_hi[order]}
+
+
+def canonical_edges(edges, canon):
+    """sha256 of the canonical table as 2-decimal text rows: the same for every N if the results are."""
+    t = canonical_table(edges, canon)
     h = hashlib.sha256()
-    for i in order:
-        h.update(b"%d\t%d\t%.2f\t%.2f\t%.2f\n" % (lo[i], hi[i], edges["ani"][i], af_lo[i], af_hi[i]))
+    for row in zip(t["a"], t["b"], t["ani"], t["af_a"], t["af_b"]):
+        h.update(b"%d\t%d\t%.2f\t%.2f\t%.2f\n" % row)
     return h.hexdigest()
+
+
+def dump_outputs(directory, prefix, columns, max_bytes=DUMP_MAX_BYTES):
+    """Columns of one output table -> DIR/<prefix>_<column>.npy in float64 (genome numbers are exact there); returns the
+    bytes written.  A table above max_bytes keeps a fixed, seeded sample of its rows, the same rows for the same length."""
+    os.makedirs(directory, exist_ok=True)
+    n = len(next(iter(columns.values())))
+    rows = np.arange(n)
+    if n * 8 * len(columns) > max_bytes:
+        rows = np.sort(np.random.default_rng(0).choice(n, max_bytes // (8 * len(columns)), replace=False))
+    for name, col in columns.items():
+        np.save(os.path.join(directory, "%s_%s.npy" % (prefix, name)), np.asarray(col, np.float64)[rows])
+    return len(rows) * 8 * len(columns)
 
 
 def parity_sample(workload, edges, per, n_clades_checked, n_each, threads, screen, min_af):
@@ -587,6 +604,8 @@ def run_ours(args):
         if world > 1:
             dist.destroy_process_group()
         return 0
+    if args.dump_outputs:  # the edge list the last timed step returned
+        dump_outputs(args.dump_outputs, "edges", canonical_table(edges, canon))
 
     ms_step = ms_dev / args.steps
     value = pairs_full / (ms_step / 1e3)
@@ -732,7 +751,7 @@ def run_ours_search(args, torch, dist, rank, world, local):
         n_db = eng.n_genomes
         all_db = np.arange(n_db, dtype=np.int32)
         accounted = np.zeros(n_full, bool)
-        reps, rep_ids = 0, []
+        reps, rep_ids, hits = 0, [], []
         # The greedy loop is sequential, but a search result does not depend on the loop's state: the next K
         # candidates in N50 order that are not accounted for YET are searched in one call (one index_append, one
         # rectangle), and their results are applied in order -- a candidate an earlier one of the same batch accounts
@@ -786,22 +805,30 @@ def run_ours_search(args, torch, dist, rank, world, local):
                 dist.all_gather_into_tensor(recv, send)
                 rec = recv[recv >= 0].cpu().numpy()
                 qi, ids = rec >> 32, rec & 0xFFFFFFFF
-            wasted = 0
+            wasted, new_reps = 0, []
             for j, g in enumerate(batch):
                 if accounted[g]:
                     wasted += 1
                     continue
                 reps += 1
                 rep_ids.append(g)
+                new_reps.append(j)
                 accounted[ids[qi == j]] = True
                 accounted[g] = True
             wasted_all += wasted
+            if keep_hits:  # this rank's rows of the searches whose results the loop used: (query, ref, ANI, AF ref, AF query)
+                q_all = ord_of_ctx[edges["b"].astype(np.int64) - n_db]
+                used = np.isin(q_all, new_reps)
+                hits.append(np.stack([np.asarray(batch, np.float64)[q_all[used]], my_ids[edges["a"][used]].astype(np.float64),
+                                      edges["ani"][used], edges["af_a"][used], edges["af_b"][used]], axis=1))
             k_batch = max(1, k_batch // 2) if wasted else min(SEARCH_BATCH_MAX, k_batch * 2)
         one_run.searched, one_run.wasted, one_run.rep_ids = searched, wasted_all, rep_ids
+        one_run.hits = np.concatenate(hits) if hits else np.zeros((0, 5))
         torch.cuda.synchronize()
         t2 = time.perf_counter()
         return reps, reps * n_full, t1 - t0, t2 - t1, eng.launches - l0
 
+    keep_hits = bool(args.dump_outputs)
     for _ in range(min(args.warmup, 1)):
         one_run()
     res = []
@@ -821,7 +848,16 @@ def run_ours_search(args, torch, dist, rank, world, local):
         launches_all = int(ll[0])
     else:
         t_loop, launches_all = float(np.mean([r[3] for r in res])), res[-1][4]
+    if keep_hits and world > 1:
+        shards = [None] * world
+        dist.all_gather_object(shards, one_run.hits)
+        one_run.hits = np.concatenate(shards)
     if rank == 0:
+        if args.dump_outputs:  # what the last timed step selected, in selection order, and its searches' rows by (query, ref)
+            used = dump_outputs(args.dump_outputs, "representatives", {"genome": one_run.rep_ids})
+            h = one_run.hits[np.lexsort((one_run.hits[:, 1], one_run.hits[:, 0]))]
+            dump_outputs(args.dump_outputs, "hits", {"query": h[:, 0], "ref": h[:, 1], "ani": h[:, 2], "af_ref": h[:, 3],
+                                                     "af_query": h[:, 4]}, DUMP_MAX_BYTES - used)
         reps, pairs, t_sk, _, launches = res[-1]
         t_step = t_all / args.steps
         line = {
@@ -864,7 +900,16 @@ def main():
     ap.add_argument("--no-parity", action="store_true", help="skip the oracle parity sample")
     ap.add_argument("--derep", choices=["off", "sample", "full"], default=os.environ.get("SKB_BENCH_DEREP", "full"),
                     help="dereplication wall time through the unmodified reference (N=1): whole workload, 10 clades, or skip")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy (float64): the edge list "
+                         "sorted by genome number (edges_a, edges_b, edges_ani, edges_af_a, edges_af_b) or, for the search "
+                         "workloads, the representatives in selection order and the rows of their searches sorted by (query, "
+                         "ref) (hits_query, hits_ref, hits_ani, hits_af_ref, hits_af_query); a seeded row sample above 64 MB")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl ours")
     return run_reference(args) if args.impl == "reference" else run_ours(args)
 
 

@@ -41,9 +41,6 @@ def genomes7():
 def genomes34():
     fs = sorted(glob.glob(os.path.join(GOLDEN, "genomes34", "*.fasta.gz")))
     if len(fs) != 34:
-        ref = "/root/reference/test_case/skder_gtdb_results/gtdb_ncbi_genomes"
-        fs = sorted(glob.glob(os.path.join(ref, "*.fasta.gz")))
-    if len(fs) != 34:
         pytest.skip("34-genome fixture set not present (only the 7-genome subset is committed)")
     return fs
 

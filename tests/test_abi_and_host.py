@@ -261,6 +261,8 @@ def test_search_through_a_running_daemon_loads_neither_numpy_nor_the_engine(tmp_
     src/skDER/skder.py:116-120).  When the database's daemon answers, the client process must stay light: no numpy,
     no libskani_b200.so.  A stand-in server speaks the daemon's protocol (authenticated Unix socket, JSON bytes)."""
     import json
+    import shutil
+    import tempfile
     import threading
     from multiprocessing.connection import Listener
 
@@ -268,9 +270,12 @@ def test_search_through_a_running_daemon_loads_neither_numpy_nor_the_engine(tmp_
 
     db = tmp_path / "skani_sketch_all.db"
     db.mkdir()
-    env = dict(os.environ, SKB_DAEMON_DIR=str(tmp_path), SKB_DEVICE="0", PYTHONPATH=ROOT)
+    # a Unix socket path holds at most 107 bytes, and pytest's tmp_path can be longer: the sockets go to a short
+    # private directory instead
+    run_dir = tempfile.mkdtemp(prefix="skb-", dir="/tmp")
+    env = dict(os.environ, SKB_DAEMON_DIR=run_dir, SKB_DEVICE="0", PYTHONPATH=ROOT)
     env.pop("SKB_NO_DAEMON", None)
-    os.environ["SKB_DAEMON_DIR"] = str(tmp_path)
+    os.environ["SKB_DAEMON_DIR"] = run_dir
     try:
         sock = daemon.socket_path(str(db), 0)
     finally:
@@ -300,9 +305,12 @@ def test_search_through_a_running_daemon_loads_neither_numpy_nor_the_engine(tmp_
     out = tmp_path / "current_search_results.tsv"
     code = ("import sys; from skder_b200.cli import main; rc = main(sys.argv[1:]); "
             "print('numpy' in sys.modules, 'skder_b200.engine' in sys.modules, rc)")
-    r = subprocess.run([sys.executable, "-c", code, "search", "query.fa", "-d", str(db), "-o", str(out), "-t", "4"],
-                       capture_output=True, text=True, env=env, cwd=str(tmp_path), timeout=60)
-    th.join(timeout=10)
+    try:
+        r = subprocess.run([sys.executable, "-c", code, "search", "query.fa", "-d", str(db), "-o", str(out), "-t", "4"],
+                           capture_output=True, text=True, env=env, cwd=str(tmp_path), timeout=60)
+        th.join(timeout=10)
+    finally:
+        shutil.rmtree(run_dir, ignore_errors=True)
     assert r.stdout.split() == ["False", "False", "0"], r.stdout + r.stderr
     assert out.read_text() == "header\n"
     assert seen and seen[0]["op"] == "search" and seen[0]["query"] == str(tmp_path / "query.fa") and seen[0]["label"] == "query.fa"

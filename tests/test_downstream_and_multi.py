@@ -22,39 +22,43 @@ def _acc(p):
 def helpers():
     import replay
 
-    h = replay.helpers()
-    if len(h) != 2:
-        pytest.skip("reference skDERsum/skDERcore not built (needs /root/reference once; oracle/_ref travels afterwards)")
+    if "skDERcore" not in replay.helpers():
+        pytest.skip("reference skDERcore not built (oracle/build_ref.py compiles it where the reference's source is present)")
     return replay
 
 
-def test_replay_reproduces_golden_representatives(helpers, tmp_path):
-    """harness check: golden edges -> golden representatives, all 30 cutoff combinations + the 7-genome run"""
+def test_replay_reproduces_golden_representatives(tmp_path):
+    """harness check: golden edges -> golden representatives, all 30 cutoff combinations + the 7-genome run, whose
+    skDERsum summary (as printed and as sorted) is the reference's own, byte for byte"""
+    import replay
+
     g = os.path.join(GOLDEN, "skder_gtdb_results")
     n_checked = 0
     for ani in ("90.0", "95.0", "97.0", "98.0", "99.0", "99.5"):
         for af in ("10.0", "25.0", "50.0", "75.0", "90.0"):
             want = [ln.strip() for ln in open(os.path.join(g, "skDER_Result", "skDER_Results_ANI%s_AF%s.txt" % (ani, af))) if ln.strip()]
-            got = helpers.greedy_reps(os.path.join(g, "Skani_Triangle_Edge_Output.txt"), os.path.join(g, "Concatenated_N50.txt"),
-                                      float(ani), float(af), str(tmp_path))
+            got = replay.greedy_reps(os.path.join(g, "Skani_Triangle_Edge_Output.txt"), os.path.join(g, "Concatenated_N50.txt"),
+                                     float(ani), float(af), str(tmp_path))
             assert got == want, (ani, af)
             n_checked += 1
     assert n_checked == 30
     g7 = os.path.join(GOLDEN, "skder_results")
+    edges, n50 = os.path.join(g7, "Skani_Triangle_Edge_Output.txt"), os.path.join(g7, "Concatenated_N50.txt")
+    gi = tmp_path / "gi.txt"
+    gi.write_text(replay.greedy_information(edges, n50, 99.0, 50.0))
+    assert gi.read_text() == open(os.path.join(g7, "Genome_Information_for_Greedy_Clustering.txt")).read()
+    srt = replay.sorted_greedy_information(str(gi), str(tmp_path))
+    assert open(srt).read() == open(os.path.join(g7, "Genome_Information_for_Greedy_Clustering.sorted.txt")).read()
     want = [ln.strip() for ln in open(os.path.join(g7, "skDER_Results.txt")) if ln.strip()]
-    got = helpers.greedy_reps(os.path.join(g7, "Skani_Triangle_Edge_Output.txt"), os.path.join(g7, "Concatenated_N50.txt"), 99.0, 50.0, str(tmp_path))
+    got = replay.greedy_reps(edges, n50, 99.0, 50.0, str(tmp_path))
     assert got == want
 
 
-def test_oracle_edges_select_golden_representatives_away_from_knife_edges(helpers, oracle, genomes7, tmp_path):
-    """test_case (config 1): oracle edge list -> reference selection code.  The golden run (-i 99.0) has two
-    rows printed exactly 99.00 (SURVEY section 4 fact 8): representatives flip on +-0.005 pp there, far inside
-    the oracle's documented residual vs skani, so the comparison is made at cutoffs with no golden row
-    within the residual (ANI 97.0 and 99.5 / AF 50), and reported, not asserted, at 99.0."""
+def _oracle_and_golden_edges(genomes7, tmp_path):
+    """the oracle's edge list of the 7 genomes and the golden one, with N50s, rewritten consistently to the local paths"""
     from oracle import skani_cpu
 
     g7 = os.path.join(GOLDEN, "skder_results")
-    # rewrite N50 + edges consistently to the local paths
     n50 = {}
     for line in open(os.path.join(g7, "Concatenated_N50.txt")):
         p, v = line.rstrip("\n").split("\t")
@@ -71,26 +75,40 @@ def test_oracle_edges_select_golden_representatives_away_from_knife_edges(helper
             t = line.split("\t")
             t[0], t[1] = local[_acc(t[0])], local[_acc(t[1])]
             o.write("\t".join(t))
+    return edges, gold_edges, n50_file
+
+
+def test_oracle_edges_select_golden_representatives_away_from_knife_edges(oracle, genomes7, tmp_path):
+    """test_case (config 1): oracle edge list -> reference selection code.  The golden run (-i 99.0) has two
+    rows printed exactly 99.00 (SURVEY section 4 fact 8): representatives flip on +-0.005 pp there, far inside
+    the oracle's documented residual vs skani, so the comparison is made at cutoffs with no golden row
+    within the residual (ANI 97.0 and 99.5 / AF 50), and reported, not asserted, at 99.0."""
+    import replay
+
+    edges, gold_edges, n50_file = _oracle_and_golden_edges(genomes7, tmp_path)
     report = {}
     for ani in (97.0, 99.0, 99.5):
-        mine = sorted(_acc(x) for x in helpers.greedy_reps(str(edges), str(n50_file), ani, 50.0, str(tmp_path)))
-        gold = sorted(_acc(x) for x in helpers.greedy_reps(str(gold_edges), str(n50_file), ani, 50.0, str(tmp_path)))
+        mine = sorted(_acc(x) for x in replay.greedy_reps(str(edges), str(n50_file), ani, 50.0, str(tmp_path)))
+        gold = sorted(_acc(x) for x in replay.greedy_reps(str(gold_edges), str(n50_file), ani, 50.0, str(tmp_path)))
         report[ani] = (mine, gold)
         if ani != 99.0:
             assert mine == gold, report
-    # dynamic mode through skDERcore on the same edge lists.  At 99.5 the only qualifying pair
-    # (GCA_001700755.2 / GCA_900186975.1: golden AF 100.00 / 99.55, oracle 99.57 / 99.92) differs by < 0.5 pp in
-    # AF and skDERcore drops "the genome with the larger AF": a documented within-tolerance flip, reported only.
-    # That pair is 99.99 % identical; whichever cutoff admits it, dynamic mode keeps ONE of the two and
-    # the choice rides on the sign of a 0.4 pp AF difference.  So: representative sets must agree once the
-    # two near-identical genomes are treated as the same genome.
+    print("representatives at the golden run's own cutoff (99.0/50):", report[99.0])
+
+
+def test_oracle_edges_select_golden_dynamic_representatives(helpers, oracle, genomes7, tmp_path):
+    """test_case (config 1), dynamic mode: the oracle's edge list and the golden one through the reference's skDERcore.
+    At 99.5 the only qualifying pair (GCA_001700755.2 / GCA_900186975.1: golden AF 100.00 / 99.55, oracle 99.57 / 99.92)
+    differs by < 0.5 pp in AF and skDERcore drops "the genome with the larger AF": a documented within-tolerance flip.
+    That pair is 99.99 % identical; whichever cutoff admits it, dynamic mode keeps ONE of the two and the choice rides on
+    the sign of a 0.4 pp AF difference.  So: representative sets must agree once the two near-identical genomes are
+    treated as the same genome."""
+    edges, gold_edges, n50_file = _oracle_and_golden_edges(genomes7, tmp_path)
     twin = {"GCA_900186975.1": "GCA_001700755.2"}
     for ani in (97.0, 98.0, 99.5):
         mine = sorted(twin.get(_acc(x), _acc(x)) for x in helpers.dynamic_reps(str(edges), str(n50_file), ani, 50.0, 10.0))
         gold = sorted(twin.get(_acc(x), _acc(x)) for x in helpers.dynamic_reps(str(gold_edges), str(n50_file), ani, 50.0, 10.0))
-        report[("dynamic", ani)] = (mine, gold)
         assert mine == gold, (ani, mine, gold)
-    print("representatives at the golden run's own cutoff (99.0/50):", report[99.0])
 
 
 def _worker(rank, world, port, q):

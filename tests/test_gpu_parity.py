@@ -525,17 +525,13 @@ def test_fragmented_genome_beyond_the_shared_memory_limits(oracle, built_lib):
 
 def test_binary_edge_handoff_equals_reference_skdersum(eng7, genomes7, built_lib, tmp_path):
     """SURVEY section 8 f3: Genome_Information_for_Greedy_Clustering.txt from binary edges (skb_greedy_summary + select.py) is
-    byte-identical to what the reference's own skDERsum prints from the TSV -- on both golden edge lists (ids assigned
-    from their paths) and on this engine's own unrounded edges against its own TSV."""
+    byte-identical to what the reference's skDERsum prints from the TSV (tests/replay.py, held to the reference's own
+    output by the CPU tests) -- on both golden edge lists (ids assigned from their paths) and on this engine's own
+    unrounded edges against its own TSV."""
     import replay
     from conftest import GOLDEN
     from skder_b200 import cli, select
     from skder_b200.engine import EDGE_DTYPE
-
-    helpers = replay.helpers()
-    if "skDERsum" not in helpers:
-        pytest.skip("reference skDERsum not built")
-    import subprocess
 
     e, packed = eng7
     for gdir, cuts in (("skder_results", [(99.0, 50.0), (97.0, 50.0)]), ("skder_gtdb_results", [(99.0, 50.0), (98.0, 90.0), (90.0, 10.0)])):
@@ -547,7 +543,7 @@ def test_binary_edge_handoff_equals_reference_skdersum(eng7, genomes7, built_lib
         edges = np.array([(idx[r[0]], idx[r[1]], float(r[2]), float(r[3]), float(r[4])) for r in rows], EDGE_DTYPE)
         n50_rows = [(ln.split("\t")[0], int(ln.split("\t")[1])) for ln in open(n50f) if ln.strip()]
         for ani, af in cuts:
-            want = subprocess.check_output([helpers["skDERsum"], tsv, n50f, str(ani), str(af)], text=True)
+            want = replay.greedy_information(tsv, n50f, ani, af)
             assert select.greedy_information(e, edges, paths, n50_rows, ani, af) == want, (gdir, ani, af)
     # this engine's own result: unrounded doubles on the device vs the 2-decimal text the shim writes
     paths = sorted(genomes7)
@@ -560,7 +556,7 @@ def test_binary_edge_handoff_equals_reference_skdersum(eng7, genomes7, built_lib
     n50_rows = [(p.path, p.n50) for p in packed]
     for ani in (97.0, 98.61, 98.73, 99.02, 99.5):  # cutoffs sitting exactly on printed values of this edge list
         for af in (50.0, 89.5, 95.04):
-            want = subprocess.check_output([helpers["skDERsum"], str(tsv), str(n50f), str(ani), str(af)], text=True)
+            want = replay.greedy_information(str(tsv), str(n50f), ani, af)
             assert select.greedy_information(e, None, paths, n50_rows, ani, af) == want, (ani, af)  # None: device-resident list
             assert select.greedy_information(e, edges, paths, n50_rows, ani, af) == want, (ani, af)
 
