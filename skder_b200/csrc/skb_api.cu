@@ -61,9 +61,11 @@ struct DevBuf {
         p = q;
         cap = ncap;
     }
-    void upload(const std::vector<T> &h, cudaStream_t st) {
-        reserve(std::max<size_t>(h.size(), 1), 0, st);
-        if (!h.empty()) CK(cudaMemcpyAsync(p, h.data(), h.size() * sizeof(T), cudaMemcpyHostToDevice, st));
+    // device copy of h whose first `from` elements are already in place (from = 0: all of it)
+    void upload(const std::vector<T> &h, size_t from, cudaStream_t st) {
+        reserve(std::max<size_t>(h.size(), 1), from, st);
+        if (h.size() > from)
+            CK(cudaMemcpyAsync(p + from, h.data() + from, (h.size() - from) * sizeof(T), cudaMemcpyHostToDevice, st));
     }
 };
 
@@ -105,17 +107,62 @@ struct skb_ctx {
     int last_anchor_launches = 0;
     cudaEvent_t t0 = nullptr, t1 = nullptr;
 
-    // ---- sketch DB (host metadata)
-    std::vector<uint64_t> h_seed_off{0};   // [n+1]
-    std::vector<uint64_t> h_total_len;     // [n]
-    std::vector<uint32_t> h_ctg_off{0};    // [n+1]
-    std::vector<uint32_t> h_ctg_len;       // kept contig lengths
-    uint64_t n_mkeys = 0;                  // raw marker keys so far
+    // ---- sketch DB (host metadata; the seeds and raw marker keys themselves are d_seeds, d_mkeys)
+    struct SketchDb {
+        std::vector<uint64_t> seed_off{0};  // [n+1]
+        std::vector<uint64_t> total_len;    // [n]
+        std::vector<uint32_t> ctg_off{0};   // [n+1]
+        std::vector<uint32_t> ctg_len;      // kept contig lengths
+        uint64_t n_mkeys = 0;               // raw marker keys so far
+
+        int32_t n() const { return (int32_t)total_len.size(); }
+        template <typename L>
+        void append(uint64_t n_seeds, uint64_t len, const L *ctg_lens, size_t n_ctg) {
+            seed_off.push_back(seed_off.back() + n_seeds);
+            total_len.push_back(len);
+            for (size_t k = 0; k < n_ctg; k++) ctg_len.push_back((uint32_t)ctg_lens[k]);
+            ctg_off.push_back((uint32_t)ctg_len.size());
+        }
+        void truncate(int32_t n, uint64_t mkeys) {
+            seed_off.resize(n + 1);
+            total_len.resize(n);
+            ctg_off.resize(n + 1);
+            ctg_len.resize(ctg_off.back());
+            n_mkeys = mkeys;
+        }
+        void clear() { *this = SketchDb(); }
+    } db;
+    // ---- host side of the index skb_index / skb_index_append built over genomes [0, n_indexed)
+    struct HostIndex {
+        int32_t n_indexed = 0;
+        int32_t n_inv_genomes = 0;     // genomes covered by the inverted marker index
+        uint64_t n_inv = 0;            // its entries
+        uint64_t n_mkeys_indexed = 0;  // raw marker keys consumed by the last (append) index
+        std::vector<uint64_t> tab_off{0}, marker_off{0};  // [n_indexed+1]
+        std::vector<uint32_t> chunk_off{0};               // [n_indexed+1]
+        std::vector<uint32_t> tab_buckets;                // [n_indexed]
+        std::vector<uint32_t> ctg_pstart, chunk_start, chunk_len;
+
+        // drop the genomes a truncated sketch DB no longer holds
+        void truncate(const SketchDb &db) {
+            const int32_t n = db.n();
+            if (n_indexed <= n) return;
+            n_indexed = n;
+            tab_off.resize(n + 1);
+            tab_buckets.resize(n);
+            ctg_pstart.resize(db.ctg_len.size());
+            chunk_off.resize(n + 1);
+            chunk_start.resize(chunk_off.back());
+            chunk_len.resize(chunk_off.back());
+            marker_off.resize(n + 1);
+            n_mkeys_indexed = std::min(n_mkeys_indexed, db.n_mkeys);
+        }
+        void clear() { *this = HostIndex(); }
+    } ix;
     // ---- device arrays
     DevBuf<uint64_t> d_seeds, d_mkeys;
     // built by skb_index
     bool indexed = false;
-    int32_t n_indexed = 0;
     int32_t own_first = 0, own_count = -1;  // genomes whose seed tables this context builds (skb_set_owned); -1: all
     // seed tables built by skb_index_seed_tables and carried across skb_clear_keep_tables: valid for a context that owns
     // exactly these genomes (count, seed records, table density)
@@ -130,15 +177,8 @@ struct skb_ctx {
     DevBuf<uint32_t> d_tab_buckets;
     DevBuf<uint32_t> d_chunk_begin, d_chunk_start, d_chunk_len, d_chunk_off, d_ctg_pstart, d_ctg_len, d_ctg_off,
         d_marker_cnt;
-    std::vector<uint64_t> h_marker_off;    // [n+1]
-    std::vector<uint64_t> h_tab_off{0};    // [n_indexed+1]
-    std::vector<uint32_t> h_tab_buckets, h_ctg_pstart, h_chunk_start, h_chunk_len;
-    int32_t n_inv_genomes = 0;             // genomes covered by the inverted marker index
-    uint64_t n_mkeys_indexed = 0;          // raw marker keys consumed by the last (append) index
     struct AddCall { int32_t n_before; uint64_t mkeys_before; };
     std::vector<AddCall> add_calls;        // for skb_pop_last_add
-    std::vector<uint32_t> h_chunk_off;     // [n+1]
-    uint64_t n_inv = 0;
     // scratch
     DevBuf<unsigned char> d_tmp;
     std::map<std::string, DevBuf<unsigned char>> pool;  // named scratch, see PoolRef
@@ -146,11 +186,16 @@ struct skb_ctx {
     DevBuf<PairInfo> d_info;
     DevBuf<uint32_t> d_nch, d_task_off;
 
-    int32_t n() const { return (int32_t)h_total_len.size(); }
+    int32_t n() const { return db.n(); }
     bool owns(int32_t g) const { return own_count < 0 || (g >= own_first && g < own_first + own_count); }
+    // the owned genomes among [g0, n): one id range [first, second)
+    std::pair<int32_t, int32_t> owned_in(int32_t g0, int32_t n) const {
+        const int32_t o0 = std::clamp(own_count < 0 ? g0 : own_first, g0, n);
+        return {o0, std::clamp(own_count < 0 ? n : own_first + own_count, o0, n)};
+    }
     DbView view() const {
         DbView v;
-        v.n_genomes = n_indexed;
+        v.n_genomes = ix.n_indexed;
         v.seeds = d_seeds.p;
         v.g_seed_off = d_seed_off.p;
         v.tab = d_tab.p;
@@ -167,7 +212,7 @@ struct skb_ctx {
         v.markers = d_markers.p;
         v.g_marker_off = d_marker_off.p;
         v.inv_keys = d_inv.p;
-        v.n_inv = (int64_t)n_inv;
+        v.n_inv = (int64_t)ix.n_inv;
         return v;
     }
     AniParams ani_params() const {
@@ -328,24 +373,21 @@ void sketch_batch(skb_ctx *c, const skb_packed *const *gen, int32_t g0, int32_t 
     CK(cudaMemcpyAsync(h_off_s.data(), d_goff.p, ((size_t)nb + 1) * 4, cudaMemcpyDeviceToHost, c->st));
     CK(cudaMemcpyAsync(&tot_m, d_off_m.p + n_warps, 4, cudaMemcpyDeviceToHost, c->st));
     CK(cudaStreamSynchronize(c->st));
-    const uint64_t cur_seeds = c->h_seed_off.back();
+    const uint64_t cur_seeds = c->db.seed_off.back();
     const uint64_t tot_s = h_off_s[nb];
     c->d_seeds.reserve(cur_seeds + tot_s + 1, cur_seeds, c->st);
-    c->d_mkeys.reserve(c->n_mkeys + tot_m + 1, c->n_mkeys, c->st);
+    c->d_mkeys.reserve(c->db.n_mkeys + tot_m + 1, c->db.n_mkeys, c->st);
     sketch_kernel<true><<<n_tiles, SK_THREADS, 0, c->st>>>(b, nullptr, nullptr, d_off_s.p, d_off_m.p,
-                                                           c->d_seeds.p + cur_seeds, c->d_mkeys.p + c->n_mkeys,
+                                                           c->d_seeds.p + cur_seeds, c->d_mkeys.p + c->db.n_mkeys,
                                                            d_masks.p);
     CK(cudaGetLastError());
     c->launches++;
     CK(cudaStreamSynchronize(c->st));  // batch-local buffers die here
     for (int32_t i = 0; i < nb; i++) {
         const skb_packed *p = gen[g0 + i];
-        c->h_seed_off.push_back(cur_seeds + h_off_s[i + 1]);
-        c->h_total_len.push_back((uint64_t)p->n_bases);
-        for (int32_t k = 0; k < p->n_contigs; k++) c->h_ctg_len.push_back((uint32_t)p->contig_lens[k]);
-        c->h_ctg_off.push_back((uint32_t)c->h_ctg_len.size());
+        c->db.append(h_off_s[i + 1] - h_off_s[i], (uint64_t)p->n_bases, p->contig_lens, (size_t)p->n_contigs);
     }
-    c->n_mkeys += tot_m;
+    c->db.n_mkeys += tot_m;
     c->indexed = false;
 }
 
@@ -473,10 +515,10 @@ void run_ani(skb_ctx *c, const unsigned long long *d_pairs, int64_t n_pairs, Pai
     // 32-bit halves and chain_kernel compares diagonals (reference position -/+ query position, sign by strand) in 32
     // bits; SKB_WIDE_DIAG=1 forces the general variants (tests run both)
     bool wide_diag = std::getenv("SKB_WIDE_DIAG") != nullptr && atoi(std::getenv("SKB_WIDE_DIAG")) != 0;
-    for (int32_t g = 0; g < c->n_indexed && !wide_diag; g++) {
-        const uint32_t k1 = c->h_ctg_off[(size_t)g + 1];
-        if (k1 > c->h_ctg_off[(size_t)g] &&
-            (uint64_t)c->h_ctg_pstart[k1 - 1] + c->h_ctg_len[k1 - 1] >= (1ull << 30) - (1ull << 21))
+    for (int32_t g = 0; g < c->ix.n_indexed && !wide_diag; g++) {
+        const uint32_t k1 = c->db.ctg_off[(size_t)g + 1];
+        if (k1 > c->db.ctg_off[(size_t)g] &&
+            (uint64_t)c->ix.ctg_pstart[k1 - 1] + c->db.ctg_len[k1 - 1] >= (1ull << 30) - (1ull << 21))
             wide_diag = true;
     }
     static const bool trace = std::getenv("SKB_TRACE") != nullptr;  // diagnosis: per-kernel timeline on stderr
@@ -794,31 +836,22 @@ int64_t skb_launch_count(const skb_ctx *ctx) { return ctx ? ctx->launches : 0; }
 void *skb_stream(const skb_ctx *ctx) { return ctx ? (void *)ctx->st : nullptr; }
 void skb_free(void *p) { std::free(p); }
 
-int skb_clear(skb_ctx *ctx) {
+static int clear_impl(skb_ctx *ctx, bool keep_tables) {
     return guarded(ctx, [&]() -> int {
         CK(cudaStreamSynchronize(ctx->st));
-        ctx->h_seed_off.assign(1, 0);
-        ctx->h_total_len.clear();
-        ctx->h_ctg_off.assign(1, 0);
-        ctx->h_ctg_len.clear();
-        ctx->n_mkeys = 0;
+        ctx->db.clear();
+        ctx->ix.clear();
         ctx->indexed = false;
-        ctx->n_indexed = 0;
-        ctx->n_inv = 0;
-        ctx->n_inv_genomes = 0;
-        ctx->n_mkeys_indexed = 0;
         ctx->add_calls.clear();
         ctx->own_first = 0;
         ctx->own_count = -1;
-        ctx->kept_n = 0;
-        ctx->h_tab_off.assign(1, 0);
-        ctx->h_tab_buckets.clear();
-        ctx->h_ctg_pstart.clear();
-        ctx->h_chunk_start.clear();
-        ctx->h_chunk_len.clear();
+        if (!keep_tables) ctx->kept_n = 0;
         return SKB_OK;
     });
 }
+
+int skb_clear(skb_ctx *ctx) { return clear_impl(ctx, false); }
+int skb_clear_keep_tables(skb_ctx *ctx) { return clear_impl(ctx, true); }
 
 int skb_timer_start(skb_ctx *ctx) {
     return guarded(ctx, [&]() -> int {
@@ -858,7 +891,7 @@ int skb_add_genomes(skb_ctx *ctx, int32_t n, const skb_packed *const *genomes) {
         // batches of <= 1 Gi bases (per-batch seed/marker totals stay far below 2^32), grouped into
         // super-batches of <= 32 (8 GiB of packed words) whose H2D copies are all enqueued up front on a second stream: batch i+1
         // uploads while batch i is being sketched.
-        ctx->add_calls.push_back({ctx->n(), ctx->n_mkeys});
+        ctx->add_calls.push_back({ctx->n(), ctx->db.n_mkeys});
         if (!ctx->st_copy) CK(cudaStreamCreateWithFlags(&ctx->st_copy, cudaStreamNonBlocking));
         PoolRef<uint64_t> d_packed(ctx->pool["add_genomes.d_packed"]);
         int32_t g0 = 0;
@@ -933,8 +966,146 @@ int skb_add_genomes(skb_ctx *ctx, int32_t n, const skb_packed *const *genomes) {
     });
 }
 
-static int index_impl(skb_ctx *c, bool tables_only) {
-    {
+// ---- the per-genome index -------------------------------------------------------------------------------------------
+// Seed tables and chunk tables of the genomes [g0, n), laid out as anchor_kernel and the chain kernels read them
+// (DESIGN.md §2): skb_index builds them with g0 = 0, skb_index_append for the genomes added since the last index.
+
+// The sparsest seed tables the device holds comfortably: a lookup is one sector read unless its bucket overflowed, and
+// at 0.5 records per bucket that is rare enough not to stall a warp (skb_probe.cuh).  SKB_TAB_X2 forces a density.
+static int table_density(skb_ctx *c, uint64_t own_seeds) {
+    if (c->tab_x2_forced) return c->tab_x2_forced;
+    // decided once per sketch-DB size: cudaMemGetInfo takes a driver-wide lock and stalls for tens of ms whenever a
+    // monitoring tool (nvidia-smi / NVML polling) holds it -- seen as 20-80 ms spikes of this call
+    if (c->x2_decided && c->x2_decided_seeds == own_seeds) return c->x2_decided;
+    size_t free_b = 0, total_b = 0;
+    CK(cudaMemGetInfo(&free_b, &total_b));
+    const double budget = std::min(0.35 * (double)total_b,
+                                   (double)free_b + (double)c->d_tab.cap * 8.0 - 40.0 * (double)(1ull << 30));
+    c->x2_decided = 1;
+    for (int x2 : {4, 2})
+        if (((double)own_seeds * x2 / 2 + (double)c->n()) * BUCKET * 8.0 <= budget) {
+            c->x2_decided = x2;
+            break;
+        }
+    c->x2_decided_seeds = own_seeds;
+    return c->x2_decided;
+}
+
+// Seed tables and repeat flags of the genomes [g0, n) at density tab_x2.  Only the genomes this context owns get a
+// table (skb_set_owned: the others are only ever queries here), so the tables of the owned genomes are laid out by
+// those genomes in id order, their seed counts and the density alone: a rank builds its tables at ids 0..k-1 before
+// the sketches are exchanged, and with `reuse` the tables already in d_tab serve the same genomes at own_first..
+static int build_seed_tables(skb_ctx *c, int32_t g0, bool reuse) {
+    const int32_t n = c->n();
+    std::vector<uint64_t> &tab_off = c->ix.tab_off;
+    std::vector<uint32_t> &buckets = c->ix.tab_buckets;
+    tab_off.resize(n + 1);
+    buckets.resize(n);
+    for (int32_t g = g0; g < n; g++) {
+        const uint64_t ns = c->db.seed_off[g + 1] - c->db.seed_off[g];
+        if (ns >= (1ull << 31)) return fail(c, SKB_ELIMIT, "genome has too many seeds");
+        buckets[g] = c->owns(g) ? (uint32_t)std::max<uint64_t>(2, ns * (uint64_t)c->tab_x2 / 2 + 1) : 0u;
+        tab_off[g + 1] = tab_off[g] + (uint64_t)buckets[g] * BUCKET;
+    }
+    c->d_seed_off.upload(c->db.seed_off, g0, c->st);
+    c->d_tab_off.upload(tab_off, g0, c->st);
+    c->d_tab_buckets.upload(buckets, g0, c->st);
+    const uint64_t t0 = tab_off[g0], t1 = tab_off[n];
+    c->d_tab.reserve(t1 + BUCKET, reuse ? t1 : t0, c->st);
+    if (reuse) return SKB_OK;
+    CK(cudaMemsetAsync(c->d_tab.p + t0, 0xFF, (t1 - t0) * 8, c->st));
+    // the owned seeds are one contiguous range; the repeat flags of the others arrived with their seeds
+    // (skb_import_sketches keeps them)
+    const auto [o0, o1] = c->owned_in(g0, n);
+    const uint64_t s0 = c->db.seed_off[o0], s1 = c->db.seed_off[o1];
+    if (s1 > s0) {
+        tab_insert_kernel<<<nblk(s1 - s0, 256), 256, 0, c->st>>>(c->d_seeds.p, s1, c->d_seed_off.p, n, c->d_tab.p,
+                                                               c->d_tab_off.p, c->d_tab_buckets.p, s0);
+        CK(cudaGetLastError());
+        rep_flag_kernel<<<nblk(s1 - s0, 256), 256, 0, c->st>>>(c->d_seeds.p, s1, c->d_seed_off.p, n, c->d_tab.p,
+                                                             c->d_tab_off.p, c->d_tab_buckets.p, c->prm.max_mult, s0);
+        CK(cudaGetLastError());
+        c->launches += 2;
+    }
+    return SKB_OK;
+}
+
+// Chunk tables of the genomes [g0, n): contigs in padded coordinates (CONTIG_PAD after each), cut into chunk_len
+// pieces, and for every chunk (and one sentinel per genome) the index of its first seed.  Counted first, then filled
+// in place, by a few host threads when the range is large (1.5 M chunks at config3: the push_back loop this replaced
+// was 4 ms of every index build, and is replicated on every rank).
+static int build_chunk_tables(skb_ctx *c, int32_t g0) {
+    const int32_t n = c->n();
+    const uint32_t CL = (uint32_t)c->prm.chunk_len;
+    const skb_ctx::SketchDb &db = c->db;
+    skb_ctx::HostIndex &ix = c->ix;
+    ix.chunk_off.resize(n + 1);
+    for (int32_t g = g0; g < n; g++) {
+        uint64_t cnt = 0;
+        for (uint32_t k = db.ctg_off[g]; k < db.ctg_off[g + 1]; k++) cnt += (db.ctg_len[k] + CL - 1) / CL;
+        if ((uint64_t)ix.chunk_off[g] + cnt >= (1ull << 32)) return fail(c, SKB_ELIMIT, "too many chunks");
+        ix.chunk_off[g + 1] = ix.chunk_off[g] + (uint32_t)cnt;
+    }
+    ix.ctg_pstart.resize(db.ctg_len.size());
+    ix.chunk_start.resize(ix.chunk_off[n]);
+    ix.chunk_len.resize(ix.chunk_off[n]);
+    auto fill = [&](int32_t ga, int32_t gb) {
+        for (int32_t g = ga; g < gb; g++) {
+            uint32_t off = 0, at = ix.chunk_off[g];
+            for (uint32_t k = db.ctg_off[g]; k < db.ctg_off[g + 1]; k++) {
+                ix.ctg_pstart[k] = off;
+                const uint32_t len = db.ctg_len[k];
+                for (uint32_t st = 0; st < len; st += CL, at++) {
+                    ix.chunk_start[at] = off + st;
+                    ix.chunk_len[at] = std::min<uint32_t>(CL, len - st);
+                }
+                off += len + CONTIG_PAD;
+            }
+        }
+    };
+    const int64_t m = n - g0;
+    const int n_thr = m >= 1024 ? 4 : 1;
+    if (n_thr == 1)
+        fill(g0, n);
+    else {
+        std::vector<std::thread> pool;
+        for (int t = 0; t < n_thr; t++)
+            pool.emplace_back(fill, g0 + (int32_t)(m * t / n_thr), g0 + (int32_t)(m * (t + 1) / n_thr));
+        for (auto &th : pool) th.join();
+    }
+    const size_t k0 = db.ctg_off[g0], ch0 = ix.chunk_off[g0];
+    c->d_total_len.upload(db.total_len, g0, c->st);
+    c->d_ctg_off.upload(db.ctg_off, g0, c->st);
+    c->d_ctg_len.upload(db.ctg_len, k0, c->st);
+    c->d_ctg_pstart.upload(ix.ctg_pstart, k0, c->st);
+    c->d_chunk_off.upload(ix.chunk_off, g0, c->st);
+    c->d_chunk_start.upload(ix.chunk_start, ch0, c->st);
+    c->d_chunk_len.upload(ix.chunk_len, ch0, c->st);
+    const uint32_t e0 = (uint32_t)ch0 + (uint32_t)g0, e1 = ix.chunk_off[n] + (uint32_t)n;
+    c->d_chunk_begin.reserve(e1, e0, c->st);
+    chunk_begin_kernel<<<nblk(e1 - e0, 256), 256, 0, c->st>>>(c->d_seeds.p, c->d_seed_off.p, c->d_chunk_off.p, n,
+                                                             c->d_chunk_start.p, c->d_chunk_begin.p, e1, e0);
+    CK(cudaGetLastError());
+    c->launches++;
+    return SKB_OK;
+}
+
+// Marker list offsets of the genomes [g0, n) from the per-genome counts the marker kernels left in d_marker_cnt
+static void marker_offsets(skb_ctx *c, int32_t g0) {
+    const int32_t n = c->n();
+    std::vector<uint32_t> cnt((size_t)(n - g0));
+    CK(cudaMemcpyAsync(cnt.data(), c->d_marker_cnt.p + g0, cnt.size() * 4, cudaMemcpyDeviceToHost, c->st));
+    CK(cudaStreamSynchronize(c->st));
+    std::vector<uint64_t> &off = c->ix.marker_off;
+    off.resize(n + 1);
+    for (int32_t g = g0; g < n; g++) off[g + 1] = off[g] + cnt[(size_t)(g - g0)];
+    c->d_marker_off.upload(off, g0, c->st);
+    CK(cudaStreamSynchronize(c->st));
+}
+
+int skb_index(skb_ctx *ctx) {
+    return guarded(ctx, [&]() -> int {
+        skb_ctx *c = ctx;
         static const bool trace = std::getenv("SKB_TRACE") != nullptr;  // diagnosis: phase times on stderr (adds syncs)
         double t_last = 0;
         auto lap = [&](const char *what) {
@@ -949,159 +1120,44 @@ static int index_impl(skb_ctx *c, bool tables_only) {
         lap(nullptr);
         const int32_t n = c->n();
         if (n == 0) return fail(c, SKB_ESTATE, "no genomes added");
-        const uint64_t n_seeds = c->h_seed_off.back();
-        (void)n_seeds;
-        uint64_t own_seeds_now = 0;
-        for (int32_t g = 0; g < n; g++)
-            if (c->owns(g)) own_seeds_now += c->h_seed_off[g + 1] - c->h_seed_off[g];
-        const int32_t own_n_now = c->own_count < 0 ? n : std::max(0, std::min(c->own_first + c->own_count, n) - std::min(c->own_first, n));
+        const auto [o0, o1] = c->owned_in(0, n);
+        const uint64_t own_seeds = c->db.seed_off[o1] - c->db.seed_off[o0];
         // tables of exactly the owned genomes are already in d_tab (built before the sketches were exchanged)
-        const bool reuse = !tables_only && c->kept_n > 0 && c->kept_n == own_n_now && c->kept_seeds == own_seeds_now;
-        // ---- host-side tables: seed hash sizes, contigs in padded coordinates, chunks
-        std::vector<uint64_t> &tab_off = c->h_tab_off;
-        std::vector<uint32_t> &tab_buckets = c->h_tab_buckets, &ctg_pstart = c->h_ctg_pstart, &chunk_start = c->h_chunk_start,
-                              &chunk_len = c->h_chunk_len;
-        // the sparsest seed tables the device holds comfortably: a lookup is one sector read unless its bucket
-        // overflowed, and at 0.5 records per bucket that is rare enough not to stall a warp (skb_probe.cuh)
-        c->tab_x2 = reuse ? c->kept_x2 : c->tab_x2_forced;
-        if (!c->tab_x2 && c->x2_decided && c->x2_decided_seeds == own_seeds_now) c->tab_x2 = c->x2_decided;
-        if (!c->tab_x2) {
-            // decided once per sketch-DB size: cudaMemGetInfo takes a driver-wide lock and stalls for tens of ms
-            // whenever a monitoring tool (nvidia-smi / NVML polling) holds it -- seen as 20-80 ms spikes of this call
-            size_t free_b = 0, total_b = 0;
-            CK(cudaMemGetInfo(&free_b, &total_b));
-            const double budget = std::min(0.35 * (double)total_b,
-                                           (double)free_b + (double)c->d_tab.cap * 8.0 - 40.0 * (double)(1ull << 30));
-            c->tab_x2 = 1;
-            uint64_t own_seeds = 0;
-            for (int32_t g = 0; g < n; g++)
-                if (c->owns(g)) own_seeds += c->h_seed_off[g + 1] - c->h_seed_off[g];
-            for (int x2 : {4, 2})
-                if (((double)own_seeds * x2 / 2 + (double)n) * BUCKET * 8.0 <= budget) {
-                    c->tab_x2 = x2;
-                    break;
-                }
-            c->x2_decided = c->tab_x2;
-            c->x2_decided_seeds = own_seeds_now;
-        }
-        tab_off.assign(n + 1, 0);
-        tab_buckets.assign(n, 0);
-        ctg_pstart.assign(c->h_ctg_len.size(), 0);
-        c->h_chunk_off.assign(n + 1, 0);
-        // chunk counts first, then the tables are filled in place by a few host threads (1.5 M chunks at config3: the
-        // push_back loop this replaces was 4 ms of every index build, and is replicated on every rank)
-        const uint32_t CL = (uint32_t)c->prm.chunk_len;
-        for (int32_t g = 0; g < n; g++) {
-            const uint64_t ns = c->h_seed_off[g + 1] - c->h_seed_off[g];
-            if (ns >= (1ull << 31)) return fail(c, SKB_ELIMIT, "genome has too many seeds");
-            // a genome this context does not own is only ever a QUERY here: no table (skb_set_owned)
-            tab_buckets[g] = c->owns(g) ? (uint32_t)std::max<uint64_t>(2, ns * (uint64_t)c->tab_x2 / 2 + 1) : 0u;
-            tab_off[g + 1] = tab_off[g] + (uint64_t)tab_buckets[g] * BUCKET;
-            uint64_t cnt = 0;
-            for (uint32_t k = c->h_ctg_off[g]; k < c->h_ctg_off[g + 1]; k++) cnt += (c->h_ctg_len[k] + CL - 1) / CL;
-            if ((uint64_t)c->h_chunk_off[g] + cnt >= (1ull << 32)) return fail(c, SKB_ELIMIT, "too many chunks");
-            c->h_chunk_off[g + 1] = c->h_chunk_off[g] + (uint32_t)cnt;
-        }
-        chunk_start.resize(c->h_chunk_off[n]);
-        chunk_len.resize(c->h_chunk_off[n]);
-        auto fill = [&](int32_t g0, int32_t g1) {
-            for (int32_t g = g0; g < g1; g++) {
-                uint32_t off = 0, at = c->h_chunk_off[g];
-                for (uint32_t k = c->h_ctg_off[g]; k < c->h_ctg_off[g + 1]; k++) {
-                    ctg_pstart[k] = off;
-                    const uint32_t len = c->h_ctg_len[k];
-                    for (uint32_t st = 0; st < len; st += CL, at++) {
-                        chunk_start[at] = off + st;
-                        chunk_len[at] = std::min<uint32_t>(CL, len - st);
-                    }
-                    off += len + CONTIG_PAD;
-                }
-            }
-        };
-        const int n_thr = n >= 1024 ? 4 : 1;
-        if (n_thr == 1)
-            fill(0, n);
-        else {
-            std::vector<std::thread> pool;
-            for (int t = 0; t < n_thr; t++)
-                pool.emplace_back(fill, (int32_t)((int64_t)n * t / n_thr), (int32_t)((int64_t)n * (t + 1) / n_thr));
-            for (auto &th : pool) th.join();
-        }
-        lap("host tables");
-        c->d_seed_off.upload(c->h_seed_off, c->st);
-        c->d_tab_off.upload(tab_off, c->st);
-        c->d_tab_buckets.upload(tab_buckets, c->st);
-        c->d_total_len.upload(c->h_total_len, c->st);
-        c->d_ctg_pstart.upload(ctg_pstart, c->st);
-        c->d_ctg_len.upload(c->h_ctg_len, c->st);
-        c->d_ctg_off.upload(c->h_ctg_off, c->st);
-        c->d_chunk_start.upload(chunk_start, c->st);
-        c->d_chunk_len.upload(chunk_len, c->st);
-        c->d_chunk_off.upload(c->h_chunk_off, c->st);
-        lap("uploads");
-        // ---- K2: seed hash indices + repeat flags + chunk_begin
-        c->d_tab.reserve(tab_off[n] + BUCKET, reuse ? tab_off[n] : 0, c->st);
-        if (!reuse) {
-            CK(cudaMemsetAsync(c->d_tab.p, 0xFF, tab_off[n] * 8, c->st));
-            // the owned genomes are one contiguous id range, so their seeds are one contiguous range too; the repeat
-            // flags of the others arrived with their seeds (skb_import_sketches keeps them)
-            const int32_t o0 = c->own_count < 0 ? 0 : std::min(c->own_first, n);
-            const int32_t o1 = c->own_count < 0 ? n : std::min(c->own_first + c->own_count, n);
-            const uint64_t s0 = c->h_seed_off[o0], s1 = c->h_seed_off[o1];
-            if (s1 > s0) {
-                tab_insert_kernel<<<nblk(s1 - s0, 256), 256, 0, c->st>>>(c->d_seeds.p, s1, c->d_seed_off.p, n, c->d_tab.p,
-                                                                       c->d_tab_off.p, c->d_tab_buckets.p, s0);
-                CK(cudaGetLastError());
-                rep_flag_kernel<<<nblk(s1 - s0, 256), 256, 0, c->st>>>(c->d_seeds.p, s1, c->d_seed_off.p, n, c->d_tab.p,
-                                                                     c->d_tab_off.p, c->d_tab_buckets.p, c->prm.max_mult, s0);
-                CK(cudaGetLastError());
-                c->launches += 3;
-            }
-        }
-        lap("seed tables");
+        const bool reuse = c->kept_n > 0 && c->kept_n == o1 - o0 && c->kept_seeds == own_seeds;
+        c->tab_x2 = reuse ? c->kept_x2 : table_density(c, own_seeds);
+        int rc = build_seed_tables(c, 0, reuse);
+        if (rc != SKB_OK) return rc;
         c->kept_n = 0;
-        if (tables_only) {  // the caller exchanges sketches next (skb_clear_keep_tables): nothing else is needed yet
-            CK(cudaStreamSynchronize(c->st));
-            c->kept_n = own_n_now;
-            c->kept_seeds = own_seeds_now;
-            c->kept_x2 = c->tab_x2;
-            c->indexed = false;
-            return SKB_OK;
-        }
-        const uint32_t n_entries = (uint32_t)chunk_start.size() + (uint32_t)n;
-        c->d_chunk_begin.reserve(n_entries, 0, c->st);
-        chunk_begin_kernel<<<nblk(n_entries, 256), 256, 0, c->st>>>(c->d_seeds.p, c->d_seed_off.p, c->d_chunk_off.p, n,
-                                                                   c->d_chunk_start.p, c->d_chunk_begin.p, n_entries, 0);
-        CK(cudaGetLastError());
-        c->launches++;
-        lap("chunk_begin");
+        lap("seed tables");
+        if ((rc = build_chunk_tables(c, 0)) != SKB_OK) return rc;
+        lap("chunk tables");
         // ---- markers: sort raw keys, unique -> inverted index; per-genome counts; per-genome lists
         c->d_marker_cnt.reserve((size_t)n, 0, c->st);
         CK(cudaMemsetAsync(c->d_marker_cnt.p, 0, (size_t)n * 4, c->st));
-        c->n_inv = 0;
-        c->h_marker_off.assign(n + 1, 0);
-        if (c->n_mkeys) {
-            if (c->n_mkeys >= (1ull << 32)) return fail(c, SKB_ELIMIT, "too many marker keys");
+        c->ix.n_inv = 0;
+        const uint64_t nk = c->db.n_mkeys;
+        if (nk) {
+            if (nk >= (1ull << 32)) return fail(c, SKB_ELIMIT, "too many marker keys");
             PoolRef<uint64_t> d_sorted(c->pool["skb_index.d_sorted"]);
             PoolRef<uint32_t> d_flag(c->pool["skb_index.d_flag"]), d_pos(c->pool["skb_index.d_pos"]);
-            d_sorted.reserve(c->n_mkeys, 0, c->st);
-            d_flag.reserve(c->n_mkeys + 1, 0, c->st);
-            d_pos.reserve(c->n_mkeys + 1, 0, c->st);
+            d_sorted.reserve(nk, 0, c->st);
+            d_flag.reserve(nk + 1, 0, c->st);
+            d_pos.reserve(nk + 1, 0, c->st);
             // raw keys arrive genome by genome (ids ascending: skb_add_genomes, skb_import_sketches, skb_db_load), so a
             // STABLE sort on the 42 marker bits alone leaves every marker's run ordered by genome id: 6 radix passes
             // instead of 8
-            sort_keys_u64(c, c->d_mkeys.p, d_sorted.p, c->n_mkeys, 64, GID_BITS);
-            unique_flag_kernel<<<nblk(c->n_mkeys, 256), 256, 0, c->st>>>(d_sorted.p, c->n_mkeys, d_flag.p);
+            sort_keys_u64(c, c->d_mkeys.p, d_sorted.p, nk, 64, GID_BITS);
+            unique_flag_kernel<<<nblk(nk, 256), 256, 0, c->st>>>(d_sorted.p, nk, d_flag.p);
             CK(cudaGetLastError());
-            CK(cudaMemsetAsync(d_flag.p + c->n_mkeys, 0, 4, c->st));
-            exclusive_scan_u32(c, d_flag.p, d_pos.p, c->n_mkeys + 1);
+            CK(cudaMemsetAsync(d_flag.p + nk, 0, 4, c->st));
+            exclusive_scan_u32(c, d_flag.p, d_pos.p, nk + 1);
             uint32_t nu = 0;
-            CK(cudaMemcpyAsync(&nu, d_pos.p + c->n_mkeys, 4, cudaMemcpyDeviceToHost, c->st));
+            CK(cudaMemcpyAsync(&nu, d_pos.p + nk, 4, cudaMemcpyDeviceToHost, c->st));
             CK(cudaStreamSynchronize(c->st));
-            c->n_inv = nu;
+            c->ix.n_inv = nu;
             c->d_inv.reserve(nu + 1, 0, c->st);
-            unique_scatter_kernel<<<nblk(c->n_mkeys, 256), 256, 0, c->st>>>(d_sorted.p, c->n_mkeys, d_flag.p, d_pos.p,
-                                                                           c->d_inv.p, c->d_marker_cnt.p);
+            unique_scatter_kernel<<<nblk(nk, 256), 256, 0, c->st>>>(d_sorted.p, nk, d_flag.p, d_pos.p, c->d_inv.p,
+                                                                  c->d_marker_cnt.p);
             CK(cudaGetLastError());
             c->launches += 3;
             lap("inverted index");
@@ -1115,123 +1171,58 @@ static int index_impl(skb_ctx *c, bool tables_only) {
             strip_gid_kernel<<<nblk(nu, 256), 256, 0, c->st>>>(c->d_markers.p, nu);
             CK(cudaGetLastError());
             c->launches += 3;
-            std::vector<uint32_t> cnt(n);
-            CK(cudaMemcpyAsync(cnt.data(), c->d_marker_cnt.p, (size_t)n * 4, cudaMemcpyDeviceToHost, c->st));
-            CK(cudaStreamSynchronize(c->st));
-            for (int32_t g = 0; g < n; g++) c->h_marker_off[g + 1] = c->h_marker_off[g] + cnt[g];
         }
-        c->d_marker_off.upload(c->h_marker_off, c->st);
-        CK(cudaStreamSynchronize(c->st));
+        marker_offsets(c, 0);
         lap("marker lists");
-        c->n_indexed = n;
-        c->n_inv_genomes = n;
-        c->n_mkeys_indexed = c->n_mkeys;
+        c->ix.n_indexed = n;
+        c->ix.n_inv_genomes = n;
+        c->ix.n_mkeys_indexed = nk;
         c->indexed = true;
         return SKB_OK;
-    }
-}
-
-int skb_index(skb_ctx *ctx) {
-    return guarded(ctx, [&]() -> int { return index_impl(ctx, false); });
+    });
 }
 
 // Seed tables and repeat flags of the genomes added so far, nothing else: the first half of skb_index, for a rank that is
 // about to exchange sketches.  With skb_clear_keep_tables the tables survive the exchange, and the skb_index that follows
 // (after skb_import_sketches + skb_set_owned for the same genomes) reuses them instead of building them again.
 int skb_index_seed_tables(skb_ctx *ctx) {
-    return guarded(ctx, [&]() -> int { return index_impl(ctx, true); });
-}
-
-int skb_clear_keep_tables(skb_ctx *ctx) {
-    if (!ctx) return SKB_EINVAL;
-    const int32_t kn = ctx->kept_n;
-    const uint64_t ks = ctx->kept_seeds;
-    const int kx = ctx->kept_x2;
-    const int rc = skb_clear(ctx);
-    if (rc == SKB_OK) {
-        ctx->kept_n = kn;
-        ctx->kept_seeds = ks;
-        ctx->kept_x2 = kx;
-    }
-    return rc;
+    return guarded(ctx, [&]() -> int {
+        skb_ctx *c = ctx;
+        const int32_t n = c->n();
+        if (n == 0) return fail(c, SKB_ESTATE, "no genomes added");
+        const auto [o0, o1] = c->owned_in(0, n);
+        const uint64_t own_seeds = c->db.seed_off[o1] - c->db.seed_off[o0];
+        c->tab_x2 = table_density(c, own_seeds);
+        const int rc = build_seed_tables(c, 0, false);
+        if (rc != SKB_OK) return rc;
+        CK(cudaStreamSynchronize(c->st));
+        c->kept_n = o1 - o0;
+        c->kept_seeds = own_seeds;
+        c->kept_x2 = c->tab_x2;
+        c->indexed = false;
+        return SKB_OK;
+    });
 }
 
 // Index the genomes added since the last skb_index / skb_index_append as QUERY-ONLY additions: their
-// seed tables, repeat flags, chunk tables and sorted marker lists are appended; the inverted marker
-// index is left alone (they can be the query side of skb_rect, not a reference, and not part of a
+// seed tables (at the density of the last skb_index), repeat flags, chunk tables and sorted marker lists are appended;
+// the inverted marker index is left alone (they can be the query side of skb_rect, not a reference, and not part of a
 // triangle).  This is what `skani search` needs: the database stays resident and indexed, one query
 // genome comes and goes (skb_pop_last_add) at the cost of its own sketch.
 int skb_index_append(skb_ctx *ctx) {
     return guarded(ctx, [&]() -> int {
         skb_ctx *c = ctx;
-        const int32_t n = c->n(), n0 = c->n_indexed;
+        const int32_t n = c->n(), n0 = c->ix.n_indexed;
         if (!c->indexed && n0 == 0) return fail(c, SKB_ESTATE, "call skb_index on the database first");
         if (n == n0) {
             c->indexed = true;
             return SKB_OK;
         }
-        const uint64_t seeds0 = c->h_seed_off[n0], seeds1 = c->h_seed_off[n];
-        const size_t ctg0 = c->h_ctg_off[n0], chunks0 = c->h_chunk_start.size();
-        c->h_tab_off.resize(n + 1);
-        c->h_tab_buckets.resize(n);
-        c->h_ctg_pstart.resize(c->h_ctg_len.size());
-        c->h_chunk_off.resize(n + 1);
-        for (int32_t g = n0; g < n; g++) {
-            const uint64_t ns = c->h_seed_off[g + 1] - c->h_seed_off[g];
-            if (ns >= (1ull << 31)) return fail(c, SKB_ELIMIT, "genome has too many seeds");
-            c->h_tab_buckets[g] = (uint32_t)std::max<uint64_t>(2, ns * (uint64_t)c->tab_x2 / 2 + 1);
-            c->h_tab_off[g + 1] = c->h_tab_off[g] + (uint64_t)c->h_tab_buckets[g] * BUCKET;
-            uint32_t off = 0;
-            for (uint32_t k = c->h_ctg_off[g]; k < c->h_ctg_off[g + 1]; k++) {
-                c->h_ctg_pstart[k] = off;
-                const uint32_t len = c->h_ctg_len[k];
-                for (uint32_t st = 0; st < len; st += (uint32_t)c->prm.chunk_len) {
-                    c->h_chunk_start.push_back(off + st);
-                    c->h_chunk_len.push_back(std::min<uint32_t>((uint32_t)c->prm.chunk_len, len - st));
-                }
-                off += len + CONTIG_PAD;
-            }
-            c->h_chunk_off[g + 1] = (uint32_t)c->h_chunk_start.size();
-        }
-        auto append = [&](auto &dev, const auto &host, size_t old_n) {
-            dev.reserve(std::max<size_t>(host.size(), 1), old_n, c->st);
-            if (host.size() > old_n)
-                CK(cudaMemcpyAsync(dev.p + old_n, host.data() + old_n, (host.size() - old_n) * sizeof(host[0]),
-                                   cudaMemcpyHostToDevice, c->st));
-        };
-        append(c->d_seed_off, c->h_seed_off, (size_t)n0 + 1);
-        append(c->d_tab_off, c->h_tab_off, (size_t)n0 + 1);
-        append(c->d_tab_buckets, c->h_tab_buckets, (size_t)n0);
-        append(c->d_total_len, c->h_total_len, (size_t)n0);
-        append(c->d_ctg_pstart, c->h_ctg_pstart, ctg0);
-        append(c->d_ctg_len, c->h_ctg_len, ctg0);
-        append(c->d_ctg_off, c->h_ctg_off, (size_t)n0 + 1);
-        append(c->d_chunk_start, c->h_chunk_start, chunks0);
-        append(c->d_chunk_len, c->h_chunk_len, chunks0);
-        append(c->d_chunk_off, c->h_chunk_off, (size_t)n0 + 1);
-        // seed tables + repeat flags of the new genomes only
-        c->d_tab.reserve(c->h_tab_off[n], c->h_tab_off[n0], c->st);
-        CK(cudaMemsetAsync(c->d_tab.p + c->h_tab_off[n0], 0xFF, (c->h_tab_off[n] - c->h_tab_off[n0]) * 8, c->st));
-        if (seeds1 > seeds0) {
-            tab_insert_kernel<<<nblk(seeds1 - seeds0, 256), 256, 0, c->st>>>(c->d_seeds.p, seeds1, c->d_seed_off.p, n, c->d_tab.p,
-                                                                           c->d_tab_off.p, c->d_tab_buckets.p, seeds0);
-            CK(cudaGetLastError());
-            rep_flag_kernel<<<nblk(seeds1 - seeds0, 256), 256, 0, c->st>>>(c->d_seeds.p, seeds1, c->d_seed_off.p, n, c->d_tab.p,
-                                                                         c->d_tab_off.p, c->d_tab_buckets.p, c->prm.max_mult,
-                                                                         seeds0);
-            CK(cudaGetLastError());
-            c->launches += 2;
-        }
-        const uint32_t ent0 = (uint32_t)chunks0 + (uint32_t)n0, ent1 = (uint32_t)c->h_chunk_start.size() + (uint32_t)n;
-        c->d_chunk_begin.reserve(ent1, ent0, c->st);
-        chunk_begin_kernel<<<nblk(ent1 - ent0, 256), 256, 0, c->st>>>(c->d_seeds.p, c->d_seed_off.p, c->d_chunk_off.p, n,
-                                                                     c->d_chunk_start.p, c->d_chunk_begin.p, ent1, ent0);
-        CK(cudaGetLastError());
-        c->launches++;
+        int rc = build_seed_tables(c, n0, false);
+        if (rc != SKB_OK) return rc;
+        if ((rc = build_chunk_tables(c, n0)) != SKB_OK) return rc;
         // sorted unique marker lists of the new genomes, appended behind the database's
-        const uint64_t nk = c->n_mkeys - c->n_mkeys_indexed;
-        c->h_marker_off.resize(n + 1);
-        for (int32_t g = n0; g < n; g++) c->h_marker_off[g + 1] = c->h_marker_off[g];
+        const uint64_t nk = c->db.n_mkeys - c->ix.n_mkeys_indexed;
         c->d_marker_cnt.reserve((size_t)n, (size_t)n0, c->st);
         CK(cudaMemsetAsync(c->d_marker_cnt.p + n0, 0, (size_t)(n - n0) * 4, c->st));
         if (nk) {
@@ -1241,7 +1232,7 @@ int skb_index_append(skb_ctx *ctx) {
             d_b.reserve(nk, 0, c->st);
             d_flag.reserve(nk + 1, 0, c->st);
             d_pos.reserve(nk + 1, 0, c->st);
-            swap_key_kernel<<<nblk(nk, 256), 256, 0, c->st>>>(c->d_mkeys.p + c->n_mkeys_indexed, nk, d_a.p);
+            swap_key_kernel<<<nblk(nk, 256), 256, 0, c->st>>>(c->d_mkeys.p + c->ix.n_mkeys_indexed, nk, d_a.p);
             CK(cudaGetLastError());
             sort_keys_u64(c, d_a.p, d_b.p, nk);
             unique_flag_kernel<<<nblk(nk, 256), 256, 0, c->st>>>(d_b.p, nk, d_flag.p);
@@ -1251,21 +1242,16 @@ int skb_index_append(skb_ctx *ctx) {
             uint32_t nu = 0;
             CK(cudaMemcpyAsync(&nu, d_pos.p + nk, 4, cudaMemcpyDeviceToHost, c->st));
             CK(cudaStreamSynchronize(c->st));
-            const uint64_t m0 = c->h_marker_off[n0];
+            const uint64_t m0 = c->ix.marker_off[n0];
             c->d_markers.reserve(m0 + nu + 1, m0, c->st);
             unique_scatter_swapped_kernel<<<nblk(nk, 256), 256, 0, c->st>>>(d_b.p, nk, d_flag.p, d_pos.p, c->d_markers.p + m0,
                                                                            c->d_marker_cnt.p);
             CK(cudaGetLastError());
             c->launches += 3;
-            std::vector<uint32_t> cnt((size_t)(n - n0));
-            CK(cudaMemcpyAsync(cnt.data(), c->d_marker_cnt.p + n0, cnt.size() * 4, cudaMemcpyDeviceToHost, c->st));
-            CK(cudaStreamSynchronize(c->st));
-            for (int32_t g = n0; g < n; g++) c->h_marker_off[g + 1] = c->h_marker_off[g] + cnt[(size_t)(g - n0)];
         }
-        append(c->d_marker_off, c->h_marker_off, (size_t)n0 + 1);
-        CK(cudaStreamSynchronize(c->st));
-        c->n_mkeys_indexed = c->n_mkeys;
-        c->n_indexed = n;
+        marker_offsets(c, n0);
+        c->ix.n_mkeys_indexed = c->db.n_mkeys;
+        c->ix.n_indexed = n;
         c->indexed = true;
         return SKB_OK;
     });
@@ -1277,27 +1263,12 @@ int skb_pop_last_add(skb_ctx *ctx) {
         skb_ctx *c = ctx;
         if (c->add_calls.empty()) return fail(c, SKB_ESTATE, "nothing to pop");
         const skb_ctx::AddCall a = c->add_calls.back();
-        if (a.n_before < c->n_inv_genomes) return fail(c, SKB_ESTATE, "cannot pop genomes that are part of the inverted index");
+        if (a.n_before < c->ix.n_inv_genomes) return fail(c, SKB_ESTATE, "cannot pop genomes that are part of the inverted index");
         CK(cudaStreamSynchronize(c->st));
         c->add_calls.pop_back();
-        const int32_t n = a.n_before;
-        c->h_seed_off.resize(n + 1);
-        c->h_total_len.resize(n);
-        c->h_ctg_off.resize(n + 1);
-        c->h_ctg_len.resize(c->h_ctg_off.back());
-        c->n_mkeys = a.mkeys_before;
-        if (c->n_indexed > n) {
-            c->n_indexed = n;
-            c->h_tab_off.resize(n + 1);
-            c->h_tab_buckets.resize(n);
-            c->h_ctg_pstart.resize(c->h_ctg_len.size());
-            c->h_chunk_off.resize(n + 1);
-            c->h_chunk_start.resize(c->h_chunk_off.back());
-            c->h_chunk_len.resize(c->h_chunk_off.back());
-            c->h_marker_off.resize(n + 1);
-            c->n_mkeys_indexed = std::min(c->n_mkeys_indexed, c->n_mkeys);
-        }
-        c->indexed = c->n_indexed == n && n > 0;
+        c->db.truncate(a.n_before, a.mkeys_before);
+        c->ix.truncate(c->db);
+        c->indexed = c->ix.n_indexed == a.n_before && a.n_before > 0;
         return SKB_OK;
     });
 }
@@ -1306,12 +1277,12 @@ int skb_sketch_sizes(skb_ctx *ctx, int32_t g, int64_t *n_seeds, int64_t *n_marke
                      int64_t *total_len) {
     if (!ctx) return SKB_EINVAL;
     if (g < 0 || g >= ctx->n()) return fail(ctx, SKB_EINVAL, "genome id out of range");
-    if (n_seeds) *n_seeds = (int64_t)(ctx->h_seed_off[g + 1] - ctx->h_seed_off[g]);
-    if (total_len) *total_len = (int64_t)ctx->h_total_len[g];
+    if (n_seeds) *n_seeds = (int64_t)(ctx->db.seed_off[g + 1] - ctx->db.seed_off[g]);
+    if (total_len) *total_len = (int64_t)ctx->db.total_len[g];
     if (n_markers || n_chunks) {
-        if (!ctx->indexed || g >= ctx->n_indexed) return fail(ctx, SKB_ESTATE, "call skb_index first");
-        if (n_markers) *n_markers = (int64_t)(ctx->h_marker_off[g + 1] - ctx->h_marker_off[g]);
-        if (n_chunks) *n_chunks = (int32_t)(ctx->h_chunk_off[g + 1] - ctx->h_chunk_off[g]);
+        if (!ctx->indexed || g >= ctx->ix.n_indexed) return fail(ctx, SKB_ESTATE, "call skb_index first");
+        if (n_markers) *n_markers = (int64_t)(ctx->ix.marker_off[g + 1] - ctx->ix.marker_off[g]);
+        if (n_chunks) *n_chunks = (int32_t)(ctx->ix.chunk_off[g + 1] - ctx->ix.chunk_off[g]);
     }
     return SKB_OK;
 }
@@ -1319,7 +1290,7 @@ int skb_sketch_sizes(skb_ctx *ctx, int32_t g, int64_t *n_seeds, int64_t *n_marke
 int skb_get_seeds(skb_ctx *ctx, int32_t g, uint64_t *out) {
     return guarded(ctx, [&]() -> int {
         if (g < 0 || g >= ctx->n() || !out) return fail(ctx, SKB_EINVAL, "bad arguments");
-        const uint64_t a = ctx->h_seed_off[g], b = ctx->h_seed_off[g + 1];
+        const uint64_t a = ctx->db.seed_off[g], b = ctx->db.seed_off[g + 1];
         CK(cudaStreamSynchronize(ctx->st));
         if (b > a) CK(cudaMemcpy(out, ctx->d_seeds.p + a, (b - a) * 8, cudaMemcpyDeviceToHost));
         return SKB_OK;
@@ -1328,8 +1299,8 @@ int skb_get_seeds(skb_ctx *ctx, int32_t g, uint64_t *out) {
 
 int skb_get_markers(skb_ctx *ctx, int32_t g, uint64_t *out) {
     return guarded(ctx, [&]() -> int {
-        if (!ctx->indexed || g < 0 || g >= ctx->n_indexed || !out) return fail(ctx, SKB_ESTATE, "not indexed / bad id");
-        const uint64_t a = ctx->h_marker_off[g], b = ctx->h_marker_off[g + 1];
+        if (!ctx->indexed || g < 0 || g >= ctx->ix.n_indexed || !out) return fail(ctx, SKB_ESTATE, "not indexed / bad id");
+        const uint64_t a = ctx->ix.marker_off[g], b = ctx->ix.marker_off[g + 1];
         CK(cudaStreamSynchronize(ctx->st));
         if (b > a) CK(cudaMemcpy(out, ctx->d_markers.p + a, (b - a) * 8, cudaMemcpyDeviceToHost));
         return SKB_OK;
@@ -1342,9 +1313,9 @@ int skb_get_markers(skb_ctx *ctx, int32_t g, uint64_t *out) {
 static int screen_triangle_impl(skb_ctx *c, double screen_pct, int32_t part, int32_t n_parts, unsigned long long **d_out,
                                 int64_t *n_out, int64_t *pairs_total_out) {
     if (n_parts < 1 || part < 0 || part >= n_parts) return fail(c, SKB_EINVAL, "bad arguments");
-    if (!c->indexed || c->n_indexed != c->n()) return fail(c, SKB_ESTATE, "call skb_index first");
-    if (c->n_inv_genomes != c->n()) return fail(c, SKB_ESTATE, "query-only genomes present: triangle needs skb_index");
-    const uint32_t n = (uint32_t)c->n_indexed;
+    if (!c->indexed || c->ix.n_indexed != c->n()) return fail(c, SKB_ESTATE, "call skb_index first");
+    if (c->ix.n_inv_genomes != c->n()) return fail(c, SKB_ESTATE, "query-only genomes present: triangle needs skb_index");
+    const uint32_t n = (uint32_t)c->ix.n_indexed;
     const uint32_t rows_local = rows_owned(n, (uint32_t)part, (uint32_t)n_parts);
     int64_t pairs_total = 0;
     for (uint32_t rl = 0; rl < rows_local; rl++) pairs_total += n - 1 - row_global(rl, (uint32_t)part, (uint32_t)n_parts);
@@ -1377,8 +1348,8 @@ static int screen_triangle_impl(skb_ctx *c, double screen_pct, int32_t part, int
                 d_cnt.reserve(cells, 0, c->st);
                 if (scale > 0.0) {
                     CK(cudaMemsetAsync(d_cnt.p, 0, cells * 4, c->st));
-                    if (c->n_inv) {
-                        screen_runs_kernel<<<nblk(c->n_inv, 256), 256, 0, c->st>>>(c->d_inv.p, c->n_inv, d_cnt.p, n, part, n_parts,
+                    if (c->ix.n_inv) {
+                        screen_runs_kernel<<<nblk(c->ix.n_inv, 256), 256, 0, c->st>>>(c->d_inv.p, c->ix.n_inv, d_cnt.p, n, part, n_parts,
                                                                                   r0, nr);
                         CK(cudaGetLastError());
                         c->launches++;
@@ -1504,7 +1475,7 @@ int skb_pairs_edges(skb_ctx *ctx, const uint64_t *dev_pairs, int64_t n_pairs, in
     return guarded(ctx, [&]() -> int {
         skb_ctx *c = ctx;
         if (!n_edges || n_pairs < 0 || (n_pairs && !dev_pairs)) return fail(c, SKB_EINVAL, "bad arguments");
-        if (!c->indexed || c->n_indexed != c->n()) return fail(c, SKB_ESTATE, "call skb_index first");
+        if (!c->indexed || c->ix.n_indexed != c->n()) return fail(c, SKB_ESTATE, "call skb_index first");
         const int64_t launches0 = c->launches;
         cudaEvent_t e0, e1, e2;
         CK(cudaEventCreate(&e0));
@@ -1556,14 +1527,14 @@ int skb_rect(skb_ctx *ctx, const int32_t *refs, int32_t n_refs, const int32_t *q
         skb_ctx *c = ctx;
         if (!edges || !n_edges || n_refs < 0 || n_queries < 0 || (n_refs && !refs) || (n_queries && !queries))
             return fail(c, SKB_EINVAL, "bad arguments");
-        if (!c->indexed || c->n_indexed != c->n()) return fail(c, SKB_ESTATE, "call skb_index first");
+        if (!c->indexed || c->ix.n_indexed != c->n()) return fail(c, SKB_ESTATE, "call skb_index first");
         if (c->own_count >= 0) return fail(c, SKB_ESTATE, "skb_rect on a context that owns only part of the seed tables (skb_set_owned)");
-        const int32_t n = c->n_indexed;
+        const int32_t n = c->ix.n_indexed;
         const int64_t launches0 = c->launches;
         std::vector<int32_t> ref_slot(n, -1);
         for (int32_t i = 0; i < n_refs; i++) {
             if (refs[i] < 0 || refs[i] >= n) return fail(c, SKB_EINVAL, "reference id out of range");
-            if (refs[i] >= c->n_inv_genomes && screen_pct > 0.0)
+            if (refs[i] >= c->ix.n_inv_genomes && screen_pct > 0.0)
                 return fail(c, SKB_ESTATE, "a query-only genome (skb_index_append) cannot be a screened reference");
             if (ref_slot[refs[i]] >= 0) return fail(c, SKB_EINVAL, "duplicate reference id");
             ref_slot[refs[i]] = i;
@@ -1571,7 +1542,7 @@ int skb_rect(skb_ctx *ctx, const int32_t *refs, int32_t n_refs, const int32_t *q
         std::vector<uint64_t> qpref(n_queries + 1, 0);
         for (int32_t i = 0; i < n_queries; i++) {
             if (queries[i] < 0 || queries[i] >= n) return fail(c, SKB_EINVAL, "query id out of range");
-            qpref[i + 1] = qpref[i] + (c->h_marker_off[queries[i] + 1] - c->h_marker_off[queries[i]]);
+            qpref[i + 1] = qpref[i] + (c->ix.marker_off[queries[i] + 1] - c->ix.marker_off[queries[i]]);
         }
         cudaEvent_t e0, e1, e2;
         CK(cudaEventCreate(&e0));
@@ -1595,9 +1566,9 @@ int skb_rect(skb_ctx *ctx, const int32_t *refs, int32_t n_refs, const int32_t *q
             d_cnt.reserve(cells, 0, c->st);
             if (scale > 0.0) {
                 CK(cudaMemsetAsync(d_cnt.p, 0, cells * 4, c->st));
-                if (qpref[n_queries] && c->n_inv) {
+                if (qpref[n_queries] && c->ix.n_inv) {
                     screen_rect_kernel<<<nblk(qpref[n_queries], 256), 256, 0, c->st>>>(
-                        c->d_inv.p, c->n_inv, c->d_markers.p, c->d_marker_off.p, d_queries.p, n_queries, d_qpref.p,
+                        c->d_inv.p, c->ix.n_inv, c->d_markers.p, c->d_marker_off.p, d_queries.p, n_queries, d_qpref.p,
                         d_slot.p, d_cnt.p, (uint32_t)n_refs);
                     CK(cudaGetLastError());
                     c->launches++;
@@ -1651,14 +1622,14 @@ int skb_pairs_detail(skb_ctx *ctx, const uint32_t *a, const uint32_t *b, int64_t
     return guarded(ctx, [&]() -> int {
         skb_ctx *c = ctx;
         if (n < 0 || (n && (!a || !b || !out))) return fail(c, SKB_EINVAL, "bad arguments");
-        if (!c->indexed || c->n_indexed != c->n()) return fail(c, SKB_ESTATE, "call skb_index first");
+        if (!c->indexed || c->ix.n_indexed != c->n()) return fail(c, SKB_ESTATE, "call skb_index first");
         if (n == 0) return SKB_OK;
         std::vector<unsigned long long> hp((size_t)n);
         for (int64_t i = 0; i < n; i++) {
-            if (a[i] >= (uint32_t)c->n_indexed || b[i] >= (uint32_t)c->n_indexed || a[i] == b[i])
+            if (a[i] >= (uint32_t)c->ix.n_indexed || b[i] >= (uint32_t)c->ix.n_indexed || a[i] == b[i])
                 return fail(c, SKB_EINVAL, "pair id out of range");
             hp[(size_t)i] = ((unsigned long long)a[i] << 32) | b[i];
-            const uint64_t nsa = c->h_seed_off[a[i] + 1] - c->h_seed_off[a[i]], nsb = c->h_seed_off[b[i] + 1] - c->h_seed_off[b[i]];
+            const uint64_t nsa = c->db.seed_off[a[i] + 1] - c->db.seed_off[a[i]], nsb = c->db.seed_off[b[i] + 1] - c->db.seed_off[b[i]];
             if (!c->owns((int32_t)(nsb < nsa ? a[i] : b[i])))
                 return fail(c, SKB_ESTATE, "the reference genome of a pair is not owned by this context (skb_set_owned)");
         }
@@ -1694,10 +1665,10 @@ int skb_shared_markers(skb_ctx *ctx, const uint32_t *a, const uint32_t *b, int64
     return guarded(ctx, [&]() -> int {
         skb_ctx *c = ctx;
         if (n < 0 || (n && (!a || !b || !shared))) return fail(c, SKB_EINVAL, "bad arguments");
-        if (!c->indexed || c->n_indexed != c->n()) return fail(c, SKB_ESTATE, "call skb_index first");
+        if (!c->indexed || c->ix.n_indexed != c->n()) return fail(c, SKB_ESTATE, "call skb_index first");
         if (n == 0) return SKB_OK;
         for (int64_t i = 0; i < n; i++)
-            if (a[i] >= (uint32_t)c->n_indexed || b[i] >= (uint32_t)c->n_indexed)
+            if (a[i] >= (uint32_t)c->ix.n_indexed || b[i] >= (uint32_t)c->ix.n_indexed)
                 return fail(c, SKB_EINVAL, "pair id out of range");
         PoolRef<uint32_t> da(c->pool["skb_shared_markers.da"]), db(c->pool["skb_shared_markers.db"]);
         PoolRef<long long> dout(c->pool["skb_shared_markers.dout"]);
@@ -1724,16 +1695,16 @@ int skb_db_save(skb_ctx *ctx, const char *dir) {
         const std::string path = std::string(dir) + "/sketches.skb";
         FILE *f = fopen(path.c_str(), "wb");
         if (!f) return fail(c, SKB_EIO, "cannot create " + path);
-        const uint64_t n = (uint64_t)c->n(), ns = c->h_seed_off.back(), nm = c->n_mkeys, nc = c->h_ctg_len.size();
+        const uint64_t n = (uint64_t)c->n(), ns = c->db.seed_off.back(), nm = c->db.n_mkeys, nc = c->db.ctg_len.size();
         std::vector<uint64_t> seeds(ns), mk(nm);
         CK(cudaStreamSynchronize(c->st));
         if (ns) CK(cudaMemcpy(seeds.data(), c->d_seeds.p, ns * 8, cudaMemcpyDeviceToHost));
         if (nm) CK(cudaMemcpy(mk.data(), c->d_mkeys.p, nm * 8, cudaMemcpyDeviceToHost));
         for (auto &s : seeds) s &= ~2ull;  // repeat flags are index state
         bool ok = write_all(f, kMagic, 8) && write_all(f, &n, 8) && write_all(f, &ns, 8) && write_all(f, &nm, 8) &&
-                  write_all(f, &nc, 8) && write_all(f, c->h_seed_off.data(), (n + 1) * 8) &&
-                  write_all(f, c->h_total_len.data(), n * 8) && write_all(f, c->h_ctg_off.data(), (n + 1) * 4) &&
-                  write_all(f, c->h_ctg_len.data(), nc * 4) && write_all(f, seeds.data(), ns * 8) &&
+                  write_all(f, &nc, 8) && write_all(f, c->db.seed_off.data(), (n + 1) * 8) &&
+                  write_all(f, c->db.total_len.data(), n * 8) && write_all(f, c->db.ctg_off.data(), (n + 1) * 4) &&
+                  write_all(f, c->db.ctg_len.data(), nc * 4) && write_all(f, seeds.data(), ns * 8) &&
                   write_all(f, mk.data(), nm * 8);
         ok = (fclose(f) == 0) && ok;
         return ok ? SKB_OK : fail(c, SKB_EIO, "short write to " + path);
@@ -1768,11 +1739,7 @@ int skb_db_load(skb_ctx *ctx, const char *dir) {
         if (ns) CK(cudaMemcpyAsync(c->d_seeds.p, seeds.data(), ns * 8, cudaMemcpyHostToDevice, c->st));
         if (nm) CK(cudaMemcpyAsync(c->d_mkeys.p, mk.data(), nm * 8, cudaMemcpyHostToDevice, c->st));
         CK(cudaStreamSynchronize(c->st));
-        c->h_seed_off = seed_off;
-        c->h_total_len = total_len;
-        c->h_ctg_off = ctg_off;
-        c->h_ctg_len = ctg_len;
-        c->n_mkeys = nm;
+        c->db = skb_ctx::SketchDb{std::move(seed_off), std::move(total_len), std::move(ctg_off), std::move(ctg_len), nm};
         c->indexed = false;
         return SKB_OK;
     });
@@ -1783,15 +1750,15 @@ int skb_sketch_view_get(skb_ctx *ctx, skb_sketch_view *v) {
     cudaSetDevice(ctx->device);
     cudaStreamSynchronize(ctx->st);
     v->n_genomes = ctx->n();
-    v->n_seeds = (int64_t)ctx->h_seed_off.back();
-    v->n_marker_keys = (int64_t)ctx->n_mkeys;
-    v->n_contigs = (int64_t)ctx->h_ctg_len.size();
+    v->n_seeds = (int64_t)ctx->db.seed_off.back();
+    v->n_marker_keys = (int64_t)ctx->db.n_mkeys;
+    v->n_contigs = (int64_t)ctx->db.ctg_len.size();
     v->dev_seeds = ctx->d_seeds.p;
     v->dev_marker_keys = ctx->d_mkeys.p;
-    v->host_seed_off = ctx->h_seed_off.data();
-    v->host_total_len = ctx->h_total_len.data();
-    v->host_ctg_off = ctx->h_ctg_off.data();
-    v->host_ctg_len = ctx->h_ctg_len.data();
+    v->host_seed_off = ctx->db.seed_off.data();
+    v->host_total_len = ctx->db.total_len.data();
+    v->host_ctg_off = ctx->db.ctg_off.data();
+    v->host_ctg_len = ctx->db.ctg_len.data();
     return SKB_OK;
 }
 
@@ -1854,10 +1821,10 @@ int skb_import_sketches(skb_ctx *ctx, int32_t n_genomes, const uint64_t *dev_see
         if (n_genomes < 0 || n_seeds < 0 || n_marker_keys < 0) return fail(c, SKB_EINVAL, "bad arguments");
         if (n_genomes == 0) return SKB_OK;
         if ((uint64_t)c->n() + (uint64_t)n_genomes >= GID_MASK) return fail(c, SKB_ELIMIT, "too many genomes");
-        const uint64_t cur = c->h_seed_off.back();
-        c->add_calls.push_back({c->n(), c->n_mkeys});  // skb_pop_last_add undoes an import like an add
+        const uint64_t cur = c->db.seed_off.back();
+        c->add_calls.push_back({c->n(), c->db.n_mkeys});  // skb_pop_last_add undoes an import like an add
         c->d_seeds.reserve(cur + (uint64_t)n_seeds + 1, cur, c->st);
-        c->d_mkeys.reserve(c->n_mkeys + (uint64_t)n_marker_keys + 1, c->n_mkeys, c->st);
+        c->d_mkeys.reserve(c->db.n_mkeys + (uint64_t)n_marker_keys + 1, c->db.n_mkeys, c->st);
         if (n_seeds && keep_repeat_flags)  // the sender indexed its genomes: their repeat flags travel with the seeds
             CK(cudaMemcpyAsync(c->d_seeds.p + cur, dev_seeds, (size_t)n_seeds * 8, cudaMemcpyDeviceToDevice, c->st));
         else if (n_seeds) {
@@ -1870,19 +1837,15 @@ int skb_import_sketches(skb_ctx *ctx, int32_t n_genomes, const uint64_t *dev_see
         if (n_marker_keys) {
             // senders export a whole context, whose ids start at 0: shift them behind this context's genomes
             retag_keys_kernel<<<nblk((uint64_t)n_marker_keys, 256), 256, 0, c->st>>>(
-                dev_marker_keys, (uint64_t)n_marker_keys, c->d_mkeys.p + c->n_mkeys, (int64_t)c->n());
+                dev_marker_keys, (uint64_t)n_marker_keys, c->d_mkeys.p + c->db.n_mkeys, (int64_t)c->n());
             CK(cudaGetLastError());
             c->launches++;
         }
         CK(cudaStreamSynchronize(c->st));
-        const uint32_t ctg_base = (uint32_t)c->h_ctg_len.size();
-        for (int32_t g = 0; g < n_genomes; g++) {
-            c->h_seed_off.push_back(cur + (host_seed_off[g + 1] - host_seed_off[0]));
-            c->h_total_len.push_back(host_total_len[g]);
-            for (uint32_t k = host_ctg_off[g]; k < host_ctg_off[g + 1]; k++) c->h_ctg_len.push_back(host_ctg_len[k]);
-            c->h_ctg_off.push_back(ctg_base + (host_ctg_off[g + 1] - host_ctg_off[0]));
-        }
-        c->n_mkeys += (uint64_t)n_marker_keys;
+        for (int32_t g = 0; g < n_genomes; g++)
+            c->db.append(host_seed_off[g + 1] - host_seed_off[g], host_total_len[g], host_ctg_len + host_ctg_off[g],
+                         host_ctg_off[g + 1] - host_ctg_off[g]);
+        c->db.n_mkeys += (uint64_t)n_marker_keys;
         c->indexed = false;
         return SKB_OK;
     });

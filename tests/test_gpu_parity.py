@@ -124,6 +124,54 @@ def test_rect_equals_triangle_values(eng7):
     assert len(rect) == 12
 
 
+# the automatic seed-table density, and two records per 4-slot bucket (SKB_TAB_X2=1), which fills overflow chains
+@pytest.mark.parametrize("tab_x2", [None, "1"], ids=["auto", "SKB_TAB_X2=1"])
+def test_appended_index_equals_full_index(genomes7, built_lib, monkeypatch, tab_x2):
+    """Genomes indexed by skb_index_append get the chunk tables, marker lists and per-pair results a full skb_index gives
+    them, and popping them leaves the database as it was."""
+    from skder_b200 import engine
+
+    if tab_x2:
+        monkeypatch.setenv("SKB_TAB_X2", tab_x2)
+    else:
+        monkeypatch.delenv("SKB_TAB_X2", raising=False)
+    packed = engine.pack_fasta_many(genomes7, threads=4)
+    with engine.Engine(0) as app, engine.Engine(0) as full:
+        app.add(packed[:5])
+        app.index()
+        app.add([packed[5]])
+        app.add([packed[6]])
+        app.index_append()
+        full.add(packed)
+        full.index()
+        for g in (5, 6):
+            assert app.sizes(g) == full.sizes(g)
+            assert np.array_equal(app.markers(g), full.markers(g))
+        assert app.rect(range(5), [5, 6])[0].tobytes() == full.rect(range(5), [5, 6])[0].tobytes()
+        pairs = [p for g in (5, 6) for x in range(5) for p in ((x, g), (g, x))]
+        a, b = [p[0] for p in pairs], [p[1] for p in pairs]
+        for p, x, y in zip(pairs, app.pairs_detail(a, b), full.pairs_detail(a, b)):
+            assert bytes(x) == bytes(y), p  # integers and doubles bit for bit
+        app.pop_last_add()
+        app.pop_last_add()
+        with engine.Engine(0) as db:
+            db.add(packed[:5])
+            db.index()
+            assert app.triangle(min_af=0.0)[0].tobytes() == db.triangle(min_af=0.0)[0].tobytes()
+    # a context that owns genomes 0-4 builds no seed table for an appended genome, and refuses it as a reference
+    with engine.Engine(0) as part:
+        part.add(packed[:5])
+        part.set_owned(0, 5)
+        part.index()
+        part.add([packed[5]])
+        part.index_append()
+        ns = [part.sizes(g)["n_seeds"] for g in range(6)]
+        for x in range(5):
+            a, b = (x, 5) if ns[5] >= ns[x] else (5, x)  # the reference is the genome with more seeds (ties: b)
+            with pytest.raises(engine.SkbError):
+                part.pairs_detail([a], [b])
+
+
 def test_db_roundtrip(eng7, tmp_path):
     from skder_b200 import engine
 
