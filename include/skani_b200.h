@@ -143,6 +143,14 @@ int skb_triangle(skb_ctx *ctx, double screen_pct, double min_af_pct, int32_t par
 int skb_rect(skb_ctx *ctx, const int32_t *refs, int32_t n_refs, const int32_t *queries, int32_t n_queries,
              double screen_pct, double min_af_pct, skb_edge **edges, int64_t *n_edges, skb_stats *stats);
 
+/* How a pair's accepted chains become one ANI (skani's default, --median, --robust; DESIGN.md section 3).  Context
+ * state, kept across skb_clear: applies to every later skb_triangle, skb_rect, skb_pairs_edges and skb_pairs_detail
+ * call.  AF, chain, anchor and seed counts are the same in every mode.  Any other value: SKB_EINVAL. */
+#define SKB_ANI_MEAN 0
+#define SKB_ANI_MEDIAN 1
+#define SKB_ANI_ROBUST 2
+int skb_set_ani_estimator(skb_ctx *ctx, int32_t estimator);
+
 /* explicit pair list, full detail, no screening / no AF filter (parity tests) */
 int skb_pairs_detail(skb_ctx *ctx, const uint32_t *a, const uint32_t *b, int64_t n, skb_pair_detail *out);
 /* shared-marker counts of an explicit pair list (prescreen parity) */

@@ -103,6 +103,7 @@ SYMBOLS = [
     "skb_rect", "skb_pairs_detail", "skb_shared_markers", "skb_sketch_view_get", "skb_import_sketches",
     "skb_free", "skb_launch_count", "skb_stream", "skb_clear", "skb_timer_start", "skb_timer_stop", "skb_index_append", "skb_pop_last_add",
     "skb_device_edges", "skb_set_owned", "skb_screen_triangle", "skb_pairs_edges", "skb_greedy_summary", "skb_index_seed_tables", "skb_clear_keep_tables",
+    "skb_set_ani_estimator",
 ]
 
 _lib = None
@@ -165,6 +166,7 @@ def lib():
     L.skb_greedy_summary.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_double, C.c_double,
                                      C.POINTER(C.POINTER(C.c_int64)), C.POINTER(C.POINTER(C.c_int64)), C.POINTER(C.POINTER(C.c_uint32))]
     L.skb_clear.argtypes = [C.c_void_p]
+    L.skb_set_ani_estimator.argtypes = [C.c_void_p, C.c_int32]
     L.skb_index_seed_tables.argtypes = [C.c_void_p]
     L.skb_clear_keep_tables.argtypes = [C.c_void_p]
     L.skb_index_append.argtypes = [C.c_void_p]

@@ -9,9 +9,11 @@ without touching skDER.  Sub-commands and flags are exactly the ones skDER spell
   skani search   QUERY.fa -d DBDIR -o OUT -t T                   (skder.py:119)
   skani dist     --rl REFS --ql QUERIES [-s S] [-t T] -o OUT     (skder.py:58-59, cidder.py:362-363)
 
-Any other skani option (-c, -m, --fast, --slow, --medium, --small-genomes, --no-learned-ani, --robust,
---median, ...) changes skani's estimator in ways this engine does not implement: the shim then exits
-non-zero WITHOUT creating the output, which is the one failure signal runCmd checks (util.py:642-645).
+skDER hands its `-p` string to skani verbatim, so two estimator flags are accepted on triangle, dist and search:
+`--median` (median chain identity) and `--robust` (mean after trimming the 10 % / 90 % tails), DESIGN.md section 3.
+Any other skani option (-c, -m, --fast, --slow, --medium, --small-genomes, --no-learned-ani, --ci, ...) changes
+skani's estimator in ways this engine does not implement: the shim then exits non-zero WITHOUT creating the output,
+which is the one failure signal runCmd checks (util.py:642-645).
 stderr is discarded by skDER, so diagnostics also go to <output>.skani_b200.log.
 """
 import json
@@ -41,6 +43,8 @@ def parse_args(argv):
         "-d": "db",
     }
     flags = {"-E": "edge_list", "--sparse": "edge_list"}
+    estimators = {"--median": "median", "--robust": "robust"}
+    chosen = []
     i = 1
     while i < len(argv):
         a = argv[i]
@@ -55,6 +59,9 @@ def parse_args(argv):
         elif a in flags:
             opt[flags[a]] = True
             i += 1
+        elif a in estimators:
+            chosen.append(a)
+            i += 1
         elif a.startswith("-"):
             raise UsageError("skani option %r is not implemented by the B200 engine" % a)
         else:
@@ -66,6 +73,11 @@ def parse_args(argv):
         opt["threads"] = max(1, int(opt["threads"]))
     except ValueError as e:
         raise UsageError("bad numeric option: %s" % e)
+    if len(set(chosen)) > 1:
+        raise UsageError("--median and --robust are mutually exclusive")
+    if chosen and sub == "sketch":
+        raise UsageError("skani sketch takes no ANI estimator option (%s)" % chosen[0])
+    opt["estimator"] = estimators[chosen[0]] if chosen else "mean"
     need = {"triangle": ["list", "out"], "sketch": ["list", "out"], "search": ["db", "out"], "dist": ["rl", "ql", "out"]}[sub]
     for k in need:
         if k not in opt:
@@ -154,6 +166,7 @@ def run_triangle(opt, engine_mod):
     paths = sorted(set(read_list(opt["list"])))
     with engine_mod.Engine(_device()) as eng:
         ph["context_s"] = time.time() - t0
+        eng.set_estimator(opt["estimator"])
         names = stream_add(eng, engine_mod, paths, opt["threads"], ph)
         t1 = time.time()
         eng.index()
@@ -193,7 +206,7 @@ def run_search(opt, engine_mod):
         from . import daemon
 
         msg = {"op": "search", "query": query, "label": opt["positional"][0],  # the row shows the path as it was given
-               "screen": opt["screen"], "min_af": opt["min_af"], "out": out}
+               "screen": opt["screen"], "min_af": opt["min_af"], "estimator": opt["estimator"], "out": out}
         rep = daemon.request(db, dev, msg)
         if rep is not None and rep.get("stale"):  # the directory was rewritten under a running server: it has just exited
             deadline = time.time() + 15.0
@@ -222,6 +235,7 @@ def run_search(opt, engine_mod):
         man = json.load(f)
     paths, names = list(man["paths"]), list(man["names"])
     with engine_mod.Engine(dev) as eng:
+        eng.set_estimator(opt["estimator"])
         eng.load(opt["db"])
         eng.index()
         qp = engine_mod.pack_fasta(query, eng.params.min_contig_len)
@@ -235,6 +249,7 @@ def run_dist(opt, engine_mod):
     paths = list(dict.fromkeys(refs + queries))
     idx = {p: i for i, p in enumerate(paths)}
     with engine_mod.Engine(_device()) as eng:
+        eng.set_estimator(opt["estimator"])
         names = stream_add(eng, engine_mod, paths, opt["threads"])
         eng.index()
         edges, st = eng.rect([idx[p] for p in dict.fromkeys(refs)], [idx[p] for p in dict.fromkeys(queries)],
@@ -252,8 +267,11 @@ PROVENANCE = ("skani %s: produced by skder_b200 (B200 engine) in %.2f s -- NOT t
 def _provenance(opt, sub, seconds):
     """Say beside the output which estimator wrote it (skDER discards stdout/stderr).  Overwritten, not appended: the
     search output is rewritten thousands of times by the low_mem_greedy loop."""
+    text = PROVENANCE % (sub, seconds)
+    if opt.get("estimator", "mean") != "mean":
+        text += "ANI estimator: --%s (DESIGN.md section 3)\n" % opt["estimator"]
     try:
-        write_atomic(opt["out"].rstrip("/") + ".skani_b200.log", PROVENANCE % (sub, seconds))
+        write_atomic(opt["out"].rstrip("/") + ".skani_b200.log", text)
     except OSError:
         pass
 

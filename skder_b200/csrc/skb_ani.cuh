@@ -744,6 +744,24 @@ __global__ void cand_pack_kernel(DbView db, AniParams prm, const PairInfo *__res
     }
 }
 
+// ANI of `a_in` anchors over `s_in` query seeds (both > 0): raw = ratio^(1/k), then the debias substitute.  The one
+// place this arithmetic lives: the pooled mean (make_pair_out) and the median / robust estimators (est_pick_kernel).
+// Two steps, so that make_pair_out keeps its order of work (the AF in between): its register allocation is unchanged.
+__device__ __forceinline__ double ani_raw_of(int64_t a_in, int64_t s_in) {
+    double ratio = (double)a_in / (double)s_in;
+    if (ratio > 1.0) ratio = 1.0;
+    return pow(ratio, 1.0 / (double)K_SEED);
+}
+__device__ __forceinline__ double ani_debiased(const AniParams &prm, double raw) {
+    const double x = 100.0 * (1.0 - raw);
+    double ani = 1.0;
+    if (x > 0.0) {
+        ani = 1.0 - prm.debias_a * pow(x, prm.debias_g) / 100.0;
+        if (ani < 0.0) ani = 0.0;
+    }
+    return ani > 1.0 ? 1.0 : ani;
+}
+
 // The pair's result from the sums over its accepted chains (one thread).
 __device__ __forceinline__ PairOut make_pair_out(const DbView &db, const AniParams &prm, const PairInfo &pi, int64_t t_a,
                                                  int64_t t_s, int64_t t_span_q, int64_t t_span_r, int n_acc) {
@@ -759,21 +777,12 @@ __device__ __forceinline__ PairOut make_pair_out(const DbView &db, const AniPara
     // the two end anchors of every chain are anchors by construction: left out of both counts (oracle ora_pair)
     const int64_t a_in = o.n_anchors - 2 * (int64_t)o.n_chains, s_in = o.n_seeds - 2 * (int64_t)o.n_chains;
     if (a_in > 0 && s_in > 0) {
-        double ratio = (double)a_in / (double)s_in;
-        if (ratio > 1.0) ratio = 1.0;
-        const double mean = pow(ratio, 1.0 / (double)K_SEED);
-        o.ani_raw = mean;
+        o.ani_raw = ani_raw_of(a_in, s_in);
         double afq = (double)o.span_q / (double)db.g_total_len[pi.q];
         double afr = (double)o.span_r / (double)db.g_total_len[pi.r];
         o.af_q = afq > 1.0 ? 1.0 : afq;
         o.af_r = afr > 1.0 ? 1.0 : afr;
-        const double x = 100.0 * (1.0 - mean);
-        double ani = 1.0;
-        if (x > 0.0) {
-            ani = 1.0 - prm.debias_a * pow(x, prm.debias_g) / 100.0;
-            if (ani < 0.0) ani = 0.0;
-        }
-        o.ani = ani > 1.0 ? 1.0 : ani;
+        o.ani = ani_debiased(prm, o.ani_raw);
     }
     return o;
 }
@@ -838,12 +847,15 @@ __device__ __forceinline__ void fw_edge(const PCand *__restrict__ list, int i, i
     if (e < (uint32_t)FW_EDGES) edges[e] = i_first ? ((uint32_t)i << 16) | (uint32_t)j : ((uint32_t)j << 16) | (uint32_t)i;
 }
 
-// ctl: [0] largest candidate count among the listed mid pairs, [1] number of big pairs, [2] number of mid pairs
+// ctl: [0] largest candidate count among the listed mid pairs, [1] number of big pairs, [2] number of mid pairs.
+// ACC (median / robust estimators): also store every candidate's accepted flag at acc[its pcands index].
+template <bool ACC>
 __global__ void __launch_bounds__(FW_WARPS * 32)
 finalize_warp_kernel(DbView db, AniParams prm, const PairInfo *__restrict__ info, const uint32_t *__restrict__ task_off,
                      uint32_t base, int64_t n_pairs, const PCand *__restrict__ pcands, const uint32_t *__restrict__ cand_off,
                      const uint32_t *__restrict__ perm, PairOut *__restrict__ out, uint32_t wcap, uint32_t *ctl,
-                     uint32_t *__restrict__ mid_list, uint32_t *__restrict__ big_list, uint32_t *__restrict__ big_nc) {
+                     uint32_t *__restrict__ mid_list, uint32_t *__restrict__ big_list, uint32_t *__restrict__ big_nc,
+                     uint8_t *__restrict__ acc) {
     extern __shared__ __align__(16) unsigned char smem[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     unsigned char *my = smem + (size_t)warp * ((fw_bytes_per_warp(wcap) + 15) & ~(size_t)15);
@@ -973,6 +985,7 @@ finalize_warp_kernel(DbView db, AniParams prm, const PairInfo *__restrict__ info
         // ---- sums over the accepted chains
         uint32_t s_q = 0, s_r = 0, s_a = 0, s_s = 0, n_acc = 0;  // a lane sums <= wcap/32 spans: far below 2^32
         for (int t = lane; t < n; t += 32) {
+            if (ACC) acc[c0 + t] = (state[t] & 3) == 1;
             if ((state[t] & 3) != 1) continue;
             const uint4 w0 = __ldcg(reinterpret_cast<const uint4 *>(list + t));
             const uint2 w1 = __ldcg(reinterpret_cast<const uint2 *>(list + t) + 2);  // score n_anchors | n_seeds ext
@@ -1008,13 +1021,14 @@ constexpr uint32_t MAX_CHUNKS_PER_GENOME = 1u << 23;
 // BIG = false: candidates / keys / states in dynamic shared memory sized for `cap` candidates (a power of two >= the
 //   largest listed pair): PCand[cap] | u64 key[cap] | u8 state[cap].
 // BIG = true: the same three arrays in global scratch at big_off[blockIdx.x] (bytes), capacity big_cap[blockIdx.x].
-template <bool BIG>
+// ACC: as in finalize_warp_kernel.
+template <bool BIG, bool ACC>
 __global__ void __launch_bounds__(FIN_THREADS)
 finalize_kernel(DbView db, AniParams prm, const PairInfo *__restrict__ info, const uint32_t *__restrict__ task_off,
                 uint32_t base, int64_t n_pairs, const PCand *__restrict__ pcands, const uint32_t *__restrict__ cand_off,
                 const uint32_t *__restrict__ perm, PairOut *__restrict__ out,
                 uint32_t cap, const uint32_t *__restrict__ list, const unsigned long long *__restrict__ big_off,
-                const uint32_t *__restrict__ big_cap, unsigned char *__restrict__ big_scratch) {
+                const uint32_t *__restrict__ big_cap, unsigned char *__restrict__ big_scratch, uint8_t *__restrict__ acc) {
     extern __shared__ __align__(16) unsigned char smem[];
     __shared__ FinCtl ctl;
     const int tid = threadIdx.x;
@@ -1101,6 +1115,7 @@ finalize_kernel(DbView db, AniParams prm, const PairInfo *__restrict__ info, con
     int n_acc_local = 0;
     double l_span_q = 0, l_span_r = 0, l_a = 0, l_s = 0;  // exact in double (< 2^53); reduced below, no atomics
     for (int t = tid; t < nc; t += FIN_THREADS) {
+        if (ACC) acc[cand_off[t0] + (skey[t] & FIN_IDX_MASK)] = state[t] == 1;
         if (state[t] != 1) continue;
         n_acc_local++;
         const PCand &c = cands[(int)(skey[t] & FIN_IDX_MASK)];
@@ -1114,6 +1129,91 @@ finalize_kernel(DbView db, AniParams prm, const PairInfo *__restrict__ info, con
     const double t_acc = block_sum((double)n_acc_local, ctl.red, tid);
     if (tid == 0)
         out[perm[p]] = make_pair_out(db, prm, pi, (int64_t)t_a, (int64_t)t_s, (int64_t)t_span_q, (int64_t)t_span_r, (int)t_acc);
+}
+
+// ---- --median / --robust (DESIGN.md section 3): after the finalize kernels, per batch --------------------------------
+// est_key_kernel (thread per candidate) -> stable segmented sort of (key, candidate index), one segment per pair ->
+// est_pick_kernel (warp per pair).  The mean needs none of it.
+//
+// key of an accepted chain: (a << 47) / s with a = n_anchors - 2, s = n_seeds - 2 (both < 2^16, so distinct ratios get
+// distinct keys and equal ratios equal keys); a rejected chain sorts last.  The sort is stable and a pair's candidates
+// are listed in (chunk, ordinal) order, which breaks ties.  seg[p] (p <= n_pairs): first candidate of pair p.
+__global__ void est_key_kernel(const PCand *__restrict__ pcands, const uint8_t *__restrict__ acc, uint32_t n_cand,
+                               const uint32_t *__restrict__ task_off, uint32_t base, int64_t n_pairs,
+                               const uint32_t *__restrict__ cand_off, unsigned long long *__restrict__ key,
+                               uint32_t *__restrict__ idx, uint32_t *__restrict__ seg) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n_cand) {
+        unsigned long long k = ~0ull;
+        if (acc[i]) {
+            const PCand &c = pcands[i];
+            k = ((unsigned long long)(c.n_anchors - 2u) << 47) / (unsigned long long)(c.n_seeds - 2u);
+        }
+        key[i] = k;
+        idx[i] = (uint32_t)i;
+    }
+    if (i <= n_pairs) seg[i] = cand_off[task_off[i] - base];
+}
+
+// One warp per pair with an estimate: its accepted chains are the first n_chains of its sorted segment.  W = sum of
+// the weights s; C = their inclusive prefix, built 32 chains a round with a warp scan.
+//   median: the first chain with 2 C >= W (ballot);  robust: pooled a / s over the chains with 10 C > W and
+//   10 (C - s) < 9 W.  Rewrites ani / ani_raw; AF and the counts stay the totals over all accepted chains.
+__global__ void __launch_bounds__(FW_WARPS * 32)
+est_pick_kernel(AniParams prm, int32_t estimator /* SKB_ANI_MEDIAN or _ROBUST */, int64_t n_pairs, const uint32_t *__restrict__ seg,
+                const uint32_t *__restrict__ sorted, const PCand *__restrict__ pcands, const uint32_t *__restrict__ perm,
+                PairOut *__restrict__ out) {
+    const int lane = threadIdx.x & 31;
+    const int64_t warps_total = (int64_t)gridDim.x * FW_WARPS;
+    for (int64_t p = (int64_t)blockIdx.x * FW_WARPS + (threadIdx.x >> 5); p < n_pairs; p += warps_total) {
+        PairOut &o = out[perm[p]];
+        if (o.ani_raw < 0.0) continue;
+        const int n = o.n_chains;
+        const long long W = o.n_seeds - 2ll * n;
+        const uint32_t *list = sorted + seg[p];
+        long long carry = 0, sa = 0, ss = 0;
+        for (int r0 = 0; r0 < n; r0 += 32) {
+            const int t = r0 + lane;
+            long long a = 0, s = 0;
+            if (t < n) {
+                const uint2 w = __ldg(reinterpret_cast<const uint2 *>(pcands + list[t]) + 2);  // score n_anchors | n_seeds ext
+                a = (long long)(w.x >> 16) - 2;
+                s = (long long)(w.y & 0xffffu) - 2;
+            }
+            long long C = s;
+#pragma unroll
+            for (int d = 1; d < 32; d <<= 1) {
+                const long long y = __shfl_up_sync(0xffffffffu, C, d);
+                if (lane >= d) C += y;
+            }
+            C += carry;
+            if (estimator == SKB_ANI_MEDIAN) {
+                const unsigned hit = __ballot_sync(0xffffffffu, t < n && 2 * C >= W);
+                if (hit) {
+                    const int src = __ffs(hit) - 1;
+                    sa = __shfl_sync(0xffffffffu, a, src);
+                    ss = __shfl_sync(0xffffffffu, s, src);
+                    break;
+                }
+            } else if (t < n && 10 * C > W && 10 * (C - s) < 9 * W) {
+                sa += a;
+                ss += s;
+            }
+            carry = __shfl_sync(0xffffffffu, C, 31);
+            if (10 * carry >= 9 * W) break;  // every later chain starts at or beyond 9W/10: trimmed (median: found)
+        }
+        if (estimator != SKB_ANI_MEDIAN) {
+#pragma unroll
+            for (int d = 16; d > 0; d >>= 1) {
+                sa += __shfl_down_sync(0xffffffffu, sa, d);
+                ss += __shfl_down_sync(0xffffffffu, ss, d);
+            }
+        }
+        if (lane == 0) {
+            o.ani_raw = ani_raw_of(sa, ss);
+            o.ani = ani_debiased(prm, o.ani_raw);
+        }
+    }
 }
 
 // K5 -- edge compaction: keep pairs with an estimate and max(AF) >= min_af; percent units.  Order-preserving

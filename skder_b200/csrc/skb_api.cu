@@ -99,6 +99,7 @@ struct skb_ctx {
     int64_t launches = 0;
     int sm_count = 148;
     bool ani_attr_set = false;
+    int32_t estimator = SKB_ANI_MEAN;  // skb_set_ani_estimator; kept across skb_clear
     const skb_edge *last_dev_edges = nullptr;  // device copy of the last triangle/rect result (skb_device_edges)
     int64_t last_n_edges = 0;
     std::vector<cudaEvent_t> anchor_ev;  // start/stop pairs around the anchor kernel launches of the current call
@@ -396,6 +397,10 @@ void sketch_batch(skb_ctx *c, const skb_packed *const *gen, int32_t g0, int32_t 
 //   info      : roles and chunk count per pair
 //   task_off  : exclusive prefix of chunk counts -> task id = (pair, chunk)
 //   cands     : SLOTS candidate slots per task;  task_ncand: how many are filled
+// kernels cub::DeviceSegmentedSort launches for one call, at most: the partition of the segments by size (two), then the
+// large- and the small/medium-segment sorts (a call with few segments runs one kernel instead)
+constexpr int EST_SORT_LAUNCHES = 4;
+
 void run_ani(skb_ctx *c, const unsigned long long *d_pairs, int64_t n_pairs, PairOut *d_out) {
     c->anchor_ev_used = 0;
     if (n_pairs == 0) return;
@@ -410,11 +415,17 @@ void run_ani(skb_ctx *c, const unsigned long long *d_pairs, int64_t n_pairs, Pai
     }();
     const size_t fw_smem = (size_t)FW_WARPS * ((fw_bytes_per_warp(fw_cap) + 15) & ~(size_t)15);
     if (!c->ani_attr_set) {
-        CK(cudaFuncSetAttribute(finalize_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+        CK(cudaFuncSetAttribute(finalize_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                 (int)(FIN_BYTES_PER_CAND * MAXP)));
-        CK(cudaFuncSetAttribute(finalize_warp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fw_smem));
+        CK(cudaFuncSetAttribute(finalize_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                (int)(FIN_BYTES_PER_CAND * MAXP)));
+        CK(cudaFuncSetAttribute(finalize_warp_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fw_smem));
+        CK(cudaFuncSetAttribute(finalize_warp_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fw_smem));
         c->ani_attr_set = true;
     }
+    // median / robust: the finalize kernels also store every candidate's accepted flag, and an estimator stage per
+    // batch turns the accepted chains into one ANI (est_key_kernel, segmented sort, est_pick_kernel)
+    const bool est = c->estimator != SKB_ANI_MEAN;
     const DbView view = c->view();
     const AniParams prm = c->ani_params();
     c->d_info.reserve((size_t)n_pairs, 0, c->st);
@@ -511,6 +522,8 @@ void run_ani(skb_ctx *c, const unsigned long long *d_pairs, int64_t n_pairs, Pai
     b_mid_list.reserve((size_t)cap_pairs, 0, c->st);
     b_big_list.reserve((size_t)cap_pairs, 0, c->st);
     b_big_nc.reserve((size_t)cap_pairs, 0, c->st);
+    PoolRef<uint8_t> e_acc(c->pool["est.acc"]);
+    if (est) e_acc.reserve((size_t)cap * SLOTS, 0, c->st);
     // When no padded position of the database comes near 2^30, anchor_kernel matches and decodes seed records by their
     // 32-bit halves and chain_kernel compares diagonals (reference position -/+ query position, sign by strand) in 32
     // bits; SKB_WIDE_DIAG=1 forces the general variants (tests run both)
@@ -589,20 +602,24 @@ void run_ani(skb_ctx *c, const unsigned long long *d_pairs, int64_t n_pairs, Pai
             CK(cudaGetLastError());
             c->launches += 1;
         }
-        finalize_warp_kernel<<<nblk((uint64_t)np, FW_WARPS), FW_WARPS * 32, fw_smem, c->st>>>(
+        (est ? finalize_warp_kernel<true> : finalize_warp_kernel<false>)<<<nblk((uint64_t)np, FW_WARPS), FW_WARPS * 32, fw_smem,
+                                                                          c->st>>>(
             view, prm, d_info_s.p + bt.p0, c->d_task_off.p + bt.p0, base, np, b_pcands.p, b_cand_off.p, d_perm.p + bt.p0, d_out,
-            fw_cap, b_fctl.p, b_mid_list.p, b_big_list.p, b_big_nc.p);
+            fw_cap, b_fctl.p, b_mid_list.p, b_big_list.p, b_big_nc.p, e_acc.p);
         CK(cudaGetLastError());
         uint32_t fctl[4] = {0, 0, 0, 0};
+        uint32_t n_cand = 0;
         CK(cudaMemcpyAsync(fctl, b_fctl.p, 16, cudaMemcpyDeviceToHost, c->st));
+        if (est && tasks) CK(cudaMemcpyAsync(&n_cand, b_cand_off.p + tasks, 4, cudaMemcpyDeviceToHost, c->st));
         CK(cudaStreamSynchronize(c->st));
         c->launches += 1;
         if (fctl[2]) {  // more than fw_cap candidates or more than FW_EDGES blocking relations: shared memory, one CTA per pair
             uint32_t fcap = 32;
             while (fcap < fctl[0]) fcap <<= 1;
-            finalize_kernel<false><<<fctl[2], FIN_THREADS, FIN_BYTES_PER_CAND * (size_t)fcap, c->st>>>(
+            (est ? finalize_kernel<false, true> : finalize_kernel<false, false>)<<<fctl[2], FIN_THREADS,
+                                                                                  FIN_BYTES_PER_CAND * (size_t)fcap, c->st>>>(
                 view, prm, d_info_s.p + bt.p0, c->d_task_off.p + bt.p0, base, np, b_pcands.p, b_cand_off.p,
-                d_perm.p + bt.p0, d_out, fcap, b_mid_list.p, nullptr, nullptr, nullptr);
+                d_perm.p + bt.p0, d_out, fcap, b_mid_list.p, nullptr, nullptr, nullptr, e_acc.p);
             CK(cudaGetLastError());
             c->launches += 1;
         }
@@ -628,14 +645,38 @@ void run_ani(skb_ctx *c, const unsigned long long *d_pairs, int64_t n_pairs, Pai
             d_big.reserve((size_t)off + 256, 0, c->st);
             d_big_off.upload(h_off, c->st);
             d_big_cap.upload(h_cap, c->st);
-            finalize_kernel<true><<<nbig, FIN_THREADS, 0, c->st>>>(view, prm, d_info_s.p + bt.p0, c->d_task_off.p + bt.p0, base, np,
-                                                                 b_pcands.p, b_cand_off.p, d_perm.p + bt.p0, d_out, 0,
-                                                                 b_big_list.p, d_big_off.p, d_big_cap.p, d_big.p);
+            (est ? finalize_kernel<true, true> : finalize_kernel<true, false>)<<<nbig, FIN_THREADS, 0, c->st>>>(
+                view, prm, d_info_s.p + bt.p0, c->d_task_off.p + bt.p0, base, np, b_pcands.p, b_cand_off.p, d_perm.p + bt.p0,
+                d_out, 0, b_big_list.p, d_big_off.p, d_big_cap.p, d_big.p, e_acc.p);
             CK(cudaGetLastError());
             c->launches++;
             CK(cudaStreamSynchronize(c->st));  // h_off / h_cap leave scope
         }
         if (trace) spans.push_back({"finalize", bi, tf, mark()});
+        if (est && n_cand) {
+            cudaEvent_t te = mark();
+            PoolRef<unsigned long long> e_key(c->pool["est.key"]), e_key_s(c->pool["est.key_sorted"]);
+            PoolRef<uint32_t> e_idx(c->pool["est.idx"]), e_idx_s(c->pool["est.idx_sorted"]), e_seg(c->pool["est.seg"]);
+            e_key.reserve(n_cand, 0, c->st);
+            e_key_s.reserve(n_cand, 0, c->st);
+            e_idx.reserve(n_cand, 0, c->st);
+            e_idx_s.reserve(n_cand, 0, c->st);
+            e_seg.reserve((size_t)np + 1, 0, c->st);
+            est_key_kernel<<<nblk(std::max<uint64_t>(n_cand, (uint64_t)np + 1), 256), 256, 0, c->st>>>(
+                b_pcands.p, e_acc.p, n_cand, c->d_task_off.p + bt.p0, base, np, b_cand_off.p, e_key.p, e_idx.p, e_seg.p);
+            CK(cudaGetLastError());
+            size_t bytes = 0;
+            CK(cub::DeviceSegmentedSort::StableSortPairs(nullptr, bytes, e_key.p, e_key_s.p, e_idx.p, e_idx_s.p, (int)n_cand,
+                                                         (int)np, e_seg.p, e_seg.p + 1, c->st));
+            c->d_tmp.reserve(bytes + 16, 0, c->st);
+            CK(cub::DeviceSegmentedSort::StableSortPairs(c->d_tmp.p, bytes, e_key.p, e_key_s.p, e_idx.p, e_idx_s.p, (int)n_cand,
+                                                         (int)np, e_seg.p, e_seg.p + 1, c->st));
+            est_pick_kernel<<<nblk((uint64_t)np, FW_WARPS), FW_WARPS * 32, 0, c->st>>>(prm, c->estimator, np, e_seg.p, e_idx_s.p,
+                                                                                     b_pcands.p, d_perm.p + bt.p0, d_out);
+            CK(cudaGetLastError());
+            c->launches += 2 + EST_SORT_LAUNCHES;
+            if (trace) spans.push_back({"estimator", bi, te, mark()});
+        }
     }
     if (trace) {
         CK(cudaStreamSynchronize(c->st));
@@ -1615,6 +1656,15 @@ int skb_rect(skb_ctx *ctx, const int32_t *refs, int32_t n_refs, const int32_t *q
             stats->sum_anchors = (int64_t)run.sums[1];
         }
         return emit_edges(c, run, edges, n_edges);
+    });
+}
+
+int skb_set_ani_estimator(skb_ctx *ctx, int32_t estimator) {
+    return guarded(ctx, [&]() -> int {
+        if (estimator != SKB_ANI_MEAN && estimator != SKB_ANI_MEDIAN && estimator != SKB_ANI_ROBUST)
+            return fail(ctx, SKB_EINVAL, "unknown ANI estimator " + std::to_string(estimator));
+        ctx->estimator = estimator;
+        return SKB_OK;
     });
 }
 

@@ -157,6 +157,7 @@ def serve(db_dir, device):
                         conn.send_bytes(json.dumps({"ok": True}).encode())
                         stop = True
                     elif msg.get("op") == "search":
+                        eng.set_estimator(msg.get("estimator", "mean"))  # per request: a resident server serves every mode
                         packed = engine.pack_fasta(msg["query"], eng.params.min_contig_len)
                         edges, st = eng.search(packed, screen=msg["screen"], min_af=msg["min_af"])
                         rows = cli.rect_rows(paths + [msg.get("label", msg["query"])], names + [packed.first_name], edges)

@@ -120,6 +120,15 @@ class Engine:
         if rc != 0:
             raise SkbError("%s failed (%d): %s" % (what, rc, self._L.skb_last_error(self._h).decode()))
 
+    ESTIMATORS = {"mean": 0, "median": 1, "robust": 2}  # SKB_ANI_MEAN / _MEDIAN / _ROBUST
+
+    def set_estimator(self, name):
+        """How a pair's accepted chains become one ANI in later triangle / rect / search / pairs calls: "mean" (skani's
+        default), "median" (--median) or "robust" (--robust); DESIGN.md section 3.  Survives clear()."""
+        if name not in self.ESTIMATORS:
+            raise ValueError("unknown ANI estimator %r (mean, median, robust)" % (name,))
+        self._ck(self._L.skb_set_ani_estimator(self._h, self.ESTIMATORS[name]), "skb_set_ani_estimator")
+
     # ---- sketching -------------------------------------------------------------------------
     def add(self, packed):
         n = len(packed)
