@@ -151,6 +151,16 @@ int skb_rect(skb_ctx *ctx, const int32_t *refs, int32_t n_refs, const int32_t *q
 #define SKB_ANI_ROBUST 2
 int skb_set_ani_estimator(skb_ctx *ctx, int32_t estimator);
 
+/* skani's --ci (DESIGN.md section 3): a percentile-bootstrap interval of every edge's ANI (100 replicates of the pair's
+ * accepted chains; 5th and 95th percentile).  Context state, kept across skb_clear: enabled != 0 applies to every later
+ * skb_triangle, skb_rect and skb_pairs_edges call, which return SKB_EINVAL while it is on and the estimator is not
+ * SKB_ANI_MEAN.  The edges themselves are the same with and without it. */
+int skb_set_ani_ci(skb_ctx *ctx, int32_t enabled);
+/* The intervals of the edge list of the last skb_triangle, skb_rect or skb_pairs_edges call on this context (also one
+ * made with edges == NULL), in edge order: lo_hi[2 i] and lo_hi[2 i + 1] are edge i's lower and upper bound, percent on
+ * the ANI's scale; *n = that call's edge count.  malloc'ed (skb_free).  SKB_ESTATE if that call ran without --ci. */
+int skb_last_edge_ci(skb_ctx *ctx, double **lo_hi, int64_t *n);
+
 /* explicit pair list, full detail, no screening / no AF filter (parity tests) */
 int skb_pairs_detail(skb_ctx *ctx, const uint32_t *a, const uint32_t *b, int64_t n, skb_pair_detail *out);
 /* shared-marker counts of an explicit pair list (prescreen parity) */

@@ -103,7 +103,7 @@ SYMBOLS = [
     "skb_rect", "skb_pairs_detail", "skb_shared_markers", "skb_sketch_view_get", "skb_import_sketches",
     "skb_free", "skb_launch_count", "skb_stream", "skb_clear", "skb_timer_start", "skb_timer_stop", "skb_index_append", "skb_pop_last_add",
     "skb_device_edges", "skb_set_owned", "skb_screen_triangle", "skb_pairs_edges", "skb_greedy_summary", "skb_index_seed_tables", "skb_clear_keep_tables",
-    "skb_set_ani_estimator",
+    "skb_set_ani_estimator", "skb_set_ani_ci", "skb_last_edge_ci",
 ]
 
 _lib = None
@@ -167,6 +167,8 @@ def lib():
                                      C.POINTER(C.POINTER(C.c_int64)), C.POINTER(C.POINTER(C.c_int64)), C.POINTER(C.POINTER(C.c_uint32))]
     L.skb_clear.argtypes = [C.c_void_p]
     L.skb_set_ani_estimator.argtypes = [C.c_void_p, C.c_int32]
+    L.skb_set_ani_ci.argtypes = [C.c_void_p, C.c_int32]
+    L.skb_last_edge_ci.argtypes = [C.c_void_p, C.POINTER(C.POINTER(C.c_double)), C.POINTER(C.c_int64)]
     L.skb_index_seed_tables.argtypes = [C.c_void_p]
     L.skb_clear_keep_tables.argtypes = [C.c_void_p]
     L.skb_index_append.argtypes = [C.c_void_p]

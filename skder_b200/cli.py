@@ -9,11 +9,14 @@ without touching skDER.  Sub-commands and flags are exactly the ones skDER spell
   skani search   QUERY.fa -d DBDIR -o OUT -t T                   (skder.py:119)
   skani dist     --rl REFS --ql QUERIES [-s S] [-t T] -o OUT     (skder.py:58-59, cidder.py:362-363)
 
-skDER hands its `-p` string to skani verbatim, so two estimator flags are accepted on triangle, dist and search:
-`--median` (median chain identity) and `--robust` (mean after trimming the 10 % / 90 % tails), DESIGN.md section 3.
-Any other skani option (-c, -m, --fast, --slow, --medium, --small-genomes, --no-learned-ani, --ci, ...) changes
-skani's estimator in ways this engine does not implement: the shim then exits non-zero WITHOUT creating the output,
-which is the one failure signal runCmd checks (util.py:642-645).
+skDER hands its `-p` string to skani verbatim, so three ANI flags are accepted on triangle, dist and search
+(DESIGN.md section 3): the estimators `--median` (median chain identity) and `--robust` (mean after trimming the
+10 % / 90 % tails), and `--ci`, which appends a bootstrap interval of the mean ANI as two columns, ANI_5_percentile and
+ANI_95_percentile (not with --median / --robust).  skDER's `-n` clustering reads exactly seven fields
+(skder.py:190), so a `-p` with --ci breaks it as it would with skani; greedy and dynamic selection are unaffected.
+Any other skani option (-c, -m, --fast, --slow, --medium, --small-genomes, --no-learned-ani, ...) changes skani's
+estimator in ways this engine does not implement: the shim then exits non-zero WITHOUT creating the output, which is
+the one failure signal runCmd checks (util.py:642-645).
 stderr is discarded by skDER, so diagnostics also go to <output>.skani_b200.log.
 """
 import json
@@ -42,7 +45,8 @@ def parse_args(argv):
         "-l": "list", "-o": "out", "-t": "threads", "-s": "screen", "--min-af": "min_af", "--rl": "rl", "--ql": "ql",
         "-d": "db",
     }
-    flags = {"-E": "edge_list", "--sparse": "edge_list"}
+    flags = {"-E": "edge_list", "--sparse": "edge_list", "--ci": "ci"}
+    opt["ci"] = False
     estimators = {"--median": "median", "--robust": "robust"}
     chosen = []
     i = 1
@@ -78,6 +82,10 @@ def parse_args(argv):
     if chosen and sub == "sketch":
         raise UsageError("skani sketch takes no ANI estimator option (%s)" % chosen[0])
     opt["estimator"] = estimators[chosen[0]] if chosen else "mean"
+    if opt["ci"] and sub == "sketch":
+        raise UsageError("skani sketch takes no --ci")
+    if opt["ci"] and chosen:
+        raise UsageError("--ci is defined for the default (mean) ANI only, not with %s" % chosen[0])
     need = {"triangle": ["list", "out"], "sketch": ["list", "out"], "search": ["db", "out"], "dist": ["rl", "ql", "out"]}[sub]
     for k in need:
         if k not in opt:
@@ -96,8 +104,13 @@ def read_list(path):
         return [ln.strip() for ln in f if ln.strip()]
 
 
-def fmt_row(ref, query, ani, af_ref, af_query, ref_name, query_name):
-    return "%s\t%s\t%.2f\t%.2f\t%.2f\t%s\t%s\n" % (ref, query, ani, af_ref, af_query, ref_name, query_name)
+def header(ci):
+    return HEADER[:-1] + "\tANI_5_percentile\tANI_95_percentile\n" if ci else HEADER
+
+
+def fmt_row(ref, query, ani, af_ref, af_query, ref_name, query_name, ci=None):
+    row = "%s\t%s\t%.2f\t%.2f\t%.2f\t%s\t%s" % (ref, query, ani, af_ref, af_query, ref_name, query_name)
+    return row + ("\n" if ci is None else "\t%.2f\t%.2f\n" % ci)
 
 
 def write_atomic(path, text):
@@ -108,18 +121,23 @@ def write_atomic(path, text):
     os.replace(tmp, path)
 
 
-def triangle_rows(paths_sorted, names, edges):
-    """edges: structured array (a < b, ids index paths_sorted).  Ref = lexicographically smaller path
-    (SURVEY.md section 4 fact 3); rows grouped by Ref."""
-    cols = [edges[k].tolist() for k in ("a", "b", "ani", "af_a", "af_b")]  # element access on structured arrays is slow
-    return [fmt_row(paths_sorted[a], paths_sorted[b], ani, afa, afb, names[a], names[b]) for a, b, ani, afa, afb in zip(*cols)]
-
-
-def rect_rows(paths, names, edges):
-    """edges: a = reference id, b = query id.  Rows grouped by query, ANI descending (SURVEY.md section 4 fact 7)."""
+def _cols(edges, ci):
+    """the edges' columns (element access on structured arrays is slow), plus (lo, hi) per edge or None without --ci"""
     cols = [edges[k].tolist() for k in ("a", "b", "ani", "af_a", "af_b")]
-    rows = sorted(zip(*cols), key=lambda t: (t[1], -t[2], t[0]))
-    return [fmt_row(paths[a], paths[b], ani, afa, afb, names[a], names[b]) for a, b, ani, afa, afb in rows]
+    return cols + [[tuple(x) for x in ci.tolist()] if ci is not None else [None] * len(edges)]
+
+
+def triangle_rows(paths_sorted, names, edges, ci=None):
+    """edges: structured array (a < b, ids index paths_sorted).  Ref = lexicographically smaller path
+    (SURVEY.md section 4 fact 3); rows grouped by Ref.  ci: Engine.last_edge_ci() for --ci's two extra columns."""
+    return [fmt_row(paths_sorted[a], paths_sorted[b], ani, afa, afb, names[a], names[b], iv)
+            for a, b, ani, afa, afb, iv in zip(*_cols(edges, ci))]
+
+
+def rect_rows(paths, names, edges, ci=None):
+    """edges: a = reference id, b = query id.  Rows grouped by query, ANI descending (SURVEY.md section 4 fact 7)."""
+    rows = sorted(zip(*_cols(edges, ci)), key=lambda t: (t[1], -t[2], t[0]))
+    return [fmt_row(paths[a], paths[b], ani, afa, afb, names[a], names[b], iv) for a, b, ani, afa, afb, iv in rows]
 
 
 def _device():
@@ -167,13 +185,15 @@ def run_triangle(opt, engine_mod):
     with engine_mod.Engine(_device()) as eng:
         ph["context_s"] = time.time() - t0
         eng.set_estimator(opt["estimator"])
+        eng.set_ci(opt["ci"])
         names = stream_add(eng, engine_mod, paths, opt["threads"], ph)
         t1 = time.time()
         eng.index()
         t2 = time.time()
         edges, st = eng.triangle(screen=opt["screen"], min_af=opt["min_af"])
+        ci = eng.last_edge_ci() if opt["ci"] else None
         t3 = time.time()
-    write_atomic(opt["out"], HEADER + "".join(triangle_rows(paths, names, edges)))
+    write_atomic(opt["out"], header(opt["ci"]) + "".join(triangle_rows(paths, names, edges, ci)))
     ph.update({"index_s": t2 - t1, "triangle_s": t3 - t2, "write_tsv_s": time.time() - t3, "total_s": time.time() - t0,
                "genomes": len(paths), "edges": int(len(edges))})
     _phase_log(opt, ph)
@@ -206,7 +226,7 @@ def run_search(opt, engine_mod):
         from . import daemon
 
         msg = {"op": "search", "query": query, "label": opt["positional"][0],  # the row shows the path as it was given
-               "screen": opt["screen"], "min_af": opt["min_af"], "estimator": opt["estimator"], "out": out}
+               "screen": opt["screen"], "min_af": opt["min_af"], "estimator": opt["estimator"], "ci": opt["ci"], "out": out}
         rep = daemon.request(db, dev, msg)
         if rep is not None and rep.get("stale"):  # the directory was rewritten under a running server: it has just exited
             deadline = time.time() + 15.0
@@ -236,11 +256,13 @@ def run_search(opt, engine_mod):
     paths, names = list(man["paths"]), list(man["names"])
     with engine_mod.Engine(dev) as eng:
         eng.set_estimator(opt["estimator"])
+        eng.set_ci(opt["ci"])
         eng.load(opt["db"])
         eng.index()
         qp = engine_mod.pack_fasta(query, eng.params.min_contig_len)
         edges, st = eng.search(qp, screen=opt["screen"], min_af=opt["min_af"])
-    write_atomic(opt["out"], HEADER + "".join(rect_rows(paths + [query], names + [qp.first_name], edges)))
+        ci = eng.last_edge_ci() if opt["ci"] else None
+    write_atomic(opt["out"], header(opt["ci"]) + "".join(rect_rows(paths + [query], names + [qp.first_name], edges, ci)))
     return st
 
 
@@ -250,11 +272,13 @@ def run_dist(opt, engine_mod):
     idx = {p: i for i, p in enumerate(paths)}
     with engine_mod.Engine(_device()) as eng:
         eng.set_estimator(opt["estimator"])
+        eng.set_ci(opt["ci"])
         names = stream_add(eng, engine_mod, paths, opt["threads"])
         eng.index()
         edges, st = eng.rect([idx[p] for p in dict.fromkeys(refs)], [idx[p] for p in dict.fromkeys(queries)],
                              screen=opt["screen"], min_af=opt["min_af"])
-    write_atomic(opt["out"], HEADER + "".join(rect_rows(paths, names, edges)))
+        ci = eng.last_edge_ci() if opt["ci"] else None
+    write_atomic(opt["out"], header(opt["ci"]) + "".join(rect_rows(paths, names, edges, ci)))
     return st
 
 
@@ -270,6 +294,9 @@ def _provenance(opt, sub, seconds):
     text = PROVENANCE % (sub, seconds)
     if opt.get("estimator", "mean") != "mean":
         text += "ANI estimator: --%s (DESIGN.md section 3)\n" % opt["estimator"]
+    if opt.get("ci"):
+        text += ("--ci: ANI_5_percentile / ANI_95_percentile are a 100-replicate bootstrap of the pair's chains as DESIGN.md "
+                 "section 3 defines it; unpinned against skani's own intervals\n")
     try:
         write_atomic(opt["out"].rstrip("/") + ".skani_b200.log", text)
     except OSError:

@@ -745,7 +745,8 @@ __global__ void cand_pack_kernel(DbView db, AniParams prm, const PairInfo *__res
 }
 
 // ANI of `a_in` anchors over `s_in` query seeds (both > 0): raw = ratio^(1/k), then the debias substitute.  The one
-// place this arithmetic lives: the pooled mean (make_pair_out) and the median / robust estimators (est_pick_kernel).
+// place this arithmetic lives: the pooled mean (make_pair_out), the median / robust estimators (est_pick_kernel) and
+// the --ci bounds (ci_kernel).
 // Two steps, so that make_pair_out keeps its order of work (the AF in between): its register allocation is unchanged.
 __device__ __forceinline__ double ani_raw_of(int64_t a_in, int64_t s_in) {
     double ratio = (double)a_in / (double)s_in;
@@ -848,7 +849,7 @@ __device__ __forceinline__ void fw_edge(const PCand *__restrict__ list, int i, i
 }
 
 // ctl: [0] largest candidate count among the listed mid pairs, [1] number of big pairs, [2] number of mid pairs.
-// ACC (median / robust estimators): also store every candidate's accepted flag at acc[its pcands index].
+// ACC (median / robust estimators, --ci): also store every candidate's accepted flag at acc[its pcands index].
 template <bool ACC>
 __global__ void __launch_bounds__(FW_WARPS * 32)
 finalize_warp_kernel(DbView db, AniParams prm, const PairInfo *__restrict__ info, const uint32_t *__restrict__ task_off,
@@ -1216,6 +1217,132 @@ est_pick_kernel(AniParams prm, int32_t estimator /* SKB_ANI_MEDIAN or _ROBUST */
     }
 }
 
+// ---- --ci (DESIGN.md section 3): percentile-bootstrap interval of the mean ANI, after the finalize kernels, per batch --
+// ci_kernel, one warp per pair with an estimate:
+//   1. its accepted chains, in candidate ((chunk, ordinal)) order, go to `chains` at the pair's candidate offset as
+//      (a << 16 | s), a = n_anchors - 2, s = n_seeds - 2 (a ballot scan over the accepted flags);
+//   2. CI_REPS replicates draw n chains each with replacement (lane per replicate, the last few split over 8 lanes);
+//   3. the replicates are ranked by A_b / S_b exactly (128-bit cross products, ties by b: a bitonic sort of their indices
+//      in shared memory), and ranks CI_LO and CI_HI become (lo, hi) through the same ratio -> raw -> debiased arithmetic
+//      as the ANI.  ci[perm[p]] = (lo, hi) as fractions; (-1, -1) for a pair without an estimate.
+// Integers throughout up to the two pow calls: s >= a >= 1 for every chain (min_anchors >= 3, one seed per anchor).
+constexpr int CI_REPS = 100, CI_LO = 5, CI_HI = 94;
+constexpr int CI_SORT = 128;  // the bitonic network's size (>= CI_REPS)
+
+__device__ __forceinline__ uint64_t ci_mix(uint64_t z) {  // splitmix64 finalizer
+    z += 0x9E3779B97F4A7C15ull;
+    z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
+    z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
+    return z ^ (z >> 31);
+}
+
+// replicate x sorts after replicate y: A_x / S_x > A_y / S_y, ties by index; indices >= CI_REPS (padding) last
+__device__ __forceinline__ bool ci_after(int x, int y, const unsigned long long *ra, const unsigned long long *rs) {
+    if (x >= CI_REPS || y >= CI_REPS) return x > y;
+    const unsigned long long hx = __umul64hi(ra[x], rs[y]), hy = __umul64hi(ra[y], rs[x]);
+    if (hx != hy) return hx > hy;
+    const unsigned long long lx = ra[x] * rs[y], ly = ra[y] * rs[x];
+    return lx != ly ? lx > ly : x > y;
+}
+
+__global__ void __launch_bounds__(FW_WARPS * 32)
+ci_kernel(AniParams prm, const PairInfo *__restrict__ info, const uint32_t *__restrict__ task_off, uint32_t base,
+          int64_t n_pairs, const PCand *__restrict__ pcands, const uint32_t *__restrict__ cand_off,
+          const uint8_t *__restrict__ acc, uint32_t *__restrict__ chains, const uint32_t *__restrict__ perm,
+          const PairOut *__restrict__ out, double2 *__restrict__ ci) {
+    __shared__ unsigned long long s_a[FW_WARPS][CI_REPS], s_s[FW_WARPS][CI_REPS];
+    __shared__ uint8_t s_idx[FW_WARPS][CI_SORT];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    unsigned long long *ra = s_a[warp], *rs = s_s[warp];
+    uint8_t *idx = s_idx[warp];
+    const int64_t warps_total = (int64_t)gridDim.x * FW_WARPS;
+    for (int64_t p = (int64_t)blockIdx.x * FW_WARPS + warp; p < n_pairs; p += warps_total) {
+        const uint32_t dst = perm[p];
+        const PairOut &o = out[dst];
+        if (o.ani_raw < 0.0) {
+            if (lane == 0) ci[dst] = make_double2(-1.0, -1.0);
+            continue;
+        }
+        // ---- 1. accepted chains, compacted
+        const PairInfo pi = info[p];
+        const uint32_t t0 = task_off[p] - base;
+        const uint32_t c0 = cand_off[t0], nc = cand_off[t0 + pi.nch] - c0;
+        uint32_t *list = chains + c0;
+        uint32_t m = 0;
+        for (uint32_t r0 = 0; r0 < nc; r0 += 32) {
+            const uint32_t t = r0 + lane;
+            const bool on = t < nc && __ldg(acc + c0 + t);
+            const unsigned bal = __ballot_sync(0xffffffffu, on);
+            if (on) {
+                const uint2 w = __ldg(reinterpret_cast<const uint2 *>(pcands + c0 + t) + 2);  // score n_anchors | n_seeds ext
+                list[m + __popc(bal & ((1u << lane) - 1u))] = (((w.x >> 16) - 2u) << 16) | ((w.y & 0xffffu) - 2u);
+            }
+            m += __popc(bal);
+        }
+        __syncwarp();
+        // ---- 2. replicates: (A_b, S_b) over n draws j = (mix(seed ^ b << 40 ^ i) * n) >> 64
+        const unsigned long long n = (unsigned long long)o.n_chains;  // == m
+        const unsigned long long A = (unsigned long long)o.n_anchors - 2 * n, S = (unsigned long long)o.n_seeds - 2 * n;
+        const unsigned long long seed = ci_mix(ci_mix(ci_mix(n) ^ A) ^ S);
+        constexpr int FULL = CI_REPS / 32 * 32;  // replicates one lane draws alone
+        for (int b = lane; b < FULL; b += 32) {
+            const unsigned long long rb = seed ^ ((unsigned long long)b << 40);
+            unsigned long long sa = 0, ss = 0;
+            for (unsigned long long i = 0; i < n; i++) {
+                const uint32_t v = list[__umul64hi(ci_mix(rb ^ i), n)];
+                sa += v >> 16;
+                ss += v & 0xffffu;
+            }
+            ra[b] = sa;
+            rs[b] = ss;
+        }
+        static_assert(CI_REPS - FULL <= 4, "the remaining replicates take 8 lanes each");
+        {
+            const int b = FULL + (lane >> 3);
+            const unsigned long long rb = seed ^ ((unsigned long long)b << 40);
+            unsigned long long sa = 0, ss = 0;
+            if (b < CI_REPS)
+                for (unsigned long long i = lane & 7; i < n; i += 8) {
+                    const uint32_t v = list[__umul64hi(ci_mix(rb ^ i), n)];
+                    sa += v >> 16;
+                    ss += v & 0xffffu;
+                }
+#pragma unroll
+            for (int d = 4; d > 0; d >>= 1) {
+                sa += __shfl_xor_sync(0xffffffffu, sa, d);
+                ss += __shfl_xor_sync(0xffffffffu, ss, d);
+            }
+            if (b < CI_REPS && (lane & 7) == 0) {
+                ra[b] = sa;
+                rs[b] = ss;
+            }
+        }
+        for (int t = lane; t < CI_SORT; t += 32) idx[t] = (uint8_t)t;
+        __syncwarp();
+        // ---- 3. rank: bitonic sort of the replicate indices
+        for (int k = 2; k <= CI_SORT; k <<= 1)
+            for (int j = k >> 1; j > 0; j >>= 1) {
+                for (int t = lane; t < CI_SORT / 2; t += 32) {
+                    const int i = ((t & ~(j - 1)) << 1) | (t & (j - 1));
+                    const int q = i | j;
+                    const bool up = (i & k) == 0;
+                    const int x = idx[i], y = idx[q];
+                    if (ci_after(x, y, ra, rs) == up) {
+                        idx[i] = (uint8_t)y;
+                        idx[q] = (uint8_t)x;
+                    }
+                }
+                __syncwarp();
+            }
+        if (lane == 0) {
+            const int lo = idx[CI_LO], hi = idx[CI_HI];
+            ci[dst] = make_double2(ani_debiased(prm, ani_raw_of((int64_t)ra[lo], (int64_t)rs[lo])),
+                                   ani_debiased(prm, ani_raw_of((int64_t)ra[hi], (int64_t)rs[hi])));
+        }
+        __syncwarp();
+    }
+}
+
 // K5 -- edge compaction: keep pairs with an estimate and max(AF) >= min_af; percent units.  Order-preserving
 // (flag -> exclusive scan -> scatter): the pair list is sorted by (a, b), so the edge list comes out sorted too.
 __device__ __forceinline__ bool edge_kept(const PairOut &o, double min_af) {
@@ -1242,6 +1369,13 @@ __global__ void edge_scatter_kernel(const unsigned long long *__restrict__ pairs
     e.af_a = (o.swapped ? o.af_r : o.af_q) * 100.0;
     e.af_b = (o.swapped ? o.af_q : o.af_r) * 100.0;
     edges[pos[t]] = e;
+}
+// --ci only: the kept pairs' intervals in edge order, percent (edge_flag_kernel's flags, their scan)
+__global__ void edge_ci_scatter_kernel(const double2 *__restrict__ ci, int64_t n_pairs, const uint32_t *__restrict__ flag,
+                                       const uint32_t *__restrict__ pos, double2 *__restrict__ edge_ci) {
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= n_pairs || !flag[t]) return;
+    edge_ci[pos[t]] = make_double2(ci[t].x * 100.0, ci[t].y * 100.0);
 }
 
 // bookkeeping: sum over pairs of the query genome's seed count and of the chained anchors (roofline bytes)

@@ -100,8 +100,11 @@ struct skb_ctx {
     int sm_count = 148;
     bool ani_attr_set = false;
     int32_t estimator = SKB_ANI_MEAN;  // skb_set_ani_estimator; kept across skb_clear
+    bool ci = false;                   // skb_set_ani_ci; kept across skb_clear
     const skb_edge *last_dev_edges = nullptr;  // device copy of the last triangle/rect result (skb_device_edges)
     int64_t last_n_edges = 0;
+    bool last_ci = false;                 // that call ran with --ci ...
+    const double2 *last_dev_ci = nullptr;  // ... and left the edges' intervals here (skb_last_edge_ci)
     std::vector<cudaEvent_t> anchor_ev;  // start/stop pairs around the anchor kernel launches of the current call
     int anchor_ev_used = 0;
     float last_ms_anchor = 0;
@@ -401,7 +404,8 @@ void sketch_batch(skb_ctx *c, const skb_packed *const *gen, int32_t g0, int32_t 
 // large- and the small/medium-segment sorts (a call with few segments runs one kernel instead)
 constexpr int EST_SORT_LAUNCHES = 4;
 
-void run_ani(skb_ctx *c, const unsigned long long *d_pairs, int64_t n_pairs, PairOut *d_out) {
+// d_ci: nullptr, or [n_pairs] for every pair's --ci interval (ci_kernel), indexed like d_out
+void run_ani(skb_ctx *c, const unsigned long long *d_pairs, int64_t n_pairs, PairOut *d_out, double2 *d_ci = nullptr) {
     c->anchor_ev_used = 0;
     if (n_pairs == 0) return;
     if (n_pairs >= (1ll << 31)) throw CudaFail{"too many surviving pairs in one call"};
@@ -426,6 +430,8 @@ void run_ani(skb_ctx *c, const unsigned long long *d_pairs, int64_t n_pairs, Pai
     // median / robust: the finalize kernels also store every candidate's accepted flag, and an estimator stage per
     // batch turns the accepted chains into one ANI (est_key_kernel, segmented sort, est_pick_kernel)
     const bool est = c->estimator != SKB_ANI_MEAN;
+    // --ci: the accepted flags too, and ci_kernel per batch bootstraps the pair's accepted chains
+    const bool acc = est || d_ci;
     const DbView view = c->view();
     const AniParams prm = c->ani_params();
     c->d_info.reserve((size_t)n_pairs, 0, c->st);
@@ -523,7 +529,7 @@ void run_ani(skb_ctx *c, const unsigned long long *d_pairs, int64_t n_pairs, Pai
     b_big_list.reserve((size_t)cap_pairs, 0, c->st);
     b_big_nc.reserve((size_t)cap_pairs, 0, c->st);
     PoolRef<uint8_t> e_acc(c->pool["est.acc"]);
-    if (est) e_acc.reserve((size_t)cap * SLOTS, 0, c->st);
+    if (acc) e_acc.reserve((size_t)cap * SLOTS, 0, c->st);
     // When no padded position of the database comes near 2^30, anchor_kernel matches and decodes seed records by their
     // 32-bit halves and chain_kernel compares diagonals (reference position -/+ query position, sign by strand) in 32
     // bits; SKB_WIDE_DIAG=1 forces the general variants (tests run both)
@@ -602,7 +608,7 @@ void run_ani(skb_ctx *c, const unsigned long long *d_pairs, int64_t n_pairs, Pai
             CK(cudaGetLastError());
             c->launches += 1;
         }
-        (est ? finalize_warp_kernel<true> : finalize_warp_kernel<false>)<<<nblk((uint64_t)np, FW_WARPS), FW_WARPS * 32, fw_smem,
+        (acc ? finalize_warp_kernel<true> : finalize_warp_kernel<false>)<<<nblk((uint64_t)np, FW_WARPS), FW_WARPS * 32, fw_smem,
                                                                           c->st>>>(
             view, prm, d_info_s.p + bt.p0, c->d_task_off.p + bt.p0, base, np, b_pcands.p, b_cand_off.p, d_perm.p + bt.p0, d_out,
             fw_cap, b_fctl.p, b_mid_list.p, b_big_list.p, b_big_nc.p, e_acc.p);
@@ -616,7 +622,7 @@ void run_ani(skb_ctx *c, const unsigned long long *d_pairs, int64_t n_pairs, Pai
         if (fctl[2]) {  // more than fw_cap candidates or more than FW_EDGES blocking relations: shared memory, one CTA per pair
             uint32_t fcap = 32;
             while (fcap < fctl[0]) fcap <<= 1;
-            (est ? finalize_kernel<false, true> : finalize_kernel<false, false>)<<<fctl[2], FIN_THREADS,
+            (acc ? finalize_kernel<false, true> : finalize_kernel<false, false>)<<<fctl[2], FIN_THREADS,
                                                                                   FIN_BYTES_PER_CAND * (size_t)fcap, c->st>>>(
                 view, prm, d_info_s.p + bt.p0, c->d_task_off.p + bt.p0, base, np, b_pcands.p, b_cand_off.p,
                 d_perm.p + bt.p0, d_out, fcap, b_mid_list.p, nullptr, nullptr, nullptr, e_acc.p);
@@ -645,7 +651,7 @@ void run_ani(skb_ctx *c, const unsigned long long *d_pairs, int64_t n_pairs, Pai
             d_big.reserve((size_t)off + 256, 0, c->st);
             d_big_off.upload(h_off, c->st);
             d_big_cap.upload(h_cap, c->st);
-            (est ? finalize_kernel<true, true> : finalize_kernel<true, false>)<<<nbig, FIN_THREADS, 0, c->st>>>(
+            (acc ? finalize_kernel<true, true> : finalize_kernel<true, false>)<<<nbig, FIN_THREADS, 0, c->st>>>(
                 view, prm, d_info_s.p + bt.p0, c->d_task_off.p + bt.p0, base, np, b_pcands.p, b_cand_off.p, d_perm.p + bt.p0,
                 d_out, 0, b_big_list.p, d_big_off.p, d_big_cap.p, d_big.p, e_acc.p);
             CK(cudaGetLastError());
@@ -653,6 +659,17 @@ void run_ani(skb_ctx *c, const unsigned long long *d_pairs, int64_t n_pairs, Pai
             CK(cudaStreamSynchronize(c->st));  // h_off / h_cap leave scope
         }
         if (trace) spans.push_back({"finalize", bi, tf, mark()});
+        if (d_ci) {
+            cudaEvent_t tc = mark();
+            PoolRef<uint32_t> ci_chains(c->pool["ci.chains"]);
+            ci_chains.reserve((size_t)cap * SLOTS, 0, c->st);
+            ci_kernel<<<nblk((uint64_t)np, FW_WARPS), FW_WARPS * 32, 0, c->st>>>(
+                prm, d_info_s.p + bt.p0, c->d_task_off.p + bt.p0, base, np, b_pcands.p, b_cand_off.p, e_acc.p, ci_chains.p,
+                d_perm.p + bt.p0, d_out, d_ci);
+            CK(cudaGetLastError());
+            c->launches += 1;
+            if (trace) spans.push_back({"ci", bi, tc, mark()});
+        }
         if (est && n_cand) {
             cudaEvent_t te = mark();
             PoolRef<unsigned long long> e_key(c->pool["est.key"]), e_key_s(c->pool["est.key_sorted"]);
@@ -711,10 +728,18 @@ void pairs_to_edges(skb_ctx *c, unsigned long long *d_pairs, int64_t n_pairs, do
     CK(cudaMemsetAsync(d_n.p, 0, 32, c->st));
     CK(cudaEventRecord(ev_mid, c->st));
     unsigned long long ne = 0;
+    c->last_ci = c->ci;
+    c->last_dev_ci = nullptr;
     if (n_pairs > 0) {
         d_out.reserve((size_t)n_pairs, 0, c->st);
         d_edges.reserve((size_t)n_pairs, 0, c->st);
-        run_ani(c, d_pairs, n_pairs, d_out.p);
+        double2 *d_ci = nullptr;
+        if (c->ci) {
+            PoolRef<double2> ci_pairs(c->pool["ci.pairs"]);
+            ci_pairs.reserve((size_t)n_pairs, 0, c->st);
+            d_ci = ci_pairs.p;
+        }
+        run_ani(c, d_pairs, n_pairs, d_out.p, d_ci);
         PoolRef<uint32_t> d_ef(c->pool["pairs_to_edges.flag"]), d_ep(c->pool["pairs_to_edges.pos"]);
         d_ef.reserve((size_t)n_pairs, 0, c->st);
         d_ep.reserve((size_t)n_pairs, 0, c->st);
@@ -725,6 +750,14 @@ void pairs_to_edges(skb_ctx *c, unsigned long long *d_pairs, int64_t n_pairs, do
                                                                             d_edges.p, d_n.p);
         CK(cudaGetLastError());
         c->launches += 2;
+        if (d_ci) {
+            PoolRef<double2> ci_edges(c->pool["ci.edges"]);
+            ci_edges.reserve((size_t)n_pairs, 0, c->st);
+            edge_ci_scatter_kernel<<<nblk((uint64_t)n_pairs, 256), 256, 0, c->st>>>(d_ci, n_pairs, d_ef.p, d_ep.p, ci_edges.p);
+            CK(cudaGetLastError());
+            c->launches += 1;
+            c->last_dev_ci = ci_edges.p;
+        }
     }
     CK(cudaEventRecord(ev_end, c->st));
     if (n_pairs > 0) {
@@ -764,6 +797,10 @@ void pairs_to_edges(skb_ctx *c, unsigned long long *d_pairs, int64_t n_pairs, do
     }
     // rect lists are sorted by (ref, query) on the device already; nothing to do on the host
 }
+
+// --ci is defined for the mean estimator only (DESIGN.md section 3)
+bool ci_conflict(skb_ctx *c) { return c->ci && c->estimator != SKB_ANI_MEAN; }
+const char *const CI_CONFLICT = "the --ci interval is defined for the mean ANI estimator only (skb_set_ani_ci, skb_set_ani_estimator)";
 
 int emit_edges(skb_ctx *c, EdgeRun &run, skb_edge **edges, int64_t *n_edges) {
     *n_edges = run.n_edges;
@@ -1440,6 +1477,7 @@ int skb_triangle(skb_ctx *ctx, double screen_pct, double min_af_pct, int32_t par
     return guarded(ctx, [&]() -> int {
         skb_ctx *c = ctx;
         if (!n_edges) return fail(c, SKB_EINVAL, "bad arguments");
+        if (ci_conflict(c)) return fail(c, SKB_EINVAL, CI_CONFLICT);
         const int64_t launches0 = c->launches;
         cudaEvent_t e0, e1, e2;
         CK(cudaEventCreate(&e0));
@@ -1516,6 +1554,7 @@ int skb_pairs_edges(skb_ctx *ctx, const uint64_t *dev_pairs, int64_t n_pairs, in
     return guarded(ctx, [&]() -> int {
         skb_ctx *c = ctx;
         if (!n_edges || n_pairs < 0 || (n_pairs && !dev_pairs)) return fail(c, SKB_EINVAL, "bad arguments");
+        if (ci_conflict(c)) return fail(c, SKB_EINVAL, CI_CONFLICT);
         if (!c->indexed || c->ix.n_indexed != c->n()) return fail(c, SKB_ESTATE, "call skb_index first");
         const int64_t launches0 = c->launches;
         cudaEvent_t e0, e1, e2;
@@ -1568,6 +1607,7 @@ int skb_rect(skb_ctx *ctx, const int32_t *refs, int32_t n_refs, const int32_t *q
         skb_ctx *c = ctx;
         if (!edges || !n_edges || n_refs < 0 || n_queries < 0 || (n_refs && !refs) || (n_queries && !queries))
             return fail(c, SKB_EINVAL, "bad arguments");
+        if (ci_conflict(c)) return fail(c, SKB_EINVAL, CI_CONFLICT);
         if (!c->indexed || c->ix.n_indexed != c->n()) return fail(c, SKB_ESTATE, "call skb_index first");
         if (c->own_count >= 0) return fail(c, SKB_ESTATE, "skb_rect on a context that owns only part of the seed tables (skb_set_owned)");
         const int32_t n = c->ix.n_indexed;
@@ -1664,6 +1704,35 @@ int skb_set_ani_estimator(skb_ctx *ctx, int32_t estimator) {
         if (estimator != SKB_ANI_MEAN && estimator != SKB_ANI_MEDIAN && estimator != SKB_ANI_ROBUST)
             return fail(ctx, SKB_EINVAL, "unknown ANI estimator " + std::to_string(estimator));
         ctx->estimator = estimator;
+        return SKB_OK;
+    });
+}
+
+int skb_set_ani_ci(skb_ctx *ctx, int32_t enabled) {
+    return guarded(ctx, [&]() -> int {
+        ctx->ci = enabled != 0;
+        return SKB_OK;
+    });
+}
+
+int skb_last_edge_ci(skb_ctx *ctx, double **lo_hi, int64_t *n) {
+    return guarded(ctx, [&]() -> int {
+        if (!lo_hi || !n) return fail(ctx, SKB_EINVAL, "bad arguments");
+        if (!ctx->last_ci)
+            return fail(ctx, SKB_ESTATE, "the last skb_triangle / skb_rect / skb_pairs_edges call ran without --ci (skb_set_ani_ci)");
+        const size_t ne = (size_t)ctx->last_n_edges;
+        double *h = (double *)std::malloc(std::max<size_t>(1, ne) * sizeof(double2));
+        if (!h) return fail(ctx, SKB_ENOMEM, "host out of memory for the intervals");
+        if (ne) {
+            cudaError_t e = cudaMemcpyAsync(h, ctx->last_dev_ci, ne * sizeof(double2), cudaMemcpyDeviceToHost, ctx->st);
+            if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->st);
+            if (e != cudaSuccess) {
+                std::free(h);
+                CK(e);
+            }
+        }
+        *lo_hi = h;
+        *n = (int64_t)ne;
         return SKB_OK;
     });
 }

@@ -158,10 +158,13 @@ def serve(db_dir, device):
                         stop = True
                     elif msg.get("op") == "search":
                         eng.set_estimator(msg.get("estimator", "mean"))  # per request: a resident server serves every mode
+                        ci = bool(msg.get("ci", False))
+                        eng.set_ci(ci)
                         packed = engine.pack_fasta(msg["query"], eng.params.min_contig_len)
                         edges, st = eng.search(packed, screen=msg["screen"], min_af=msg["min_af"])
-                        rows = cli.rect_rows(paths + [msg.get("label", msg["query"])], names + [packed.first_name], edges)
-                        cli.write_atomic(msg["out"], cli.HEADER + "".join(rows))
+                        rows = cli.rect_rows(paths + [msg.get("label", msg["query"])], names + [packed.first_name], edges,
+                                             eng.last_edge_ci() if ci else None)
+                        cli.write_atomic(msg["out"], cli.header(ci) + "".join(rows))
                         conn.send_bytes(json.dumps({"ok": True, "rows": len(rows), "ms": st.ms_total}).encode())
                     else:
                         conn.send_bytes(json.dumps({"ok": False, "error": "unknown op"}).encode())

@@ -129,6 +129,21 @@ class Engine:
             raise ValueError("unknown ANI estimator %r (mean, median, robust)" % (name,))
         self._ck(self._L.skb_set_ani_estimator(self._h, self.ESTIMATORS[name]), "skb_set_ani_estimator")
 
+    def set_ci(self, on):
+        """skani's --ci: later triangle / rect / search / pairs_edges calls also compute a bootstrap interval of every
+        edge's ANI (last_edge_ci); DESIGN.md section 3.  Mean estimator only.  Survives clear()."""
+        self._ck(self._L.skb_set_ani_ci(self._h, 1 if on else 0), "skb_set_ani_ci")
+
+    def last_edge_ci(self):
+        """(n, 2) float64 array: the 5th and 95th percentile ANI (percent) of every edge of the last triangle / rect /
+        search / pairs_edges call, in edge order.  That call must have run with set_ci(True)."""
+        ptr, n = C.POINTER(C.c_double)(), C.c_int64()
+        self._ck(self._L.skb_last_edge_ci(self._h, C.byref(ptr), C.byref(n)), "skb_last_edge_ci")
+        try:
+            return np.ctypeslib.as_array(ptr, shape=(max(1, 2 * n.value),))[: 2 * n.value].reshape(n.value, 2).copy()
+        finally:
+            self._L.skb_free(ptr)
+
     # ---- sketching -------------------------------------------------------------------------
     def add(self, packed):
         n = len(packed)
