@@ -110,6 +110,7 @@ struct skb_ctx {
     float last_ms_anchor = 0;
     int last_anchor_launches = 0;
     cudaEvent_t t0 = nullptr, t1 = nullptr;
+    cudaEvent_t call_ev[3] = {};  // start, pairs ready, edges ready of one screen or edge call (call_events)
 
     // ---- sketch DB (host metadata; the seeds and raw marker keys themselves are d_seeds, d_mkeys)
     struct SketchDb {
@@ -262,12 +263,30 @@ int fail(skb_ctx *ctx, int code, const std::string &m) {
     return code;
 }
 
-void exclusive_scan_u32(skb_ctx *c, const uint32_t *in, uint32_t *out, size_t n) {
+// Every kernel launch of the library: enqueued on the context's stream and counted (skb_stats.launches).  `kern` may be
+// a pointer to one of a kernel's instantiations chosen at run time.
+template <typename K, typename... A>
+void launch(skb_ctx *c, K kern, dim3 grid, dim3 block, size_t smem, A... args) {
+    kern<<<grid, block, smem, c->st>>>(args...);
+    CK(cudaGetLastError());
+    c->launches++;
+}
+
+// A CUB device call f(tmp, bytes): once for the temp size, once on the context's d_tmp.  CUB does not report its
+// launches; n_launches is the caller's estimate of them.
+template <typename F>
+void cub_run(skb_ctx *c, int n_launches, F &&f) {
     size_t bytes = 0;
-    CK(cub::DeviceScan::ExclusiveSum(nullptr, bytes, in, out, (int)n, c->st));
+    CK(f(nullptr, bytes));
     c->d_tmp.reserve(bytes + 16, 0, c->st);
-    CK(cub::DeviceScan::ExclusiveSum(c->d_tmp.p, bytes, in, out, (int)n, c->st));
-    c->launches += 2;
+    CK(f(c->d_tmp.p, bytes));
+    c->launches += n_launches;
+}
+
+void exclusive_scan_u32(skb_ctx *c, const uint32_t *in, uint32_t *out, size_t n) {
+    cub_run(c, 2, [&](void *tmp, size_t &bytes) {
+        return cub::DeviceScan::ExclusiveSum(tmp, bytes, in, out, (int)n, c->st);
+    });
 }
 
 __global__ void widen_u8_kernel(const uint8_t *__restrict__ in, uint32_t *__restrict__ out, size_t n) {
@@ -276,19 +295,36 @@ __global__ void widen_u8_kernel(const uint8_t *__restrict__ in, uint32_t *__rest
 }
 // out[i] = sum of in[0..i), in place over the widened copy
 void exclusive_scan_u8(skb_ctx *c, const uint8_t *in, uint32_t *out, size_t n) {
-    widen_u8_kernel<<<(unsigned)((n + 255) / 256), 256, 0, c->st>>>(in, out, n);
-    CK(cudaGetLastError());
-    c->launches++;
+    launch(c, widen_u8_kernel, (unsigned)((n + 255) / 256), 256, 0, in, out, n);
     exclusive_scan_u32(c, out, out, n);
 }
 
 // stable LSD radix sort on key bits [begin_bit, end_bit)
 void sort_keys_u64(skb_ctx *c, const uint64_t *in, uint64_t *out, size_t n, int end_bit = 64, int begin_bit = 0) {
-    size_t bytes = 0;
-    CK(cub::DeviceRadixSort::SortKeys(nullptr, bytes, in, out, (int64_t)n, begin_bit, end_bit, c->st));
-    c->d_tmp.reserve(bytes + 16, 0, c->st);
-    CK(cub::DeviceRadixSort::SortKeys(c->d_tmp.p, bytes, in, out, (int64_t)n, begin_bit, end_bit, c->st));
-    c->launches += (end_bit - begin_bit + 7) / 8 + 1;
+    cub_run(c, (end_bit - begin_bit + 7) / 8 + 1, [&](void *tmp, size_t &bytes) {
+        return cub::DeviceRadixSort::SortKeys(tmp, bytes, in, out, (int64_t)n, begin_bit, end_bit, c->st);
+    });
+}
+
+// radix sort of (key, value) pairs on all 64 key bits, counted as sort_keys_u64 counts a 64-bit sort
+void sort_pairs_u64(skb_ctx *c, unsigned long long *keys_in, unsigned long long *keys_out, uint32_t *vals_in,
+                    uint32_t *vals_out, size_t n) {
+    cub_run(c, 9, [&](void *tmp, size_t &bytes) {
+        return cub::DeviceRadixSort::SortPairs(tmp, bytes, keys_in, keys_out, vals_in, vals_out, (int64_t)n, 0, 64, c->st);
+    });
+}
+
+// kernels cub::DeviceSegmentedSort launches for one call, at most: the partition of the segments by size (two), then the
+// large- and the small/medium-segment sorts (a call with few segments runs one kernel instead)
+constexpr int EST_SORT_LAUNCHES = 4;
+
+// stable sort of (key, value) pairs within each of the segments [off[s], off[s + 1]), s < n_seg
+void segmented_sort_pairs(skb_ctx *c, unsigned long long *keys_in, unsigned long long *keys_out, uint32_t *vals_in,
+                          uint32_t *vals_out, int n, int n_seg, uint32_t *off) {
+    cub_run(c, EST_SORT_LAUNCHES, [&](void *tmp, size_t &bytes) {
+        return cub::DeviceSegmentedSort::StableSortPairs(tmp, bytes, keys_in, keys_out, vals_in, vals_out, n, n_seg, off,
+                                                         off + 1, c->st);
+    });
 }
 
 // ---- sketch a batch of packed genomes [g0, g1) of the caller's list ------------------------------
@@ -360,10 +396,8 @@ void sketch_batch(skb_ctx *c, const skb_packed *const *gen, int32_t g0, int32_t 
     b.first_gid = (uint32_t)c->n();
     PoolRef<ulonglong2> d_masks(c->pool["sketch_batch.d_masks"]);
     d_masks.reserve(n_warps * 32, 0, c->st);
-    sketch_kernel<false><<<n_tiles, SK_THREADS, 0, c->st>>>(b, d_cnt_s.p, d_cnt_m.p, nullptr, nullptr, nullptr, nullptr,
-                                                            d_masks.p);
-    CK(cudaGetLastError());
-    c->launches++;
+    launch(c, sketch_kernel<false>, n_tiles, SK_THREADS, 0, b, d_cnt_s.p, d_cnt_m.p, nullptr, nullptr, nullptr, nullptr,
+           d_masks.p);
     exclusive_scan_u32(c, d_cnt_s.p, d_off_s.p, n_warps + 1);
     exclusive_scan_u32(c, d_cnt_m.p, d_off_m.p, n_warps + 1);
     // per-genome seed offsets = scanned offsets at genome tile boundaries
@@ -371,9 +405,7 @@ void sketch_batch(skb_ctx *c, const skb_packed *const *gen, int32_t g0, int32_t 
     uint32_t tot_m = 0;
     PoolRef<uint32_t> d_goff(c->pool["sketch_batch.d_goff"]);
     d_goff.reserve((size_t)nb + 1, 0, c->st);
-    gather_strided_kernel<<<nblk((uint64_t)nb + 1, 256), 256, 0, c->st>>>(d_off_s.p, b.tile_off, SK_WARPS, nb + 1, d_goff.p);
-    CK(cudaGetLastError());
-    c->launches++;
+    launch(c, gather_strided_kernel, nblk((uint64_t)nb + 1, 256), 256, 0, d_off_s.p, b.tile_off, SK_WARPS, nb + 1, d_goff.p);
     CK(cudaMemcpyAsync(h_off_s.data(), d_goff.p, ((size_t)nb + 1) * 4, cudaMemcpyDeviceToHost, c->st));
     CK(cudaMemcpyAsync(&tot_m, d_off_m.p + n_warps, 4, cudaMemcpyDeviceToHost, c->st));
     CK(cudaStreamSynchronize(c->st));
@@ -381,11 +413,8 @@ void sketch_batch(skb_ctx *c, const skb_packed *const *gen, int32_t g0, int32_t 
     const uint64_t tot_s = h_off_s[nb];
     c->d_seeds.reserve(cur_seeds + tot_s + 1, cur_seeds, c->st);
     c->d_mkeys.reserve(c->db.n_mkeys + tot_m + 1, c->db.n_mkeys, c->st);
-    sketch_kernel<true><<<n_tiles, SK_THREADS, 0, c->st>>>(b, nullptr, nullptr, d_off_s.p, d_off_m.p,
-                                                           c->d_seeds.p + cur_seeds, c->d_mkeys.p + c->db.n_mkeys,
-                                                           d_masks.p);
-    CK(cudaGetLastError());
-    c->launches++;
+    launch(c, sketch_kernel<true>, n_tiles, SK_THREADS, 0, b, nullptr, nullptr, d_off_s.p, d_off_m.p,
+           c->d_seeds.p + cur_seeds, c->d_mkeys.p + c->db.n_mkeys, d_masks.p);
     CK(cudaStreamSynchronize(c->st));  // batch-local buffers die here
     for (int32_t i = 0; i < nb; i++) {
         const skb_packed *p = gen[g0 + i];
@@ -400,9 +429,6 @@ void sketch_batch(skb_ctx *c, const skb_packed *const *gen, int32_t g0, int32_t 
 //   info      : roles and chunk count per pair
 //   task_off  : exclusive prefix of chunk counts -> task id = (pair, chunk)
 //   cands     : SLOTS candidate slots per task;  task_ncand: how many are filled
-// kernels cub::DeviceSegmentedSort launches for one call, at most: the partition of the segments by size (two), then the
-// large- and the small/medium-segment sorts (a call with few segments runs one kernel instead)
-constexpr int EST_SORT_LAUNCHES = 4;
 
 // d_ci: nullptr, or [n_pairs] for every pair's --ci interval (ci_kernel), indexed like d_out
 void run_ani(skb_ctx *c, const unsigned long long *d_pairs, int64_t n_pairs, PairOut *d_out, double2 *d_ci = nullptr) {
@@ -445,21 +471,11 @@ void run_ani(skb_ctx *c, const unsigned long long *d_pairs, int64_t n_pairs, Pai
     d_idx.reserve((size_t)n_pairs, 0, c->st);
     d_perm.reserve((size_t)n_pairs, 0, c->st);
     d_info_s.reserve((size_t)n_pairs, 0, c->st);
-    pair_setup_kernel<<<nblk((uint64_t)n_pairs, 256), 256, 0, c->st>>>(view, d_pairs, n_pairs, c->d_info.p, d_key.p,
-                                                                      d_idx.p);
-    CK(cudaGetLastError());
-    {
-        size_t bytes = 0;
-        CK(cub::DeviceRadixSort::SortPairs(nullptr, bytes, d_key.p, d_key2.p, d_idx.p, d_perm.p, (int64_t)n_pairs, 0, 64,
-                                           c->st));
-        c->d_tmp.reserve(bytes + 16, 0, c->st);
-        CK(cub::DeviceRadixSort::SortPairs(c->d_tmp.p, bytes, d_key.p, d_key2.p, d_idx.p, d_perm.p, (int64_t)n_pairs, 0,
-                                           64, c->st));
-    }
-    pair_gather_kernel<<<nblk((uint64_t)n_pairs, 256), 256, 0, c->st>>>(c->d_info.p, d_perm.p, n_pairs, d_info_s.p,
-                                                                       c->d_nch.p);
-    CK(cudaGetLastError());
-    c->launches += 11;
+    launch(c, pair_setup_kernel, nblk((uint64_t)n_pairs, 256), 256, 0, view, d_pairs, n_pairs, c->d_info.p, d_key.p,
+           d_idx.p);
+    sort_pairs_u64(c, d_key.p, d_key2.p, d_idx.p, d_perm.p, (size_t)n_pairs);
+    launch(c, pair_gather_kernel, nblk((uint64_t)n_pairs, 256), 256, 0, c->d_info.p, d_perm.p, n_pairs, d_info_s.p,
+           c->d_nch.p);
     // global task offsets (exclusive scan of the chunk counts in processing order)
     CK(cudaMemsetAsync(c->d_nch.p + n_pairs, 0, 4, c->st));
     exclusive_scan_u32(c, c->d_nch.p, c->d_task_off.p, (size_t)n_pairs + 1);
@@ -562,9 +578,8 @@ void run_ani(skb_ctx *c, const unsigned long long *d_pairs, int64_t n_pairs, Pai
             CK(cudaMemsetAsync(b_ncand.p, 0, (size_t)tasks + 1, c->st));
             CK(cudaMemsetAsync(b_slow.p, 0, 4, c->st));
             CK(cudaMemsetAsync(b_next.p, 0, 4, c->st));
-            task_setup_kernel<<<nblk(tasks, 256), 256, 0, c->st>>>(view, d_info_s.p + bt.p0, c->d_task_off.p + bt.p0, base, np,
-                                                                   tasks, b_desc.p, b_task_pair.p);
-            CK(cudaGetLastError());
+            launch(c, task_setup_kernel, nblk(tasks, 256), 256, 0, view, d_info_s.p + bt.p0, c->d_task_off.p + bt.p0, base, np,
+                   tasks, b_desc.p, b_task_pair.p);
             // a persistent grid fed by the task counter
             const unsigned g1 = std::min<unsigned>(nblk(tasks, (ANC_THREADS / 32) * ANC_GRAB), (unsigned)c->sm_count * 32u);
             if ((int)c->anchor_ev.size() < c->anchor_ev_used + 2) {
@@ -576,58 +591,40 @@ void run_ani(skb_ctx *c, const unsigned long long *d_pairs, int64_t n_pairs, Pai
             }
             CK(cudaEventRecord(c->anchor_ev[c->anchor_ev_used], c->st));
             cudaEvent_t t0 = mark();
-            if (wide_diag)
-                anchor_kernel<false><<<g1, ANC_THREADS, 0, c->st>>>(view, prm, b_desc.p, tasks, b_anc.p, b_tn.p, b_next.p);
-            else
-                anchor_kernel<true><<<g1, ANC_THREADS, 0, c->st>>>(view, prm, b_desc.p, tasks, b_anc.p, b_tn.p, b_next.p);
-            CK(cudaGetLastError());
+            launch(c, wide_diag ? anchor_kernel<false> : anchor_kernel<true>, g1, ANC_THREADS, 0, view, prm, b_desc.p, tasks,
+                   b_anc.p, b_tn.p, b_next.p);
             if (trace) spans.push_back({"anchor", bi, t0, mark()});
             CK(cudaEventRecord(c->anchor_ev[c->anchor_ev_used + 1], c->st));
             c->anchor_ev_used += 2;
             t0 = mark();
-            if (wide_diag)
-                chain_kernel<true><<<nblk(tasks, DP_THREADS), DP_THREADS, 0, c->st>>>(prm, tasks, b_anc.p, b_tn.p, b_res.p, b_desc.p,
-                                                                                      b_cands.p, b_ncand.p, b_slow.p);
-            else
-                chain_kernel<false><<<nblk(tasks, DP_THREADS), DP_THREADS, 0, c->st>>>(prm, tasks, b_anc.p, b_tn.p, b_res.p, b_desc.p,
-                                                                                       b_cands.p, b_ncand.p, b_slow.p);
-            CK(cudaGetLastError());
+            launch(c, wide_diag ? chain_kernel<true> : chain_kernel<false>, nblk(tasks, DP_THREADS), DP_THREADS, 0, prm, tasks,
+                   b_anc.p, b_tn.p, b_res.p, b_desc.p, b_cands.p, b_ncand.p, b_slow.p);
             if (trace) spans.push_back({"chain", bi, t0, mark()});
             const unsigned g3 = std::min<unsigned>(nblk(tasks, END_THREADS / 32), (unsigned)c->sm_count * 4u);
-            ends_kernel<<<g3, END_THREADS, 0, c->st>>>(prm, tasks, b_anc.p, b_res.p, b_tn.p, b_desc.p, b_slow.p, b_cands.p,
-                                                       b_ncand.p);
-            CK(cudaGetLastError());
-            c->launches += 4;
+            launch(c, ends_kernel, g3, END_THREADS, 0, prm, tasks, b_anc.p, b_res.p, b_tn.p, b_desc.p, b_slow.p, b_cands.p,
+                   b_ncand.p);
         }
         cudaEvent_t tf = mark();
         // selection + ANI/AF: a warp per pair; the kernel lists the pairs it leaves to the CTA-per-pair kernels
         if (tasks) {
             exclusive_scan_u8(c, b_ncand.p, b_cand_off.p, (size_t)tasks + 1);  // b_ncand[tasks] = 0
-            cand_pack_kernel<<<nblk(tasks, 256), 256, 0, c->st>>>(view, prm, d_info_s.p + bt.p0, tasks, b_task_pair.p, b_ncand.p,
-                                                                  b_cand_off.p, b_cands.p, b_pcands.p);
-            CK(cudaGetLastError());
-            c->launches += 1;
+            launch(c, cand_pack_kernel, nblk(tasks, 256), 256, 0, view, prm, d_info_s.p + bt.p0, tasks, b_task_pair.p, b_ncand.p,
+                   b_cand_off.p, b_cands.p, b_pcands.p);
         }
-        (acc ? finalize_warp_kernel<true> : finalize_warp_kernel<false>)<<<nblk((uint64_t)np, FW_WARPS), FW_WARPS * 32, fw_smem,
-                                                                          c->st>>>(
-            view, prm, d_info_s.p + bt.p0, c->d_task_off.p + bt.p0, base, np, b_pcands.p, b_cand_off.p, d_perm.p + bt.p0, d_out,
-            fw_cap, b_fctl.p, b_mid_list.p, b_big_list.p, b_big_nc.p, e_acc.p);
-        CK(cudaGetLastError());
+        launch(c, acc ? finalize_warp_kernel<true> : finalize_warp_kernel<false>, nblk((uint64_t)np, FW_WARPS), FW_WARPS * 32,
+               fw_smem, view, prm, d_info_s.p + bt.p0, c->d_task_off.p + bt.p0, base, np, b_pcands.p, b_cand_off.p,
+               d_perm.p + bt.p0, d_out, fw_cap, b_fctl.p, b_mid_list.p, b_big_list.p, b_big_nc.p, e_acc.p);
         uint32_t fctl[4] = {0, 0, 0, 0};
         uint32_t n_cand = 0;
         CK(cudaMemcpyAsync(fctl, b_fctl.p, 16, cudaMemcpyDeviceToHost, c->st));
         if (est && tasks) CK(cudaMemcpyAsync(&n_cand, b_cand_off.p + tasks, 4, cudaMemcpyDeviceToHost, c->st));
         CK(cudaStreamSynchronize(c->st));
-        c->launches += 1;
         if (fctl[2]) {  // more than fw_cap candidates or more than FW_EDGES blocking relations: shared memory, one CTA per pair
             uint32_t fcap = 32;
             while (fcap < fctl[0]) fcap <<= 1;
-            (acc ? finalize_kernel<false, true> : finalize_kernel<false, false>)<<<fctl[2], FIN_THREADS,
-                                                                                  FIN_BYTES_PER_CAND * (size_t)fcap, c->st>>>(
-                view, prm, d_info_s.p + bt.p0, c->d_task_off.p + bt.p0, base, np, b_pcands.p, b_cand_off.p,
-                d_perm.p + bt.p0, d_out, fcap, b_mid_list.p, nullptr, nullptr, nullptr, e_acc.p);
-            CK(cudaGetLastError());
-            c->launches += 1;
+            launch(c, acc ? finalize_kernel<false, true> : finalize_kernel<false, false>, fctl[2], FIN_THREADS,
+                   FIN_BYTES_PER_CAND * (size_t)fcap, view, prm, d_info_s.p + bt.p0, c->d_task_off.p + bt.p0, base, np,
+                   b_pcands.p, b_cand_off.p, d_perm.p + bt.p0, d_out, fcap, b_mid_list.p, nullptr, nullptr, nullptr, e_acc.p);
         }
         if (fctl[1]) {  // pairs beyond MAXP candidates: same kernel body on global scratch, one CTA per pair
             const uint32_t nbig = fctl[1];
@@ -651,11 +648,9 @@ void run_ani(skb_ctx *c, const unsigned long long *d_pairs, int64_t n_pairs, Pai
             d_big.reserve((size_t)off + 256, 0, c->st);
             d_big_off.upload(h_off, c->st);
             d_big_cap.upload(h_cap, c->st);
-            (acc ? finalize_kernel<true, true> : finalize_kernel<true, false>)<<<nbig, FIN_THREADS, 0, c->st>>>(
-                view, prm, d_info_s.p + bt.p0, c->d_task_off.p + bt.p0, base, np, b_pcands.p, b_cand_off.p, d_perm.p + bt.p0,
-                d_out, 0, b_big_list.p, d_big_off.p, d_big_cap.p, d_big.p, e_acc.p);
-            CK(cudaGetLastError());
-            c->launches++;
+            launch(c, acc ? finalize_kernel<true, true> : finalize_kernel<true, false>, nbig, FIN_THREADS, 0, view, prm,
+                   d_info_s.p + bt.p0, c->d_task_off.p + bt.p0, base, np, b_pcands.p, b_cand_off.p, d_perm.p + bt.p0, d_out, 0,
+                   b_big_list.p, d_big_off.p, d_big_cap.p, d_big.p, e_acc.p);
             CK(cudaStreamSynchronize(c->st));  // h_off / h_cap leave scope
         }
         if (trace) spans.push_back({"finalize", bi, tf, mark()});
@@ -663,11 +658,9 @@ void run_ani(skb_ctx *c, const unsigned long long *d_pairs, int64_t n_pairs, Pai
             cudaEvent_t tc = mark();
             PoolRef<uint32_t> ci_chains(c->pool["ci.chains"]);
             ci_chains.reserve((size_t)cap * SLOTS, 0, c->st);
-            ci_kernel<<<nblk((uint64_t)np, FW_WARPS), FW_WARPS * 32, 0, c->st>>>(
-                prm, d_info_s.p + bt.p0, c->d_task_off.p + bt.p0, base, np, b_pcands.p, b_cand_off.p, e_acc.p, ci_chains.p,
-                d_perm.p + bt.p0, d_out, d_ci);
-            CK(cudaGetLastError());
-            c->launches += 1;
+            launch(c, ci_kernel, nblk((uint64_t)np, FW_WARPS), FW_WARPS * 32, 0, prm, d_info_s.p + bt.p0,
+                   c->d_task_off.p + bt.p0, base, np, b_pcands.p, b_cand_off.p, e_acc.p, ci_chains.p, d_perm.p + bt.p0, d_out,
+                   d_ci);
             if (trace) spans.push_back({"ci", bi, tc, mark()});
         }
         if (est && n_cand) {
@@ -679,19 +672,11 @@ void run_ani(skb_ctx *c, const unsigned long long *d_pairs, int64_t n_pairs, Pai
             e_idx.reserve(n_cand, 0, c->st);
             e_idx_s.reserve(n_cand, 0, c->st);
             e_seg.reserve((size_t)np + 1, 0, c->st);
-            est_key_kernel<<<nblk(std::max<uint64_t>(n_cand, (uint64_t)np + 1), 256), 256, 0, c->st>>>(
-                b_pcands.p, e_acc.p, n_cand, c->d_task_off.p + bt.p0, base, np, b_cand_off.p, e_key.p, e_idx.p, e_seg.p);
-            CK(cudaGetLastError());
-            size_t bytes = 0;
-            CK(cub::DeviceSegmentedSort::StableSortPairs(nullptr, bytes, e_key.p, e_key_s.p, e_idx.p, e_idx_s.p, (int)n_cand,
-                                                         (int)np, e_seg.p, e_seg.p + 1, c->st));
-            c->d_tmp.reserve(bytes + 16, 0, c->st);
-            CK(cub::DeviceSegmentedSort::StableSortPairs(c->d_tmp.p, bytes, e_key.p, e_key_s.p, e_idx.p, e_idx_s.p, (int)n_cand,
-                                                         (int)np, e_seg.p, e_seg.p + 1, c->st));
-            est_pick_kernel<<<nblk((uint64_t)np, FW_WARPS), FW_WARPS * 32, 0, c->st>>>(prm, c->estimator, np, e_seg.p, e_idx_s.p,
-                                                                                     b_pcands.p, d_perm.p + bt.p0, d_out);
-            CK(cudaGetLastError());
-            c->launches += 2 + EST_SORT_LAUNCHES;
+            launch(c, est_key_kernel, nblk(std::max<uint64_t>(n_cand, (uint64_t)np + 1), 256), 256, 0, b_pcands.p, e_acc.p,
+                   n_cand, c->d_task_off.p + bt.p0, base, np, b_cand_off.p, e_key.p, e_idx.p, e_seg.p);
+            segmented_sort_pairs(c, e_key.p, e_key_s.p, e_idx.p, e_idx_s.p, (int)n_cand, (int)np, e_seg.p);
+            launch(c, est_pick_kernel, nblk((uint64_t)np, FW_WARPS), FW_WARPS * 32, 0, prm, c->estimator, np, e_seg.p,
+                   e_idx_s.p, b_pcands.p, d_perm.p + bt.p0, d_out);
             if (trace) spans.push_back({"estimator", bi, te, mark()});
         }
     }
@@ -709,25 +694,16 @@ void run_ani(skb_ctx *c, const unsigned long long *d_pairs, int64_t n_pairs, Pai
     }
 }
 
-struct EdgeRun {
-    bool to_host = true;        // false: the caller only wants the device copy (skb_device_edges)
-    skb_edge *host = nullptr;   // malloc'ed result, handed to the caller by emit_edges
-    int64_t n_edges = 0;
-    int64_t n_screened = 0;
-    float ms_screen = 0, ms_ani = 0;
-    unsigned long long sums[2] = {0, 0};  // sum query seeds, sum anchors
-};
-
-// pairs on device -> ANI -> compacted edges on host
-void pairs_to_edges(skb_ctx *c, unsigned long long *d_pairs, int64_t n_pairs, double min_af_pct, EdgeRun &run,
-                    cudaEvent_t ev_mid, cudaEvent_t ev_end) {
+// pairs on device -> ANI -> compacted edges on device (c->last_dev_edges, c->last_n_edges); sums: sum query seeds, sum
+// anchors
+void pairs_to_edges(skb_ctx *c, unsigned long long *d_pairs, int64_t n_pairs, double min_af_pct,
+                    unsigned long long sums[2], cudaEvent_t ev_mid, cudaEvent_t ev_end) {
     PoolRef<PairOut> d_out(c->pool["pairs_to_edges.d_out"]);
     PoolRef<skb_edge> d_edges(c->pool["pairs_to_edges.d_edges"]);
     PoolRef<unsigned long long> d_n(c->pool["pairs_to_edges.d_n"]);
     d_n.reserve(4, 0, c->st);
     CK(cudaMemsetAsync(d_n.p, 0, 32, c->st));
     CK(cudaEventRecord(ev_mid, c->st));
-    unsigned long long ne = 0;
     c->last_ci = c->ci;
     c->last_dev_ci = nullptr;
     if (n_pairs > 0) {
@@ -743,35 +719,26 @@ void pairs_to_edges(skb_ctx *c, unsigned long long *d_pairs, int64_t n_pairs, do
         PoolRef<uint32_t> d_ef(c->pool["pairs_to_edges.flag"]), d_ep(c->pool["pairs_to_edges.pos"]);
         d_ef.reserve((size_t)n_pairs, 0, c->st);
         d_ep.reserve((size_t)n_pairs, 0, c->st);
-        edge_flag_kernel<<<nblk((uint64_t)n_pairs, 256), 256, 0, c->st>>>(d_out.p, n_pairs, min_af_pct / 100.0, d_ef.p);
-        CK(cudaGetLastError());
+        launch(c, edge_flag_kernel, nblk((uint64_t)n_pairs, 256), 256, 0, d_out.p, n_pairs, min_af_pct / 100.0, d_ef.p);
         exclusive_scan_u32(c, d_ef.p, d_ep.p, (size_t)n_pairs);
-        edge_scatter_kernel<<<nblk((uint64_t)n_pairs, 256), 256, 0, c->st>>>(d_pairs, d_out.p, n_pairs, d_ef.p, d_ep.p,
-                                                                            d_edges.p, d_n.p);
-        CK(cudaGetLastError());
-        c->launches += 2;
+        launch(c, edge_scatter_kernel, nblk((uint64_t)n_pairs, 256), 256, 0, d_pairs, d_out.p, n_pairs, d_ef.p, d_ep.p,
+               d_edges.p, d_n.p);
         if (d_ci) {
             PoolRef<double2> ci_edges(c->pool["ci.edges"]);
             ci_edges.reserve((size_t)n_pairs, 0, c->st);
-            edge_ci_scatter_kernel<<<nblk((uint64_t)n_pairs, 256), 256, 0, c->st>>>(d_ci, n_pairs, d_ef.p, d_ep.p, ci_edges.p);
-            CK(cudaGetLastError());
-            c->launches += 1;
+            launch(c, edge_ci_scatter_kernel, nblk((uint64_t)n_pairs, 256), 256, 0, d_ci, n_pairs, d_ef.p, d_ep.p, ci_edges.p);
             c->last_dev_ci = ci_edges.p;
         }
     }
     CK(cudaEventRecord(ev_end, c->st));
-    if (n_pairs > 0) {
-        pair_sums_kernel<<<nblk((uint64_t)n_pairs, 256), 256, 0, c->st>>>(c->d_info.p, d_out.p, n_pairs,
-                                                                         c->d_seed_off.p, d_n.p + 1);
-        CK(cudaGetLastError());
-        c->launches++;
-    }
+    if (n_pairs > 0)
+        launch(c, pair_sums_kernel, nblk((uint64_t)n_pairs, 256), 256, 0, c->d_info.p, d_out.p, n_pairs, c->d_seed_off.p,
+               d_n.p + 1);
     unsigned long long h3[4] = {0, 0, 0, 0};
     CK(cudaMemcpyAsync(h3, d_n.p, 32, cudaMemcpyDeviceToHost, c->st));
     CK(cudaStreamSynchronize(c->st));
-    ne = h3[0];
-    run.sums[0] = h3[1];
-    run.sums[1] = h3[2];
+    sums[0] = h3[1];
+    sums[1] = h3[2];
     c->last_ms_anchor = 0;
     c->last_anchor_launches = c->anchor_ev_used / 2;
     for (int i = 0; i + 1 < c->anchor_ev_used; i += 2) {
@@ -780,31 +747,71 @@ void pairs_to_edges(skb_ctx *c, unsigned long long *d_pairs, int64_t n_pairs, do
         c->last_ms_anchor += ms;
     }
     c->anchor_ev_used = 0;
-    run.n_edges = (int64_t)ne;
     c->last_dev_edges = d_edges.p;
-    c->last_n_edges = (int64_t)ne;
-    if (run.to_host) {
-        run.host = (skb_edge *)std::malloc(std::max<size_t>(1, (size_t)ne) * sizeof(skb_edge));
-        if (!run.host) throw CudaFail{"host out of memory for edges"};
+    c->last_n_edges = (int64_t)h3[0];
+}
+
+// The context's events around the stages of one screen or edge call: start, pairs ready, edges ready
+cudaEvent_t *call_events(skb_ctx *c) {
+    for (cudaEvent_t &e : c->call_ev)
+        if (!e) CK(cudaEventCreate(&e));
+    return c->call_ev;
+}
+
+// The pairs an edge call evaluates (sorted, on the device) and the pair count its stats report as n_pairs_total
+struct EdgePairs {
+    unsigned long long *d_pairs = nullptr;
+    int64_t n = 0, total = 0;
+};
+
+// skb_triangle, skb_pairs_edges and skb_rect after their argument checks: `pairs(EdgePairs &)` checks the context's state
+// and leaves the pairs to evaluate (ms_screen), pairs_to_edges evaluates them (ms_ani), and the edges go to the caller --
+// a malloc'ed host copy when `edges` is given, the device copy in any case (skb_device_edges)
+template <typename F>
+int edge_call(skb_ctx *c, double min_af_pct, skb_edge **edges, int64_t *n_edges, skb_stats *stats, F &&pairs) {
+    // --ci is defined for the mean estimator only (DESIGN.md section 3)
+    if (c->ci && c->estimator != SKB_ANI_MEAN)
+        return fail(c, SKB_EINVAL,
+                    "the --ci interval is defined for the mean ANI estimator only (skb_set_ani_ci, skb_set_ani_estimator)");
+    const int64_t launches0 = c->launches;
+    cudaEvent_t *ev = call_events(c);
+    CK(cudaEventRecord(ev[0], c->st));
+    EdgePairs p;
+    const int rc = pairs(p);
+    if (rc != SKB_OK) return rc;
+    unsigned long long sums[2];
+    pairs_to_edges(c, p.d_pairs, p.n, min_af_pct, sums, ev[1], ev[2]);
+    float ms_screen = 0, ms_ani = 0;
+    CK(cudaEventElapsedTime(&ms_screen, ev[0], ev[1]));
+    CK(cudaEventElapsedTime(&ms_ani, ev[1], ev[2]));
+    const int64_t ne = c->last_n_edges;
+    // rect lists are sorted by (ref, query) on the device already; nothing to do on the host
+    if (edges) {
+        skb_edge *h = (skb_edge *)std::malloc(std::max<size_t>(1, (size_t)ne) * sizeof(skb_edge));
+        if (!h) throw CudaFail{"host out of memory for edges"};
         if (ne) {
-            const cudaError_t e = cudaMemcpy(run.host, d_edges.p, (size_t)ne * sizeof(skb_edge), cudaMemcpyDeviceToHost);
+            const cudaError_t e = cudaMemcpy(h, c->last_dev_edges, (size_t)ne * sizeof(skb_edge), cudaMemcpyDeviceToHost);
             if (e != cudaSuccess) {
-                std::free(run.host);
-                run.host = nullptr;
+                std::free(h);
                 CK(e);
             }
         }
+        *edges = h;
     }
-    // rect lists are sorted by (ref, query) on the device already; nothing to do on the host
-}
-
-// --ci is defined for the mean estimator only (DESIGN.md section 3)
-bool ci_conflict(skb_ctx *c) { return c->ci && c->estimator != SKB_ANI_MEAN; }
-const char *const CI_CONFLICT = "the --ci interval is defined for the mean ANI estimator only (skb_set_ani_ci, skb_set_ani_estimator)";
-
-int emit_edges(skb_ctx *c, EdgeRun &run, skb_edge **edges, int64_t *n_edges) {
-    *n_edges = run.n_edges;
-    if (edges) *edges = run.host;
+    if (stats) {
+        stats->n_pairs_total = p.total;
+        stats->n_pairs_screened = p.n;
+        stats->n_edges = ne;
+        stats->ms_screen = ms_screen;
+        stats->ms_ani = ms_ani;
+        stats->ms_total = ms_screen + ms_ani;
+        stats->ms_anchor = c->last_ms_anchor;
+        stats->n_anchor_launches = c->last_anchor_launches;
+        stats->launches = c->launches - launches0;
+        stats->sum_query_seeds = (int64_t)sums[0];
+        stats->sum_anchors = (int64_t)sums[1];
+    }
+    *n_edges = ne;
     return SKB_OK;
 }
 
@@ -892,6 +899,8 @@ void skb_destroy(skb_ctx *ctx) {
     if (ctx->st_copy) cudaStreamDestroy(ctx->st_copy);
     if (ctx->t0) cudaEventDestroy(ctx->t0);
     if (ctx->t1) cudaEventDestroy(ctx->t1);
+    for (cudaEvent_t e : ctx->call_ev)
+        if (e) cudaEventDestroy(e);
     if (ctx->st) {
         cudaStreamSynchronize(ctx->st);
         cudaStreamDestroy(ctx->st);
@@ -1097,13 +1106,10 @@ static int build_seed_tables(skb_ctx *c, int32_t g0, bool reuse) {
     const auto [o0, o1] = c->owned_in(g0, n);
     const uint64_t s0 = c->db.seed_off[o0], s1 = c->db.seed_off[o1];
     if (s1 > s0) {
-        tab_insert_kernel<<<nblk(s1 - s0, 256), 256, 0, c->st>>>(c->d_seeds.p, s1, c->d_seed_off.p, n, c->d_tab.p,
-                                                               c->d_tab_off.p, c->d_tab_buckets.p, s0);
-        CK(cudaGetLastError());
-        rep_flag_kernel<<<nblk(s1 - s0, 256), 256, 0, c->st>>>(c->d_seeds.p, s1, c->d_seed_off.p, n, c->d_tab.p,
-                                                             c->d_tab_off.p, c->d_tab_buckets.p, c->prm.max_mult, s0);
-        CK(cudaGetLastError());
-        c->launches += 2;
+        launch(c, tab_insert_kernel, nblk(s1 - s0, 256), 256, 0, c->d_seeds.p, s1, c->d_seed_off.p, n, c->d_tab.p,
+               c->d_tab_off.p, c->d_tab_buckets.p, s0);
+        launch(c, rep_flag_kernel, nblk(s1 - s0, 256), 256, 0, c->d_seeds.p, s1, c->d_seed_off.p, n, c->d_tab.p,
+               c->d_tab_off.p, c->d_tab_buckets.p, c->prm.max_mult, s0);
     }
     return SKB_OK;
 }
@@ -1161,10 +1167,8 @@ static int build_chunk_tables(skb_ctx *c, int32_t g0) {
     c->d_chunk_len.upload(ix.chunk_len, ch0, c->st);
     const uint32_t e0 = (uint32_t)ch0 + (uint32_t)g0, e1 = ix.chunk_off[n] + (uint32_t)n;
     c->d_chunk_begin.reserve(e1, e0, c->st);
-    chunk_begin_kernel<<<nblk(e1 - e0, 256), 256, 0, c->st>>>(c->d_seeds.p, c->d_seed_off.p, c->d_chunk_off.p, n,
-                                                             c->d_chunk_start.p, c->d_chunk_begin.p, e1, e0);
-    CK(cudaGetLastError());
-    c->launches++;
+    launch(c, chunk_begin_kernel, nblk(e1 - e0, 256), 256, 0, c->d_seeds.p, c->d_seed_off.p, c->d_chunk_off.p, n,
+           c->d_chunk_start.p, c->d_chunk_begin.p, e1, e0);
     return SKB_OK;
 }
 
@@ -1225,8 +1229,7 @@ int skb_index(skb_ctx *ctx) {
             // STABLE sort on the 42 marker bits alone leaves every marker's run ordered by genome id: 6 radix passes
             // instead of 8
             sort_keys_u64(c, c->d_mkeys.p, d_sorted.p, nk, 64, GID_BITS);
-            unique_flag_kernel<<<nblk(nk, 256), 256, 0, c->st>>>(d_sorted.p, nk, d_flag.p);
-            CK(cudaGetLastError());
+            launch(c, unique_flag_kernel, nblk(nk, 256), 256, 0, d_sorted.p, nk, d_flag.p);
             CK(cudaMemsetAsync(d_flag.p + nk, 0, 4, c->st));
             exclusive_scan_u32(c, d_flag.p, d_pos.p, nk + 1);
             uint32_t nu = 0;
@@ -1234,21 +1237,16 @@ int skb_index(skb_ctx *ctx) {
             CK(cudaStreamSynchronize(c->st));
             c->ix.n_inv = nu;
             c->d_inv.reserve(nu + 1, 0, c->st);
-            unique_scatter_kernel<<<nblk(nk, 256), 256, 0, c->st>>>(d_sorted.p, nk, d_flag.p, d_pos.p, c->d_inv.p,
-                                                                  c->d_marker_cnt.p);
-            CK(cudaGetLastError());
-            c->launches += 3;
+            launch(c, unique_scatter_kernel, nblk(nk, 256), 256, 0, d_sorted.p, nk, d_flag.p, d_pos.p, c->d_inv.p,
+                   c->d_marker_cnt.p);
             lap("inverted index");
             // per-genome sorted lists: swap key halves, sort again, strip ids
             c->d_markers.reserve(nu + 1, 0, c->st);
-            swap_key_kernel<<<nblk(nu, 256), 256, 0, c->st>>>(c->d_inv.p, nu, d_sorted.p);
-            CK(cudaGetLastError());
+            launch(c, swap_key_kernel, nblk(nu, 256), 256, 0, c->d_inv.p, nu, d_sorted.p);
             // the input is ordered by marker: a stable sort on the 22 genome bits alone keeps each genome's markers
             // ascending (3 passes instead of 8)
             sort_keys_u64(c, d_sorted.p, c->d_markers.p, nu, 64, 2 * K_MARKER);
-            strip_gid_kernel<<<nblk(nu, 256), 256, 0, c->st>>>(c->d_markers.p, nu);
-            CK(cudaGetLastError());
-            c->launches += 3;
+            launch(c, strip_gid_kernel, nblk(nu, 256), 256, 0, c->d_markers.p, nu);
         }
         marker_offsets(c, 0);
         lap("marker lists");
@@ -1310,11 +1308,9 @@ int skb_index_append(skb_ctx *ctx) {
             d_b.reserve(nk, 0, c->st);
             d_flag.reserve(nk + 1, 0, c->st);
             d_pos.reserve(nk + 1, 0, c->st);
-            swap_key_kernel<<<nblk(nk, 256), 256, 0, c->st>>>(c->d_mkeys.p + c->ix.n_mkeys_indexed, nk, d_a.p);
-            CK(cudaGetLastError());
+            launch(c, swap_key_kernel, nblk(nk, 256), 256, 0, c->d_mkeys.p + c->ix.n_mkeys_indexed, nk, d_a.p);
             sort_keys_u64(c, d_a.p, d_b.p, nk);
-            unique_flag_kernel<<<nblk(nk, 256), 256, 0, c->st>>>(d_b.p, nk, d_flag.p);
-            CK(cudaGetLastError());
+            launch(c, unique_flag_kernel, nblk(nk, 256), 256, 0, d_b.p, nk, d_flag.p);
             CK(cudaMemsetAsync(d_flag.p + nk, 0, 4, c->st));
             exclusive_scan_u32(c, d_flag.p, d_pos.p, nk + 1);
             uint32_t nu = 0;
@@ -1322,10 +1318,8 @@ int skb_index_append(skb_ctx *ctx) {
             CK(cudaStreamSynchronize(c->st));
             const uint64_t m0 = c->ix.marker_off[n0];
             c->d_markers.reserve(m0 + nu + 1, m0, c->st);
-            unique_scatter_swapped_kernel<<<nblk(nk, 256), 256, 0, c->st>>>(d_b.p, nk, d_flag.p, d_pos.p, c->d_markers.p + m0,
-                                                                           c->d_marker_cnt.p);
-            CK(cudaGetLastError());
-            c->launches += 3;
+            launch(c, unique_scatter_swapped_kernel, nblk(nk, 256), 256, 0, d_b.p, nk, d_flag.p, d_pos.p, c->d_markers.p + m0,
+                   c->d_marker_cnt.p);
         }
         marker_offsets(c, n0);
         c->ix.n_mkeys_indexed = c->db.n_mkeys;
@@ -1388,8 +1382,7 @@ int skb_get_markers(skb_ctx *ctx, int32_t g, uint64_t *out) {
 // Marker prescreen of this partition's rows of the triangle; leaves the surviving pairs (a << 32 | b, a < b, sorted)
 // on the device.  Rows of the dense count matrix are processed in tiles that fit a memory budget, so the matrix
 // never has to hold rows x n counters at once (n = 50,000: 10 GB).
-static int screen_triangle_impl(skb_ctx *c, double screen_pct, int32_t part, int32_t n_parts, unsigned long long **d_out,
-                                int64_t *n_out, int64_t *pairs_total_out) {
+static int screen_triangle_impl(skb_ctx *c, double screen_pct, int32_t part, int32_t n_parts, EdgePairs &out) {
     if (n_parts < 1 || part < 0 || part >= n_parts) return fail(c, SKB_EINVAL, "bad arguments");
     if (!c->indexed || c->ix.n_indexed != c->n()) return fail(c, SKB_ESTATE, "call skb_index first");
     if (c->ix.n_inv_genomes != c->n()) return fail(c, SKB_ESTATE, "query-only genomes present: triangle needs skb_index");
@@ -1397,7 +1390,7 @@ static int screen_triangle_impl(skb_ctx *c, double screen_pct, int32_t part, int
     const uint32_t rows_local = rows_owned(n, (uint32_t)part, (uint32_t)n_parts);
     int64_t pairs_total = 0;
     for (uint32_t rl = 0; rl < rows_local; rl++) pairs_total += n - 1 - row_global(rl, (uint32_t)part, (uint32_t)n_parts);
-    if (pairs_total_out) *pairs_total_out = pairs_total;
+    out.total = pairs_total;
     PoolRef<uint32_t> d_cnt(c->pool["skb_triangle.d_cnt"]);
     PoolRef<unsigned long long> d_pairs(c->pool["skb_triangle.d_pairs"]), d_pairs_sorted(c->pool["skb_triangle.d_pairs_sorted"]), d_np(c->pool["skb_triangle.d_np"]);
     d_np.reserve(1, 0, c->st);
@@ -1426,20 +1419,14 @@ static int screen_triangle_impl(skb_ctx *c, double screen_pct, int32_t part, int
                 d_cnt.reserve(cells, 0, c->st);
                 if (scale > 0.0) {
                     CK(cudaMemsetAsync(d_cnt.p, 0, cells * 4, c->st));
-                    if (c->ix.n_inv) {
-                        screen_runs_kernel<<<nblk(c->ix.n_inv, 256), 256, 0, c->st>>>(c->d_inv.p, c->ix.n_inv, d_cnt.p, n, part, n_parts,
-                                                                                  r0, nr);
-                        CK(cudaGetLastError());
-                        c->launches++;
-                    }
+                    if (c->ix.n_inv)
+                        launch(c, screen_runs_kernel, nblk(c->ix.n_inv, 256), 256, 0, c->d_inv.p, c->ix.n_inv, d_cnt.p, n, part,
+                               n_parts, r0, nr);
                 }
             }
             CK(cudaMemsetAsync(d_np.p, 0, 8, c->st));
-            screen_compact_kernel<<<nblk(cells, 256), 256, 0, c->st>>>(d_cnt.p, n, nr, r0, part, n_parts, c->d_marker_cnt.p, scale,
-                                                                      pass ? d_pairs.p + at : nullptr, d_np.p,
-                                                                      pass ? tile_np[ti] : 0ull);
-            CK(cudaGetLastError());
-            c->launches++;
+            launch(c, screen_compact_kernel, nblk(cells, 256), 256, 0, d_cnt.p, n, nr, r0, part, n_parts, c->d_marker_cnt.p,
+                   scale, pass ? d_pairs.p + at : nullptr, d_np.p, pass ? tile_np[ti] : 0ull);
             if (pass == 0) {
                 unsigned long long t = 0;
                 CK(cudaMemcpyAsync(&t, d_np.p, 8, cudaMemcpyDeviceToHost, c->st));
@@ -1451,55 +1438,17 @@ static int screen_triangle_impl(skb_ctx *c, double screen_pct, int32_t part, int
         }
     }
     if (np) sort_keys_u64(c, (const uint64_t *)d_pairs.p, (uint64_t *)d_pairs_sorted.p, np);
-    *d_out = d_pairs_sorted.p;
-    *n_out = (int64_t)np;
+    out.d_pairs = d_pairs_sorted.p;
+    out.n = (int64_t)np;
     return SKB_OK;
-}
-
-static void fill_stats(skb_ctx *c, skb_stats *stats, int64_t pairs_total, const EdgeRun &run, float ms01, float ms12,
-                       int64_t launches0) {
-    if (!stats) return;
-    stats->n_pairs_total = pairs_total;
-    stats->n_pairs_screened = run.n_screened;
-    stats->n_edges = run.n_edges;
-    stats->ms_screen = ms01;
-    stats->ms_ani = ms12;
-    stats->ms_total = ms01 + ms12;
-    stats->ms_anchor = c->last_ms_anchor;
-    stats->n_anchor_launches = c->last_anchor_launches;
-    stats->launches = c->launches - launches0;
-    stats->sum_query_seeds = (int64_t)run.sums[0];
-    stats->sum_anchors = (int64_t)run.sums[1];
 }
 
 int skb_triangle(skb_ctx *ctx, double screen_pct, double min_af_pct, int32_t part, int32_t n_parts,
                  skb_edge **edges, int64_t *n_edges, skb_stats *stats) {
     return guarded(ctx, [&]() -> int {
-        skb_ctx *c = ctx;
-        if (!n_edges) return fail(c, SKB_EINVAL, "bad arguments");
-        if (ci_conflict(c)) return fail(c, SKB_EINVAL, CI_CONFLICT);
-        const int64_t launches0 = c->launches;
-        cudaEvent_t e0, e1, e2;
-        CK(cudaEventCreate(&e0));
-        CK(cudaEventCreate(&e1));
-        CK(cudaEventCreate(&e2));
-        CK(cudaEventRecord(e0, c->st));
-        unsigned long long *d_pairs = nullptr;
-        int64_t np = 0, pairs_total = 0;
-        const int rc = screen_triangle_impl(c, screen_pct, part, n_parts, &d_pairs, &np, &pairs_total);
-        if (rc != SKB_OK) return rc;
-        EdgeRun run;
-        run.to_host = edges != nullptr;
-        run.n_screened = np;
-        pairs_to_edges(c, d_pairs, np, min_af_pct, run, e1, e2);
-        float ms01 = 0, ms12 = 0;
-        CK(cudaEventElapsedTime(&ms01, e0, e1));
-        CK(cudaEventElapsedTime(&ms12, e1, e2));
-        cudaEventDestroy(e0);
-        cudaEventDestroy(e1);
-        cudaEventDestroy(e2);
-        fill_stats(c, stats, pairs_total, run, ms01, ms12, launches0);
-        return emit_edges(c, run, edges, n_edges);
+        if (!n_edges) return fail(ctx, SKB_EINVAL, "bad arguments");
+        return edge_call(ctx, min_af_pct, edges, n_edges, stats,
+                         [&](EdgePairs &p) { return screen_triangle_impl(ctx, screen_pct, part, n_parts, p); });
     });
 }
 
@@ -1522,26 +1471,21 @@ int skb_screen_triangle(skb_ctx *ctx, double screen_pct, int32_t part, int32_t n
         skb_ctx *c = ctx;
         if (!dev_pairs || !n_pairs) return fail(c, SKB_EINVAL, "bad arguments");
         const int64_t launches0 = c->launches;
-        cudaEvent_t e0, e1;
-        CK(cudaEventCreate(&e0));
-        CK(cudaEventCreate(&e1));
-        CK(cudaEventRecord(e0, c->st));
-        unsigned long long *d_pairs = nullptr;
-        int64_t np = 0, pairs_total = 0;
-        const int rc = screen_triangle_impl(c, screen_pct, part, n_parts, &d_pairs, &np, &pairs_total);
+        cudaEvent_t *ev = call_events(c);
+        CK(cudaEventRecord(ev[0], c->st));
+        EdgePairs p;
+        const int rc = screen_triangle_impl(c, screen_pct, part, n_parts, p);
         if (rc != SKB_OK) return rc;
-        CK(cudaEventRecord(e1, c->st));
-        CK(cudaEventSynchronize(e1));
+        CK(cudaEventRecord(ev[1], c->st));
+        CK(cudaEventSynchronize(ev[1]));
         float ms = 0;
-        CK(cudaEventElapsedTime(&ms, e0, e1));
-        cudaEventDestroy(e0);
-        cudaEventDestroy(e1);
-        *dev_pairs = (const uint64_t *)d_pairs;
-        *n_pairs = np;
+        CK(cudaEventElapsedTime(&ms, ev[0], ev[1]));
+        *dev_pairs = (const uint64_t *)p.d_pairs;
+        *n_pairs = p.n;
         if (stats) {
             std::memset(stats, 0, sizeof(*stats));
-            stats->n_pairs_total = pairs_total;
-            stats->n_pairs_screened = np;
+            stats->n_pairs_total = p.total;
+            stats->n_pairs_screened = p.n;
             stats->ms_screen = stats->ms_total = ms;
             stats->launches = c->launches - launches0;
         }
@@ -1554,148 +1498,101 @@ int skb_pairs_edges(skb_ctx *ctx, const uint64_t *dev_pairs, int64_t n_pairs, in
     return guarded(ctx, [&]() -> int {
         skb_ctx *c = ctx;
         if (!n_edges || n_pairs < 0 || (n_pairs && !dev_pairs)) return fail(c, SKB_EINVAL, "bad arguments");
-        if (ci_conflict(c)) return fail(c, SKB_EINVAL, CI_CONFLICT);
-        if (!c->indexed || c->ix.n_indexed != c->n()) return fail(c, SKB_ESTATE, "call skb_index first");
-        const int64_t launches0 = c->launches;
-        cudaEvent_t e0, e1, e2;
-        CK(cudaEventCreate(&e0));
-        CK(cudaEventCreate(&e1));
-        CK(cudaEventCreate(&e2));
-        CK(cudaEventRecord(e0, c->st));
-        unsigned long long *d_pairs = (unsigned long long *)dev_pairs;
-        int64_t np = n_pairs;
-        if (n_pairs && (owned_only || c->own_count >= 0)) {
-            // keep the pairs whose reference genome (more seeds; ties: b) this context owns, order preserved
-            PoolRef<uint32_t> d_f(c->pool["pairs_edges.flag"]), d_p(c->pool["pairs_edges.pos"]);
-            PoolRef<unsigned long long> d_keep(c->pool["pairs_edges.keep"]);
-            d_f.reserve((size_t)n_pairs + 1, 0, c->st);
-            d_p.reserve((size_t)n_pairs + 1, 0, c->st);
-            d_keep.reserve((size_t)n_pairs, 0, c->st);
-            const int32_t o0 = c->own_count < 0 ? 0 : c->own_first, o1 = c->own_count < 0 ? c->n() : c->own_first + c->own_count;
-            pair_owned_flag_kernel<<<nblk((uint64_t)n_pairs, 256), 256, 0, c->st>>>(c->d_seed_off.p, d_pairs, n_pairs, (uint32_t)c->n(),
-                                                                                   (uint32_t)o0, (uint32_t)o1, d_f.p);
-            CK(cudaGetLastError());
-            CK(cudaMemsetAsync(d_f.p + n_pairs, 0, 4, c->st));
-            exclusive_scan_u32(c, d_f.p, d_p.p, (size_t)n_pairs + 1);
-            pair_keep_kernel<<<nblk((uint64_t)n_pairs, 256), 256, 0, c->st>>>(d_pairs, n_pairs, d_f.p, d_p.p, d_keep.p);
-            CK(cudaGetLastError());
-            uint32_t kept = 0;
-            CK(cudaMemcpyAsync(&kept, d_p.p + n_pairs, 4, cudaMemcpyDeviceToHost, c->st));
-            CK(cudaStreamSynchronize(c->st));
-            c->launches += 2;
-            d_pairs = d_keep.p;
-            np = kept;
-        }
-        EdgeRun run;
-        run.to_host = edges != nullptr;
-        run.n_screened = np;
-        pairs_to_edges(c, d_pairs, np, min_af_pct, run, e1, e2);
-        float ms01 = 0, ms12 = 0;
-        CK(cudaEventElapsedTime(&ms01, e0, e1));
-        CK(cudaEventElapsedTime(&ms12, e1, e2));
-        cudaEventDestroy(e0);
-        cudaEventDestroy(e1);
-        cudaEventDestroy(e2);
-        fill_stats(c, stats, n_pairs, run, ms01, ms12, launches0);
-        return emit_edges(c, run, edges, n_edges);
+        return edge_call(c, min_af_pct, edges, n_edges, stats, [&](EdgePairs &p) -> int {
+            if (!c->indexed || c->ix.n_indexed != c->n()) return fail(c, SKB_ESTATE, "call skb_index first");
+            p.d_pairs = (unsigned long long *)dev_pairs;
+            p.n = p.total = n_pairs;
+            if (n_pairs && (owned_only || c->own_count >= 0)) {
+                // keep the pairs whose reference genome (more seeds; ties: b) this context owns, order preserved
+                PoolRef<uint32_t> d_f(c->pool["pairs_edges.flag"]), d_p(c->pool["pairs_edges.pos"]);
+                PoolRef<unsigned long long> d_keep(c->pool["pairs_edges.keep"]);
+                d_f.reserve((size_t)n_pairs + 1, 0, c->st);
+                d_p.reserve((size_t)n_pairs + 1, 0, c->st);
+                d_keep.reserve((size_t)n_pairs, 0, c->st);
+                const int32_t o0 = c->own_count < 0 ? 0 : c->own_first, o1 = c->own_count < 0 ? c->n() : c->own_first + c->own_count;
+                launch(c, pair_owned_flag_kernel, nblk((uint64_t)n_pairs, 256), 256, 0, c->d_seed_off.p, p.d_pairs, n_pairs,
+                       (uint32_t)c->n(), (uint32_t)o0, (uint32_t)o1, d_f.p);
+                CK(cudaMemsetAsync(d_f.p + n_pairs, 0, 4, c->st));
+                exclusive_scan_u32(c, d_f.p, d_p.p, (size_t)n_pairs + 1);
+                launch(c, pair_keep_kernel, nblk((uint64_t)n_pairs, 256), 256, 0, p.d_pairs, n_pairs, d_f.p, d_p.p, d_keep.p);
+                uint32_t kept = 0;
+                CK(cudaMemcpyAsync(&kept, d_p.p + n_pairs, 4, cudaMemcpyDeviceToHost, c->st));
+                CK(cudaStreamSynchronize(c->st));
+                p.d_pairs = d_keep.p;
+                p.n = kept;
+            }
+            return SKB_OK;
+        });
     });
+}
+
+// Marker prescreen of the rectangle refs x queries; leaves the surviving pairs (ref << 32 | query, sorted) on the device
+static int screen_rect_impl(skb_ctx *c, const int32_t *refs, int32_t n_refs, const int32_t *queries, int32_t n_queries,
+                            double screen_pct, EdgePairs &out) {
+    if (!c->indexed || c->ix.n_indexed != c->n()) return fail(c, SKB_ESTATE, "call skb_index first");
+    if (c->own_count >= 0) return fail(c, SKB_ESTATE, "skb_rect on a context that owns only part of the seed tables (skb_set_owned)");
+    const int32_t n = c->ix.n_indexed;
+    std::vector<int32_t> ref_slot(n, -1);
+    for (int32_t i = 0; i < n_refs; i++) {
+        if (refs[i] < 0 || refs[i] >= n) return fail(c, SKB_EINVAL, "reference id out of range");
+        if (refs[i] >= c->ix.n_inv_genomes && screen_pct > 0.0)
+            return fail(c, SKB_ESTATE, "a query-only genome (skb_index_append) cannot be a screened reference");
+        if (ref_slot[refs[i]] >= 0) return fail(c, SKB_EINVAL, "duplicate reference id");
+        ref_slot[refs[i]] = i;
+    }
+    std::vector<uint64_t> qpref(n_queries + 1, 0);
+    for (int32_t i = 0; i < n_queries; i++) {
+        if (queries[i] < 0 || queries[i] >= n) return fail(c, SKB_EINVAL, "query id out of range");
+        qpref[i + 1] = qpref[i] + (c->ix.marker_off[queries[i] + 1] - c->ix.marker_off[queries[i]]);
+    }
+    PoolRef<int32_t> d_refs(c->pool["skb_rect.d_refs"]), d_queries(c->pool["skb_rect.d_queries"]), d_slot(c->pool["skb_rect.d_slot"]);
+    PoolRef<uint64_t> d_qpref(c->pool["skb_rect.d_qpref"]);
+    PoolRef<uint32_t> d_cnt(c->pool["skb_rect.d_cnt"]);
+    PoolRef<unsigned long long> d_pairs(c->pool["skb_rect.d_pairs"]), d_pairs_sorted(c->pool["skb_rect.d_pairs_sorted"]), d_np(c->pool["skb_rect.d_np"]);
+    const uint64_t cells = (uint64_t)n_refs * (uint64_t)n_queries;
+    unsigned long long np = 0;
+    d_np.reserve(1, 0, c->st);
+    CK(cudaMemsetAsync(d_np.p, 0, 8, c->st));
+    const double scale = screen_pct > 0.0 ? std::pow(screen_pct / 100.0, (double)K_MARKER) : 0.0;
+    if (cells) {
+        d_refs.upload(std::vector<int32_t>(refs, refs + n_refs), c->st);
+        d_queries.upload(std::vector<int32_t>(queries, queries + n_queries), c->st);
+        d_slot.upload(ref_slot, c->st);
+        d_qpref.upload(qpref, c->st);
+        d_cnt.reserve(cells, 0, c->st);
+        if (scale > 0.0) {
+            CK(cudaMemsetAsync(d_cnt.p, 0, cells * 4, c->st));
+            if (qpref[n_queries] && c->ix.n_inv)
+                launch(c, screen_rect_kernel, nblk(qpref[n_queries], 256), 256, 0, c->d_inv.p, c->ix.n_inv, c->d_markers.p,
+                       c->d_marker_off.p, d_queries.p, n_queries, d_qpref.p, d_slot.p, d_cnt.p, (uint32_t)n_refs);
+        }
+        launch(c, screen_rect_compact_kernel, nblk(cells, 256), 256, 0, d_cnt.p, d_refs.p, (uint32_t)n_refs, d_queries.p,
+               (uint32_t)n_queries, c->d_marker_cnt.p, scale, nullptr, d_np.p, 0ull);
+        CK(cudaMemcpyAsync(&np, d_np.p, 8, cudaMemcpyDeviceToHost, c->st));
+        CK(cudaStreamSynchronize(c->st));
+        if (np) {
+            d_pairs.reserve(np, 0, c->st);
+            d_pairs_sorted.reserve(np, 0, c->st);
+            CK(cudaMemsetAsync(d_np.p, 0, 8, c->st));
+            launch(c, screen_rect_compact_kernel, nblk(cells, 256), 256, 0, d_cnt.p, d_refs.p, (uint32_t)n_refs, d_queries.p,
+                   (uint32_t)n_queries, c->d_marker_cnt.p, scale, d_pairs.p, d_np.p, np);
+            sort_keys_u64(c, (const uint64_t *)d_pairs.p, (uint64_t *)d_pairs_sorted.p, np);
+        }
+    }
+    out.d_pairs = d_pairs_sorted.p;
+    out.n = (int64_t)np;
+    out.total = (int64_t)cells;
+    return SKB_OK;
 }
 
 int skb_rect(skb_ctx *ctx, const int32_t *refs, int32_t n_refs, const int32_t *queries, int32_t n_queries,
              double screen_pct, double min_af_pct, skb_edge **edges, int64_t *n_edges, skb_stats *stats) {
     return guarded(ctx, [&]() -> int {
-        skb_ctx *c = ctx;
         if (!edges || !n_edges || n_refs < 0 || n_queries < 0 || (n_refs && !refs) || (n_queries && !queries))
-            return fail(c, SKB_EINVAL, "bad arguments");
-        if (ci_conflict(c)) return fail(c, SKB_EINVAL, CI_CONFLICT);
-        if (!c->indexed || c->ix.n_indexed != c->n()) return fail(c, SKB_ESTATE, "call skb_index first");
-        if (c->own_count >= 0) return fail(c, SKB_ESTATE, "skb_rect on a context that owns only part of the seed tables (skb_set_owned)");
-        const int32_t n = c->ix.n_indexed;
-        const int64_t launches0 = c->launches;
-        std::vector<int32_t> ref_slot(n, -1);
-        for (int32_t i = 0; i < n_refs; i++) {
-            if (refs[i] < 0 || refs[i] >= n) return fail(c, SKB_EINVAL, "reference id out of range");
-            if (refs[i] >= c->ix.n_inv_genomes && screen_pct > 0.0)
-                return fail(c, SKB_ESTATE, "a query-only genome (skb_index_append) cannot be a screened reference");
-            if (ref_slot[refs[i]] >= 0) return fail(c, SKB_EINVAL, "duplicate reference id");
-            ref_slot[refs[i]] = i;
-        }
-        std::vector<uint64_t> qpref(n_queries + 1, 0);
-        for (int32_t i = 0; i < n_queries; i++) {
-            if (queries[i] < 0 || queries[i] >= n) return fail(c, SKB_EINVAL, "query id out of range");
-            qpref[i + 1] = qpref[i] + (c->ix.marker_off[queries[i] + 1] - c->ix.marker_off[queries[i]]);
-        }
-        cudaEvent_t e0, e1, e2;
-        CK(cudaEventCreate(&e0));
-        CK(cudaEventCreate(&e1));
-        CK(cudaEventCreate(&e2));
-        CK(cudaEventRecord(e0, c->st));
-        PoolRef<int32_t> d_refs(c->pool["skb_rect.d_refs"]), d_queries(c->pool["skb_rect.d_queries"]), d_slot(c->pool["skb_rect.d_slot"]);
-        PoolRef<uint64_t> d_qpref(c->pool["skb_rect.d_qpref"]);
-        PoolRef<uint32_t> d_cnt(c->pool["skb_rect.d_cnt"]);
-        PoolRef<unsigned long long> d_pairs(c->pool["skb_rect.d_pairs"]), d_pairs_sorted(c->pool["skb_rect.d_pairs_sorted"]), d_np(c->pool["skb_rect.d_np"]);
-        const uint64_t cells = (uint64_t)n_refs * (uint64_t)n_queries;
-        unsigned long long np = 0;
-        d_np.reserve(1, 0, c->st);
-        CK(cudaMemsetAsync(d_np.p, 0, 8, c->st));
-        const double scale = screen_pct > 0.0 ? std::pow(screen_pct / 100.0, (double)K_MARKER) : 0.0;
-        if (cells) {
-            d_refs.upload(std::vector<int32_t>(refs, refs + n_refs), c->st);
-            d_queries.upload(std::vector<int32_t>(queries, queries + n_queries), c->st);
-            d_slot.upload(ref_slot, c->st);
-            d_qpref.upload(qpref, c->st);
-            d_cnt.reserve(cells, 0, c->st);
-            if (scale > 0.0) {
-                CK(cudaMemsetAsync(d_cnt.p, 0, cells * 4, c->st));
-                if (qpref[n_queries] && c->ix.n_inv) {
-                    screen_rect_kernel<<<nblk(qpref[n_queries], 256), 256, 0, c->st>>>(
-                        c->d_inv.p, c->ix.n_inv, c->d_markers.p, c->d_marker_off.p, d_queries.p, n_queries, d_qpref.p,
-                        d_slot.p, d_cnt.p, (uint32_t)n_refs);
-                    CK(cudaGetLastError());
-                    c->launches++;
-                }
-            }
-            screen_rect_compact_kernel<<<nblk(cells, 256), 256, 0, c->st>>>(d_cnt.p, d_refs.p, (uint32_t)n_refs,
-                                                                           d_queries.p, (uint32_t)n_queries,
-                                                                           c->d_marker_cnt.p, scale, nullptr, d_np.p, 0ull);
-            CK(cudaGetLastError());
-            c->launches++;
-            CK(cudaMemcpyAsync(&np, d_np.p, 8, cudaMemcpyDeviceToHost, c->st));
-            CK(cudaStreamSynchronize(c->st));
-            if (np) {
-                d_pairs.reserve(np, 0, c->st);
-                d_pairs_sorted.reserve(np, 0, c->st);
-                CK(cudaMemsetAsync(d_np.p, 0, 8, c->st));
-                screen_rect_compact_kernel<<<nblk(cells, 256), 256, 0, c->st>>>(
-                    d_cnt.p, d_refs.p, (uint32_t)n_refs, d_queries.p, (uint32_t)n_queries, c->d_marker_cnt.p, scale,
-                    d_pairs.p, d_np.p, np);
-                CK(cudaGetLastError());
-                c->launches++;
-                sort_keys_u64(c, (const uint64_t *)d_pairs.p, (uint64_t *)d_pairs_sorted.p, np);
-            }
-        }
-        EdgeRun run;
-        pairs_to_edges(c, d_pairs_sorted.p, (int64_t)np, min_af_pct, run, e1, e2);
-        float ms01 = 0, ms12 = 0;
-        CK(cudaEventElapsedTime(&ms01, e0, e1));
-        CK(cudaEventElapsedTime(&ms12, e1, e2));
-        cudaEventDestroy(e0);
-        cudaEventDestroy(e1);
-        cudaEventDestroy(e2);
-        if (stats) {
-            stats->n_pairs_total = (int64_t)cells;
-            stats->n_pairs_screened = (int64_t)np;
-            stats->n_edges = run.n_edges;
-            stats->ms_screen = ms01;
-            stats->ms_ani = ms12;
-            stats->ms_total = ms01 + ms12;
-            stats->ms_anchor = c->last_ms_anchor;
-            stats->n_anchor_launches = c->last_anchor_launches;
-            stats->launches = c->launches - launches0;
-            stats->sum_query_seeds = (int64_t)run.sums[0];
-            stats->sum_anchors = (int64_t)run.sums[1];
-        }
-        return emit_edges(c, run, edges, n_edges);
+            return fail(ctx, SKB_EINVAL, "bad arguments");
+        return edge_call(ctx, min_af_pct, edges, n_edges, stats, [&](EdgePairs &p) {
+            return screen_rect_impl(ctx, refs, n_refs, queries, n_queries, screen_pct, p);
+        });
     });
 }
 
@@ -1794,10 +1691,8 @@ int skb_shared_markers(skb_ctx *ctx, const uint32_t *a, const uint32_t *b, int64
         da.upload(std::vector<uint32_t>(a, a + n), c->st);
         db.upload(std::vector<uint32_t>(b, b + n), c->st);
         dout.reserve((size_t)n, 0, c->st);
-        shared_markers_kernel<<<nblk((uint64_t)n * 32, 256), 256, 0, c->st>>>(c->d_markers.p, c->d_marker_off.p, da.p,
-                                                                             db.p, n, dout.p);
-        CK(cudaGetLastError());
-        c->launches++;
+        launch(c, shared_markers_kernel, nblk((uint64_t)n * 32, 256), 256, 0, c->d_markers.p, c->d_marker_off.p, da.p, db.p, n,
+               dout.p);
         CK(cudaMemcpyAsync(shared, dout.p, (size_t)n * 8, cudaMemcpyDeviceToHost, c->st));
         CK(cudaStreamSynchronize(c->st));
         return SKB_OK;
@@ -1946,19 +1841,13 @@ int skb_import_sketches(skb_ctx *ctx, int32_t n_genomes, const uint64_t *dev_see
         c->d_mkeys.reserve(c->db.n_mkeys + (uint64_t)n_marker_keys + 1, c->db.n_mkeys, c->st);
         if (n_seeds && keep_repeat_flags)  // the sender indexed its genomes: their repeat flags travel with the seeds
             CK(cudaMemcpyAsync(c->d_seeds.p + cur, dev_seeds, (size_t)n_seeds * 8, cudaMemcpyDeviceToDevice, c->st));
-        else if (n_seeds) {
-            clear_rep_kernel<<<nblk((uint64_t)n_seeds, 256), 256, 0, c->st>>>(dev_seeds, (uint64_t)n_seeds,
-                                                                             c->d_seeds.p + cur);
-            CK(cudaGetLastError());
-            c->launches++;
-        }
+        else if (n_seeds)
+            launch(c, clear_rep_kernel, nblk((uint64_t)n_seeds, 256), 256, 0, dev_seeds, (uint64_t)n_seeds, c->d_seeds.p + cur);
         // the sender tagged its keys with ids first_src .. ; the first imported genome becomes c->n()
         if (n_marker_keys) {
             // senders export a whole context, whose ids start at 0: shift them behind this context's genomes
-            retag_keys_kernel<<<nblk((uint64_t)n_marker_keys, 256), 256, 0, c->st>>>(
-                dev_marker_keys, (uint64_t)n_marker_keys, c->d_mkeys.p + c->db.n_mkeys, (int64_t)c->n());
-            CK(cudaGetLastError());
-            c->launches++;
+            launch(c, retag_keys_kernel, nblk((uint64_t)n_marker_keys, 256), 256, 0, dev_marker_keys, (uint64_t)n_marker_keys,
+                   c->d_mkeys.p + c->db.n_mkeys, (int64_t)c->n());
         }
         CK(cudaStreamSynchronize(c->st));
         for (int32_t g = 0; g < n_genomes; g++)
@@ -2003,10 +1892,8 @@ int skb_greedy_summary(skb_ctx *ctx, const skb_edge *edges, int64_t n_edges, int
         CK(cudaMemsetAsync(d_conn.p, 0, ((size_t)n_genomes + 1) * 4, c->st));
         std::vector<unsigned int> h_conn((size_t)n_genomes);
         if (n_edges) {
-            summary_keys_kernel<<<nblk((uint64_t)n_edges, 256), 256, 0, c->st>>>(d_edges, n_edges, min_ani, min_af, d_k.p, d_conn.p);
-            CK(cudaGetLastError());
+            launch(c, summary_keys_kernel, nblk((uint64_t)n_edges, 256), 256, 0, d_edges, n_edges, min_ani, min_af, d_k.p, d_conn.p);
             sort_keys_u64(c, (const uint64_t *)d_k.p, (uint64_t *)d_ks.p, nk, 56);  // unused keys (all ones) sort last
-            c->launches++;
         }
         if (n_genomes) CK(cudaMemcpyAsync(h_conn.data(), d_conn.p, (size_t)n_genomes * 4, cudaMemcpyDeviceToHost, c->st));
         CK(cudaStreamSynchronize(c->st));
@@ -2030,9 +1917,7 @@ int skb_greedy_summary(skb_ctx *ctx, const skb_edge *edges, int64_t n_edges, int
             return fail(c, SKB_ENOMEM, "host out of memory");
         }
         if (total) {
-            summary_members_kernel<<<nblk((uint64_t)total, 256), 256, 0, c->st>>>(d_edges, d_ks.p, total, d_mem.p);
-            CK(cudaGetLastError());
-            c->launches++;
+            launch(c, summary_members_kernel, nblk((uint64_t)total, 256), 256, 0, d_edges, d_ks.p, total, d_mem.p);
             CK(cudaMemcpyAsync(mem, d_mem.p, (size_t)total * 4, cudaMemcpyDeviceToHost, c->st));
             CK(cudaStreamSynchronize(c->st));
         }
