@@ -161,6 +161,27 @@ int skb_set_ani_ci(skb_ctx *ctx, int32_t enabled);
  * the ANI's scale; *n = that call's edge count.  malloc'ed (skb_free).  SKB_ESTATE if that call ran without --ci. */
 int skb_last_edge_ci(skb_ctx *ctx, double **lo_hi, int64_t *n);
 
+/* skani's --detailed (DESIGN.md section 3): per edge, what the extra columns need beyond the contig statistics below.
+ * "a" / "b" are the edge's genomes (skb_edge.a / .b). */
+typedef struct {
+    double ani_lo, ani_hi;          /* percent: the --ci interval, the same bits skb_last_edge_ci gives */
+    double sd;                      /* percent: seed-weighted standard deviation of the accepted chains' ANI */
+    int64_t covered_a, covered_b;   /* bases of genome a / b in the accepted chains' extended spans (AF numerators) */
+    int32_t n_chains, pad;          /* accepted chains */
+} skb_edge_detail;                  /* 48 bytes */
+/* Context state, kept across skb_clear: enabled != 0 applies to every later skb_triangle, skb_rect and skb_pairs_edges
+ * call, which return SKB_EINVAL while it is on and the estimator is not SKB_ANI_MEAN.  The edges themselves are the same
+ * with and without it. */
+int skb_set_detailed(skb_ctx *ctx, int32_t enabled);
+/* The details of the edge list of the last skb_triangle, skb_rect or skb_pairs_edges call on this context (also one
+ * made with edges == NULL), in edge order; *n = that call's edge count.  malloc'ed (skb_free).  SKB_ESTATE if that call
+ * ran without --detailed. */
+int skb_last_edge_detail(skb_ctx *ctx, skb_edge_detail **out, int64_t *n);
+/* Host-side statistics of the kept contigs (those of at least min_contig_len: what the sketch DB holds) of genomes
+ * first .. first + n - 1: n_contigs[i], and nx[3 i .. 3 i + 2] = N90, N50, N10 (DESIGN.md section 3; 0 for a genome
+ * without kept contigs).  Serves added, loaded and imported genomes alike. */
+int skb_genome_contig_stats(skb_ctx *ctx, int32_t first, int32_t n, int32_t *n_contigs, int64_t *nx);
+
 /* explicit pair list, full detail, no screening / no AF filter (parity tests) */
 int skb_pairs_detail(skb_ctx *ctx, const uint32_t *a, const uint32_t *b, int64_t n, skb_pair_detail *out);
 /* shared-marker counts of an explicit pair list (prescreen parity) */

@@ -64,6 +64,11 @@ class PairDetail(C.Structure):
     ]
 
 
+class EdgeDetail(C.Structure):  # skb_edge_detail
+    _fields_ = [("ani_lo", C.c_double), ("ani_hi", C.c_double), ("sd", C.c_double), ("covered_a", C.c_int64),
+                ("covered_b", C.c_int64), ("n_chains", C.c_int32), ("pad", C.c_int32)]
+
+
 class Stats(C.Structure):
     _fields_ = [
         ("n_pairs_total", C.c_int64),
@@ -103,7 +108,8 @@ SYMBOLS = [
     "skb_rect", "skb_pairs_detail", "skb_shared_markers", "skb_sketch_view_get", "skb_import_sketches",
     "skb_free", "skb_launch_count", "skb_stream", "skb_clear", "skb_timer_start", "skb_timer_stop", "skb_index_append", "skb_pop_last_add",
     "skb_device_edges", "skb_set_owned", "skb_screen_triangle", "skb_pairs_edges", "skb_greedy_summary", "skb_index_seed_tables", "skb_clear_keep_tables",
-    "skb_set_ani_estimator", "skb_set_ani_ci", "skb_last_edge_ci",
+    "skb_set_ani_estimator", "skb_set_ani_ci", "skb_last_edge_ci", "skb_set_detailed", "skb_last_edge_detail",
+    "skb_genome_contig_stats",
 ]
 
 _lib = None
@@ -168,6 +174,9 @@ def lib():
     L.skb_clear.argtypes = [C.c_void_p]
     L.skb_set_ani_estimator.argtypes = [C.c_void_p, C.c_int32]
     L.skb_set_ani_ci.argtypes = [C.c_void_p, C.c_int32]
+    L.skb_set_detailed.argtypes = [C.c_void_p, C.c_int32]
+    L.skb_last_edge_detail.argtypes = [C.c_void_p, C.POINTER(C.POINTER(EdgeDetail)), C.POINTER(C.c_int64)]
+    L.skb_genome_contig_stats.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.POINTER(C.c_int32), C.POINTER(C.c_int64)]
     L.skb_last_edge_ci.argtypes = [C.c_void_p, C.POINTER(C.POINTER(C.c_double)), C.POINTER(C.c_int64)]
     L.skb_index_seed_tables.argtypes = [C.c_void_p]
     L.skb_clear_keep_tables.argtypes = [C.c_void_p]

@@ -9,11 +9,13 @@ without touching skDER.  Sub-commands and flags are exactly the ones skDER spell
   skani search   QUERY.fa -d DBDIR -o OUT -t T                   (skder.py:119)
   skani dist     --rl REFS --ql QUERIES [-s S] [-t T] -o OUT     (skder.py:58-59, cidder.py:362-363)
 
-skDER hands its `-p` string to skani verbatim, so three ANI flags are accepted on triangle, dist and search
+skDER hands its `-p` string to skani verbatim, so four ANI flags are accepted on triangle, dist and search
 (DESIGN.md section 3): the estimators `--median` (median chain identity) and `--robust` (mean after trimming the
-10 % / 90 % tails), and `--ci`, which appends a bootstrap interval of the mean ANI as two columns, ANI_5_percentile and
-ANI_95_percentile (not with --median / --robust).  skDER's `-n` clustering reads exactly seven fields
-(skder.py:190), so a `-p` with --ci breaks it as it would with skani; greedy and dynamic selection are unaffected.
+10 % / 90 % tails); `--ci`, which appends a bootstrap interval of the mean ANI as two columns, ANI_5_percentile and
+ANI_95_percentile; and `--detailed`, which appends 13 columns (contig counts and N90/N50/N10 of both genomes, that
+interval, the spread of the chain identities, the chains' average length and the query bases they cover).  --ci and
+--detailed are not taken with --median / --robust.  skDER's `-n` clustering reads exactly seven fields (skder.py:190),
+so a `-p` with --ci or --detailed breaks it as it would with skani; greedy and dynamic selection are unaffected.
 Any other skani option (-c, -m, --fast, --slow, --medium, --small-genomes, --no-learned-ani, ...) changes skani's
 estimator in ways this engine does not implement: the shim then exits non-zero WITHOUT creating the output, which is
 the one failure signal runCmd checks (util.py:642-645).
@@ -25,6 +27,11 @@ import sys
 import time
 
 HEADER = "Ref_file\tQuery_file\tANI\tAlign_fraction_ref\tAlign_fraction_query\tRef_name\tQuery_name\n"
+# --detailed's columns after the seven above (DESIGN.md section 3); Ref = the edge's genome a, Query = its genome b
+DETAILED_COLUMNS = ("Num_ref_contigs", "Num_query_contigs", "ANI_5_percentile", "ANI_95_percentile", "Standard_deviation",
+                    "Ref_90_ctg_len", "Ref_50_ctg_len", "Ref_10_ctg_len", "Query_90_ctg_len", "Query_50_ctg_len",
+                    "Query_10_ctg_len", "Avg_chain_len", "Total_bases_covered")
+DETAILED_FMT = "\t%d\t%d\t%.2f\t%.2f\t%.2f\t%d\t%d\t%d\t%d\t%d\t%d\t%d\t%d\n"
 DEFAULT_SCREEN = 80.0  # skani -s default
 DEFAULT_MIN_AF = 15.0  # skani --min-af default
 
@@ -45,8 +52,8 @@ def parse_args(argv):
         "-l": "list", "-o": "out", "-t": "threads", "-s": "screen", "--min-af": "min_af", "--rl": "rl", "--ql": "ql",
         "-d": "db",
     }
-    flags = {"-E": "edge_list", "--sparse": "edge_list", "--ci": "ci"}
-    opt["ci"] = False
+    flags = {"-E": "edge_list", "--sparse": "edge_list", "--ci": "ci", "--detailed": "detailed"}
+    opt["ci"] = opt["detailed"] = False
     estimators = {"--median": "median", "--robust": "robust"}
     chosen = []
     i = 1
@@ -86,6 +93,10 @@ def parse_args(argv):
         raise UsageError("skani sketch takes no --ci")
     if opt["ci"] and chosen:
         raise UsageError("--ci is defined for the default (mean) ANI only, not with %s" % chosen[0])
+    if opt["detailed"] and sub == "sketch":
+        raise UsageError("skani sketch takes no --detailed")
+    if opt["detailed"] and chosen:
+        raise UsageError("--detailed is defined for the default (mean) ANI only, not with %s" % chosen[0])
     need = {"triangle": ["list", "out"], "sketch": ["list", "out"], "search": ["db", "out"], "dist": ["rl", "ql", "out"]}[sub]
     for k in need:
         if k not in opt:
@@ -104,13 +115,26 @@ def read_list(path):
         return [ln.strip() for ln in f if ln.strip()]
 
 
-def header(ci):
+def header(ci, detailed=False):
+    if detailed:  # the --ci interval is two of its columns
+        return HEADER[:-1] + "".join("\t" + c for c in DETAILED_COLUMNS) + "\n"
     return HEADER[:-1] + "\tANI_5_percentile\tANI_95_percentile\n" if ci else HEADER
 
 
-def fmt_row(ref, query, ani, af_ref, af_query, ref_name, query_name, ci=None):
+def fmt_row(ref, query, ani, af_ref, af_query, ref_name, query_name, ci=None, detail=None):
     row = "%s\t%s\t%.2f\t%.2f\t%.2f\t%s\t%s" % (ref, query, ani, af_ref, af_query, ref_name, query_name)
+    if detail is not None:
+        return row + DETAILED_FMT % detail
     return row + ("\n" if ci is None else "\t%.2f\t%.2f\n" % ci)
+
+
+def edge_details(edges, det, n_contigs, nx):
+    """--detailed's 13 values per edge, in DETAILED_COLUMNS order.  det: Engine.last_edge_detail() of `edges`;
+    n_contigs, nx: Engine.contig_stats() of every genome id the edges hold."""
+    nc, nx = n_contigs.tolist(), nx.tolist()
+    cols = [edges["a"].tolist(), edges["b"].tolist()]
+    cols += [det[k].tolist() for k in ("ani_lo", "ani_hi", "sd", "covered_b", "n_chains")]
+    return [(nc[a], nc[b], lo, hi, sd, *nx[a], *nx[b], cov // k, cov) for a, b, lo, hi, sd, cov, k in zip(*cols)]
 
 
 def write_atomic(path, text):
@@ -121,23 +145,35 @@ def write_atomic(path, text):
     os.replace(tmp, path)
 
 
-def _cols(edges, ci):
-    """the edges' columns (element access on structured arrays is slow), plus (lo, hi) per edge or None without --ci"""
+def _cols(edges, ci, detail):
+    """the edges' columns (element access on structured arrays is slow), plus (lo, hi) per edge or None without --ci,
+    plus edge_details() per edge or None without --detailed"""
     cols = [edges[k].tolist() for k in ("a", "b", "ani", "af_a", "af_b")]
-    return cols + [[tuple(x) for x in ci.tolist()] if ci is not None else [None] * len(edges)]
+    cols.append([tuple(x) for x in ci.tolist()] if ci is not None else [None] * len(edges))
+    return cols + [detail if detail is not None else [None] * len(edges)]
 
 
-def triangle_rows(paths_sorted, names, edges, ci=None):
+def triangle_rows(paths_sorted, names, edges, ci=None, detail=None):
     """edges: structured array (a < b, ids index paths_sorted).  Ref = lexicographically smaller path
-    (SURVEY.md section 4 fact 3); rows grouped by Ref.  ci: Engine.last_edge_ci() for --ci's two extra columns."""
-    return [fmt_row(paths_sorted[a], paths_sorted[b], ani, afa, afb, names[a], names[b], iv)
-            for a, b, ani, afa, afb, iv in zip(*_cols(edges, ci))]
+    (SURVEY.md section 4 fact 3); rows grouped by Ref.  ci: Engine.last_edge_ci() for --ci's two extra columns;
+    detail: edge_details() for --detailed's 13 (they replace ci's)."""
+    return [fmt_row(paths_sorted[a], paths_sorted[b], ani, afa, afb, names[a], names[b], iv, dt)
+            for a, b, ani, afa, afb, iv, dt in zip(*_cols(edges, ci, detail))]
 
 
-def rect_rows(paths, names, edges, ci=None):
+def rect_rows(paths, names, edges, ci=None, detail=None):
     """edges: a = reference id, b = query id.  Rows grouped by query, ANI descending (SURVEY.md section 4 fact 7)."""
-    rows = sorted(zip(*_cols(edges, ci)), key=lambda t: (t[1], -t[2], t[0]))
-    return [fmt_row(paths[a], paths[b], ani, afa, afb, names[a], names[b], iv) for a, b, ani, afa, afb, iv in rows]
+    rows = sorted(zip(*_cols(edges, ci, detail)), key=lambda t: (t[1], -t[2], t[0]))
+    return [fmt_row(paths[a], paths[b], ani, afa, afb, names[a], names[b], iv, dt)
+            for a, b, ani, afa, afb, iv, dt in rows]
+
+
+def edge_extras(eng, ci, detailed, edges, stats=None):
+    """(ci, detail) for triangle_rows / rect_rows after an edge call run with --ci / --detailed as given: stats =
+    (n_contigs, nx) of the edges' genome ids, by default Engine.contig_stats of the whole context"""
+    if detailed:
+        return None, edge_details(edges, eng.last_edge_detail(), *(stats or eng.contig_stats(0, eng.n_genomes)))
+    return (eng.last_edge_ci() if ci else None), None
 
 
 def _device():
@@ -186,14 +222,15 @@ def run_triangle(opt, engine_mod):
         ph["context_s"] = time.time() - t0
         eng.set_estimator(opt["estimator"])
         eng.set_ci(opt["ci"])
+        eng.set_detailed(opt["detailed"])
         names = stream_add(eng, engine_mod, paths, opt["threads"], ph)
         t1 = time.time()
         eng.index()
         t2 = time.time()
         edges, st = eng.triangle(screen=opt["screen"], min_af=opt["min_af"])
-        ci = eng.last_edge_ci() if opt["ci"] else None
+        ci, detail = edge_extras(eng, opt["ci"], opt["detailed"], edges)
         t3 = time.time()
-    write_atomic(opt["out"], header(opt["ci"]) + "".join(triangle_rows(paths, names, edges, ci)))
+    write_atomic(opt["out"], header(opt["ci"], opt["detailed"]) + "".join(triangle_rows(paths, names, edges, ci, detail)))
     ph.update({"index_s": t2 - t1, "triangle_s": t3 - t2, "write_tsv_s": time.time() - t3, "total_s": time.time() - t0,
                "genomes": len(paths), "edges": int(len(edges))})
     _phase_log(opt, ph)
@@ -226,7 +263,8 @@ def run_search(opt, engine_mod):
         from . import daemon
 
         msg = {"op": "search", "query": query, "label": opt["positional"][0],  # the row shows the path as it was given
-               "screen": opt["screen"], "min_af": opt["min_af"], "estimator": opt["estimator"], "ci": opt["ci"], "out": out}
+               "screen": opt["screen"], "min_af": opt["min_af"], "estimator": opt["estimator"], "ci": opt["ci"],
+               "detailed": opt["detailed"], "out": out}
         rep = daemon.request(db, dev, msg)
         if rep is not None and rep.get("stale"):  # the directory was rewritten under a running server: it has just exited
             deadline = time.time() + 15.0
@@ -257,13 +295,25 @@ def run_search(opt, engine_mod):
     with engine_mod.Engine(dev) as eng:
         eng.set_estimator(opt["estimator"])
         eng.set_ci(opt["ci"])
+        eng.set_detailed(opt["detailed"])
         eng.load(opt["db"])
         eng.index()
         qp = engine_mod.pack_fasta(query, eng.params.min_contig_len)
         edges, st = eng.search(qp, screen=opt["screen"], min_af=opt["min_af"])
-        ci = eng.last_edge_ci() if opt["ci"] else None
-    write_atomic(opt["out"], header(opt["ci"]) + "".join(rect_rows(paths + [query], names + [qp.first_name], edges, ci)))
+        ci, detail = edge_extras(eng, opt["ci"], opt["detailed"], edges, search_contig_stats(eng) if opt["detailed"] else None)
+    write_atomic(opt["out"], header(opt["ci"], opt["detailed"]) +
+                 "".join(rect_rows(paths + [query], names + [qp.first_name], edges, ci, detail)))
     return st
+
+
+def search_contig_stats(eng, db_stats=None):
+    """contig statistics of the database genomes (db_stats, or read from the context) and, last, of the query the
+    previous Engine.search saw: indexed like the ids of that search's edges"""
+    import numpy as np
+
+    cnt, nx = db_stats or eng.contig_stats(0, eng.n_genomes)
+    qc, qnx = eng.last_query_contig_stats
+    return np.concatenate([cnt, qc]), np.concatenate([nx, qnx])
 
 
 def run_dist(opt, engine_mod):
@@ -273,12 +323,13 @@ def run_dist(opt, engine_mod):
     with engine_mod.Engine(_device()) as eng:
         eng.set_estimator(opt["estimator"])
         eng.set_ci(opt["ci"])
+        eng.set_detailed(opt["detailed"])
         names = stream_add(eng, engine_mod, paths, opt["threads"])
         eng.index()
         edges, st = eng.rect([idx[p] for p in dict.fromkeys(refs)], [idx[p] for p in dict.fromkeys(queries)],
                              screen=opt["screen"], min_af=opt["min_af"])
-        ci = eng.last_edge_ci() if opt["ci"] else None
-    write_atomic(opt["out"], header(opt["ci"]) + "".join(rect_rows(paths, names, edges, ci)))
+        ci, detail = edge_extras(eng, opt["ci"], opt["detailed"], edges)
+    write_atomic(opt["out"], header(opt["ci"], opt["detailed"]) + "".join(rect_rows(paths, names, edges, ci, detail)))
     return st
 
 
@@ -297,6 +348,9 @@ def _provenance(opt, sub, seconds):
     if opt.get("ci"):
         text += ("--ci: ANI_5_percentile / ANI_95_percentile are a 100-replicate bootstrap of the pair's chains as DESIGN.md "
                  "section 3 defines it; unpinned against skani's own intervals\n")
+    if opt.get("detailed"):
+        text += ("--detailed: the 13 extra columns as DESIGN.md section 3 defines them; their names, order and definitions "
+                 "are recalled, unpinned against skani's own --detailed output\n")
     try:
         write_atomic(opt["out"].rstrip("/") + ".skani_b200.log", text)
     except OSError:

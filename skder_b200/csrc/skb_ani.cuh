@@ -745,8 +745,8 @@ __global__ void cand_pack_kernel(DbView db, AniParams prm, const PairInfo *__res
 }
 
 // ANI of `a_in` anchors over `s_in` query seeds (both > 0): raw = ratio^(1/k), then the debias substitute.  The one
-// place this arithmetic lives: the pooled mean (make_pair_out), the median / robust estimators (est_pick_kernel) and
-// the --ci bounds (ci_kernel).
+// place this arithmetic lives: the pooled mean (make_pair_out), the median / robust estimators (est_pick_kernel),
+// the --ci bounds (ci_kernel) and --detailed's per-chain ANI (sd_kernel).
 // Two steps, so that make_pair_out keeps its order of work (the AF in between): its register allocation is unchanged.
 __device__ __forceinline__ double ani_raw_of(int64_t a_in, int64_t s_in) {
     double ratio = (double)a_in / (double)s_in;
@@ -849,7 +849,7 @@ __device__ __forceinline__ void fw_edge(const PCand *__restrict__ list, int i, i
 }
 
 // ctl: [0] largest candidate count among the listed mid pairs, [1] number of big pairs, [2] number of mid pairs.
-// ACC (median / robust estimators, --ci): also store every candidate's accepted flag at acc[its pcands index].
+// ACC (median / robust, --ci, --detailed): also store every candidate's accepted flag at acc[its pcands index].
 template <bool ACC>
 __global__ void __launch_bounds__(FW_WARPS * 32)
 finalize_warp_kernel(DbView db, AniParams prm, const PairInfo *__restrict__ info, const uint32_t *__restrict__ task_off,
@@ -1343,6 +1343,51 @@ ci_kernel(AniParams prm, const PairInfo *__restrict__ info, const uint32_t *__re
     }
 }
 
+// ---- --detailed (DESIGN.md section 3): spread of the chain identities, after ci_kernel, per batch ------------------
+// sd_kernel, one warp per pair with an estimate, over the chain list ci_kernel compacted at the pair's candidate offset
+// ((a << 16 | s), n_chains of them, no cap): d_c = the ANI of chain c alone (ratio -> raw -> debiased, as the ANI),
+// mu = sum s_c d_c / W, sd = sqrt(sum s_c (d_c - mu)^2 / W), W = sum s_c; two passes (d_c recomputed in the second).
+// sd[perm[p]] as a fraction; 0 for a one-chain pair, -1 for a pair without an estimate.
+__device__ __forceinline__ double sd_chain_ani(const AniParams &prm, uint32_t v) {
+    return ani_debiased(prm, ani_raw_of((int64_t)(v >> 16), (int64_t)(v & 0xffffu)));
+}
+
+__global__ void __launch_bounds__(FW_WARPS * 32)
+sd_kernel(AniParams prm, const uint32_t *__restrict__ task_off, uint32_t base, int64_t n_pairs,
+          const uint32_t *__restrict__ cand_off, const uint32_t *__restrict__ chains, const uint32_t *__restrict__ perm,
+          const PairOut *__restrict__ out, double *__restrict__ sd) {
+    const int lane = threadIdx.x & 31;
+    const int64_t warps_total = (int64_t)gridDim.x * FW_WARPS;
+    for (int64_t p = (int64_t)blockIdx.x * FW_WARPS + (threadIdx.x >> 5); p < n_pairs; p += warps_total) {
+        const uint32_t dst = perm[p];
+        const PairOut &o = out[dst];
+        const int n = o.n_chains;
+        if (o.ani_raw < 0.0 || n == 1) {
+            if (lane == 0) sd[dst] = o.ani_raw < 0.0 ? -1.0 : 0.0;
+            continue;
+        }
+        const uint32_t *list = chains + cand_off[task_off[p] - base];
+        const double W = (double)(o.n_seeds - 2ll * n);  // exact: < 2^53
+        double m = 0.0;
+        for (int t = lane; t < n; t += 32) {
+            const uint32_t v = list[t];
+            m += (double)(v & 0xffffu) * sd_chain_ani(prm, v);
+        }
+#pragma unroll
+        for (int d = 16; d > 0; d >>= 1) m += __shfl_xor_sync(0xffffffffu, m, d);
+        const double mu = m / W;
+        double q = 0.0;
+        for (int t = lane; t < n; t += 32) {
+            const uint32_t v = list[t];
+            const double e = sd_chain_ani(prm, v) - mu;
+            q += (double)(v & 0xffffu) * e * e;
+        }
+#pragma unroll
+        for (int d = 16; d > 0; d >>= 1) q += __shfl_down_sync(0xffffffffu, q, d);
+        if (lane == 0) sd[dst] = sqrt(q / W);
+    }
+}
+
 // K5 -- edge compaction: keep pairs with an estimate and max(AF) >= min_af; percent units.  Order-preserving
 // (flag -> exclusive scan -> scatter): the pair list is sorted by (a, b), so the edge list comes out sorted too.
 __device__ __forceinline__ bool edge_kept(const PairOut &o, double min_af) {
@@ -1376,6 +1421,25 @@ __global__ void edge_ci_scatter_kernel(const double2 *__restrict__ ci, int64_t n
     const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= n_pairs || !flag[t]) return;
     edge_ci[pos[t]] = make_double2(ci[t].x * 100.0, ci[t].y * 100.0);
+}
+// --detailed only: the kept pairs' details in edge order (edge_flag_kernel's flags, their scan): the interval as
+// edge_ci_scatter_kernel writes it, sd in percent, and the AF numerators picked by `swapped` as edge_scatter_kernel
+// picks the AF
+__global__ void edge_detail_scatter_kernel(const PairOut *__restrict__ po, const double2 *__restrict__ ci,
+                                           const double *__restrict__ sd, int64_t n_pairs, const uint32_t *__restrict__ flag,
+                                           const uint32_t *__restrict__ pos, skb_edge_detail *__restrict__ detail) {
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= n_pairs || !flag[t]) return;
+    const PairOut &o = po[t];
+    skb_edge_detail d;
+    d.ani_lo = ci[t].x * 100.0;
+    d.ani_hi = ci[t].y * 100.0;
+    d.sd = sd[t] * 100.0;
+    d.covered_a = o.swapped ? o.span_r : o.span_q;
+    d.covered_b = o.swapped ? o.span_q : o.span_r;
+    d.n_chains = o.n_chains;
+    d.pad = 0;
+    detail[pos[t]] = d;
 }
 
 // bookkeeping: sum over pairs of the query genome's seed count and of the chained anchors (roofline bytes)

@@ -7,6 +7,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <functional>
 #include <ctime>
 #include <cub/cub.cuh>
 #include <map>
@@ -101,10 +102,13 @@ struct skb_ctx {
     bool ani_attr_set = false;
     int32_t estimator = SKB_ANI_MEAN;  // skb_set_ani_estimator; kept across skb_clear
     bool ci = false;                   // skb_set_ani_ci; kept across skb_clear
+    bool detailed = false;             // skb_set_detailed; kept across skb_clear
     const skb_edge *last_dev_edges = nullptr;  // device copy of the last triangle/rect result (skb_device_edges)
     int64_t last_n_edges = 0;
     bool last_ci = false;                 // that call ran with --ci ...
     const double2 *last_dev_ci = nullptr;  // ... and left the edges' intervals here (skb_last_edge_ci)
+    bool last_detailed = false;                       // that call ran with --detailed ...
+    const skb_edge_detail *last_dev_detail = nullptr;  // ... and left the edges' details here (skb_last_edge_detail)
     std::vector<cudaEvent_t> anchor_ev;  // start/stop pairs around the anchor kernel launches of the current call
     int anchor_ev_used = 0;
     float last_ms_anchor = 0;
@@ -431,7 +435,9 @@ void sketch_batch(skb_ctx *c, const skb_packed *const *gen, int32_t g0, int32_t 
 //   cands     : SLOTS candidate slots per task;  task_ncand: how many are filled
 
 // d_ci: nullptr, or [n_pairs] for every pair's --ci interval (ci_kernel), indexed like d_out
-void run_ani(skb_ctx *c, const unsigned long long *d_pairs, int64_t n_pairs, PairOut *d_out, double2 *d_ci = nullptr) {
+// d_sd: nullptr, or (with d_ci) [n_pairs] for every pair's --detailed standard deviation (sd_kernel), indexed like d_out
+void run_ani(skb_ctx *c, const unsigned long long *d_pairs, int64_t n_pairs, PairOut *d_out, double2 *d_ci = nullptr,
+             double *d_sd = nullptr) {
     c->anchor_ev_used = 0;
     if (n_pairs == 0) return;
     if (n_pairs >= (1ll << 31)) throw CudaFail{"too many surviving pairs in one call"};
@@ -456,7 +462,8 @@ void run_ani(skb_ctx *c, const unsigned long long *d_pairs, int64_t n_pairs, Pai
     // median / robust: the finalize kernels also store every candidate's accepted flag, and an estimator stage per
     // batch turns the accepted chains into one ANI (est_key_kernel, segmented sort, est_pick_kernel)
     const bool est = c->estimator != SKB_ANI_MEAN;
-    // --ci: the accepted flags too, and ci_kernel per batch bootstraps the pair's accepted chains
+    // --ci (and --detailed, which prints the interval too): the accepted flags too, and ci_kernel per batch bootstraps
+    // the pair's accepted chains; --detailed's sd_kernel then reads the chain list ci_kernel compacted
     const bool acc = est || d_ci;
     const DbView view = c->view();
     const AniParams prm = c->ani_params();
@@ -662,6 +669,12 @@ void run_ani(skb_ctx *c, const unsigned long long *d_pairs, int64_t n_pairs, Pai
                    c->d_task_off.p + bt.p0, base, np, b_pcands.p, b_cand_off.p, e_acc.p, ci_chains.p, d_perm.p + bt.p0, d_out,
                    d_ci);
             if (trace) spans.push_back({"ci", bi, tc, mark()});
+            if (d_sd) {
+                cudaEvent_t ts = mark();
+                launch(c, sd_kernel, nblk((uint64_t)np, FW_WARPS), FW_WARPS * 32, 0, prm, c->d_task_off.p + bt.p0, base, np,
+                       b_cand_off.p, ci_chains.p, d_perm.p + bt.p0, d_out, d_sd);
+                if (trace) spans.push_back({"detail", bi, ts, mark()});
+            }
         }
         if (est && n_cand) {
             cudaEvent_t te = mark();
@@ -706,16 +719,24 @@ void pairs_to_edges(skb_ctx *c, unsigned long long *d_pairs, int64_t n_pairs, do
     CK(cudaEventRecord(ev_mid, c->st));
     c->last_ci = c->ci;
     c->last_dev_ci = nullptr;
+    c->last_detailed = c->detailed;
+    c->last_dev_detail = nullptr;
     if (n_pairs > 0) {
         d_out.reserve((size_t)n_pairs, 0, c->st);
         d_edges.reserve((size_t)n_pairs, 0, c->st);
         double2 *d_ci = nullptr;
-        if (c->ci) {
+        if (c->ci || c->detailed) {
             PoolRef<double2> ci_pairs(c->pool["ci.pairs"]);
             ci_pairs.reserve((size_t)n_pairs, 0, c->st);
             d_ci = ci_pairs.p;
         }
-        run_ani(c, d_pairs, n_pairs, d_out.p, d_ci);
+        double *d_sd = nullptr;
+        if (c->detailed) {
+            PoolRef<double> sd_pairs(c->pool["detail.sd"]);
+            sd_pairs.reserve((size_t)n_pairs, 0, c->st);
+            d_sd = sd_pairs.p;
+        }
+        run_ani(c, d_pairs, n_pairs, d_out.p, d_ci, d_sd);
         PoolRef<uint32_t> d_ef(c->pool["pairs_to_edges.flag"]), d_ep(c->pool["pairs_to_edges.pos"]);
         d_ef.reserve((size_t)n_pairs, 0, c->st);
         d_ep.reserve((size_t)n_pairs, 0, c->st);
@@ -723,11 +744,18 @@ void pairs_to_edges(skb_ctx *c, unsigned long long *d_pairs, int64_t n_pairs, do
         exclusive_scan_u32(c, d_ef.p, d_ep.p, (size_t)n_pairs);
         launch(c, edge_scatter_kernel, nblk((uint64_t)n_pairs, 256), 256, 0, d_pairs, d_out.p, n_pairs, d_ef.p, d_ep.p,
                d_edges.p, d_n.p);
-        if (d_ci) {
+        if (c->ci) {
             PoolRef<double2> ci_edges(c->pool["ci.edges"]);
             ci_edges.reserve((size_t)n_pairs, 0, c->st);
             launch(c, edge_ci_scatter_kernel, nblk((uint64_t)n_pairs, 256), 256, 0, d_ci, n_pairs, d_ef.p, d_ep.p, ci_edges.p);
             c->last_dev_ci = ci_edges.p;
+        }
+        if (c->detailed) {
+            PoolRef<skb_edge_detail> det_edges(c->pool["detail.edges"]);
+            det_edges.reserve((size_t)n_pairs, 0, c->st);
+            launch(c, edge_detail_scatter_kernel, nblk((uint64_t)n_pairs, 256), 256, 0, d_out.p, d_ci, d_sd, n_pairs, d_ef.p,
+                   d_ep.p, det_edges.p);
+            c->last_dev_detail = det_edges.p;
         }
     }
     CK(cudaEventRecord(ev_end, c->st));
@@ -773,6 +801,10 @@ int edge_call(skb_ctx *c, double min_af_pct, skb_edge **edges, int64_t *n_edges,
     if (c->ci && c->estimator != SKB_ANI_MEAN)
         return fail(c, SKB_EINVAL,
                     "the --ci interval is defined for the mean ANI estimator only (skb_set_ani_ci, skb_set_ani_estimator)");
+    // --detailed prints that interval too (DESIGN.md section 3)
+    if (c->detailed && c->estimator != SKB_ANI_MEAN)
+        return fail(c, SKB_EINVAL,
+                    "the --detailed columns are defined for the mean ANI estimator only (skb_set_detailed, skb_set_ani_estimator)");
     const int64_t launches0 = c->launches;
     cudaEvent_t *ev = call_events(c);
     CK(cudaEventRecord(ev[0], c->st));
@@ -813,6 +845,21 @@ int edge_call(skb_ctx *c, double min_af_pct, skb_edge **edges, int64_t *n_edges,
     }
     *n_edges = ne;
     return SKB_OK;
+}
+
+// malloc'ed host copy of the `rec_bytes`-byte records the last edge call left on the device, one per edge, or nullptr
+// when the host is out of memory (skb_last_edge_ci, skb_last_edge_detail)
+void *last_edges_to_host(skb_ctx *c, const void *dev, size_t rec_bytes) {
+    const size_t bytes = (size_t)c->last_n_edges * rec_bytes;
+    void *h = std::malloc(std::max<size_t>(1, bytes));
+    if (!h || !bytes) return h;
+    cudaError_t e = cudaMemcpyAsync(h, dev, bytes, cudaMemcpyDeviceToHost, c->st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(c->st);
+    if (e != cudaSuccess) {
+        std::free(h);
+        CK(e);
+    }
+    return h;
 }
 
 bool write_all(FILE *f, const void *p, size_t n) { return n == 0 || fwrite(p, 1, n, f) == n; }
@@ -1617,19 +1664,62 @@ int skb_last_edge_ci(skb_ctx *ctx, double **lo_hi, int64_t *n) {
         if (!lo_hi || !n) return fail(ctx, SKB_EINVAL, "bad arguments");
         if (!ctx->last_ci)
             return fail(ctx, SKB_ESTATE, "the last skb_triangle / skb_rect / skb_pairs_edges call ran without --ci (skb_set_ani_ci)");
-        const size_t ne = (size_t)ctx->last_n_edges;
-        double *h = (double *)std::malloc(std::max<size_t>(1, ne) * sizeof(double2));
+        double *h = (double *)last_edges_to_host(ctx, ctx->last_dev_ci, sizeof(double2));
         if (!h) return fail(ctx, SKB_ENOMEM, "host out of memory for the intervals");
-        if (ne) {
-            cudaError_t e = cudaMemcpyAsync(h, ctx->last_dev_ci, ne * sizeof(double2), cudaMemcpyDeviceToHost, ctx->st);
-            if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->st);
-            if (e != cudaSuccess) {
-                std::free(h);
-                CK(e);
-            }
-        }
         *lo_hi = h;
-        *n = (int64_t)ne;
+        *n = ctx->last_n_edges;
+        return SKB_OK;
+    });
+}
+
+int skb_set_detailed(skb_ctx *ctx, int32_t enabled) {
+    return guarded(ctx, [&]() -> int {
+        ctx->detailed = enabled != 0;
+        return SKB_OK;
+    });
+}
+
+int skb_last_edge_detail(skb_ctx *ctx, skb_edge_detail **out, int64_t *n) {
+    return guarded(ctx, [&]() -> int {
+        if (!out || !n) return fail(ctx, SKB_EINVAL, "bad arguments");
+        if (!ctx->last_detailed)
+            return fail(ctx, SKB_ESTATE,
+                        "the last skb_triangle / skb_rect / skb_pairs_edges call ran without --detailed (skb_set_detailed)");
+        skb_edge_detail *h = (skb_edge_detail *)last_edges_to_host(ctx, ctx->last_dev_detail, sizeof(skb_edge_detail));
+        if (!h) return fail(ctx, SKB_ENOMEM, "host out of memory for the edge details");
+        *out = h;
+        *n = ctx->last_n_edges;
+        return SKB_OK;
+    });
+}
+
+int skb_genome_contig_stats(skb_ctx *ctx, int32_t first, int32_t n, int32_t *n_contigs, int64_t *nx) {
+    return guarded(ctx, [&]() -> int {
+        if (n < 0 || first < 0 || first > ctx->n() - n || (n && (!n_contigs || !nx))) return fail(ctx, SKB_EINVAL, "bad arguments");
+        const skb_ctx::SketchDb &db = ctx->db;
+        std::vector<uint32_t> len;
+        for (int32_t i = 0; i < n; i++) {
+            const int32_t g = first + i;
+            len.assign(db.ctg_len.begin() + db.ctg_off[g], db.ctg_len.begin() + db.ctg_off[g + 1]);
+            std::sort(len.begin(), len.end(), std::greater<uint32_t>());
+            uint64_t total = 0;
+            for (uint32_t l : len) total += l;
+            // Nx: the length l_k of the first k (lengths descending) with 100 (l_1 + ... + l_k) >= x T
+            const int xs[3] = {90, 50, 10};
+            for (int j = 0; j < 3; j++) {
+                uint64_t cum = 0;
+                int64_t v = 0;
+                for (uint32_t l : len) {
+                    cum += l;
+                    if (100 * cum >= (uint64_t)xs[j] * total) {
+                        v = l;
+                        break;
+                    }
+                }
+                nx[3 * (size_t)i + j] = v;
+            }
+            n_contigs[i] = (int32_t)len.size();
+        }
         return SKB_OK;
     });
 }

@@ -124,6 +124,7 @@ def serve(db_dir, device):
     eng.load(db_dir)
     eng.index()
     n_db = eng.n_genomes
+    db_stats = None  # contig statistics of the database genomes, read on the first --detailed request
     key = secrets.token_bytes(32)
     kp = _key_path(db_dir, device)
     fd = os.open(kp + ".tmp", os.O_WRONLY | os.O_CREAT | os.O_TRUNC, 0o600)
@@ -158,13 +159,18 @@ def serve(db_dir, device):
                         stop = True
                     elif msg.get("op") == "search":
                         eng.set_estimator(msg.get("estimator", "mean"))  # per request: a resident server serves every mode
-                        ci = bool(msg.get("ci", False))
+                        ci, detailed = bool(msg.get("ci", False)), bool(msg.get("detailed", False))
                         eng.set_ci(ci)
+                        eng.set_detailed(detailed)
                         packed = engine.pack_fasta(msg["query"], eng.params.min_contig_len)
                         edges, st = eng.search(packed, screen=msg["screen"], min_af=msg["min_af"])
+                        stats = None
+                        if detailed:
+                            db_stats = db_stats or eng.contig_stats(0, n_db)  # the database's, once per server
+                            stats = cli.search_contig_stats(eng, db_stats)
                         rows = cli.rect_rows(paths + [msg.get("label", msg["query"])], names + [packed.first_name], edges,
-                                             eng.last_edge_ci() if ci else None)
-                        cli.write_atomic(msg["out"], cli.header(ci) + "".join(rows))
+                                             *cli.edge_extras(eng, ci, detailed, edges, stats))
+                        cli.write_atomic(msg["out"], cli.header(ci, detailed) + "".join(rows))
                         conn.send_bytes(json.dumps({"ok": True, "rows": len(rows), "ms": st.ms_total}).encode())
                     else:
                         conn.send_bytes(json.dumps({"ok": False, "error": "unknown op"}).encode())

@@ -20,6 +20,12 @@ EDGE_DTYPE = np.dtype(
      "offsets": [0, 4, 8, 16, 24], "itemsize": 32}
 )
 assert C.sizeof(_lib.Edge) == EDGE_DTYPE.itemsize
+# skb_edge_detail: --detailed's per-edge record (Engine.last_edge_detail)
+DETAIL_DTYPE = np.dtype(
+    {"names": ["ani_lo", "ani_hi", "sd", "covered_a", "covered_b", "n_chains"],
+     "formats": ["<f8", "<f8", "<f8", "<i8", "<i8", "<i4"], "offsets": [0, 8, 16, 24, 32, 40], "itemsize": 48}
+)
+assert C.sizeof(_lib.EdgeDetail) == DETAIL_DTYPE.itemsize
 
 
 def default_params():
@@ -102,6 +108,8 @@ class Engine:
         if rc != 0:
             raise SkbError("skb_create failed (%d): %s" % (rc, self._L.skb_last_error(None).decode()))
         self.device = int(device)
+        self.detailed = False  # set_detailed
+        self.last_query_contig_stats = None  # contig_stats of the last search's query, with set_detailed(True)
 
     def close(self):
         if getattr(self, "_h", None):
@@ -144,6 +152,34 @@ class Engine:
         finally:
             self._L.skb_free(ptr)
 
+    def set_detailed(self, on):
+        """skani's --detailed: later triangle / rect / search / pairs_edges calls also leave a detail record per edge
+        (last_edge_detail), and search keeps the query's contig statistics (last_query_contig_stats); DESIGN.md section
+        3.  Mean estimator only.  Survives clear()."""
+        self._ck(self._L.skb_set_detailed(self._h, 1 if on else 0), "skb_set_detailed")
+        self.detailed = bool(on)
+
+    def last_edge_detail(self):
+        """DETAIL_DTYPE array of every edge of the last triangle / rect / search / pairs_edges call, in edge order: the
+        --ci interval and the chains' standard deviation (percent), the AF numerators of genomes a and b, the accepted
+        chain count.  That call must have run with set_detailed(True)."""
+        ptr, n = C.POINTER(_lib.EdgeDetail)(), C.c_int64()
+        self._ck(self._L.skb_last_edge_detail(self._h, C.byref(ptr), C.byref(n)), "skb_last_edge_detail")
+        try:
+            if n.value == 0:
+                return np.zeros(0, DETAIL_DTYPE)
+            buf = C.cast(ptr, C.POINTER(C.c_char * (n.value * DETAIL_DTYPE.itemsize))).contents
+            return np.frombuffer(buf, dtype=DETAIL_DTYPE, count=n.value).copy()
+        finally:
+            self._L.skb_free(ptr)
+
+    def contig_stats(self, first, n):
+        """(n_contigs [n] int32, nx [n, 3] int64: N90, N50, N10) over the kept contigs of genomes first .. first+n-1"""
+        cnt, nx = np.zeros(n, np.int32), np.zeros((n, 3), np.int64)
+        self._ck(self._L.skb_genome_contig_stats(self._h, first, n, cnt.ctypes.data_as(C.POINTER(C.c_int32)),
+                                                 nx.ctypes.data_as(C.POINTER(C.c_int64))), "skb_genome_contig_stats")
+        return cnt, nx
+
     # ---- sketching -------------------------------------------------------------------------
     def add(self, packed):
         n = len(packed)
@@ -185,10 +221,13 @@ class Engine:
 
     def search(self, query_packed, screen=80.0, min_af=15.0):
         """`skani search`: one query genome against the resident, indexed database (ids 0..n-1).  The query
-        is sketched, indexed query-only, compared, and removed again.  Edges: a = database genome, b = query."""
+        is sketched, indexed query-only, compared, and removed again.  Edges: a = database genome, b = query.
+        With set_detailed(True) the query's contig_stats are kept in last_query_contig_stats."""
         n_db = self.n_genomes
         self.add([query_packed])
         try:
+            if self.detailed:  # contig_stats of the query: it leaves the context below
+                self.last_query_contig_stats = self.contig_stats(n_db, 1)
             self.index_append()
             return self.rect(np.arange(n_db, dtype=np.int32), [n_db], screen=screen, min_af=min_af)
         finally:
