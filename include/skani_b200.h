@@ -101,7 +101,17 @@ int skb_sketch_sizes(skb_ctx *ctx, int32_t g, int64_t *n_seeds, int64_t *n_marke
 int skb_get_seeds(skb_ctx *ctx, int32_t g, uint64_t *out);   /* position-ordered packed seed records */
 int skb_get_markers(skb_ctx *ctx, int32_t g, uint64_t *out); /* sorted unique canonical 21-mers */
 
-/* persistence of the sketch DB: `skani sketch -o <dir>` writes it, `skani search -d <dir>` loads it */
+/* skani's -m (DESIGN.md section 3): a canonical 21-mer is a marker iff its hash is below UINT64_MAX / m (integer
+ * division; default m = 1000).  Markers only decide which pairs the prescreen passes; seeds, chains and the ANI/AF of a
+ * pair are the same at every m.  Context state, kept across skb_clear, applied to every later skb_add_genomes.  m < 1:
+ * SKB_EINVAL; a different m while the context holds genomes: SKB_ESTATE (setting the current value is fine).  A small
+ * m makes many markers: like any other allocation, one the device cannot hold fails the call that needs it. */
+int skb_set_marker_compression(skb_ctx *ctx, int64_t m);
+int skb_marker_compression(const skb_ctx *ctx, int64_t *m);
+
+/* persistence of the sketch DB: `skani sketch -o <dir>` writes it, `skani search -d <dir>` loads it.  The file records
+ * the marker compression (format SKB200v1 at m = 1000, SKB200v2 otherwise); skb_db_load reads both and sets the
+ * context's m to the file's, so genomes added afterwards (a search's query) are sketched at the database's density. */
 int skb_db_save(skb_ctx *ctx, const char *dir);
 int skb_db_load(skb_ctx *ctx, const char *dir);
 
@@ -201,7 +211,8 @@ typedef struct {
 } skb_sketch_view;
 int skb_sketch_view_get(skb_ctx *ctx, skb_sketch_view *view);
 /* append genomes whose sketches were produced by another context (device pointers on THIS device);
- * marker keys are re-tagged with the receiving context's genome ids */
+ * marker keys are re-tagged with the receiving context's genome ids.  The sender's marker compression is not part of
+ * the view: the caller must give both contexts the same one (skb_set_marker_compression; multi.py checks it). */
 int skb_import_sketches(skb_ctx *ctx, int32_t n_genomes, const uint64_t *dev_seeds, int64_t n_seeds,
                         const uint64_t *dev_marker_keys, int64_t n_marker_keys, const uint64_t *host_seed_off,
                         const uint64_t *host_total_len, const uint32_t *host_ctg_off, const uint32_t *host_ctg_len,

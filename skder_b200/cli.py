@@ -16,13 +16,18 @@ ANI_95_percentile; and `--detailed`, which appends 13 columns (contig counts and
 interval, the spread of the chain identities, the chains' average length and the query bases they cover).  --ci and
 --detailed are not taken with --median / --robust.  skDER's `-n` clustering reads exactly seven fields (skder.py:190),
 so a `-p` with --ci or --detailed breaks it as it would with skani; greedy and dynamic selection are unaffected.
-Any other skani option (-c, -m, --fast, --slow, --medium, --small-genomes, --no-learned-ani, ...) changes skani's
+`-m M` (triangle, dist, sketch) is skani's marker compression: a canonical 21-mer is a marker iff its hash is below
+2^64 / M (default 1000).  Markers only decide which pairs the prescreen passes, so a smaller M (skani suggests
+~200-300 for plasmids and viruses) lets small genomes that share no marker at 1000 be compared; a pair's ANI/AF does
+not depend on it.  A database records its M, and `search` sketches the query at that M, so search takes no -m.
+Any other skani option (-c, --fast, --slow, --medium, --small-genomes, --no-learned-ani, ...) changes skani's
 estimator in ways this engine does not implement: the shim then exits non-zero WITHOUT creating the output, which is
 the one failure signal runCmd checks (util.py:642-645).
 stderr is discarded by skDER, so diagnostics also go to <output>.skani_b200.log.
 """
 import json
 import os
+import re
 import sys
 import time
 
@@ -34,6 +39,7 @@ DETAILED_COLUMNS = ("Num_ref_contigs", "Num_query_contigs", "ANI_5_percentile", 
 DETAILED_FMT = "\t%d\t%d\t%.2f\t%.2f\t%.2f\t%d\t%d\t%d\t%d\t%d\t%d\t%d\t%d\n"
 DEFAULT_SCREEN = 80.0  # skani -s default
 DEFAULT_MIN_AF = 15.0  # skani --min-af default
+DEFAULT_MARKER_C = 1000  # skani -m default
 
 
 class UsageError(Exception):
@@ -50,7 +56,7 @@ def parse_args(argv):
     opt = {"screen": DEFAULT_SCREEN, "min_af": DEFAULT_MIN_AF, "threads": 3, "edge_list": False, "positional": []}
     valued = {
         "-l": "list", "-o": "out", "-t": "threads", "-s": "screen", "--min-af": "min_af", "--rl": "rl", "--ql": "ql",
-        "-d": "db",
+        "-d": "db", "-m": "marker_c",
     }
     flags = {"-E": "edge_list", "--sparse": "edge_list", "--ci": "ci", "--detailed": "detailed"}
     opt["ci"] = opt["detailed"] = False
@@ -84,6 +90,15 @@ def parse_args(argv):
         opt["threads"] = max(1, int(opt["threads"]))
     except ValueError as e:
         raise UsageError("bad numeric option: %s" % e)
+    if "marker_c" in opt:
+        if sub == "search":
+            raise UsageError("skani search takes no -m: the query is sketched at the database's marker compression")
+        m = opt["marker_c"]
+        if not re.fullmatch(r"[0-9]+", m) or not 1 <= int(m) < 2 ** 63:
+            raise UsageError("-m needs an integer of at least 1, not %r" % m)
+        opt["marker_c"] = int(m)
+    else:
+        opt["marker_c"] = DEFAULT_MARKER_C
     if len(set(chosen)) > 1:
         raise UsageError("--median and --robust are mutually exclusive")
     if chosen and sub == "sketch":
@@ -223,6 +238,7 @@ def run_triangle(opt, engine_mod):
         eng.set_estimator(opt["estimator"])
         eng.set_ci(opt["ci"])
         eng.set_detailed(opt["detailed"])
+        eng.set_marker_compression(opt["marker_c"])
         names = stream_add(eng, engine_mod, paths, opt["threads"], ph)
         t1 = time.time()
         eng.index()
@@ -244,6 +260,7 @@ def run_sketch(opt, engine_mod):
 
     daemon.stop_for(opt["out"])  # a server still holding the previous contents of this directory must not answer for the new ones
     with engine_mod.Engine(_device()) as eng:
+        eng.set_marker_compression(opt["marker_c"])  # recorded in the database: its searches sketch queries at it
         names = stream_add(eng, engine_mod, paths, opt["threads"])
         eng.save(opt["out"])
     write_atomic(os.path.join(opt["out"], "manifest.json"), json.dumps({"paths": paths, "names": names}))
@@ -324,6 +341,7 @@ def run_dist(opt, engine_mod):
         eng.set_estimator(opt["estimator"])
         eng.set_ci(opt["ci"])
         eng.set_detailed(opt["detailed"])
+        eng.set_marker_compression(opt["marker_c"])
         names = stream_add(eng, engine_mod, paths, opt["threads"])
         eng.index()
         edges, st = eng.rect([idx[p] for p in dict.fromkeys(refs)], [idx[p] for p in dict.fromkeys(queries)],
@@ -348,6 +366,9 @@ def _provenance(opt, sub, seconds):
     if opt.get("ci"):
         text += ("--ci: ANI_5_percentile / ANI_95_percentile are a 100-replicate bootstrap of the pair's chains as DESIGN.md "
                  "section 3 defines it; unpinned against skani's own intervals\n")
+    if opt.get("marker_c", DEFAULT_MARKER_C) != DEFAULT_MARKER_C:
+        text += ("-m %d: markers are the canonical 21-mers whose hash is below 2^64 / %d (skani's default is 1000); they "
+                 "decide only which pairs pass the prescreen, not a pair's ANI/AF\n" % (opt["marker_c"], opt["marker_c"]))
     if opt.get("detailed"):
         text += ("--detailed: the 13 extra columns as DESIGN.md section 3 defines them; their names, order and definitions "
                  "are recalled, unpinned against skani's own --detailed output\n")

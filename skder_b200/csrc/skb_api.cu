@@ -103,6 +103,7 @@ struct skb_ctx {
     int32_t estimator = SKB_ANI_MEAN;  // skb_set_ani_estimator; kept across skb_clear
     bool ci = false;                   // skb_set_ani_ci; kept across skb_clear
     bool detailed = false;             // skb_set_detailed; kept across skb_clear
+    uint64_t marker_c = C_MARKER;      // skb_set_marker_compression / skb_db_load; kept across skb_clear
     const skb_edge *last_dev_edges = nullptr;  // device copy of the last triangle/rect result (skb_device_edges)
     int64_t last_n_edges = 0;
     bool last_ci = false;                 // that call ran with --ci ...
@@ -398,6 +399,7 @@ void sketch_batch(skb_ctx *c, const skb_packed *const *gen, int32_t g0, int32_t 
     CK(cudaMemsetAsync(d_cnt_m.p + n_warps, 0, 4, c->st));
     SketchBatch b = meta.b;
     b.first_gid = (uint32_t)c->n();
+    b.thr_marker = marker_threshold(c->marker_c);
     PoolRef<ulonglong2> d_masks(c->pool["sketch_batch.d_masks"]);
     d_masks.reserve(n_warps * 32, 0, c->st);
     launch(c, sketch_kernel<false>, n_tiles, SK_THREADS, 0, b, d_cnt_s.p, d_cnt_m.p, nullptr, nullptr, nullptr, nullptr,
@@ -1679,6 +1681,23 @@ int skb_set_detailed(skb_ctx *ctx, int32_t enabled) {
     });
 }
 
+int skb_set_marker_compression(skb_ctx *ctx, int64_t m) {
+    return guarded(ctx, [&]() -> int {
+        if (m < 1) return fail(ctx, SKB_EINVAL, "marker compression must be at least 1");
+        if ((uint64_t)m == ctx->marker_c) return SKB_OK;
+        // every genome of a context is sketched at one density: the screen compares marker counts across genomes
+        if (ctx->n() != 0) return fail(ctx, SKB_ESTATE, "context already holds genomes sketched at another marker compression");
+        ctx->marker_c = (uint64_t)m;
+        return SKB_OK;
+    });
+}
+
+int skb_marker_compression(const skb_ctx *ctx, int64_t *m) {
+    if (!ctx || !m) return SKB_EINVAL;
+    *m = (int64_t)ctx->marker_c;
+    return SKB_OK;
+}
+
 int skb_last_edge_detail(skb_ctx *ctx, skb_edge_detail **out, int64_t *n) {
     return guarded(ctx, [&]() -> int {
         if (!out || !n) return fail(ctx, SKB_EINVAL, "bad arguments");
@@ -1790,7 +1809,11 @@ int skb_shared_markers(skb_ctx *ctx, const uint32_t *a, const uint32_t *b, int64
 }
 
 // ---- persistence: raw sketches (seeds + marker keys + host tables); the index is rebuilt on load
+// v1: magic | n | n_seeds | n_marker_keys | n_contigs | tables | seeds | marker keys, sketched at m = 1000.
+// v2: the same with the marker compression m (u64) between the magic and n; written only when m != 1000, so a
+// default database stays a v1 file byte for byte.
 static const char kMagic[8] = {'S', 'K', 'B', '2', '0', '0', 'v', '1'};
+static const char kMagic2[8] = {'S', 'K', 'B', '2', '0', '0', 'v', '2'};
 
 int skb_db_save(skb_ctx *ctx, const char *dir) {
     return guarded(ctx, [&]() -> int {
@@ -1805,7 +1828,9 @@ int skb_db_save(skb_ctx *ctx, const char *dir) {
         if (ns) CK(cudaMemcpy(seeds.data(), c->d_seeds.p, ns * 8, cudaMemcpyDeviceToHost));
         if (nm) CK(cudaMemcpy(mk.data(), c->d_mkeys.p, nm * 8, cudaMemcpyDeviceToHost));
         for (auto &s : seeds) s &= ~2ull;  // repeat flags are index state
-        bool ok = write_all(f, kMagic, 8) && write_all(f, &n, 8) && write_all(f, &ns, 8) && write_all(f, &nm, 8) &&
+        const bool v1 = c->marker_c == C_MARKER;
+        bool ok = (v1 ? write_all(f, kMagic, 8) : write_all(f, kMagic2, 8) && write_all(f, &c->marker_c, 8)) &&
+                  write_all(f, &n, 8) && write_all(f, &ns, 8) && write_all(f, &nm, 8) &&
                   write_all(f, &nc, 8) && write_all(f, c->db.seed_off.data(), (n + 1) * 8) &&
                   write_all(f, c->db.total_len.data(), n * 8) && write_all(f, c->db.ctg_off.data(), (n + 1) * 4) &&
                   write_all(f, c->db.ctg_len.data(), nc * 4) && write_all(f, seeds.data(), ns * 8) &&
@@ -1824,10 +1849,11 @@ int skb_db_load(skb_ctx *ctx, const char *dir) {
         FILE *f = fopen(path.c_str(), "rb");
         if (!f) return fail(c, SKB_EIO, "cannot open " + path);
         char magic[8];
-        uint64_t n = 0, ns = 0, nm = 0, nc = 0;
-        bool ok = read_all(f, magic, 8) && std::memcmp(magic, kMagic, 8) == 0 && read_all(f, &n, 8) &&
-                  read_all(f, &ns, 8) && read_all(f, &nm, 8) && read_all(f, &nc, 8);
-        if (!ok || n >= GID_MASK) {
+        uint64_t n = 0, ns = 0, nm = 0, nc = 0, m = C_MARKER;
+        bool ok = read_all(f, magic, 8) &&
+                  (std::memcmp(magic, kMagic, 8) == 0 || (std::memcmp(magic, kMagic2, 8) == 0 && read_all(f, &m, 8))) &&
+                  read_all(f, &n, 8) && read_all(f, &ns, 8) && read_all(f, &nm, 8) && read_all(f, &nc, 8);
+        if (!ok || n >= GID_MASK || m < 1 || m > (uint64_t)INT64_MAX) {
             fclose(f);
             return fail(c, SKB_EIO, "not a sketch DB: " + path);
         }
@@ -1844,6 +1870,7 @@ int skb_db_load(skb_ctx *ctx, const char *dir) {
         if (nm) CK(cudaMemcpyAsync(c->d_mkeys.p, mk.data(), nm * 8, cudaMemcpyHostToDevice, c->st));
         CK(cudaStreamSynchronize(c->st));
         c->db = skb_ctx::SketchDb{std::move(seed_off), std::move(total_len), std::move(ctg_off), std::move(ctg_len), nm};
+        c->marker_c = m;  // genomes added later (a search's query) are sketched at the database's density
         c->indexed = false;
         return SKB_OK;
     });

@@ -11,9 +11,10 @@ namespace skb {
 constexpr int K_SEED = 15;
 constexpr int K_MARKER = 21;
 constexpr uint64_t C_SEED = 125;
-constexpr uint64_t C_MARKER = 1000;
+constexpr uint64_t C_MARKER = 1000;  // skani's -m default; a context's value is skb_set_marker_compression's
 constexpr uint64_t THR_SEED = 0xFFFFFFFFFFFFFFFFull / C_SEED;
-constexpr uint64_t THR_MARKER = 0xFFFFFFFFFFFFFFFFull / C_MARKER;
+// markers are kept iff mm_hash64 < marker_threshold(m) (SketchBatch::thr_marker)
+__host__ __device__ inline uint64_t marker_threshold(uint64_t m) { return 0xFFFFFFFFFFFFFFFFull / m; }
 constexpr uint64_t MASK_MARKER = (~0ull) >> (64 - 2 * K_MARKER);
 constexpr uint64_t MASK_SEED = (~0ull) >> (64 - 2 * K_SEED);
 constexpr uint32_t CONTIG_PAD = 4096;  // virtual gap between contigs in genome coordinates

@@ -1,4 +1,4 @@
-// K1 -- FracMinHash sketching kernel (seeds k=15 c=125, markers k=21 c=1000).
+// K1 -- FracMinHash sketching kernel (seeds k=15 c=125, markers k=21 c=m: 1000 unless skb_set_marker_compression).
 //
 // Stands in for skani's sketching pass, reached from skDER at src/skDER/skder.py:16 (triangle),
 // :58 (dist), :103 (sketch) and :119 (search).  Bit-exact against oracle/skani_oracle.c
@@ -33,6 +33,7 @@ struct SketchBatch {
     const uint32_t *tile_off;    // [n+1] CTA-tile prefix sum
     int32_t n;
     uint32_t first_gid;          // DB id of batch genome 0
+    uint64_t thr_marker;         // a canonical 21-mer is a marker iff its hash is below this (marker_threshold)
 };
 
 // reverse the order of the 21 two-bit groups held in the low 42 bits of x
@@ -137,7 +138,7 @@ sketch_kernel(SketchBatch b, uint32_t *__restrict__ warp_seed_cnt, uint32_t *__r
                 if (mm_hash64((uint64_t)cseed) < THR_SEED) sm16 |= 1u << u;
                 const uint64_t f = ((uint64_t)fhi << 32) | flo, r = ((uint64_t)rhi << 32) | rlo;
                 const uint64_t cm = f < r ? f : r;
-                if (mm_hash64(cm) < THR_MARKER) mm16 |= 1u << u;
+                if (mm_hash64(cm) < b.thr_marker) mm16 |= 1u << u;
             }
             seed_mask |= (uint64_t)sm16 << (16 * jb);
             marker_mask |= (uint64_t)mm16 << (16 * jb);

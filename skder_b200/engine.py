@@ -173,6 +173,18 @@ class Engine:
         finally:
             self._L.skb_free(ptr)
 
+    def set_marker_compression(self, m):
+        """skani's -m: genomes added from now on keep a canonical 21-mer as a marker iff its hash is below 2^64 // m
+        (default 1000; DESIGN.md section 3).  Markers only decide which pairs pass the prescreen.  The context must be
+        empty unless m is its current value; load() takes the database's m.  Survives clear()."""
+        self._ck(self._L.skb_set_marker_compression(self._h, int(m)), "skb_set_marker_compression")
+
+    @property
+    def marker_compression(self):
+        m = C.c_int64()
+        self._ck(self._L.skb_marker_compression(self._h, C.byref(m)), "skb_marker_compression")
+        return m.value
+
     def contig_stats(self, first, n):
         """(n_contigs [n] int32, nx [n, 3] int64: N90, N50, N10) over the kept contigs of genomes first .. first+n-1"""
         cnt, nx = np.zeros(n, np.int32), np.zeros((n, 3), np.int64)

@@ -70,7 +70,7 @@ def _allgather_sketches(eng, dist, torch, lap=lambda: None):
     n = v.n_genomes
     nctg = int(v.n_contigs)
     meta = {  # an empty context (a rank without queries in this batch) has null host tables
-        "n": n, "n_seeds": v.n_seeds, "n_mkeys": v.n_marker_keys,
+        "n": n, "n_seeds": v.n_seeds, "n_mkeys": v.n_marker_keys, "marker_c": eng.marker_compression,
         "seed_off": np.ctypeslib.as_array(v.host_seed_off, shape=(n + 1,)).copy() if n else np.zeros(1, np.uint64),
         "total_len": np.ctypeslib.as_array(v.host_total_len, shape=(n,)).copy() if n else np.zeros(0, np.uint64),
         "ctg_off": np.ctypeslib.as_array(v.host_ctg_off, shape=(n + 1,)).copy() if n else np.zeros(1, np.uint32),
@@ -96,6 +96,9 @@ def _allgather_sketches(eng, dist, torch, lap=lambda: None):
 def _import_gathered(eng, metas, gathered, keep_flags=False):
     """Append every rank's gathered sketches to `eng`, rank-major; returns the number of import (= add) calls made."""
     (seeds, s_stride), (mkeys, m_stride) = gathered
+    if metas and metas[0]["marker_c"] != eng.marker_compression:  # the sketch view does not carry it (skb_import_sketches)
+        raise ValueError("sketches made at marker compression %d cannot join a context at %d"
+                         % (metas[0]["marker_c"], eng.marker_compression))
     calls = 0
     for r, m in enumerate(metas):
         if m["n"] == 0:
@@ -125,13 +128,17 @@ def append_gathered_sketches(src, dst, dist, torch):
 
 def _exchange_meta(meta, dist, torch, device):
     """The per-rank host tables of replicate_sketches as two tensor all-gathers (sizes, then one padded int64 blob)
-    instead of pickled objects: no Python object serialisation in the per-step path."""
+    instead of pickled objects: no Python object serialisation in the per-step path.  Every rank must have sketched at
+    the same marker compression (the screen compares marker counts across genomes): ValueError on every rank if not."""
     world = dist.get_world_size()
     n, nctg = int(meta["n"]), len(meta["ctg_len"])
-    head = torch.tensor([n, int(meta["n_seeds"]), int(meta["n_mkeys"]), nctg], dtype=torch.int64, device=device)
-    heads = torch.zeros(world * 4, dtype=torch.int64, device=device)
+    mc = int(meta.get("marker_c", 1000))  # tables without it were sketched at skani's default
+    head = torch.tensor([n, int(meta["n_seeds"]), int(meta["n_mkeys"]), nctg, mc], dtype=torch.int64, device=device)
+    heads = torch.zeros(world * 5, dtype=torch.int64, device=device)
     dist.all_gather_into_tensor(heads, head)
-    heads = heads.cpu().numpy().reshape(world, 4)
+    heads = heads.cpu().numpy().reshape(world, 5)
+    if len(set(heads[:, 4].tolist())) > 1:
+        raise ValueError("ranks sketched at different marker compressions (-m): %s" % heads[:, 4].tolist())
     size = lambda h: (int(h[0]) + 1) + int(h[0]) + (int(h[0]) + 1) + int(h[3])
     mx = max(1, max(size(h) for h in heads))
     blob = np.zeros(mx, np.int64)
@@ -145,14 +152,14 @@ def _exchange_meta(meta, dist, torch, device):
     recv = recv.cpu().numpy().reshape(world, mx)
     out = []
     for r in range(world):
-        n_r, ns, nm, nc = (int(x) for x in heads[r])
+        n_r, ns, nm, nc, mc = (int(x) for x in heads[r])
         o = 0
         seed_off = recv[r, o:o + n_r + 1].view(np.uint64).copy(); o += n_r + 1
         total_len = recv[r, o:o + n_r].view(np.uint64).copy(); o += n_r
         ctg_off = recv[r, o:o + n_r + 1].astype(np.uint32); o += n_r + 1
         ctg_len = recv[r, o:o + nc].astype(np.uint32)
-        out.append({"n": n_r, "n_seeds": ns, "n_mkeys": nm, "seed_off": seed_off, "total_len": total_len, "ctg_off": ctg_off,
-                    "ctg_len": ctg_len})
+        out.append({"n": n_r, "n_seeds": ns, "n_mkeys": nm, "marker_c": mc, "seed_off": seed_off, "total_len": total_len,
+                    "ctg_off": ctg_off, "ctg_len": ctg_len})
     return out
 
 
