@@ -153,6 +153,14 @@ int skb_triangle(skb_ctx *ctx, double screen_pct, double min_af_pct, int32_t par
 int skb_rect(skb_ctx *ctx, const int32_t *refs, int32_t n_refs, const int32_t *queries, int32_t n_queries,
              double screen_pct, double min_af_pct, skb_edge **edges, int64_t *n_edges, skb_stats *stats);
 
+/* skani's -n on dist / search (DESIGN.md section 3): every later skb_rect keeps, for each query genome, only its first n
+ * edges in row order -- ANI descending (the unrounded double), ties to the lower reference id -- after the screen,
+ * --min-af and the active estimator.  The kept edges stay in skb_rect's (a, b) order, and skb_device_edges,
+ * skb_last_edge_ci, skb_last_edge_detail and skb_greedy_summary(edges = NULL) see only them.  n = 0 (the default): all
+ * edges.  Context state, kept across skb_clear.  skb_triangle and skb_pairs_edges are unaffected: skani's triangle has
+ * no -n.  n < 0: SKB_EINVAL. */
+int skb_set_max_results(skb_ctx *ctx, int64_t n);
+
 /* How a pair's accepted chains become one ANI (skani's default, --median, --robust; DESIGN.md section 3).  Context
  * state, kept across skb_clear: applies to every later skb_triangle, skb_rect, skb_pairs_edges and skb_pairs_detail
  * call.  AF, chain, anchor and seed counts are the same in every mode.  Any other value: SKB_EINVAL. */

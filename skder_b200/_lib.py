@@ -109,7 +109,7 @@ SYMBOLS = [
     "skb_free", "skb_launch_count", "skb_stream", "skb_clear", "skb_timer_start", "skb_timer_stop", "skb_index_append", "skb_pop_last_add",
     "skb_device_edges", "skb_set_owned", "skb_screen_triangle", "skb_pairs_edges", "skb_greedy_summary", "skb_index_seed_tables", "skb_clear_keep_tables",
     "skb_set_ani_estimator", "skb_set_ani_ci", "skb_last_edge_ci", "skb_set_detailed", "skb_last_edge_detail",
-    "skb_genome_contig_stats", "skb_set_marker_compression", "skb_marker_compression",
+    "skb_genome_contig_stats", "skb_set_marker_compression", "skb_marker_compression", "skb_set_max_results",
 ]
 
 _lib = None
@@ -178,6 +178,7 @@ def lib():
     L.skb_last_edge_detail.argtypes = [C.c_void_p, C.POINTER(C.POINTER(EdgeDetail)), C.POINTER(C.c_int64)]
     L.skb_set_marker_compression.argtypes = [C.c_void_p, C.c_int64]
     L.skb_marker_compression.argtypes = [C.c_void_p, C.POINTER(C.c_int64)]
+    L.skb_set_max_results.argtypes = [C.c_void_p, C.c_int64]
     L.skb_genome_contig_stats.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.POINTER(C.c_int32), C.POINTER(C.c_int64)]
     L.skb_last_edge_ci.argtypes = [C.c_void_p, C.POINTER(C.POINTER(C.c_double)), C.POINTER(C.c_int64)]
     L.skb_index_seed_tables.argtypes = [C.c_void_p]

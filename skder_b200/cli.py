@@ -9,6 +9,11 @@ without touching skDER.  Sub-commands and flags are exactly the ones skDER spell
   skani search   QUERY.fa -d DBDIR -o OUT -t T                   (skder.py:119)
   skani dist     --rl REFS --ql QUERIES [-s S] [-t T] -o OUT     (skder.py:58-59, cidder.py:362-363)
 
+`search` also takes several query FASTAs, as positionals and/or a list file `--ql` (positionals first, then the list in
+file order, a repeated path once at its first position), answered in one device pass; rows are grouped by query in that
+order.  `-n N` (dist, search) keeps each query's first N rows -- its N best hits by unrounded ANI, ties to the reference
+listed first; `-n 1` asks for each query's best hit (DESIGN.md section 3).
+
 skDER hands its `-p` string to skani verbatim, so four ANI flags are accepted on triangle, dist and search
 (DESIGN.md section 3): the estimators `--median` (median chain identity) and `--robust` (mean after trimming the
 10 % / 90 % tails); `--ci`, which appends a bootstrap interval of the mean ANI as two columns, ANI_5_percentile and
@@ -56,7 +61,7 @@ def parse_args(argv):
     opt = {"screen": DEFAULT_SCREEN, "min_af": DEFAULT_MIN_AF, "threads": 3, "edge_list": False, "positional": []}
     valued = {
         "-l": "list", "-o": "out", "-t": "threads", "-s": "screen", "--min-af": "min_af", "--rl": "rl", "--ql": "ql",
-        "-d": "db", "-m": "marker_c",
+        "-d": "db", "-m": "marker_c", "-n": "max_results",
     }
     flags = {"-E": "edge_list", "--sparse": "edge_list", "--ci": "ci", "--detailed": "detailed"}
     opt["ci"] = opt["detailed"] = False
@@ -99,6 +104,15 @@ def parse_args(argv):
         opt["marker_c"] = int(m)
     else:
         opt["marker_c"] = DEFAULT_MARKER_C
+    if "max_results" in opt:
+        if sub not in ("search", "dist"):
+            raise UsageError("skani %s takes no -n: it is the number of results per query of dist and search" % sub)
+        n = opt["max_results"]
+        if not re.fullmatch(r"[0-9]+", n) or not 1 <= int(n) < 2 ** 63:
+            raise UsageError("-n needs an integer of at least 1, not %r" % n)
+        opt["max_results"] = int(n)
+    else:
+        opt["max_results"] = 0  # every row
     if len(set(chosen)) > 1:
         raise UsageError("--median and --robust are mutually exclusive")
     if chosen and sub == "sketch":
@@ -118,7 +132,7 @@ def parse_args(argv):
             raise UsageError("skani %s: missing required option for %r" % (sub, k))
     if sub == "triangle" and not opt["edge_list"]:
         raise UsageError("skani triangle without -E (matrix output) is not implemented; skDER always passes -E")
-    if sub == "search" and len(opt["positional"]) < 1:
+    if sub == "search" and not opt["positional"] and "ql" not in opt:
         raise UsageError("skani search: no query FASTA given")
     if sub != "search" and opt["positional"]:
         raise UsageError("unexpected positional arguments: %r" % opt["positional"])
@@ -128,6 +142,15 @@ def parse_args(argv):
 def read_list(path):
     with open(path) as f:
         return [ln.strip() for ln in f if ln.strip()]
+
+
+def search_queries(opt):
+    """search's query FASTAs as given: the positionals, then the --ql list's entries, each path once at its first
+    position"""
+    qs = list(dict.fromkeys(opt["positional"] + (read_list(opt["ql"]) if "ql" in opt else [])))
+    if not qs:
+        raise UsageError("skani search: no query FASTA given")
+    return qs
 
 
 def header(ci, detailed=False):
@@ -267,11 +290,12 @@ def run_sketch(opt, engine_mod):
 
 
 def run_search(opt, engine_mod):
-    """`skani search q.fa -d DB -o OUT` (reference src/skDER/skder.py:119).  Served by the database's resident
-    daemon (skder_b200/daemon.py; started here on first use) unless SKB_NO_DAEMON=1, in which case the database is
-    loaded, indexed and searched in this process."""
+    """`skani search q.fa [q2.fa ...] [--ql LIST] -d DB -o OUT` (reference src/skDER/skder.py:119).  Served by the
+    database's resident daemon (skder_b200/daemon.py; started here on first use) unless SKB_NO_DAEMON=1, in which case
+    the database is loaded, indexed and searched in this process.  All queries go through one Engine.search."""
+    labels = search_queries(opt)  # each query's rows show its path as it was given
     # the server runs in another working directory: every path goes over absolute
-    query, db, out = os.path.abspath(opt["positional"][0]), os.path.abspath(opt["db"]), os.path.abspath(opt["out"])
+    db, out = os.path.abspath(opt["db"]), os.path.abspath(opt["out"])
     opt = dict(opt, db=db, out=out)
     dev = _device()
     if os.environ.get("SKB_NO_DAEMON") != "1":
@@ -279,9 +303,14 @@ def run_search(opt, engine_mod):
 
         from . import daemon
 
-        msg = {"op": "search", "query": query, "label": opt["positional"][0],  # the row shows the path as it was given
-               "screen": opt["screen"], "min_af": opt["min_af"], "estimator": opt["estimator"], "ci": opt["ci"],
-               "detailed": opt["detailed"], "out": out}
+        msg = {"op": "search", "screen": opt["screen"], "min_af": opt["min_af"], "estimator": opt["estimator"],
+               "ci": opt["ci"], "detailed": opt["detailed"], "out": out}
+        if len(labels) == 1:  # the single-query message every server version answers
+            msg.update(query=os.path.abspath(labels[0]), label=labels[0])
+        else:
+            msg.update(queries=[os.path.abspath(q) for q in labels], labels=labels)
+        if opt["max_results"]:
+            msg["max_results"] = opt["max_results"]
         rep = daemon.request(db, dev, msg)
         if rep is not None and rep.get("stale"):  # the directory was rewritten under a running server: it has just exited
             deadline = time.time() + 15.0
@@ -305,7 +334,6 @@ def run_search(opt, engine_mod):
         return None
     if engine_mod is None:
         from . import engine as engine_mod
-    query = opt["positional"][0]
     with open(os.path.join(opt["db"], "manifest.json")) as f:
         man = json.load(f)
     paths, names = list(man["paths"]), list(man["names"])
@@ -313,18 +341,19 @@ def run_search(opt, engine_mod):
         eng.set_estimator(opt["estimator"])
         eng.set_ci(opt["ci"])
         eng.set_detailed(opt["detailed"])
+        eng.set_max_results(opt["max_results"])
         eng.load(opt["db"])
         eng.index()
-        qp = engine_mod.pack_fasta(query, eng.params.min_contig_len)
+        qp = engine_mod.pack_fasta_many(labels, opt["threads"], eng.params.min_contig_len)
         edges, st = eng.search(qp, screen=opt["screen"], min_af=opt["min_af"])
         ci, detail = edge_extras(eng, opt["ci"], opt["detailed"], edges, search_contig_stats(eng) if opt["detailed"] else None)
     write_atomic(opt["out"], header(opt["ci"], opt["detailed"]) +
-                 "".join(rect_rows(paths + [query], names + [qp.first_name], edges, ci, detail)))
+                 "".join(rect_rows(paths + labels, names + [p.first_name for p in qp], edges, ci, detail)))
     return st
 
 
 def search_contig_stats(eng, db_stats=None):
-    """contig statistics of the database genomes (db_stats, or read from the context) and, last, of the query the
+    """contig statistics of the database genomes (db_stats, or read from the context) and, last, of the queries the
     previous Engine.search saw: indexed like the ids of that search's edges"""
     import numpy as np
 
@@ -342,6 +371,7 @@ def run_dist(opt, engine_mod):
         eng.set_ci(opt["ci"])
         eng.set_detailed(opt["detailed"])
         eng.set_marker_compression(opt["marker_c"])
+        eng.set_max_results(opt["max_results"])
         names = stream_add(eng, engine_mod, paths, opt["threads"])
         eng.index()
         edges, st = eng.rect([idx[p] for p in dict.fromkeys(refs)], [idx[p] for p in dict.fromkeys(queries)],
@@ -369,6 +399,9 @@ def _provenance(opt, sub, seconds):
     if opt.get("marker_c", DEFAULT_MARKER_C) != DEFAULT_MARKER_C:
         text += ("-m %d: markers are the canonical 21-mers whose hash is below 2^64 / %d (skani's default is 1000); they "
                  "decide only which pairs pass the prescreen, not a pair's ANI/AF\n" % (opt["marker_c"], opt["marker_c"]))
+    if opt.get("max_results"):
+        text += ("-n %d: each query keeps its first %d rows, by unrounded ANI descending, ties to the lower reference "
+                 "id (DESIGN.md section 3); unpinned against skani's own -n\n" % (opt["max_results"], opt["max_results"]))
     if opt.get("detailed"):
         text += ("--detailed: the 13 extra columns as DESIGN.md section 3 defines them; their names, order and definitions "
                  "are recalled, unpinned against skani's own --detailed output\n")

@@ -16,6 +16,7 @@
 #include <vector>
 
 #include "skb_ani.cuh"
+#include "skb_best_n.cuh"
 #include "skb_common.cuh"
 #include "skb_index.cuh"
 #include "skb_sketch.cuh"
@@ -104,6 +105,7 @@ struct skb_ctx {
     bool ci = false;                   // skb_set_ani_ci; kept across skb_clear
     bool detailed = false;             // skb_set_detailed; kept across skb_clear
     uint64_t marker_c = C_MARKER;      // skb_set_marker_compression / skb_db_load; kept across skb_clear
+    int64_t max_results = 0;           // skb_set_max_results (skb_rect's -n; 0: all); kept across skb_clear
     const skb_edge *last_dev_edges = nullptr;  // device copy of the last triangle/rect result (skb_device_edges)
     int64_t last_n_edges = 0;
     bool last_ci = false;                 // that call ran with --ci ...
@@ -115,7 +117,8 @@ struct skb_ctx {
     float last_ms_anchor = 0;
     int last_anchor_launches = 0;
     cudaEvent_t t0 = nullptr, t1 = nullptr;
-    cudaEvent_t call_ev[3] = {};  // start, pairs ready, edges ready of one screen or edge call (call_events)
+    cudaEvent_t call_ev[5] = {};  // start, pairs ready, edges ready of one screen or edge call, and around its -n stage
+                                  // (call_events)
 
     // ---- sketch DB (host metadata; the seeds and raw marker keys themselves are d_seeds, d_mkeys)
     struct SketchDb {
@@ -311,11 +314,13 @@ void sort_keys_u64(skb_ctx *c, const uint64_t *in, uint64_t *out, size_t n, int 
     });
 }
 
-// radix sort of (key, value) pairs on all 64 key bits, counted as sort_keys_u64 counts a 64-bit sort
-void sort_pairs_u64(skb_ctx *c, unsigned long long *keys_in, unsigned long long *keys_out, uint32_t *vals_in,
-                    uint32_t *vals_out, size_t n) {
-    cub_run(c, 9, [&](void *tmp, size_t &bytes) {
-        return cub::DeviceRadixSort::SortPairs(tmp, bytes, keys_in, keys_out, vals_in, vals_out, (int64_t)n, 0, 64, c->st);
+// stable radix sort of (key, value) pairs on key bits [0, end_bit), counted as sort_keys_u64 counts its sort
+template <typename K>
+void sort_pairs(skb_ctx *c, K *keys_in, K *keys_out, uint32_t *vals_in, uint32_t *vals_out, size_t n,
+                int end_bit = 8 * sizeof(K)) {
+    cub_run(c, (end_bit + 7) / 8 + 1, [&](void *tmp, size_t &bytes) {
+        return cub::DeviceRadixSort::SortPairs(tmp, bytes, keys_in, keys_out, vals_in, vals_out, (int64_t)n, 0, end_bit,
+                                               c->st);
     });
 }
 
@@ -482,7 +487,7 @@ void run_ani(skb_ctx *c, const unsigned long long *d_pairs, int64_t n_pairs, Pai
     d_info_s.reserve((size_t)n_pairs, 0, c->st);
     launch(c, pair_setup_kernel, nblk((uint64_t)n_pairs, 256), 256, 0, view, d_pairs, n_pairs, c->d_info.p, d_key.p,
            d_idx.p);
-    sort_pairs_u64(c, d_key.p, d_key2.p, d_idx.p, d_perm.p, (size_t)n_pairs);
+    sort_pairs(c, d_key.p, d_key2.p, d_idx.p, d_perm.p, (size_t)n_pairs);
     launch(c, pair_gather_kernel, nblk((uint64_t)n_pairs, 256), 256, 0, c->d_info.p, d_perm.p, n_pairs, d_info_s.p,
            c->d_nch.p);
     // global task offsets (exclusive scan of the chunk counts in processing order)
@@ -781,6 +786,52 @@ void pairs_to_edges(skb_ctx *c, unsigned long long *d_pairs, int64_t n_pairs, do
     c->last_n_edges = (int64_t)h3[0];
 }
 
+// skani's -n (skb_set_max_results): cut the last edge call's list, and its --ci / --detailed records, to each query's
+// first max_n edges in row order (query, ANI descending, reference ascending); skb_best_n.cuh.  The kept edges keep
+// their (a, b) order.
+void best_n_edges(skb_ctx *c, int64_t max_n) {
+    const int64_t n = c->last_n_edges;
+    PoolRef<unsigned long long> d_key(c->pool["best_n.key"]), d_key_s(c->pool["best_n.key_sorted"]);
+    PoolRef<uint32_t> d_idx(c->pool["best_n.idx"]), d_idx_a(c->pool["best_n.idx_ani"]), d_idx_q(c->pool["best_n.idx_row"]);
+    PoolRef<uint32_t> d_q(c->pool["best_n.query"]), d_q_s(c->pool["best_n.query_sorted"]);
+    PoolRef<uint32_t> d_f(c->pool["best_n.flag"]), d_p(c->pool["best_n.pos"]);
+    for (auto *b : {&d_idx, &d_idx_a, &d_idx_q, &d_q, &d_q_s}) b->reserve((size_t)n, 0, c->st);
+    d_key.reserve((size_t)n, 0, c->st);
+    d_key_s.reserve((size_t)n, 0, c->st);
+    d_f.reserve((size_t)n + 1, 0, c->st);
+    d_p.reserve((size_t)n + 1, 0, c->st);
+    const unsigned nb = nblk((uint64_t)n, 256);
+    launch(c, best_n_key_kernel, nb, 256, 0, c->last_dev_edges, n, d_key.p, d_idx.p);
+    sort_pairs(c, d_key.p, d_key_s.p, d_idx.p, d_idx_a.p, (size_t)n);
+    launch(c, best_n_query_kernel, nb, 256, 0, c->last_dev_edges, d_idx_a.p, n, d_q.p);
+    int q_bits = 1;  // query ids are genome ids < n()
+    while (q_bits < 32 && (1ll << q_bits) < (int64_t)c->n()) q_bits++;
+    sort_pairs(c, d_q.p, d_q_s.p, d_idx_a.p, d_idx_q.p, (size_t)n, q_bits);
+    launch(c, best_n_flag_kernel, nb, 256, 0, d_q_s.p, d_idx_q.p, n, max_n, d_f.p);
+    CK(cudaMemsetAsync(d_f.p + n, 0, 4, c->st));
+    exclusive_scan_u32(c, d_f.p, d_p.p, (size_t)n + 1);
+    PoolRef<skb_edge> kept(c->pool["best_n.edges"]);
+    kept.reserve((size_t)n, 0, c->st);
+    launch(c, best_n_scatter_kernel<skb_edge>, nb, 256, 0, c->last_dev_edges, n, d_f.p, d_p.p, kept.p);
+    c->last_dev_edges = kept.p;
+    if (c->last_dev_ci) {
+        PoolRef<double2> kept_ci(c->pool["best_n.ci"]);
+        kept_ci.reserve((size_t)n, 0, c->st);
+        launch(c, best_n_scatter_kernel<double2>, nb, 256, 0, c->last_dev_ci, n, d_f.p, d_p.p, kept_ci.p);
+        c->last_dev_ci = kept_ci.p;
+    }
+    if (c->last_dev_detail) {
+        PoolRef<skb_edge_detail> kept_det(c->pool["best_n.detail"]);
+        kept_det.reserve((size_t)n, 0, c->st);
+        launch(c, best_n_scatter_kernel<skb_edge_detail>, nb, 256, 0, c->last_dev_detail, n, d_f.p, d_p.p, kept_det.p);
+        c->last_dev_detail = kept_det.p;
+    }
+    uint32_t n_kept = 0;
+    CK(cudaMemcpyAsync(&n_kept, d_p.p + n, 4, cudaMemcpyDeviceToHost, c->st));
+    CK(cudaStreamSynchronize(c->st));
+    c->last_n_edges = n_kept;
+}
+
 // The context's events around the stages of one screen or edge call: start, pairs ready, edges ready
 cudaEvent_t *call_events(skb_ctx *c) {
     for (cudaEvent_t &e : c->call_ev)
@@ -795,10 +846,12 @@ struct EdgePairs {
 };
 
 // skb_triangle, skb_pairs_edges and skb_rect after their argument checks: `pairs(EdgePairs &)` checks the context's state
-// and leaves the pairs to evaluate (ms_screen), pairs_to_edges evaluates them (ms_ani), and the edges go to the caller --
-// a malloc'ed host copy when `edges` is given, the device copy in any case (skb_device_edges)
+// and leaves the pairs to evaluate (ms_screen), pairs_to_edges evaluates them (ms_ani), max_n > 0 cuts them to each
+// query's best max_n (best_n_edges; its time counts in ms_total only), and the edges go to the caller -- a malloc'ed host
+// copy when `edges` is given, the device copy in any case (skb_device_edges)
 template <typename F>
-int edge_call(skb_ctx *c, double min_af_pct, skb_edge **edges, int64_t *n_edges, skb_stats *stats, F &&pairs) {
+int edge_call(skb_ctx *c, double min_af_pct, skb_edge **edges, int64_t *n_edges, skb_stats *stats, F &&pairs,
+              int64_t max_n = 0) {
     // --ci is defined for the mean estimator only (DESIGN.md section 3)
     if (c->ci && c->estimator != SKB_ANI_MEAN)
         return fail(c, SKB_EINVAL,
@@ -815,9 +868,16 @@ int edge_call(skb_ctx *c, double min_af_pct, skb_edge **edges, int64_t *n_edges,
     if (rc != SKB_OK) return rc;
     unsigned long long sums[2];
     pairs_to_edges(c, p.d_pairs, p.n, min_af_pct, sums, ev[1], ev[2]);
-    float ms_screen = 0, ms_ani = 0;
+    float ms_screen = 0, ms_ani = 0, ms_best_n = 0;
     CK(cudaEventElapsedTime(&ms_screen, ev[0], ev[1]));
     CK(cudaEventElapsedTime(&ms_ani, ev[1], ev[2]));
+    if (max_n > 0 && c->last_n_edges > max_n) {  // fewer edges than max_n: no query has more
+        CK(cudaEventRecord(ev[3], c->st));
+        best_n_edges(c, max_n);
+        CK(cudaEventRecord(ev[4], c->st));
+        CK(cudaEventSynchronize(ev[4]));
+        CK(cudaEventElapsedTime(&ms_best_n, ev[3], ev[4]));
+    }
     const int64_t ne = c->last_n_edges;
     // rect lists are sorted by (ref, query) on the device already; nothing to do on the host
     if (edges) {
@@ -838,7 +898,7 @@ int edge_call(skb_ctx *c, double min_af_pct, skb_edge **edges, int64_t *n_edges,
         stats->n_edges = ne;
         stats->ms_screen = ms_screen;
         stats->ms_ani = ms_ani;
-        stats->ms_total = ms_screen + ms_ani;
+        stats->ms_total = ms_screen + ms_ani + ms_best_n;
         stats->ms_anchor = c->last_ms_anchor;
         stats->n_anchor_launches = c->last_anchor_launches;
         stats->launches = c->launches - launches0;
@@ -1639,9 +1699,10 @@ int skb_rect(skb_ctx *ctx, const int32_t *refs, int32_t n_refs, const int32_t *q
     return guarded(ctx, [&]() -> int {
         if (!edges || !n_edges || n_refs < 0 || n_queries < 0 || (n_refs && !refs) || (n_queries && !queries))
             return fail(ctx, SKB_EINVAL, "bad arguments");
-        return edge_call(ctx, min_af_pct, edges, n_edges, stats, [&](EdgePairs &p) {
-            return screen_rect_impl(ctx, refs, n_refs, queries, n_queries, screen_pct, p);
-        });
+        return edge_call(
+            ctx, min_af_pct, edges, n_edges, stats,
+            [&](EdgePairs &p) { return screen_rect_impl(ctx, refs, n_refs, queries, n_queries, screen_pct, p); },
+            ctx->max_results);
     });
 }
 
@@ -1677,6 +1738,14 @@ int skb_last_edge_ci(skb_ctx *ctx, double **lo_hi, int64_t *n) {
 int skb_set_detailed(skb_ctx *ctx, int32_t enabled) {
     return guarded(ctx, [&]() -> int {
         ctx->detailed = enabled != 0;
+        return SKB_OK;
+    });
+}
+
+int skb_set_max_results(skb_ctx *ctx, int64_t n) {
+    return guarded(ctx, [&]() -> int {
+        if (n < 0) return fail(ctx, SKB_EINVAL, "the number of results per query must be at least 0 (0: all)");
+        ctx->max_results = n;
         return SKB_OK;
     });
 }

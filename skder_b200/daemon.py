@@ -5,7 +5,9 @@ skDER's low_mem_greedy mode launches one `skani search <genome> -d <db>` process
 CUDA context, read the database from disk, upload it and build its index.  The first `search` against a
 database starts this server (one per database directory, per GPU); it keeps the indexed database in HBM
 and answers each later search with one sketch + one rectangle (Engine.search), then exits after
-SKB_DAEMON_IDLE seconds without requests.
+SKB_DAEMON_IDLE seconds without requests.  A request names its query FASTAs as "queries" (absolute paths) and
+"labels" (the paths its rows show), or a single one as "query" and "label"; every query of a request is answered in
+one device pass.  "max_results" is skani's -n (0 or absent: every row).
 
 Trust and staleness:
 * The Unix socket lives in a directory only the user can enter (mode 0700, ownership checked: $XDG_RUNTIME_DIR
@@ -107,6 +109,18 @@ def stop_for(db_dir, wait=15.0):
             pass
 
 
+def search_queries(msg):
+    """(query paths, row labels) of a search request: its "queries" / "labels" lists, or its single "query" / "label"
+    (the label defaults to the path)"""
+    if "queries" in msg:
+        queries, labels = list(msg["queries"]), list(msg.get("labels", msg["queries"]))
+    else:
+        queries, labels = [msg["query"]], [msg.get("label", msg["query"])]
+    if not queries or len(labels) != len(queries):
+        raise ValueError("a search request needs at least one query and one label per query")
+    return queries, labels
+
+
 def serve(db_dir, device):
     from . import cli, engine
 
@@ -162,13 +176,15 @@ def serve(db_dir, device):
                         ci, detailed = bool(msg.get("ci", False)), bool(msg.get("detailed", False))
                         eng.set_ci(ci)
                         eng.set_detailed(detailed)
-                        packed = engine.pack_fasta(msg["query"], eng.params.min_contig_len)
+                        eng.set_max_results(int(msg.get("max_results", 0)))
+                        queries, labels = search_queries(msg)
+                        packed = engine.pack_fasta_many(queries, None, eng.params.min_contig_len)
                         edges, st = eng.search(packed, screen=msg["screen"], min_af=msg["min_af"])
                         stats = None
                         if detailed:
                             db_stats = db_stats or eng.contig_stats(0, n_db)  # the database's, once per server
                             stats = cli.search_contig_stats(eng, db_stats)
-                        rows = cli.rect_rows(paths + [msg.get("label", msg["query"])], names + [packed.first_name], edges,
+                        rows = cli.rect_rows(paths + labels, names + [p.first_name for p in packed], edges,
                                              *cli.edge_extras(eng, ci, detailed, edges, stats))
                         cli.write_atomic(msg["out"], cli.header(ci, detailed) + "".join(rows))
                         conn.send_bytes(json.dumps({"ok": True, "rows": len(rows), "ms": st.ms_total}).encode())

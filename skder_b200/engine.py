@@ -109,7 +109,7 @@ class Engine:
             raise SkbError("skb_create failed (%d): %s" % (rc, self._L.skb_last_error(None).decode()))
         self.device = int(device)
         self.detailed = False  # set_detailed
-        self.last_query_contig_stats = None  # contig_stats of the last search's query, with set_detailed(True)
+        self.last_query_contig_stats = None  # contig_stats of the last search's queries, with set_detailed(True)
 
     def close(self):
         if getattr(self, "_h", None):
@@ -179,6 +179,12 @@ class Engine:
         empty unless m is its current value; load() takes the database's m.  Survives clear()."""
         self._ck(self._L.skb_set_marker_compression(self._h, int(m)), "skb_set_marker_compression")
 
+    def set_max_results(self, n):
+        """skani's -n: later rect / search calls keep each query's first n edges in row order (ANI descending, ties to
+        the lower reference id), with their last_edge_ci / last_edge_detail records; 0 (the default): all.  triangle and
+        pairs_edges are unaffected.  DESIGN.md section 3.  Survives clear()."""
+        self._ck(self._L.skb_set_max_results(self._h, int(n)), "skb_set_max_results")
+
     @property
     def marker_compression(self):
         m = C.c_int64()
@@ -232,16 +238,19 @@ class Engine:
         self._ck(self._L.skb_pop_last_add(self._h), "skb_pop_last_add")
 
     def search(self, query_packed, screen=80.0, min_af=15.0):
-        """`skani search`: one query genome against the resident, indexed database (ids 0..n-1).  The query
-        is sketched, indexed query-only, compared, and removed again.  Edges: a = database genome, b = query.
-        With set_detailed(True) the query's contig_stats are kept in last_query_contig_stats."""
+        """`skani search`: query genomes (one PackedGenome, or a list of them) against the resident, indexed database
+        (ids 0..n-1), in one device pass.  The queries are sketched, indexed query-only, compared, and removed again.
+        Edges: a = database genome, b = query (ids n, n+1, ... in list order).  With set_detailed(True) the queries'
+        contig_stats are kept in last_query_contig_stats, in list order."""
+        queries = list(query_packed) if isinstance(query_packed, (list, tuple)) else [query_packed]
         n_db = self.n_genomes
-        self.add([query_packed])
+        self.add(queries)
         try:
-            if self.detailed:  # contig_stats of the query: it leaves the context below
-                self.last_query_contig_stats = self.contig_stats(n_db, 1)
+            if self.detailed:  # contig_stats of the queries: they leave the context below
+                self.last_query_contig_stats = self.contig_stats(n_db, len(queries))
             self.index_append()
-            return self.rect(np.arange(n_db, dtype=np.int32), [n_db], screen=screen, min_af=min_af)
+            return self.rect(np.arange(n_db, dtype=np.int32), np.arange(n_db, n_db + len(queries), dtype=np.int32),
+                             screen=screen, min_af=min_af)
         finally:
             self.pop_last_add()
 
