@@ -60,6 +60,7 @@ typedef struct {
     char *first_name;     /* header line of first kept record, without '>' */
     int64_t n50;          /* N50 over ALL records (reference src/skDER/util.py:686-724 n50_calc) */
     int64_t total_bases_all; /* over all records */
+    char **contig_names;  /* [n_contigs] header lines of the kept records, without '>' (skb_pack_contigs: NULL) */
 } skb_packed;
 int skb_pack_fasta(const char *path, int32_t min_contig_len, skb_packed **out);
 /* n files on n_threads host threads; out[i] is NULL where file i failed (return value = #failures) */
@@ -80,6 +81,12 @@ const char *skb_last_error(const skb_ctx *ctx); /* ctx may be NULL: last creatio
 /* Upload n packed genomes (host pointers, pinned or pageable), sketch them on the device and
  * append them to the context's sketch DB.  Genome ids are assigned in call order. */
 int skb_add_genomes(skb_ctx *ctx, int32_t n, const skb_packed *const *genomes);
+/* skani's per-sequence mode (-i, --qi, --ri; DESIGN.md section 3): every kept contig of every one of the n_files packed
+ * files becomes a genome of its own with one contig, ids in (file, record) order -- its sketch is exactly the one the
+ * record gets as a one-contig genome of skb_add_genomes.  Uploads and batches as skb_add_genomes; one skb_pop_last_add
+ * undoes the whole call.  SKB_ELIMIT: more genomes than 22-bit ids, a record too large for 31-bit padded coordinates,
+ * or a file of 2^32 bases or more. */
+int skb_add_sequences(skb_ctx *ctx, int32_t n_files, const skb_packed *const *files);
 /* Build the search structures (inverted marker index, per-genome seed hash indices, chunk tables)
  * over every genome added so far.  Must be called before triangle/rect; may be called again after
  * more genomes were added. */
@@ -89,7 +96,7 @@ int skb_index(skb_ctx *ctx);
  * not references and not part of a triangle.  With skb_pop_last_add this is `skani search` (skder.py:119)
  * against a resident database: one query genome comes and goes at the cost of its own sketch. */
 int skb_index_append(skb_ctx *ctx);
-/* Undo the most recent skb_add_genomes call (only genomes that are not in the inverted index). */
+/* Undo the most recent skb_add_genomes / skb_add_sequences call (only genomes that are not in the inverted index). */
 int skb_pop_last_add(skb_ctx *ctx);
 int32_t skb_n_genomes(const skb_ctx *ctx);
 /* drop every genome and index but keep the device allocations (repeated runs on one context) */

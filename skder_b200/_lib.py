@@ -40,6 +40,7 @@ class Packed(C.Structure):
         ("first_name", C.c_char_p),
         ("n50", C.c_int64),
         ("total_bases_all", C.c_int64),
+        ("contig_names", C.POINTER(C.c_char_p)),
     ]
 
 
@@ -110,6 +111,7 @@ SYMBOLS = [
     "skb_device_edges", "skb_set_owned", "skb_screen_triangle", "skb_pairs_edges", "skb_greedy_summary", "skb_index_seed_tables", "skb_clear_keep_tables",
     "skb_set_ani_estimator", "skb_set_ani_ci", "skb_last_edge_ci", "skb_set_detailed", "skb_last_edge_detail",
     "skb_genome_contig_stats", "skb_set_marker_compression", "skb_marker_compression", "skb_set_max_results",
+    "skb_add_sequences",
 ]
 
 _lib = None
@@ -139,6 +141,7 @@ def lib():
     L.skb_last_error.argtypes = [C.c_void_p]
     L.skb_last_error.restype = C.c_char_p
     L.skb_add_genomes.argtypes = [C.c_void_p, C.c_int32, PP]
+    L.skb_add_sequences.argtypes = [C.c_void_p, C.c_int32, PP]
     L.skb_index.argtypes = [C.c_void_p]
     L.skb_n_genomes.argtypes = [C.c_void_p]
     L.skb_n_genomes.restype = C.c_int32

@@ -25,6 +25,9 @@ so a `-p` with --ci or --detailed breaks it as it would with skani; greedy and d
 2^64 / M (default 1000).  Markers only decide which pairs the prescreen passes, so a smaller M (skani suggests
 ~200-300 for plasmids and viruses) lets small genomes that share no marker at 1000 be compared; a pair's ANI/AF does
 not depend on it.  A database records its M, and `search` sketches the query at that M, so search takes no -m.
+skani's per-sequence mode -- `-i` (triangle, sketch), `--qi` (dist, search), `--ri` (dist) -- makes every record of at
+least 500 bp of the flagged files a genome of its own, named by its file and header (DESIGN.md section 3); skDER keys
+its selection on whole files, so a `-p` with -i breaks it.
 Any other skani option (-c, --fast, --slow, --medium, --small-genomes, --no-learned-ani, ...) changes skani's
 estimator in ways this engine does not implement: the shim then exits non-zero WITHOUT creating the output, which is
 the one failure signal runCmd checks (util.py:642-645).
@@ -63,8 +66,9 @@ def parse_args(argv):
         "-l": "list", "-o": "out", "-t": "threads", "-s": "screen", "--min-af": "min_af", "--rl": "rl", "--ql": "ql",
         "-d": "db", "-m": "marker_c", "-n": "max_results",
     }
-    flags = {"-E": "edge_list", "--sparse": "edge_list", "--ci": "ci", "--detailed": "detailed"}
-    opt["ci"] = opt["detailed"] = False
+    flags = {"-E": "edge_list", "--sparse": "edge_list", "--ci": "ci", "--detailed": "detailed", "-i": "per_seq",
+             "--qi": "query_per_seq", "--ri": "ref_per_seq"}
+    opt["ci"] = opt["detailed"] = opt["per_seq"] = opt["query_per_seq"] = opt["ref_per_seq"] = False
     estimators = {"--median": "median", "--robust": "robust"}
     chosen = []
     i = 1
@@ -126,6 +130,10 @@ def parse_args(argv):
         raise UsageError("skani sketch takes no --detailed")
     if opt["detailed"] and chosen:
         raise UsageError("--detailed is defined for the default (mean) ANI only, not with %s" % chosen[0])
+    for flag, key, subs in (("-i", "per_seq", ("triangle", "sketch")), ("--qi", "query_per_seq", ("dist", "search")),
+                            ("--ri", "ref_per_seq", ("dist",))):
+        if opt[key] and sub not in subs:
+            raise UsageError("skani %s takes no %s (per-sequence mode: %s)" % (sub, flag, ", ".join(subs)))
     need = {"triangle": ["list", "out"], "sketch": ["list", "out"], "search": ["db", "out"], "dist": ["rl", "ql", "out"]}[sub]
     for k in need:
         if k not in opt:
@@ -221,13 +229,15 @@ def _device():
 INGEST_BATCH = 256  # genomes packed per host batch: batch k+1 is parsed while batch k uploads and is sketched
 
 
-def stream_add(eng, engine_mod, paths, threads, phases=None):
+def stream_add(eng, engine_mod, paths, threads, phases=None, per_sequence=False):
     """FASTA files -> sketches on the device, streamed: host threads parse and 2-bit pack batch k+1
     (skb_pack_fasta_many) while the device uploads and sketches batch k (skb_add_genomes), so at most two batches of
-    packed genomes are resident on the host and the ingest hides behind the upload.  Returns the first-record names."""
+    packed genomes are resident on the host and the ingest hides behind the upload.  Returns the first-record names.
+    per_sequence (-i, --qi, --ri): every kept record is a genome (skb_add_sequences); returns the (file path, record
+    name) lists of the genomes added, in id order."""
     from concurrent.futures import ThreadPoolExecutor
 
-    names, t_wait, t_add = [], 0.0, 0.0
+    names, gpaths, t_wait, t_add = [], [], 0.0, 0.0
     mcl = eng.params.min_contig_len
     with ThreadPoolExecutor(1) as ex:
         fut = ex.submit(engine_mod.pack_fasta_many, paths[:INGEST_BATCH], threads, mcl) if paths else None
@@ -237,15 +247,20 @@ def stream_add(eng, engine_mod, paths, threads, phases=None):
             nxt = paths[i + INGEST_BATCH:i + 2 * INGEST_BATCH]
             fut = ex.submit(engine_mod.pack_fasta_many, nxt, threads, mcl) if nxt else None
             t1 = time.time()
-            names += [p.first_name for p in packed]
-            eng.add(packed)
+            if per_sequence:
+                for p in packed:
+                    gpaths += [p.path] * p.n_contigs
+                    names += p.contig_names
+            else:
+                names += [p.first_name for p in packed]
+            eng.add(packed, per_sequence)
             del packed
             t_wait += t1 - t0
             t_add += time.time() - t1
     if phases is not None:
         phases["ingest_wait_s"] = t_wait  # time the device side waited for the parser (first batch + any shortfall)
         phases["upload_sketch_s"] = t_add
-    return names
+    return (gpaths, names) if per_sequence else names
 
 
 def _phase_log(opt, phases):
@@ -262,7 +277,10 @@ def run_triangle(opt, engine_mod):
         eng.set_ci(opt["ci"])
         eng.set_detailed(opt["detailed"])
         eng.set_marker_compression(opt["marker_c"])
-        names = stream_add(eng, engine_mod, paths, opt["threads"], ph)
+        if opt["per_seq"]:  # genomes: each file's kept records, files in sorted order
+            paths, names = stream_add(eng, engine_mod, paths, opt["threads"], ph, per_sequence=True)
+        else:
+            names = stream_add(eng, engine_mod, paths, opt["threads"], ph)
         t1 = time.time()
         eng.index()
         t2 = time.time()
@@ -284,7 +302,10 @@ def run_sketch(opt, engine_mod):
     daemon.stop_for(opt["out"])  # a server still holding the previous contents of this directory must not answer for the new ones
     with engine_mod.Engine(_device()) as eng:
         eng.set_marker_compression(opt["marker_c"])  # recorded in the database: its searches sketch queries at it
-        names = stream_add(eng, engine_mod, paths, opt["threads"])
+        if opt["per_seq"]:  # the database's genomes are records: paths[i] is genome i's file, names[i] its header
+            paths, names = stream_add(eng, engine_mod, paths, opt["threads"], per_sequence=True)
+        else:
+            names = stream_add(eng, engine_mod, paths, opt["threads"])
         eng.save(opt["out"])
     write_atomic(os.path.join(opt["out"], "manifest.json"), json.dumps({"paths": paths, "names": names}))
 
@@ -303,15 +324,20 @@ def run_search(opt, engine_mod):
 
         from . import daemon
 
-        msg = {"op": "search", "screen": opt["screen"], "min_af": opt["min_af"], "estimator": opt["estimator"],
+        # a per-sequence search is an op of its own, which a server predating it refuses as unknown instead of
+        # answering it as a whole-file search
+        msg = {"op": "search_records" if opt["query_per_seq"] else "search", "screen": opt["screen"], "min_af": opt["min_af"], "estimator": opt["estimator"],
                "ci": opt["ci"], "detailed": opt["detailed"], "out": out}
-        if len(labels) == 1:  # the single-query message every server version answers
+        if len(labels) == 1 and not opt["query_per_seq"]:  # the single-query message every server version answers
             msg.update(query=os.path.abspath(labels[0]), label=labels[0])
         else:
             msg.update(queries=[os.path.abspath(q) for q in labels], labels=labels)
         if opt["max_results"]:
             msg["max_results"] = opt["max_results"]
         rep = daemon.request(db, dev, msg)
+        if rep is not None and rep.get("error") == "unknown op":  # a server from before this op: replace it, once
+            daemon.stop_for(db)
+            rep = None
         if rep is not None and rep.get("stale"):  # the directory was rewritten under a running server: it has just exited
             deadline = time.time() + 15.0
             while time.time() < deadline and daemon.request(db, dev, {"op": "ping"}, timeout=1.0) is not None:
@@ -345,11 +371,20 @@ def run_search(opt, engine_mod):
         eng.load(opt["db"])
         eng.index()
         qp = engine_mod.pack_fasta_many(labels, opt["threads"], eng.params.min_contig_len)
-        edges, st = eng.search(qp, screen=opt["screen"], min_af=opt["min_af"])
+        edges, st = eng.search(qp, screen=opt["screen"], min_af=opt["min_af"], per_sequence=opt["query_per_seq"])
         ci, detail = edge_extras(eng, opt["ci"], opt["detailed"], edges, search_contig_stats(eng) if opt["detailed"] else None)
+    qlabels, qnames = query_columns(labels, qp, opt["query_per_seq"])
     write_atomic(opt["out"], header(opt["ci"], opt["detailed"]) +
-                 "".join(rect_rows(paths + labels, names + [p.first_name for p in qp], edges, ci, detail)))
+                 "".join(rect_rows(paths + qlabels, names + qnames, edges, ci, detail)))
     return st
+
+
+def query_columns(labels, packed, per_sequence):
+    """(Query_file, Query_name) of every query genome of a search: one per file, or with --qi one per kept record"""
+    if not per_sequence:
+        return list(labels), [p.first_name for p in packed]
+    return ([lb for lb, p in zip(labels, packed) for _ in range(p.n_contigs)],
+            [n for p in packed for n in p.contig_names])
 
 
 def search_contig_stats(eng, db_stats=None):
@@ -363,18 +398,35 @@ def search_contig_stats(eng, db_stats=None):
 
 
 def run_dist(opt, engine_mod):
+    """--ri / --qi split that side's files into records: a (file, split) pair is one unit of genomes, so a file split
+    on one side only is compared as records against itself as a whole, and one split on both sides shares its ids"""
+    import itertools
+
     refs, queries = read_list(opt["rl"]), read_list(opt["ql"])
-    paths = list(dict.fromkeys(refs + queries))
-    idx = {p: i for i, p in enumerate(paths)}
+    units = list(dict.fromkeys([(p, opt["ref_per_seq"]) for p in refs] + [(p, opt["query_per_seq"]) for p in queries]))
+    ids, paths, names = {}, [], []
     with engine_mod.Engine(_device()) as eng:
         eng.set_estimator(opt["estimator"])
         eng.set_ci(opt["ci"])
         eng.set_detailed(opt["detailed"])
         eng.set_marker_compression(opt["marker_c"])
         eng.set_max_results(opt["max_results"])
-        names = stream_add(eng, engine_mod, paths, opt["threads"])
+        for split, run in itertools.groupby(units, key=lambda u: u[1]):
+            run = [p for p, _ in run]
+            if split:
+                gp, gn = stream_add(eng, engine_mod, run, opt["threads"], per_sequence=True)
+            else:
+                gp, gn = run, stream_add(eng, engine_mod, run, opt["threads"])
+            for p in gp:
+                ids.setdefault((p, split), []).append(len(paths))
+                paths.append(p)
+            names += gn
+
+        def genome_ids(side, split):
+            return [g for p in dict.fromkeys(side) for g in ids.get((p, split), [])]
+
         eng.index()
-        edges, st = eng.rect([idx[p] for p in dict.fromkeys(refs)], [idx[p] for p in dict.fromkeys(queries)],
+        edges, st = eng.rect(genome_ids(refs, opt["ref_per_seq"]), genome_ids(queries, opt["query_per_seq"]),
                              screen=opt["screen"], min_af=opt["min_af"])
         ci, detail = edge_extras(eng, opt["ci"], opt["detailed"], edges)
     write_atomic(opt["out"], header(opt["ci"], opt["detailed"]) + "".join(rect_rows(paths, names, edges, ci, detail)))
@@ -402,6 +454,11 @@ def _provenance(opt, sub, seconds):
     if opt.get("max_results"):
         text += ("-n %d: each query keeps its first %d rows, by unrounded ANI descending, ties to the lower reference "
                  "id (DESIGN.md section 3); unpinned against skani's own -n\n" % (opt["max_results"], opt["max_results"]))
+    if opt.get("per_seq") or opt.get("query_per_seq") or opt.get("ref_per_seq"):
+        text += ("%s: per-sequence mode, every record of at least 500 bp is a genome of its own (DESIGN.md section 3); "
+                 "skani turns its learned ANI debias off in this mode, this engine keeps its debias substitute on -- the "
+                 "difference is unpinned against skani\n"
+                 % " ".join(f for f, k in (("-i", "per_seq"), ("--qi", "query_per_seq"), ("--ri", "ref_per_seq")) if opt[k]))
     if opt.get("detailed"):
         text += ("--detailed: the 13 extra columns as DESIGN.md section 3 defines them; their names, order and definitions "
                  "are recalled, unpinned against skani's own --detailed output\n")

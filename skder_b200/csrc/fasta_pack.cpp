@@ -168,8 +168,9 @@ int64_t n50_of(std::vector<int64_t> lens) {
     return lens.back();
 }
 
+// names: the kept records' header lines ([kept.size()]), or nullptr for contigs without headers (skb_pack_contigs)
 skb_packed *make_packed(Packer &pk, std::vector<int64_t> &kept, const std::string &name,
-                        const std::vector<int64_t> &all_lens) {
+                        const std::vector<int64_t> &all_lens, const std::vector<std::string> *names) {
     pk.finish();
     skb_packed *p = (skb_packed *)std::calloc(1, sizeof(skb_packed));
     if (!p) return nullptr;
@@ -185,6 +186,10 @@ skb_packed *make_packed(Packer &pk, std::vector<int64_t> &kept, const std::strin
     int64_t t = 0;
     for (int64_t l : all_lens) t += l;
     p->total_bases_all = t;
+    if (names) {
+        p->contig_names = (char **)std::calloc(std::max<size_t>(names->size(), 1), sizeof(char *));
+        for (size_t k = 0; k < names->size(); k++) p->contig_names[k] = strdup((*names)[k].c_str());
+    }
     return p;
 }
 
@@ -233,8 +238,9 @@ int skb_pack_fasta(const char *path, int32_t min_contig_len, skb_packed **out) {
         ~GiveBack() { pk.words.swap(home); }
     } give_back{pk, scratch_words};
     std::vector<int64_t> kept, all_lens;
-    std::string first_name, cur_name;
-    bool have_first = false, in_header = false, in_record = false;
+    std::vector<std::string> kept_names;
+    std::string cur_name;
+    bool in_header = false, in_record = false;
     int64_t rec_len = 0, rec_start_bases = 0;
     size_t rec_start_words = 0;
     uint64_t rec_start_cur = 0;
@@ -243,10 +249,7 @@ int skb_pack_fasta(const char *path, int32_t min_contig_len, skb_packed **out) {
         all_lens.push_back(rec_len);
         if (rec_len >= min_contig_len && rec_len > 0) {
             kept.push_back(rec_len);
-            if (!have_first) {
-                first_name = cur_name;
-                have_first = true;
-            }
+            kept_names.push_back(cur_name);
         } else {  // roll back
             pk.words.resize(rec_start_words);
             pk.cur = rec_start_cur;
@@ -301,7 +304,7 @@ int skb_pack_fasta(const char *path, int32_t min_contig_len, skb_packed **out) {
     }
     close_input();
     close_record();
-    *out = make_packed(pk, kept, first_name, all_lens);
+    *out = make_packed(pk, kept, kept_names.empty() ? std::string() : kept_names[0], all_lens, &kept_names);
     return *out ? SKB_OK : SKB_ENOMEM;
 }
 
@@ -316,7 +319,7 @@ int skb_pack_contigs(const char *const *seqs, const int64_t *lens, int32_t n, in
         const uint8_t *s = (const uint8_t *)seqs[i];
         kept.push_back(pk.put_line(s, lens[i], s + lens[i]));  // the whole contig as one line (blanks, if any, are dropped)
     }
-    *out = make_packed(pk, kept, "", all_lens);
+    *out = make_packed(pk, kept, "", all_lens, nullptr);
     return *out ? SKB_OK : SKB_ENOMEM;
 }
 
@@ -345,6 +348,9 @@ void skb_packed_free(skb_packed *p) {
     std::free(p->words);
     std::free(p->contig_lens);
     std::free(p->first_name);
+    if (p->contig_names)
+        for (int32_t k = 0; k < p->n_contigs; k++) std::free(p->contig_names[k]);
+    std::free(p->contig_names);
     std::free(p);
 }
 

@@ -342,6 +342,7 @@ struct BatchMeta {
     SketchBatch b;
     uint32_t n_tiles = 0;
     size_t n_warps = 0;
+    size_t n_ctg = 0;  // contigs of the batch (ctg_start entries)
 };
 
 // Host-side layout of a batch -> device, one copy per batch (slot = position in the super-batch).  Issued for every
@@ -360,7 +361,6 @@ BatchMeta sketch_meta(skb_ctx *c, const skb_packed *const *gen, int32_t g0, int3
             ctg_start.push_back(s);
             s += (uint64_t)p->contig_lens[k];
         }
-        if (p->n_contigs == 0) ctg_start.push_back(0);  // keep one entry so the kernel's search is well-defined
         ctg_off[i + 1] = (uint32_t)ctg_start.size();
         tile_off[i + 1] = tile_off[i] + (uint32_t)std::max<uint64_t>(1, (nbases[i] + SK_TILE_BASES - 1) / SK_TILE_BASES);
     }
@@ -378,6 +378,7 @@ BatchMeta sketch_meta(skb_ctx *c, const skb_packed *const *gen, int32_t g0, int3
     BatchMeta m;
     m.n_tiles = tile_off[nb];
     m.n_warps = (size_t)m.n_tiles * SK_WARPS;
+    m.n_ctg = ctg_start.size();
     m.b.packed = d_words;
     m.b.g_word_off = d_meta.p;
     m.b.g_nbases = d_meta.p + o_nb;
@@ -389,8 +390,9 @@ BatchMeta sketch_meta(skb_ctx *c, const skb_packed *const *gen, int32_t g0, int3
     return m;
 }
 
+// per_seq (skb_add_sequences): every contig of the batch is appended as a genome of its own
 void sketch_batch(skb_ctx *c, const skb_packed *const *gen, int32_t g0, int32_t g1, const BatchMeta &meta,
-                  cudaEvent_t uploaded) {
+                  cudaEvent_t uploaded, bool per_seq) {
     const int32_t nb = g1 - g0;
     const uint32_t n_tiles = meta.n_tiles;
     const size_t n_warps = meta.n_warps;
@@ -411,25 +413,37 @@ void sketch_batch(skb_ctx *c, const skb_packed *const *gen, int32_t g0, int32_t 
            d_masks.p);
     exclusive_scan_u32(c, d_cnt_s.p, d_off_s.p, n_warps + 1);
     exclusive_scan_u32(c, d_cnt_m.p, d_off_m.p, n_warps + 1);
-    // per-genome seed offsets = scanned offsets at genome tile boundaries
-    std::vector<uint32_t> h_off_s(nb + 1);
+    // per-genome seed offsets = scanned offsets at genome tile boundaries; per-sequence: at every contig's first base
+    const size_t n_units = per_seq ? meta.n_ctg : (size_t)nb;
+    std::vector<uint32_t> h_off_s(n_units + 1);
     uint32_t tot_m = 0;
     PoolRef<uint32_t> d_goff(c->pool["sketch_batch.d_goff"]);
-    d_goff.reserve((size_t)nb + 1, 0, c->st);
-    launch(c, gather_strided_kernel, nblk((uint64_t)nb + 1, 256), 256, 0, d_off_s.p, b.tile_off, SK_WARPS, nb + 1, d_goff.p);
-    CK(cudaMemcpyAsync(h_off_s.data(), d_goff.p, ((size_t)nb + 1) * 4, cudaMemcpyDeviceToHost, c->st));
+    d_goff.reserve(n_units + 1, 0, c->st);
+    if (per_seq)
+        launch(c, record_seed_off_kernel, nblk((uint64_t)n_units + 1, 256), 256, 0, b, d_off_s.p, d_masks.p,
+               (int)n_units, n_warps, d_goff.p);
+    else
+        launch(c, gather_strided_kernel, nblk((uint64_t)nb + 1, 256), 256, 0, d_off_s.p, b.tile_off, SK_WARPS, nb + 1,
+               d_goff.p);
+    CK(cudaMemcpyAsync(h_off_s.data(), d_goff.p, (n_units + 1) * 4, cudaMemcpyDeviceToHost, c->st));
     CK(cudaMemcpyAsync(&tot_m, d_off_m.p + n_warps, 4, cudaMemcpyDeviceToHost, c->st));
     CK(cudaStreamSynchronize(c->st));
     const uint64_t cur_seeds = c->db.seed_off.back();
-    const uint64_t tot_s = h_off_s[nb];
+    const uint64_t tot_s = h_off_s[n_units];
     c->d_seeds.reserve(cur_seeds + tot_s + 1, cur_seeds, c->st);
     c->d_mkeys.reserve(c->db.n_mkeys + tot_m + 1, c->db.n_mkeys, c->st);
-    launch(c, sketch_kernel<true>, n_tiles, SK_THREADS, 0, b, nullptr, nullptr, d_off_s.p, d_off_m.p,
-           c->d_seeds.p + cur_seeds, c->d_mkeys.p + c->db.n_mkeys, d_masks.p);
+    launch(c, per_seq ? sketch_kernel<true, true> : sketch_kernel<true>, n_tiles, SK_THREADS, 0, b, nullptr, nullptr,
+           d_off_s.p, d_off_m.p, c->d_seeds.p + cur_seeds, c->d_mkeys.p + c->db.n_mkeys, d_masks.p);
     CK(cudaStreamSynchronize(c->st));  // batch-local buffers die here
+    size_t u = 0;
     for (int32_t i = 0; i < nb; i++) {
         const skb_packed *p = gen[g0 + i];
-        c->db.append(h_off_s[i + 1] - h_off_s[i], (uint64_t)p->n_bases, p->contig_lens, (size_t)p->n_contigs);
+        if (!per_seq) {
+            c->db.append(h_off_s[u + 1] - h_off_s[u], (uint64_t)p->n_bases, p->contig_lens, (size_t)p->n_contigs);
+            u++;
+        } else
+            for (int32_t k = 0; k < p->n_contigs; k++, u++)
+                c->db.append(h_off_s[u + 1] - h_off_s[u], (uint64_t)p->contig_lens[k], p->contig_lens + k, 1);
     }
     c->db.n_mkeys += tot_m;
     c->indexed = false;
@@ -1070,20 +1084,30 @@ int skb_timer_stop(skb_ctx *ctx, float *ms) {
     });
 }
 
-int skb_add_genomes(skb_ctx *ctx, int32_t n, const skb_packed *const *genomes) {
+// skb_add_genomes (per_seq = false: one genome per packed file) and skb_add_sequences (per_seq: one per kept contig)
+static int add_impl(skb_ctx *ctx, int32_t n, const skb_packed *const *genomes, bool per_seq) {
     return guarded(ctx, [&]() -> int {
         if (n < 0 || (n > 0 && !genomes)) return fail(ctx, SKB_EINVAL, "bad genome list");
-        if ((uint64_t)ctx->n() + (uint64_t)n >= GID_MASK) return fail(ctx, SKB_ELIMIT, "too many genomes (22-bit ids)");
+        uint64_t n_new = per_seq ? 0 : (uint64_t)n;
         for (int32_t i = 0; i < n; i++) {
             const skb_packed *p = genomes[i];
-            if (!p || !p->words || (p->n_words & 1) || p->n_words * 32 < p->n_bases)
+            if (!p || !p->words || (p->n_words & 1) || p->n_words * 32 < p->n_bases || p->n_contigs < 0)
                 return fail(ctx, SKB_EINVAL, "genome " + std::to_string(i) + ": malformed packed buffer");
             uint64_t s = 0;
-            for (int32_t k = 0; k < p->n_contigs; k++) s += (uint64_t)p->contig_lens[k];
+            for (int32_t k = 0; k < p->n_contigs; k++) {
+                s += (uint64_t)p->contig_lens[k];
+                if (per_seq && p->contig_lens[k] <= 0) return fail(ctx, SKB_EINVAL, "empty contig");
+                if (per_seq && (uint64_t)p->contig_lens[k] + CONTIG_PAD >= (1ull << 31))
+                    return fail(ctx, SKB_ELIMIT, "sequence too large for 31-bit padded coordinates");
+            }
             if (s != (uint64_t)p->n_bases) return fail(ctx, SKB_EINVAL, "contig lengths do not sum to n_bases");
-            if ((uint64_t)p->n_bases + (uint64_t)p->n_contigs * CONTIG_PAD >= (1ull << 31))
+            if (!per_seq && (uint64_t)p->n_bases + (uint64_t)p->n_contigs * CONTIG_PAD >= (1ull << 31))
                 return fail(ctx, SKB_ELIMIT, "genome too large for 31-bit padded coordinates");
+            if (per_seq && (uint64_t)p->n_bases >= (1ull << 32))  // a batch's seed and marker counts are 32-bit
+                return fail(ctx, SKB_ELIMIT, "file too large for one sketch batch");
+            if (per_seq) n_new += (uint64_t)p->n_contigs;
         }
+        if ((uint64_t)ctx->n() + n_new >= GID_MASK) return fail(ctx, SKB_ELIMIT, "too many genomes (22-bit ids)");
         // batches of <= 1 Gi bases (per-batch seed/marker totals stay far below 2^32), grouped into
         // super-batches of <= 32 (8 GiB of packed words) whose H2D copies are all enqueued up front on a second stream: batch i+1
         // uploads while batch i is being sketched.
@@ -1143,7 +1167,7 @@ int skb_add_genomes(skb_ctx *ctx, int32_t n, const skb_packed *const *genomes) {
                 mark(ctx->st_copy);
             }
             for (size_t bi = 0; bi < nbatch; bi++) {
-                sketch_batch(ctx, genomes, cut[bi], cut[bi + 1], metas[bi], ctx->up_ev[bi]);
+                sketch_batch(ctx, genomes, cut[bi], cut[bi + 1], metas[bi], ctx->up_ev[bi], per_seq);
                 mark(ctx->st);
             }
             if (trace) {
@@ -1160,6 +1184,11 @@ int skb_add_genomes(skb_ctx *ctx, int32_t n, const skb_packed *const *genomes) {
         }
         return SKB_OK;
     });
+}
+
+int skb_add_genomes(skb_ctx *ctx, int32_t n, const skb_packed *const *genomes) { return add_impl(ctx, n, genomes, false); }
+int skb_add_sequences(skb_ctx *ctx, int32_t n_files, const skb_packed *const *files) {
+    return add_impl(ctx, n_files, files, true);
 }
 
 // ---- the per-genome index -------------------------------------------------------------------------------------------
@@ -1438,7 +1467,7 @@ int skb_index_append(skb_ctx *ctx) {
     });
 }
 
-// Undo the most recent skb_add_genomes call (and its index entries): the query genome of a search leaves.
+// Undo the most recent skb_add_genomes / skb_add_sequences call (and its index entries): the query genomes of a search leave.
 int skb_pop_last_add(skb_ctx *ctx) {
     return guarded(ctx, [&]() -> int {
         skb_ctx *c = ctx;

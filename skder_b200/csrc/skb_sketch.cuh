@@ -28,7 +28,7 @@ struct SketchBatch {
     const uint64_t *packed;      // all genomes of the batch, each starting on an even word
     const uint64_t *g_word_off;  // [n+1]
     const uint64_t *g_nbases;    // [n]
-    const uint32_t *g_ctg_off;   // [n+1] into ctg_start
+    const uint32_t *g_ctg_off;   // [n+1] into ctg_start; per-sequence mode: also the batch-local id of each file's first record
     const uint64_t *ctg_start;   // unpadded first-base offset of each contig inside its genome
     const uint32_t *tile_off;    // [n+1] CTA-tile prefix sum
     int32_t n;
@@ -49,7 +49,10 @@ __device__ __forceinline__ uint32_t rev2_32(uint32_t x) {
     return ((y >> 1) & 0x55555555u) | ((y & 0x55555555u) << 1);
 }
 
-template <bool EMIT>
+// PER_SEQ (emit pass only; skb_add_sequences): every contig of a batch entry is its own genome -- its marker keys carry
+// the genome id first_gid + g_ctg_off[g] + ci and its seeds the record-local position p - ctg_start[ci] (contig index
+// 0), which is what the same record sketched as a one-contig genome gets.  The hash pass does not depend on the mode.
+template <bool EMIT, bool PER_SEQ = false>
 __global__ void __launch_bounds__(SK_THREADS)
 sketch_kernel(SketchBatch b, uint32_t *__restrict__ warp_seed_cnt, uint32_t *__restrict__ warp_marker_cnt,
               const uint32_t *__restrict__ warp_seed_off, const uint32_t *__restrict__ warp_marker_off,
@@ -184,7 +187,7 @@ sketch_kernel(SketchBatch b, uint32_t *__restrict__ warp_seed_cnt, uint32_t *__r
         size_t so = (size_t)warp_seed_off[wgid] + (ps - ns);
         size_t mo = (size_t)warp_marker_off[wgid] + (pm - nm);
         if ((seed_mask | marker_mask) == 0) return;
-        const uint64_t gid = (uint64_t)b.first_gid + g;
+        const uint64_t gid = PER_SEQ ? (uint64_t)b.first_gid + b.g_ctg_off[g] : (uint64_t)b.first_gid + g;
         int ci = ci0;
         uint64_t hits = seed_mask | marker_mask;
         while (hits) {
@@ -206,12 +209,12 @@ sketch_kernel(SketchBatch b, uint32_t *__restrict__ warp_seed_cnt, uint32_t *__r
                 const uint64_t fs = f & MASK_SEED, rs = r >> (2 * (K_MARKER - K_SEED));
                 const int fwd = fs < rs;
                 const uint64_t cseed = fwd ? fs : rs;
-                const uint64_t ppos = p + (uint64_t)ci * CONTIG_PAD;
+                const uint64_t ppos = PER_SEQ ? p - cs[ci] : p + (uint64_t)ci * CONTIG_PAD;
                 seeds_out[so++] = (cseed << 34) | (ppos << 2) | (uint64_t)fwd;
             }
             if ((marker_mask >> j) & 1) {
                 const uint64_t cm = f < r ? f : r;
-                mkeys_out[mo++] = (cm << GID_BITS) | gid;
+                mkeys_out[mo++] = (cm << GID_BITS) | (PER_SEQ ? gid + ci : gid);
             }
         }
     }
@@ -222,6 +225,32 @@ __global__ void gather_strided_kernel(const uint32_t *__restrict__ src, const ui
                                       int n, uint32_t *__restrict__ out) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) out[i] = src[(size_t)idx[i] * mult];
+}
+
+// Per-sequence mode: out[r] = batch-local offset of the first seed of contig r of the batch (ctg_start order), and
+// out[n_rec] = the batch's seed total.  Seeds come out in position order, so a contig's seeds start where the seeds
+// before its first base end: the scanned offset of the warp holding that base plus the seed bits the hash pass left in
+// the masks of the lanes, and the bits of its own lane, before it.
+__global__ void record_seed_off_kernel(SketchBatch b, const uint32_t *__restrict__ warp_seed_off,
+                                       const ulonglong2 *__restrict__ masks, int n_rec, size_t n_warps,
+                                       uint32_t *__restrict__ out) {
+    const int r = blockIdx.x * blockDim.x + threadIdx.x;
+    if (r == 0) out[n_rec] = warp_seed_off[n_warps];
+    if (r >= n_rec) return;
+    int lo = 0, hi = b.n - 1;  // batch entry of contig r: last g with g_ctg_off[g] <= r
+    while (lo < hi) {
+        int mid = (lo + hi + 1) >> 1;
+        if (b.g_ctg_off[mid] <= (uint32_t)r)
+            lo = mid;
+        else
+            hi = mid - 1;
+    }
+    const uint64_t s = b.ctg_start[r];
+    const size_t wgid = ((size_t)b.tile_off[lo] + s / SK_TILE_BASES) * SK_WARPS + (s % SK_TILE_BASES) / SK_WARP_BASES;
+    const int lane = (int)((s % SK_WARP_BASES) / SK_LANE_BASES), j = (int)(s % SK_LANE_BASES);
+    uint32_t o = warp_seed_off[wgid];
+    for (int l = 0; l < lane; l++) o += __popcll(masks[wgid * 32 + l].x);
+    out[r] = o + __popcll(masks[wgid * 32 + lane].x & ((1ull << j) - 1));
 }
 
 }  // namespace skb

@@ -7,7 +7,9 @@ database starts this server (one per database directory, per GPU); it keeps the 
 and answers each later search with one sketch + one rectangle (Engine.search), then exits after
 SKB_DAEMON_IDLE seconds without requests.  A request names its query FASTAs as "queries" (absolute paths) and
 "labels" (the paths its rows show), or a single one as "query" and "label"; every query of a request is answered in
-one device pass.  "max_results" is skani's -n (0 or absent: every row).
+one device pass.  "max_results" is skani's -n (0 or absent: every row).  The op "search_records" is the same request in
+skani's per-sequence mode (--qi): every kept record of the query files is a query.  It is an op of its own so that a
+server predating it refuses it as unknown rather than answering it as a whole-file search.
 
 Trust and staleness:
 * The Unix socket lives in a directory only the user can enter (mode 0700, ownership checked: $XDG_RUNTIME_DIR
@@ -171,7 +173,8 @@ def serve(db_dir, device):
                     elif msg.get("op") == "stop":
                         conn.send_bytes(json.dumps({"ok": True}).encode())
                         stop = True
-                    elif msg.get("op") == "search":
+                    elif msg.get("op") in ("search", "search_records"):
+                        per_seq = msg["op"] == "search_records"
                         eng.set_estimator(msg.get("estimator", "mean"))  # per request: a resident server serves every mode
                         ci, detailed = bool(msg.get("ci", False)), bool(msg.get("detailed", False))
                         eng.set_ci(ci)
@@ -179,12 +182,13 @@ def serve(db_dir, device):
                         eng.set_max_results(int(msg.get("max_results", 0)))
                         queries, labels = search_queries(msg)
                         packed = engine.pack_fasta_many(queries, None, eng.params.min_contig_len)
-                        edges, st = eng.search(packed, screen=msg["screen"], min_af=msg["min_af"])
+                        edges, st = eng.search(packed, screen=msg["screen"], min_af=msg["min_af"], per_sequence=per_seq)
                         stats = None
                         if detailed:
                             db_stats = db_stats or eng.contig_stats(0, n_db)  # the database's, once per server
                             stats = cli.search_contig_stats(eng, db_stats)
-                        rows = cli.rect_rows(paths + labels, names + [p.first_name for p in packed], edges,
+                        qlabels, qnames = cli.query_columns(labels, packed, per_seq)
+                        rows = cli.rect_rows(paths + qlabels, names + qnames, edges,
                                              *cli.edge_extras(eng, ci, detailed, edges, stats))
                         cli.write_atomic(msg["out"], cli.header(ci, detailed) + "".join(rows))
                         conn.send_bytes(json.dumps({"ok": True, "rows": len(rows), "ms": st.ms_total}).encode())

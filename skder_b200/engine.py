@@ -56,6 +56,14 @@ class PackedGenome:
     def first_name(self):
         return (self._p.contents.first_name or b"").decode("utf-8", "replace")
 
+    @property
+    def contig_names(self):
+        """header lines (without '>') of the kept records, in file order; empty for pack_contigs' genomes"""
+        names = self._p.contents.contig_names
+        if not names:
+            return []
+        return [(names[k] or b"").decode("utf-8", "replace") for k in range(self.n_contigs)]
+
     def contig_lens(self):
         n = self.n_contigs
         return np.ctypeslib.as_array(self._p.contents.contig_lens, shape=(n,)).copy() if n else np.zeros(0, np.int64)
@@ -199,12 +207,15 @@ class Engine:
         return cnt, nx
 
     # ---- sketching -------------------------------------------------------------------------
-    def add(self, packed):
+    def add(self, packed, per_sequence=False):
+        """Sketch packed genomes into the context.  per_sequence (skani's -i / --qi / --ri; DESIGN.md section 3): every
+        kept record of every packed file becomes a genome of its own, ids in (file, record) order."""
         n = len(packed)
         if n == 0:
             return
         arr = (C.POINTER(_lib.Packed) * n)(*[p._p for p in packed])
-        self._ck(self._L.skb_add_genomes(self._h, n, arr), "skb_add_genomes")
+        fn = "skb_add_sequences" if per_sequence else "skb_add_genomes"
+        self._ck(getattr(self._L, fn)(self._h, n, arr), fn)
 
     def add_fasta(self, paths, threads=None):
         packed = pack_fasta_many(list(paths), threads, self.params.min_contig_len)
@@ -237,19 +248,21 @@ class Engine:
     def pop_last_add(self):
         self._ck(self._L.skb_pop_last_add(self._h), "skb_pop_last_add")
 
-    def search(self, query_packed, screen=80.0, min_af=15.0):
+    def search(self, query_packed, screen=80.0, min_af=15.0, per_sequence=False):
         """`skani search`: query genomes (one PackedGenome, or a list of them) against the resident, indexed database
         (ids 0..n-1), in one device pass.  The queries are sketched, indexed query-only, compared, and removed again.
-        Edges: a = database genome, b = query (ids n, n+1, ... in list order).  With set_detailed(True) the queries'
-        contig_stats are kept in last_query_contig_stats, in list order."""
+        Edges: a = database genome, b = query (ids n, n+1, ... in list order).  per_sequence (skani's --qi): every kept
+        record of the query files is a query, in (file, record) order.  With set_detailed(True) the queries'
+        contig_stats are kept in last_query_contig_stats, in query order."""
         queries = list(query_packed) if isinstance(query_packed, (list, tuple)) else [query_packed]
         n_db = self.n_genomes
-        self.add(queries)
+        self.add(queries, per_sequence)
         try:
+            n_q = self.n_genomes - n_db
             if self.detailed:  # contig_stats of the queries: they leave the context below
-                self.last_query_contig_stats = self.contig_stats(n_db, len(queries))
+                self.last_query_contig_stats = self.contig_stats(n_db, n_q)
             self.index_append()
-            return self.rect(np.arange(n_db, dtype=np.int32), np.arange(n_db, n_db + len(queries), dtype=np.int32),
+            return self.rect(np.arange(n_db, dtype=np.int32), np.arange(n_db, n_db + n_q, dtype=np.int32),
                              screen=screen, min_af=min_af)
         finally:
             self.pop_last_add()
