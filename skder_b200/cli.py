@@ -9,6 +9,19 @@ without touching skDER.  Sub-commands and flags are exactly the ones skDER spell
   skani search   QUERY.fa -d DBDIR -o OUT -t T                   (skder.py:119)
   skani dist     --rl REFS --ql QUERIES [-s S] [-t T] -o OUT     (skder.py:58-59, cidder.py:362-363)
 
+skani's own command forms work too (DESIGN.md section 3):
+
+  skani triangle [FASTA ...] [-l LIST] -E [-o OUT]       genomes: both sources, deduplicated and sorted
+  skani sketch   [FASTA ...] [-l LIST] -o DBDIR          genomes: the FASTAs in order, then the list; nothing deduplicated
+  skani dist     [-q FASTA ...] [--ql LIST] [-r FASTA ...] [--rl LIST] [-o OUT]
+  skani dist     QUERY REF [REF ...] [-o OUT]
+  skani search   QUERY ... [--ql LIST] -d DBDIR [-o OUT]
+
+`-q` / `-r` (dist only) take every following argument up to the next one starting with '-'; each side is its values,
+then its list's entries, a path twice on one side counting once.  The positional dist form takes no -q, -r, --ql or
+--rl.  Without -o, triangle, dist and search write the TSV to stdout -- the bytes the -o file would hold, nothing on
+failure -- and the provenance note below goes to stderr.
+
 `search` also takes several query FASTAs, as positionals and/or a list file `--ql` (positionals first, then the list in
 file order, a repeated path once at its first position), answered in one device pass; rows are grouped by query in that
 order.  `-n N` (dist, search) keeps each query's first N rows -- its N best hits by unrounded ANI, ties to the reference
@@ -66,6 +79,7 @@ def parse_args(argv):
         "-l": "list", "-o": "out", "-t": "threads", "-s": "screen", "--min-af": "min_af", "--rl": "rl", "--ql": "ql",
         "-d": "db", "-m": "marker_c", "-n": "max_results",
     }
+    multi = {"-q": "q", "-r": "r"}  # dist's FASTA lists: every following token up to the next one starting with '-'
     flags = {"-E": "edge_list", "--sparse": "edge_list", "--ci": "ci", "--detailed": "detailed", "-i": "per_seq",
              "--qi": "query_per_seq", "--ri": "ref_per_seq"}
     opt["ci"] = opt["detailed"] = opt["per_seq"] = opt["query_per_seq"] = opt["ref_per_seq"] = False
@@ -82,6 +96,15 @@ def parse_args(argv):
                 raise UsageError("option %s needs a value" % a)
             opt[valued[a]] = argv[i + 1]
             i += 2
+        elif a in multi:
+            vals = opt.setdefault(multi[a], [])
+            n0, i = len(vals), i + 1
+            while i < len(argv) and not argv[i].startswith("-"):
+                if argv[i]:
+                    vals.append(argv[i])
+                i += 1
+            if len(vals) == n0:
+                raise UsageError("option %s needs at least one FASTA" % a)
         elif a in flags:
             opt[flags[a]] = True
             i += 1
@@ -134,16 +157,29 @@ def parse_args(argv):
                             ("--ri", "ref_per_seq", ("dist",))):
         if opt[key] and sub not in subs:
             raise UsageError("skani %s takes no %s (per-sequence mode: %s)" % (sub, flag, ", ".join(subs)))
-    need = {"triangle": ["list", "out"], "sketch": ["list", "out"], "search": ["db", "out"], "dist": ["rl", "ql", "out"]}[sub]
+    if sub != "dist" and ("q" in opt or "r" in opt):
+        raise UsageError("skani %s takes no -q / -r: they name dist's query and reference FASTAs" % sub)
+    # without -o, triangle, dist and search write the TSV to stdout; sketch writes a directory
+    need = {"sketch": ["out"], "search": ["db"]}.get(sub, [])
     for k in need:
         if k not in opt:
             raise UsageError("skani %s: missing required option for %r" % (sub, k))
+    if sub in ("triangle", "sketch") and "list" not in opt and not opt["positional"]:
+        raise UsageError("skani %s: no genome given (FASTA arguments and/or -l LIST)" % sub)
     if sub == "triangle" and not opt["edge_list"]:
         raise UsageError("skani triangle without -E (matrix output) is not implemented; skDER always passes -E")
     if sub == "search" and not opt["positional"] and "ql" not in opt:
         raise UsageError("skani search: no query FASTA given")
-    if sub != "search" and opt["positional"]:
-        raise UsageError("unexpected positional arguments: %r" % opt["positional"])
+    if sub == "dist":
+        lists = [a for a, k in (("-q", "q"), ("-r", "r"), ("--ql", "ql"), ("--rl", "rl")) if k in opt]
+        if opt["positional"] and lists:
+            raise UsageError("skani dist QUERY REF...: positional FASTAs %r do not combine with %s"
+                             % (opt["positional"], ", ".join(lists)))
+        if opt["positional"] and len(opt["positional"]) < 2:
+            raise UsageError("skani dist QUERY REF [REF ...] needs a query and at least one reference")
+        for side, keys in (("query", ("q", "ql")), ("reference", ("r", "rl"))):
+            if not opt["positional"] and not any(k in opt for k in keys):
+                raise UsageError("skani dist: no %s FASTA given (-%s and/or --%s)" % (side, keys[0], keys[1]))
     return sub, opt
 
 
@@ -159,6 +195,43 @@ def search_queries(opt):
     if not qs:
         raise UsageError("skani search: no query FASTA given")
     return qs
+
+
+def inputs(sub, opt):
+    """The FASTA paths a command names, as given, whatever form named them (DESIGN.md section 3):
+    triangle: the FASTA arguments and the -l entries, deduplicated and sorted (the triangle's genome order);
+    sketch: the FASTA arguments in order, then the -l entries, nothing deduplicated;
+    dist: (refs, queries), each -r / -q's values followed by --rl / --ql's entries, or for `dist Q R1 [R2 ...]` the
+    first argument as the query and the rest as references (a path twice on one side counts once, in run_dist);
+    search: search_queries()."""
+    def entries(values_key, list_key):
+        return opt.get(values_key, []) + (read_list(opt[list_key]) if list_key in opt else [])
+
+    if sub == "triangle":
+        return sorted(set(entries("positional", "list")))
+    if sub == "sketch":
+        return entries("positional", "list")
+    if sub == "dist":
+        if opt["positional"]:
+            return opt["positional"][1:], opt["positional"][:1]
+        return entries("r", "rl"), entries("q", "ql")
+    return search_queries(opt)
+
+
+def emit(opt, text):
+    """The TSV into -o, atomically, or without -o onto stdout, written once as a whole so a failure leaves none of it"""
+    if "out" in opt:
+        write_atomic(opt["out"], text)
+    else:
+        to_stdout(text)
+
+
+def to_stdout(data):
+    """data, built whole before any of it is written, onto stdout: bytes as they are, text encoded as write_atomic's
+    file would be"""
+    sys.stdout.flush()
+    with open(sys.stdout.fileno(), "wb" if isinstance(data, bytes) else "w", closefd=False) as f:
+        f.write(data)
 
 
 def header(ci, detailed=False):
@@ -264,13 +337,13 @@ def stream_add(eng, engine_mod, paths, threads, phases=None, per_sequence=False)
 
 
 def _phase_log(opt, phases):
-    if os.environ.get("SKB_PHASE_LOG") == "1":
+    if os.environ.get("SKB_PHASE_LOG") == "1" and "out" in opt:  # nothing to put it beside with stdout output
         write_atomic(opt["out"].rstrip("/") + ".skani_b200.phases.json", json.dumps(phases))
 
 
 def run_triangle(opt, engine_mod):
     ph, t0 = {}, time.time()
-    paths = sorted(set(read_list(opt["list"])))
+    paths = inputs("triangle", opt)
     with engine_mod.Engine(_device()) as eng:
         ph["context_s"] = time.time() - t0
         eng.set_estimator(opt["estimator"])
@@ -287,7 +360,7 @@ def run_triangle(opt, engine_mod):
         edges, st = eng.triangle(screen=opt["screen"], min_af=opt["min_af"])
         ci, detail = edge_extras(eng, opt["ci"], opt["detailed"], edges)
         t3 = time.time()
-    write_atomic(opt["out"], header(opt["ci"], opt["detailed"]) + "".join(triangle_rows(paths, names, edges, ci, detail)))
+    emit(opt, header(opt["ci"], opt["detailed"]) + "".join(triangle_rows(paths, names, edges, ci, detail)))
     ph.update({"index_s": t2 - t1, "triangle_s": t3 - t2, "write_tsv_s": time.time() - t3, "total_s": time.time() - t0,
                "genomes": len(paths), "edges": int(len(edges))})
     _phase_log(opt, ph)
@@ -295,7 +368,7 @@ def run_triangle(opt, engine_mod):
 
 
 def run_sketch(opt, engine_mod):
-    paths = read_list(opt["list"])
+    paths = inputs("sketch", opt)
     os.makedirs(opt["out"], exist_ok=True)
     from . import daemon
 
@@ -310,53 +383,78 @@ def run_sketch(opt, engine_mod):
     write_atomic(os.path.join(opt["out"], "manifest.json"), json.dumps({"paths": paths, "names": names}))
 
 
+def _daemon_search(opt, labels, dev, out):
+    """search through the database's resident daemon (started here if none answers), its TSV written to `out`, an
+    absolute path; raises if no server answers or the search fails"""
+    import subprocess
+
+    from . import daemon
+
+    db = opt["db"]
+    # a per-sequence search is an op of its own, which a server predating it refuses as unknown instead of
+    # answering it as a whole-file search
+    msg = {"op": "search_records" if opt["query_per_seq"] else "search", "screen": opt["screen"], "min_af": opt["min_af"], "estimator": opt["estimator"],
+           "ci": opt["ci"], "detailed": opt["detailed"], "out": out}
+    if len(labels) == 1 and not opt["query_per_seq"]:  # the single-query message every server version answers
+        msg.update(query=os.path.abspath(labels[0]), label=labels[0])
+    else:
+        msg.update(queries=[os.path.abspath(q) for q in labels], labels=labels)
+    if opt["max_results"]:
+        msg["max_results"] = opt["max_results"]
+    rep = daemon.request(db, dev, msg)
+    if rep is not None and rep.get("error") == "unknown op":  # a server from before this op: replace it, once
+        daemon.stop_for(db)
+        rep = None
+    if rep is not None and rep.get("stale"):  # the directory was rewritten under a running server: it has just exited
+        deadline = time.time() + 15.0
+        while time.time() < deadline and daemon.request(db, dev, {"op": "ping"}, timeout=1.0) is not None:
+            time.sleep(0.05)
+        rep = None
+    if rep is None:
+        log = open(os.path.join(db, "skani_b200_daemon.log"), "a")
+        subprocess.Popen([sys.executable, "-m", "skder_b200.daemon", db, str(dev)], stdout=log, stderr=log,
+                         stdin=subprocess.DEVNULL, start_new_session=True,
+                         cwd=os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+        deadline = time.time() + float(os.environ.get("SKB_DAEMON_START_TIMEOUT", "600"))
+        while rep is None and time.time() < deadline:
+            time.sleep(0.2)
+            if daemon.request(db, dev, {"op": "ping"}, timeout=5.0):
+                rep = daemon.request(db, dev, msg)
+    if rep is None:
+        raise RuntimeError("search daemon did not come up (see %s/skani_b200_daemon.log)" % db)
+    if not rep.get("ok"):
+        raise RuntimeError("search daemon: %s" % rep.get("error"))
+
+
 def run_search(opt, engine_mod):
-    """`skani search q.fa [q2.fa ...] [--ql LIST] -d DB -o OUT` (reference src/skDER/skder.py:119).  Served by the
+    """`skani search q.fa [q2.fa ...] [--ql LIST] -d DB [-o OUT]` (reference src/skDER/skder.py:119).  Served by the
     database's resident daemon (skder_b200/daemon.py; started here on first use) unless SKB_NO_DAEMON=1, in which case
     the database is loaded, indexed and searched in this process.  All queries go through one Engine.search."""
-    labels = search_queries(opt)  # each query's rows show its path as it was given
+    labels = inputs("search", opt)  # each query's rows show its path as it was given
     # the server runs in another working directory: every path goes over absolute
-    db, out = os.path.abspath(opt["db"]), os.path.abspath(opt["out"])
-    opt = dict(opt, db=db, out=out)
+    opt = dict(opt, db=os.path.abspath(opt["db"]))
+    if "out" in opt:
+        opt["out"] = os.path.abspath(opt["out"])
     dev = _device()
     if os.environ.get("SKB_NO_DAEMON") != "1":
-        import subprocess
+        if "out" in opt:
+            _daemon_search(opt, labels, dev, opt["out"])
+            return None
+        # stdout: the server writes into a fresh private (0700) directory, whose file is copied out; the directory goes
+        # on failure too.  No protocol change, so any running server version answers, and the copy is plain file I/O
+        # that keeps numpy and the engine out of this process.
+        import shutil
+        import tempfile
 
-        from . import daemon
-
-        # a per-sequence search is an op of its own, which a server predating it refuses as unknown instead of
-        # answering it as a whole-file search
-        msg = {"op": "search_records" if opt["query_per_seq"] else "search", "screen": opt["screen"], "min_af": opt["min_af"], "estimator": opt["estimator"],
-               "ci": opt["ci"], "detailed": opt["detailed"], "out": out}
-        if len(labels) == 1 and not opt["query_per_seq"]:  # the single-query message every server version answers
-            msg.update(query=os.path.abspath(labels[0]), label=labels[0])
-        else:
-            msg.update(queries=[os.path.abspath(q) for q in labels], labels=labels)
-        if opt["max_results"]:
-            msg["max_results"] = opt["max_results"]
-        rep = daemon.request(db, dev, msg)
-        if rep is not None and rep.get("error") == "unknown op":  # a server from before this op: replace it, once
-            daemon.stop_for(db)
-            rep = None
-        if rep is not None and rep.get("stale"):  # the directory was rewritten under a running server: it has just exited
-            deadline = time.time() + 15.0
-            while time.time() < deadline and daemon.request(db, dev, {"op": "ping"}, timeout=1.0) is not None:
-                time.sleep(0.05)
-            rep = None
-        if rep is None:
-            log = open(os.path.join(db, "skani_b200_daemon.log"), "a")
-            subprocess.Popen([sys.executable, "-m", "skder_b200.daemon", db, str(dev)], stdout=log, stderr=log,
-                             stdin=subprocess.DEVNULL, start_new_session=True,
-                             cwd=os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-            deadline = time.time() + float(os.environ.get("SKB_DAEMON_START_TIMEOUT", "600"))
-            while rep is None and time.time() < deadline:
-                time.sleep(0.2)
-                if daemon.request(db, dev, {"op": "ping"}, timeout=5.0):
-                    rep = daemon.request(db, dev, msg)
-        if rep is None:
-            raise RuntimeError("search daemon did not come up (see %s/skani_b200_daemon.log)" % db)
-        if not rep.get("ok"):
-            raise RuntimeError("search daemon: %s" % rep.get("error"))
+        tmp = tempfile.mkdtemp(prefix="skani_b200.search.")
+        try:
+            out = os.path.join(tmp, "out.tsv")
+            _daemon_search(opt, labels, dev, out)
+            with open(out, "rb") as f:
+                data = f.read()
+        finally:
+            shutil.rmtree(tmp, ignore_errors=True)
+        to_stdout(data)
         return None
     if engine_mod is None:
         from . import engine as engine_mod
@@ -374,8 +472,7 @@ def run_search(opt, engine_mod):
         edges, st = eng.search(qp, screen=opt["screen"], min_af=opt["min_af"], per_sequence=opt["query_per_seq"])
         ci, detail = edge_extras(eng, opt["ci"], opt["detailed"], edges, search_contig_stats(eng) if opt["detailed"] else None)
     qlabels, qnames = query_columns(labels, qp, opt["query_per_seq"])
-    write_atomic(opt["out"], header(opt["ci"], opt["detailed"]) +
-                 "".join(rect_rows(paths + qlabels, names + qnames, edges, ci, detail)))
+    emit(opt, header(opt["ci"], opt["detailed"]) + "".join(rect_rows(paths + qlabels, names + qnames, edges, ci, detail)))
     return st
 
 
@@ -402,7 +499,7 @@ def run_dist(opt, engine_mod):
     on one side only is compared as records against itself as a whole, and one split on both sides shares its ids"""
     import itertools
 
-    refs, queries = read_list(opt["rl"]), read_list(opt["ql"])
+    refs, queries = inputs("dist", opt)
     units = list(dict.fromkeys([(p, opt["ref_per_seq"]) for p in refs] + [(p, opt["query_per_seq"]) for p in queries]))
     ids, paths, names = {}, [], []
     with engine_mod.Engine(_device()) as eng:
@@ -429,7 +526,7 @@ def run_dist(opt, engine_mod):
         edges, st = eng.rect(genome_ids(refs, opt["ref_per_seq"]), genome_ids(queries, opt["query_per_seq"]),
                              screen=opt["screen"], min_af=opt["min_af"])
         ci, detail = edge_extras(eng, opt["ci"], opt["detailed"], edges)
-    write_atomic(opt["out"], header(opt["ci"], opt["detailed"]) + "".join(rect_rows(paths, names, edges, ci, detail)))
+    emit(opt, header(opt["ci"], opt["detailed"]) + "".join(rect_rows(paths, names, edges, ci, detail)))
     return st
 
 
@@ -462,6 +559,9 @@ def _provenance(opt, sub, seconds):
     if opt.get("detailed"):
         text += ("--detailed: the 13 extra columns as DESIGN.md section 3 defines them; their names, order and definitions "
                  "are recalled, unpinned against skani's own --detailed output\n")
+    if "out" not in opt:  # the TSV went to stdout: there is no file to put the note beside
+        sys.stderr.write(text)
+        return
     try:
         write_atomic(opt["out"].rstrip("/") + ".skani_b200.log", text)
     except OSError:
