@@ -183,13 +183,14 @@ int skb_set_ani_estimator(skb_ctx *ctx, int32_t estimator);
 int skb_set_ani_ci(skb_ctx *ctx, int32_t enabled);
 /* The intervals of the edge list of the last skb_triangle, skb_rect or skb_pairs_edges call on this context (also one
  * made with edges == NULL), in edge order: lo_hi[2 i] and lo_hi[2 i + 1] are edge i's lower and upper bound, percent on
- * the ANI's scale; *n = that call's edge count.  malloc'ed (skb_free).  SKB_ESTATE if that call ran without --ci. */
+ * the ANI's scale, copied from the per-edge records skb_last_edge_detail serves (ani_lo, ani_hi); *n = that call's
+ * edge count.  malloc'ed (skb_free).  SKB_ESTATE if that call ran without --ci, also when it ran with --detailed. */
 int skb_last_edge_ci(skb_ctx *ctx, double **lo_hi, int64_t *n);
 
 /* skani's --detailed (DESIGN.md section 3): per edge, what the extra columns need beyond the contig statistics below.
  * "a" / "b" are the edge's genomes (skb_edge.a / .b). */
 typedef struct {
-    double ani_lo, ani_hi;          /* percent: the --ci interval, the same bits skb_last_edge_ci gives */
+    double ani_lo, ani_hi;          /* percent: the --ci interval; skb_last_edge_ci reads it from here */
     double sd;                      /* percent: seed-weighted standard deviation of the accepted chains' ANI */
     int64_t covered_a, covered_b;   /* bases of genome a / b in the accepted chains' extended spans (AF numerators) */
     int32_t n_chains, pad;          /* accepted chains */
@@ -200,7 +201,7 @@ typedef struct {
 int skb_set_detailed(skb_ctx *ctx, int32_t enabled);
 /* The details of the edge list of the last skb_triangle, skb_rect or skb_pairs_edges call on this context (also one
  * made with edges == NULL), in edge order; *n = that call's edge count.  malloc'ed (skb_free).  SKB_ESTATE if that call
- * ran without --detailed. */
+ * ran without --detailed, also when it ran with --ci. */
 int skb_last_edge_detail(skb_ctx *ctx, skb_edge_detail **out, int64_t *n);
 /* Host-side statistics of the kept contigs (those of at least min_contig_len: what the sketch DB holds) of genomes
  * first .. first + n - 1: n_contigs[i], and nx[3 i .. 3 i + 2] = N90, N50, N10 (DESIGN.md section 3; 0 for a genome

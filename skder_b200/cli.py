@@ -240,20 +240,21 @@ def header(ci, detailed=False):
     return HEADER[:-1] + "\tANI_5_percentile\tANI_95_percentile\n" if ci else HEADER
 
 
-def fmt_row(ref, query, ani, af_ref, af_query, ref_name, query_name, ci=None, detail=None):
-    row = "%s\t%s\t%.2f\t%.2f\t%.2f\t%s\t%s" % (ref, query, ani, af_ref, af_query, ref_name, query_name)
-    if detail is not None:
-        return row + DETAILED_FMT % detail
-    return row + ("\n" if ci is None else "\t%.2f\t%.2f\n" % ci)
-
-
-def edge_details(edges, det, n_contigs, nx):
-    """--detailed's 13 values per edge, in DETAILED_COLUMNS order.  det: Engine.last_edge_detail() of `edges`;
-    n_contigs, nx: Engine.contig_stats() of every genome id the edges hold."""
-    nc, nx = n_contigs.tolist(), nx.tolist()
-    cols = [edges["a"].tolist(), edges["b"].tolist()]
-    cols += [det[k].tolist() for k in ("ani_lo", "ani_hi", "sd", "covered_b", "n_chains")]
-    return [(nc[a], nc[b], lo, hi, sd, *nx[a], *nx[b], cov // k, cov) for a, b, lo, hi, sd, cov, k in zip(*cols)]
+def row_suffixes(eng, opt, edges, stats=None):
+    """What follows the seven columns in each row of `edges`, newline included, after an edge call run with opt's --ci
+    and --detailed: None without either (the line ends there), --ci's two columns, or --detailed's 13 in
+    DETAILED_COLUMNS order (they hold the interval, so they replace --ci's).  stats = (n_contigs, nx) of every genome
+    id the edges hold, by default Engine.contig_stats of the whole context."""
+    if opt["detailed"]:
+        det = eng.last_edge_detail()
+        nc, nx = (x.tolist() for x in (stats or eng.contig_stats(0, eng.n_genomes)))
+        cols = [edges["a"].tolist(), edges["b"].tolist()]
+        cols += [det[k].tolist() for k in ("ani_lo", "ani_hi", "sd", "covered_b", "n_chains")]
+        return [DETAILED_FMT % (nc[a], nc[b], lo, hi, sd, *nx[a], *nx[b], cov // k, cov)
+                for a, b, lo, hi, sd, cov, k in zip(*cols)]
+    if opt["ci"]:
+        return ["\t%.2f\t%.2f\n" % (lo, hi) for lo, hi in eng.last_edge_ci().tolist()]
+    return None
 
 
 def write_atomic(path, text):
@@ -264,35 +265,28 @@ def write_atomic(path, text):
     os.replace(tmp, path)
 
 
-def _cols(edges, ci, detail):
-    """the edges' columns (element access on structured arrays is slow), plus (lo, hi) per edge or None without --ci,
-    plus edge_details() per edge or None without --detailed"""
-    cols = [edges[k].tolist() for k in ("a", "b", "ani", "af_a", "af_b")]
-    cols.append([tuple(x) for x in ci.tolist()] if ci is not None else [None] * len(edges))
-    return cols + [detail if detail is not None else [None] * len(edges)]
+def triangle_rows(paths, names, edges, suffixes=None):
+    """One row per edge, in edge order.  edges: structured array (a < b, ids index paths, which are sorted).  Ref =
+    lexicographically smaller path (SURVEY.md section 4 fact 3); rows grouped by Ref.  suffixes: row_suffixes() of
+    `edges`, each ending its row."""
+    cols = [edges[k].tolist() for k in ("a", "b", "ani", "af_a", "af_b")]  # element access on structured arrays is slow
+    return ["%s\t%s\t%.2f\t%.2f\t%.2f\t%s\t%s%s" % (paths[a], paths[b], ani, afa, afb, names[a], names[b], s)
+            for a, b, ani, afa, afb, s in zip(*cols, suffixes or ["\n"] * len(edges))]
 
 
-def triangle_rows(paths_sorted, names, edges, ci=None, detail=None):
-    """edges: structured array (a < b, ids index paths_sorted).  Ref = lexicographically smaller path
-    (SURVEY.md section 4 fact 3); rows grouped by Ref.  ci: Engine.last_edge_ci() for --ci's two extra columns;
-    detail: edge_details() for --detailed's 13 (they replace ci's)."""
-    return [fmt_row(paths_sorted[a], paths_sorted[b], ani, afa, afb, names[a], names[b], iv, dt)
-            for a, b, ani, afa, afb, iv, dt in zip(*_cols(edges, ci, detail))]
-
-
-def rect_rows(paths, names, edges, ci=None, detail=None):
+def rect_rows(paths, names, edges, suffixes=None):
     """edges: a = reference id, b = query id.  Rows grouped by query, ANI descending (SURVEY.md section 4 fact 7)."""
-    rows = sorted(zip(*_cols(edges, ci, detail)), key=lambda t: (t[1], -t[2], t[0]))
-    return [fmt_row(paths[a], paths[b], ani, afa, afb, names[a], names[b], iv, dt)
-            for a, b, ani, afa, afb, iv, dt in rows]
+    rows = triangle_rows(paths, names, edges, suffixes)
+    a, b, ani = (edges[k].tolist() for k in ("a", "b", "ani"))
+    return [rows[i] for i in sorted(range(len(rows)), key=lambda i: (b[i], -ani[i], a[i]))]
 
 
-def edge_extras(eng, ci, detailed, edges, stats=None):
-    """(ci, detail) for triangle_rows / rect_rows after an edge call run with --ci / --detailed as given: stats =
-    (n_contigs, nx) of the edges' genome ids, by default Engine.contig_stats of the whole context"""
-    if detailed:
-        return None, edge_details(edges, eng.last_edge_detail(), *(stats or eng.contig_stats(0, eng.n_genomes)))
-    return (eng.last_edge_ci() if ci else None), None
+def apply_options(eng, opt):
+    """opt's ANI and output options onto `eng` for its next edge calls: the estimator, --ci, --detailed and -n"""
+    eng.set_estimator(opt["estimator"])
+    eng.set_ci(opt["ci"])
+    eng.set_detailed(opt["detailed"])
+    eng.set_max_results(opt["max_results"])
 
 
 def _device():
@@ -346,9 +340,7 @@ def run_triangle(opt, engine_mod):
     paths = inputs("triangle", opt)
     with engine_mod.Engine(_device()) as eng:
         ph["context_s"] = time.time() - t0
-        eng.set_estimator(opt["estimator"])
-        eng.set_ci(opt["ci"])
-        eng.set_detailed(opt["detailed"])
+        apply_options(eng, opt)
         eng.set_marker_compression(opt["marker_c"])
         if opt["per_seq"]:  # genomes: each file's kept records, files in sorted order
             paths, names = stream_add(eng, engine_mod, paths, opt["threads"], ph, per_sequence=True)
@@ -358,9 +350,9 @@ def run_triangle(opt, engine_mod):
         eng.index()
         t2 = time.time()
         edges, st = eng.triangle(screen=opt["screen"], min_af=opt["min_af"])
-        ci, detail = edge_extras(eng, opt["ci"], opt["detailed"], edges)
+        suffixes = row_suffixes(eng, opt, edges)
         t3 = time.time()
-    emit(opt, header(opt["ci"], opt["detailed"]) + "".join(triangle_rows(paths, names, edges, ci, detail)))
+    emit(opt, header(opt["ci"], opt["detailed"]) + "".join(triangle_rows(paths, names, edges, suffixes)))
     ph.update({"index_s": t2 - t1, "triangle_s": t3 - t2, "write_tsv_s": time.time() - t3, "total_s": time.time() - t0,
                "genomes": len(paths), "edges": int(len(edges))})
     _phase_log(opt, ph)
@@ -462,18 +454,24 @@ def run_search(opt, engine_mod):
         man = json.load(f)
     paths, names = list(man["paths"]), list(man["names"])
     with engine_mod.Engine(dev) as eng:
-        eng.set_estimator(opt["estimator"])
-        eng.set_ci(opt["ci"])
-        eng.set_detailed(opt["detailed"])
-        eng.set_max_results(opt["max_results"])
         eng.load(opt["db"])
         eng.index()
-        qp = engine_mod.pack_fasta_many(labels, opt["threads"], eng.params.min_contig_len)
-        edges, st = eng.search(qp, screen=opt["screen"], min_af=opt["min_af"], per_sequence=opt["query_per_seq"])
-        ci, detail = edge_extras(eng, opt["ci"], opt["detailed"], edges, search_contig_stats(eng) if opt["detailed"] else None)
-    qlabels, qnames = query_columns(labels, qp, opt["query_per_seq"])
-    emit(opt, header(opt["ci"], opt["detailed"]) + "".join(rect_rows(paths + qlabels, names + qnames, edges, ci, detail)))
+        text, st = search_tsv(eng, engine_mod, paths, names, labels, labels, opt)
+    emit(opt, text)
     return st
+
+
+def search_tsv(eng, engine_mod, paths, names, queries, labels, opt, db_stats=None):
+    """(TSV text, stats) of one Engine.search of the query FASTAs `queries`, whose rows show `labels`, under opt's
+    options (parse_args' keys) against the indexed database in `eng` (its genomes' `paths` and `names`).  db_stats:
+    the database's contig statistics for --detailed when the caller keeps them, else read from the context."""
+    apply_options(eng, opt)
+    packed = engine_mod.pack_fasta_many(queries, opt["threads"], eng.params.min_contig_len)
+    edges, st = eng.search(packed, screen=opt["screen"], min_af=opt["min_af"], per_sequence=opt["query_per_seq"])
+    suffixes = row_suffixes(eng, opt, edges, search_contig_stats(eng, db_stats) if opt["detailed"] else None)
+    qlabels, qnames = query_columns(labels, packed, opt["query_per_seq"])
+    rows = rect_rows(paths + qlabels, names + qnames, edges, suffixes)
+    return header(opt["ci"], opt["detailed"]) + "".join(rows), st
 
 
 def query_columns(labels, packed, per_sequence):
@@ -503,11 +501,8 @@ def run_dist(opt, engine_mod):
     units = list(dict.fromkeys([(p, opt["ref_per_seq"]) for p in refs] + [(p, opt["query_per_seq"]) for p in queries]))
     ids, paths, names = {}, [], []
     with engine_mod.Engine(_device()) as eng:
-        eng.set_estimator(opt["estimator"])
-        eng.set_ci(opt["ci"])
-        eng.set_detailed(opt["detailed"])
+        apply_options(eng, opt)
         eng.set_marker_compression(opt["marker_c"])
-        eng.set_max_results(opt["max_results"])
         for split, run in itertools.groupby(units, key=lambda u: u[1]):
             run = [p for p, _ in run]
             if split:
@@ -525,8 +520,8 @@ def run_dist(opt, engine_mod):
         eng.index()
         edges, st = eng.rect(genome_ids(refs, opt["ref_per_seq"]), genome_ids(queries, opt["query_per_seq"]),
                              screen=opt["screen"], min_af=opt["min_af"])
-        ci, detail = edge_extras(eng, opt["ci"], opt["detailed"], edges)
-    emit(opt, header(opt["ci"], opt["detailed"]) + "".join(rect_rows(paths, names, edges, ci, detail)))
+        suffixes = row_suffixes(eng, opt, edges)
+    emit(opt, header(opt["ci"], opt["detailed"]) + "".join(rect_rows(paths, names, edges, suffixes)))
     return st
 
 

@@ -1415,16 +1415,9 @@ __global__ void edge_scatter_kernel(const unsigned long long *__restrict__ pairs
     e.af_b = (o.swapped ? o.af_q : o.af_r) * 100.0;
     edges[pos[t]] = e;
 }
-// --ci only: the kept pairs' intervals in edge order, percent (edge_flag_kernel's flags, their scan)
-__global__ void edge_ci_scatter_kernel(const double2 *__restrict__ ci, int64_t n_pairs, const uint32_t *__restrict__ flag,
-                                       const uint32_t *__restrict__ pos, double2 *__restrict__ edge_ci) {
-    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= n_pairs || !flag[t]) return;
-    edge_ci[pos[t]] = make_double2(ci[t].x * 100.0, ci[t].y * 100.0);
-}
-// --detailed only: the kept pairs' details in edge order (edge_flag_kernel's flags, their scan): the interval as
-// edge_ci_scatter_kernel writes it, sd in percent, and the AF numerators picked by `swapped` as edge_scatter_kernel
-// picks the AF
+// --ci or --detailed: the kept pairs' details in edge order (edge_flag_kernel's flags, their scan): the interval and
+// sd in percent, and the AF numerators picked by `swapped` as edge_scatter_kernel picks the AF.  sd == nullptr (--ci
+// alone, no sd_kernel): sd = 0, read by nobody
 __global__ void edge_detail_scatter_kernel(const PairOut *__restrict__ po, const double2 *__restrict__ ci,
                                            const double *__restrict__ sd, int64_t n_pairs, const uint32_t *__restrict__ flag,
                                            const uint32_t *__restrict__ pos, skb_edge_detail *__restrict__ detail) {
@@ -1434,12 +1427,17 @@ __global__ void edge_detail_scatter_kernel(const PairOut *__restrict__ po, const
     skb_edge_detail d;
     d.ani_lo = ci[t].x * 100.0;
     d.ani_hi = ci[t].y * 100.0;
-    d.sd = sd[t] * 100.0;
+    d.sd = sd ? sd[t] * 100.0 : 0.0;
     d.covered_a = o.swapped ? o.span_r : o.span_q;
     d.covered_b = o.swapped ? o.span_q : o.span_r;
     d.n_chains = o.n_chains;
     d.pad = 0;
     detail[pos[t]] = d;
+}
+// skb_last_edge_ci: the interval of every edge's detail record, packed so that only it crosses to the host
+__global__ void detail_ci_gather_kernel(const skb_edge_detail *__restrict__ detail, int64_t n, double2 *__restrict__ lo_hi) {
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t < n) lo_hi[t] = make_double2(detail[t].ani_lo, detail[t].ani_hi);
 }
 
 // bookkeeping: sum over pairs of the query genome's seed count and of the chained anchors (roofline bytes)

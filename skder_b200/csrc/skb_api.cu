@@ -108,10 +108,9 @@ struct skb_ctx {
     int64_t max_results = 0;           // skb_set_max_results (skb_rect's -n; 0: all); kept across skb_clear
     const skb_edge *last_dev_edges = nullptr;  // device copy of the last triangle/rect result (skb_device_edges)
     int64_t last_n_edges = 0;
-    bool last_ci = false;                 // that call ran with --ci ...
-    const double2 *last_dev_ci = nullptr;  // ... and left the edges' intervals here (skb_last_edge_ci)
-    bool last_detailed = false;                       // that call ran with --detailed ...
-    const skb_edge_detail *last_dev_detail = nullptr;  // ... and left the edges' details here (skb_last_edge_detail)
+    bool last_ci = false, last_detailed = false;       // that call ran with --ci / --detailed ...
+    const skb_edge_detail *last_dev_detail = nullptr;  // ... and, with either, left the edges' details here
+                                                       // (skb_last_edge_ci, skb_last_edge_detail)
     std::vector<cudaEvent_t> anchor_ev;  // start/stop pairs around the anchor kernel launches of the current call
     int anchor_ev_used = 0;
     float last_ms_anchor = 0;
@@ -739,7 +738,6 @@ void pairs_to_edges(skb_ctx *c, unsigned long long *d_pairs, int64_t n_pairs, do
     CK(cudaMemsetAsync(d_n.p, 0, 32, c->st));
     CK(cudaEventRecord(ev_mid, c->st));
     c->last_ci = c->ci;
-    c->last_dev_ci = nullptr;
     c->last_detailed = c->detailed;
     c->last_dev_detail = nullptr;
     if (n_pairs > 0) {
@@ -765,13 +763,7 @@ void pairs_to_edges(skb_ctx *c, unsigned long long *d_pairs, int64_t n_pairs, do
         exclusive_scan_u32(c, d_ef.p, d_ep.p, (size_t)n_pairs);
         launch(c, edge_scatter_kernel, nblk((uint64_t)n_pairs, 256), 256, 0, d_pairs, d_out.p, n_pairs, d_ef.p, d_ep.p,
                d_edges.p, d_n.p);
-        if (c->ci) {
-            PoolRef<double2> ci_edges(c->pool["ci.edges"]);
-            ci_edges.reserve((size_t)n_pairs, 0, c->st);
-            launch(c, edge_ci_scatter_kernel, nblk((uint64_t)n_pairs, 256), 256, 0, d_ci, n_pairs, d_ef.p, d_ep.p, ci_edges.p);
-            c->last_dev_ci = ci_edges.p;
-        }
-        if (c->detailed) {
+        if (d_ci) {  // one record per edge serves both skb_last_edge_ci and skb_last_edge_detail
             PoolRef<skb_edge_detail> det_edges(c->pool["detail.edges"]);
             det_edges.reserve((size_t)n_pairs, 0, c->st);
             launch(c, edge_detail_scatter_kernel, nblk((uint64_t)n_pairs, 256), 256, 0, d_out.p, d_ci, d_sd, n_pairs, d_ef.p,
@@ -828,12 +820,6 @@ void best_n_edges(skb_ctx *c, int64_t max_n) {
     kept.reserve((size_t)n, 0, c->st);
     launch(c, best_n_scatter_kernel<skb_edge>, nb, 256, 0, c->last_dev_edges, n, d_f.p, d_p.p, kept.p);
     c->last_dev_edges = kept.p;
-    if (c->last_dev_ci) {
-        PoolRef<double2> kept_ci(c->pool["best_n.ci"]);
-        kept_ci.reserve((size_t)n, 0, c->st);
-        launch(c, best_n_scatter_kernel<double2>, nb, 256, 0, c->last_dev_ci, n, d_f.p, d_p.p, kept_ci.p);
-        c->last_dev_ci = kept_ci.p;
-    }
     if (c->last_dev_detail) {
         PoolRef<skb_edge_detail> kept_det(c->pool["best_n.detail"]);
         kept_det.reserve((size_t)n, 0, c->st);
@@ -866,14 +852,10 @@ struct EdgePairs {
 template <typename F>
 int edge_call(skb_ctx *c, double min_af_pct, skb_edge **edges, int64_t *n_edges, skb_stats *stats, F &&pairs,
               int64_t max_n = 0) {
-    // --ci is defined for the mean estimator only (DESIGN.md section 3)
-    if (c->ci && c->estimator != SKB_ANI_MEAN)
-        return fail(c, SKB_EINVAL,
-                    "the --ci interval is defined for the mean ANI estimator only (skb_set_ani_ci, skb_set_ani_estimator)");
-    // --detailed prints that interval too (DESIGN.md section 3)
-    if (c->detailed && c->estimator != SKB_ANI_MEAN)
-        return fail(c, SKB_EINVAL,
-                    "the --detailed columns are defined for the mean ANI estimator only (skb_set_detailed, skb_set_ani_estimator)");
+    // --ci is defined for the mean estimator only, and --detailed prints that interval too (DESIGN.md section 3)
+    if ((c->ci || c->detailed) && c->estimator != SKB_ANI_MEAN)
+        return fail(c, SKB_EINVAL, "the --ci interval and the --detailed columns are defined for the mean ANI estimator "
+                                   "only (skb_set_ani_ci, skb_set_detailed, skb_set_ani_estimator)");
     const int64_t launches0 = c->launches;
     cudaEvent_t *ev = call_events(c);
     CK(cudaEventRecord(ev[0], c->st));
@@ -1756,10 +1738,17 @@ int skb_last_edge_ci(skb_ctx *ctx, double **lo_hi, int64_t *n) {
         if (!lo_hi || !n) return fail(ctx, SKB_EINVAL, "bad arguments");
         if (!ctx->last_ci)
             return fail(ctx, SKB_ESTATE, "the last skb_triangle / skb_rect / skb_pairs_edges call ran without --ci (skb_set_ani_ci)");
-        double *h = (double *)last_edges_to_host(ctx, ctx->last_dev_ci, sizeof(double2));
+        // the interval is the one --detailed prints: gathered from the same records, 16 of their 48 bytes copied
+        const int64_t ne = ctx->last_n_edges;
+        PoolRef<double2> d_lo_hi(ctx->pool["ci.lo_hi"]);
+        if (ne) {
+            d_lo_hi.reserve((size_t)ne, 0, ctx->st);
+            launch(ctx, detail_ci_gather_kernel, nblk((uint64_t)ne, 256), 256, 0, ctx->last_dev_detail, ne, d_lo_hi.p);
+        }
+        double *h = (double *)last_edges_to_host(ctx, d_lo_hi.p, sizeof(double2));
         if (!h) return fail(ctx, SKB_ENOMEM, "host out of memory for the intervals");
         *lo_hi = h;
-        *n = ctx->last_n_edges;
+        *n = ne;
         return SKB_OK;
     });
 }

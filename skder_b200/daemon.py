@@ -123,6 +123,15 @@ def search_queries(msg):
     return queries, labels
 
 
+def search_options(msg):
+    """a search request's options under cli.parse_args' keys (cli.search_tsv); an absent key means its default, as an
+    older shim that never sends it intends"""
+    return {"screen": msg["screen"], "min_af": msg["min_af"], "threads": None,
+            "query_per_seq": msg["op"] == "search_records", "estimator": msg.get("estimator", "mean"),
+            "ci": bool(msg.get("ci", False)), "detailed": bool(msg.get("detailed", False)),
+            "max_results": int(msg.get("max_results", 0))}
+
+
 def serve(db_dir, device):
     from . import cli, engine
 
@@ -174,24 +183,13 @@ def serve(db_dir, device):
                         conn.send_bytes(json.dumps({"ok": True}).encode())
                         stop = True
                     elif msg.get("op") in ("search", "search_records"):
-                        per_seq = msg["op"] == "search_records"
-                        eng.set_estimator(msg.get("estimator", "mean"))  # per request: a resident server serves every mode
-                        ci, detailed = bool(msg.get("ci", False)), bool(msg.get("detailed", False))
-                        eng.set_ci(ci)
-                        eng.set_detailed(detailed)
-                        eng.set_max_results(int(msg.get("max_results", 0)))
+                        opt = search_options(msg)  # per request: a resident server serves every mode
                         queries, labels = search_queries(msg)
-                        packed = engine.pack_fasta_many(queries, None, eng.params.min_contig_len)
-                        edges, st = eng.search(packed, screen=msg["screen"], min_af=msg["min_af"], per_sequence=per_seq)
-                        stats = None
-                        if detailed:
+                        if opt["detailed"]:
                             db_stats = db_stats or eng.contig_stats(0, n_db)  # the database's, once per server
-                            stats = cli.search_contig_stats(eng, db_stats)
-                        qlabels, qnames = cli.query_columns(labels, packed, per_seq)
-                        rows = cli.rect_rows(paths + qlabels, names + qnames, edges,
-                                             *cli.edge_extras(eng, ci, detailed, edges, stats))
-                        cli.write_atomic(msg["out"], cli.header(ci, detailed) + "".join(rows))
-                        conn.send_bytes(json.dumps({"ok": True, "rows": len(rows), "ms": st.ms_total}).encode())
+                        text, st = cli.search_tsv(eng, engine, paths, names, queries, labels, opt, db_stats)
+                        cli.write_atomic(msg["out"], text)
+                        conn.send_bytes(json.dumps({"ok": True, "rows": st.n_edges, "ms": st.ms_total}).encode())
                     else:
                         conn.send_bytes(json.dumps({"ok": False, "error": "unknown op"}).encode())
                 except Exception as e:  # the shim turns this into "no output file"

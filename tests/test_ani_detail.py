@@ -6,6 +6,7 @@ import itertools
 import os
 import subprocess
 import sys
+import types
 
 import numpy as np
 import pytest
@@ -82,7 +83,7 @@ def test_parser_accepts_detailed():
     assert cli.header(True) == cli.HEADER[:-1] + "\tANI_5_percentile\tANI_95_percentile\n"
 
 
-def test_rows_carry_the_detail_through_the_sort():
+def test_row_suffixes_follow_their_edges_through_the_sort():
     from skder_b200 import cli
     from skder_b200.engine import DETAIL_DTYPE, EDGE_DTYPE
 
@@ -92,14 +93,19 @@ def test_rows_carry_the_detail_through_the_sort():
                                                                             (98.5, 99.5, 0.5, 20, 3000, 3)]
     cnt = np.array([3, 4, 5], np.int32)
     nx = np.array([[1, 2, 3], [4, 5, 6], [7, 8, 9]], np.int64)
-    detail = cli.edge_details(edges, det, cnt, nx)
-    assert detail == [(3, 5, 96.5, 97.5, 1.25, 1, 2, 3, 7, 8, 9, 500, 1001),
-                      (4, 5, 98.5, 99.5, 0.5, 4, 5, 6, 7, 8, 9, 1000, 3000)]
-    rows = cli.rect_rows(["/r1", "/r2", "/q"], ["n1", "n2", "nq"], edges, None, detail)  # ANI descending: r2 first
+    # the two Engine calls row_suffixes makes after an edge call
+    eng = types.SimpleNamespace(last_edge_detail=lambda: det, last_edge_ci=lambda: np.array([[1.0, 2.0], [3.0, 4.0]]))
+    detail = cli.row_suffixes(eng, {"ci": False, "detailed": True}, edges, (cnt, nx))
+    assert detail == [cli.DETAILED_FMT % (3, 5, 96.5, 97.5, 1.25, 1, 2, 3, 7, 8, 9, 500, 1001),
+                      cli.DETAILED_FMT % (4, 5, 98.5, 99.5, 0.5, 4, 5, 6, 7, 8, 9, 1000, 3000)]
+    rows = cli.rect_rows(["/r1", "/r2", "/q"], ["n1", "n2", "nq"], edges, detail)  # ANI descending: r2 first
     assert rows == ["/r2\t/q\t99.00\t90.00\t91.00\tn2\tnq\t4\t5\t98.50\t99.50\t0.50\t4\t5\t6\t7\t8\t9\t1000\t3000\n",
                     "/r1\t/q\t97.00\t80.00\t81.00\tn1\tnq\t3\t5\t96.50\t97.50\t1.25\t1\t2\t3\t7\t8\t9\t500\t1001\n"]
-    assert cli.triangle_rows(["/a", "/b", "/c"], ["na", "nb", "nc"], edges, np.array([[1.0, 2.0], [3.0, 4.0]]),
-                             detail)[0].endswith("\t1\t2\t3\t7\t8\t9\t500\t1001\n")  # the detail replaces --ci's columns
+    assert cli.row_suffixes(eng, {"ci": True, "detailed": False}, edges) == ["\t1.00\t2.00\n", "\t3.00\t4.00\n"]
+    assert cli.row_suffixes(eng, {"ci": False, "detailed": False}, edges) is None
+    both = cli.row_suffixes(eng, {"ci": True, "detailed": True}, edges, (cnt, nx))
+    assert cli.triangle_rows(["/a", "/b", "/c"], ["na", "nb", "nc"], edges,
+                             both)[0].endswith("\t1\t2\t3\t7\t8\t9\t500\t1001\n")  # the detail replaces --ci's columns
 
 
 def test_cpu_reference_follows_the_definition(oracle, genomes7):

@@ -247,7 +247,12 @@ def test_skani_shim_triangle_dist_search_bytes_equal_oracle(genomes7, oracle, bu
     assert _run_shim(["sketch", "-l", str(lst), "-o", str(db), "-t", "4"]) == 0 and db.is_dir()
     sout = tmp_path / "current_search_results.tsv"
     q = genomes7[2]
-    assert _run_shim(["search", q, "-d", str(db), "-o", str(sout), "-t", "4"]) == 0
+    from skder_b200 import daemon
+
+    try:
+        assert _run_shim(["search", q, "-d", str(db), "-o", str(sout), "-t", "4"]) == 0
+    finally:
+        daemon.stop_for(str(db))  # the search started the database's server: it must not outlive the test
     rows = [ln.split("\t") for ln in sout.read_text().splitlines()[1:]]
     assert len(rows) == 7 and all(r[1] == q for r in rows)  # 6 partners + the genome's own copy in the DB
     self_row = [r for r in rows if r[0] == q][0]

@@ -152,7 +152,7 @@ def test_cpu_reference_against_restatement(oracle, tmp_path):
 
 # ---- the daemon protocol ------------------------------------------------------------------------------------------------
 def test_daemon_request_forms():
-    from skder_b200 import daemon
+    from skder_b200 import cli, daemon
 
     assert daemon.search_queries({"query": "/a.fa", "label": "a.fa"}) == (["/a.fa"], ["a.fa"])
     assert daemon.search_queries({"query": "/a.fa"}) == (["/a.fa"], ["/a.fa"])
@@ -160,6 +160,14 @@ def test_daemon_request_forms():
     for bad in ({"queries": []}, {"queries": ["/a", "/b"], "labels": ["a"]}):
         with pytest.raises(ValueError):
             daemon.search_queries(bad)
+    # a request's options under the parser's keys; an absent one (an older shim's request) at the parser's default
+    keys = ("estimator", "ci", "detailed", "max_results", "query_per_seq")
+    for argv, msg in (("", {"op": "search"}), (" --median", {"op": "search", "estimator": "median"}),
+                      (" --ci --detailed -n 2 --qi",
+                       {"op": "search_records", "ci": True, "detailed": True, "max_results": 2})):
+        opt = daemon.search_options(dict(msg, screen=80.0, min_af=15.0))
+        want = cli.parse_args(("search q.fa -d db" + argv).split())[1]
+        assert [opt[k] for k in keys] == [want[k] for k in keys], argv
 
 
 def _shim_through_stand_in(tmp_path, args):
