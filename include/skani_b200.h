@@ -272,6 +272,29 @@ int skb_device_edges(skb_ctx *ctx, const skb_edge **dev_edges, int64_t *n_edges)
 int skb_greedy_summary(skb_ctx *ctx, const skb_edge *edges, int64_t n_edges, int32_t n_genomes, double min_ani, double min_af,
                        int64_t **connectivity, int64_t **member_off, uint32_t **members);
 
+/* ---- skani's `triangle --full-matrix [--distance]` (DESIGN.md section 3) -------------------------------------------
+ * Writes the whole file at `path`: the line "N\n" (N = n_genomes), then per genome r in id order its label (labels
+ * bytes label_off[r] .. label_off[r + 1]), for every genome c in id order '\t' and the cell (r, c) as `%.2f` text, then
+ * '\n'.  The value of a cell is read from the edge {r, c}'s printed `%.2f` text, in hundredths:
+ *   SKB_MATRIX_ANI       r = c: 100.00; an edge: its ANI; no edge: 0.00.
+ *   SKB_MATRIX_DISTANCE  100.00 minus the SKB_MATRIX_ANI cell, computed on the printed hundredths (10000 - cents), so
+ *                        the two files are exact complements: the diagonal 0.00, no edge 100.00.
+ *   SKB_MATRIX_AF        r = c: 100.00; an edge: genome r's aligned fraction (af_a if r is the edge's a, else af_b), so
+ *                        the matrix is not symmetric; no edge: 0.00.
+ * edges == NULL: the device edge list of the last skb_triangle (the one skb_device_edges serves); n_edges is ignored and
+ * n_genomes must equal the context's genome count.  SKB_ESTATE if the last edge call was skb_rect or skb_pairs_edges,
+ * a partition of the triangle (n_parts > 1), or if genomes were added, removed or cleared since.
+ * edges != NULL: a host list, strictly increasing in (a, b), a < b < n_genomes, every value finite in [0, 100];
+ * otherwise SKB_EINVAL.  A multi-GPU rank holding a gathered list passes it this way.
+ * The text is rendered on the device in blocks of rows (at most SKB_MATRIX_BLOCK_MB MiB of device scratch, default
+ * 1024) and written while the next block renders.  SKB_EINVAL for an unknown kind, SKB_EIO on a write failure (the file
+ * may then be partial: the caller makes the write atomic), SKB_ELIMIT if one row does not fit the device. */
+#define SKB_MATRIX_ANI 0
+#define SKB_MATRIX_DISTANCE 1
+#define SKB_MATRIX_AF 2
+int skb_write_matrix(skb_ctx *ctx, const char *path, int32_t kind, const skb_edge *edges, int64_t n_edges,
+                     int32_t n_genomes, const char *labels, const int64_t *label_off /* [n_genomes + 1] */);
+
 void skb_free(void *p);
 
 /* total kernels launched by this context so far (bench.py's gpu_launches) */

@@ -111,7 +111,7 @@ SYMBOLS = [
     "skb_device_edges", "skb_set_owned", "skb_screen_triangle", "skb_pairs_edges", "skb_greedy_summary", "skb_index_seed_tables", "skb_clear_keep_tables",
     "skb_set_ani_estimator", "skb_set_ani_ci", "skb_last_edge_ci", "skb_set_detailed", "skb_last_edge_detail",
     "skb_genome_contig_stats", "skb_set_marker_compression", "skb_marker_compression", "skb_set_max_results",
-    "skb_add_sequences",
+    "skb_add_sequences", "skb_write_matrix",
 ]
 
 _lib = None
@@ -174,6 +174,8 @@ def lib():
                                   C.POINTER(C.c_int64), C.POINTER(Stats)]
     L.skb_greedy_summary.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_double, C.c_double,
                                      C.POINTER(C.POINTER(C.c_int64)), C.POINTER(C.POINTER(C.c_int64)), C.POINTER(C.POINTER(C.c_uint32))]
+    L.skb_write_matrix.argtypes = [C.c_void_p, C.c_char_p, C.c_int32, C.c_void_p, C.c_int64, C.c_int32, C.c_char_p,
+                                   C.c_void_p]
     L.skb_clear.argtypes = [C.c_void_p]
     L.skb_set_ani_estimator.argtypes = [C.c_void_p, C.c_int32]
     L.skb_set_ani_ci.argtypes = [C.c_void_p, C.c_int32]

@@ -41,6 +41,10 @@ not depend on it.  A database records its M, and `search` sketches the query at 
 skani's per-sequence mode -- `-i` (triangle, sketch), `--qi` (dist, search), `--ri` (dist) -- makes every record of at
 least 500 bp of the flagged files a genome of its own, named by its file and header (DESIGN.md section 3); skDER keys
 its selection on whole files, so a `-p` with -i breaks it.
+`triangle --full-matrix [--distance]` (instead of -E) writes skani's square matrices, rendered on the device
+(DESIGN.md section 3): the ANI matrix to -o OUT or stdout (with --distance 100 minus each printed ANI), the AF matrix to
+OUT.af, or without -o to ./skani_matrix.af.  Both go to temporaries and are renamed only when both are complete.  The
+lower-triangular default and --diagonal are not implemented, nor --full-matrix with --ci or --detailed.
 Any other skani option (-c, --fast, --slow, --medium, --small-genomes, --no-learned-ani, ...) changes skani's
 estimator in ways this engine does not implement: the shim then exits non-zero WITHOUT creating the output, which is
 the one failure signal runCmd checks (util.py:642-645).
@@ -81,8 +85,9 @@ def parse_args(argv):
     }
     multi = {"-q": "q", "-r": "r"}  # dist's FASTA lists: every following token up to the next one starting with '-'
     flags = {"-E": "edge_list", "--sparse": "edge_list", "--ci": "ci", "--detailed": "detailed", "-i": "per_seq",
-             "--qi": "query_per_seq", "--ri": "ref_per_seq"}
+             "--qi": "query_per_seq", "--ri": "ref_per_seq", "--full-matrix": "full_matrix", "--distance": "distance"}
     opt["ci"] = opt["detailed"] = opt["per_seq"] = opt["query_per_seq"] = opt["ref_per_seq"] = False
+    opt["full_matrix"] = opt["distance"] = False
     estimators = {"--median": "median", "--robust": "robust"}
     chosen = []
     i = 1
@@ -166,8 +171,18 @@ def parse_args(argv):
             raise UsageError("skani %s: missing required option for %r" % (sub, k))
     if sub in ("triangle", "sketch") and "list" not in opt and not opt["positional"]:
         raise UsageError("skani %s: no genome given (FASTA arguments and/or -l LIST)" % sub)
-    if sub == "triangle" and not opt["edge_list"]:
-        raise UsageError("skani triangle without -E (matrix output) is not implemented; skDER always passes -E")
+    for flag, key in (("--full-matrix", "full_matrix"), ("--distance", "distance")):
+        if opt[key] and sub != "triangle":
+            raise UsageError("skani %s takes no %s: it is an output form of triangle" % (sub, flag))
+    if opt["full_matrix"] and opt["edge_list"]:
+        raise UsageError("--full-matrix and -E are two output forms of triangle: give one")
+    if opt["distance"] and not opt["full_matrix"]:
+        raise UsageError("--distance is implemented for --full-matrix only")
+    if opt["full_matrix"] and (opt["ci"] or opt["detailed"]):
+        raise UsageError("--full-matrix has no place for the %s columns" % ("--ci" if opt["ci"] else "--detailed"))
+    if sub == "triangle" and not opt["edge_list"] and not opt["full_matrix"]:
+        raise UsageError("skani triangle without -E (lower-triangular matrix output) is not implemented; use -E or "
+                         "--full-matrix")
     if sub == "search" and not opt["positional"] and "ql" not in opt:
         raise UsageError("skani search: no query FASTA given")
     if sub == "dist":
@@ -257,9 +272,13 @@ def row_suffixes(eng, opt, edges, stats=None):
     return None
 
 
+def tmp_beside(path):
+    """the temporary that write_atomic and write_matrices fill before renaming it to `path`"""
+    return os.path.join(os.path.dirname(os.path.abspath(path)), ".%s.tmp.%d" % (os.path.basename(path), os.getpid()))
+
+
 def write_atomic(path, text):
-    d = os.path.dirname(os.path.abspath(path))
-    tmp = os.path.join(d, ".%s.tmp.%d" % (os.path.basename(path), os.getpid()))
+    tmp = tmp_beside(path)
     with open(tmp, "w") as f:
         f.write(text)
     os.replace(tmp, path)
@@ -349,14 +368,55 @@ def run_triangle(opt, engine_mod):
         t1 = time.time()
         eng.index()
         t2 = time.time()
-        edges, st = eng.triangle(screen=opt["screen"], min_af=opt["min_af"])
-        suffixes = row_suffixes(eng, opt, edges)
-        t3 = time.time()
-    emit(opt, header(opt["ci"], opt["detailed"]) + "".join(triangle_rows(paths, names, edges, suffixes)))
-    ph.update({"index_s": t2 - t1, "triangle_s": t3 - t2, "write_tsv_s": time.time() - t3, "total_s": time.time() - t0,
-               "genomes": len(paths), "edges": int(len(edges))})
+        edges, st = eng.triangle(screen=opt["screen"], min_af=opt["min_af"], to_host=not opt["full_matrix"])
+        if opt["full_matrix"]:  # rendered from the device edge list, so while the context lives
+            t3 = time.time()
+            write_matrices(eng, opt, names if opt["per_seq"] else paths)
+        else:
+            suffixes = row_suffixes(eng, opt, edges)
+            t3 = time.time()
+    if not opt["full_matrix"]:
+        emit(opt, header(opt["ci"], opt["detailed"]) + "".join(triangle_rows(paths, names, edges, suffixes)))
+    ph.update({"index_s": t2 - t1, "triangle_s": t3 - t2, "write_matrix_s" if opt["full_matrix"] else "write_tsv_s":
+               time.time() - t3, "total_s": time.time() - t0, "genomes": len(paths), "edges": int(st.n_edges)})
     _phase_log(opt, ph)
     return st
+
+
+MATRIX_AF_DEFAULT = "skani_matrix.af"  # the AF matrix without -o, in the working directory
+
+
+def write_matrices(eng, opt, labels):
+    """--full-matrix after a whole Engine.triangle: the ANI matrix (--distance: 100 minus each printed ANI) for -o or
+    stdout, the AF matrix for OUT.af or ./skani_matrix.af, one row per genome labelled `labels[i]` (DESIGN.md section
+    3).  Both are rendered into temporaries beside their targets and renamed only once both are complete; without -o
+    the finished ANI file is then copied to stdout.  On failure neither target is created and the temporaries go."""
+    import shutil
+    import tempfile
+
+    af_path = opt["out"] + ".af" if "out" in opt else MATRIX_AF_DEFAULT
+    tmps = []
+    try:
+        if "out" in opt:
+            tmps.append(tmp_beside(opt["out"]))
+        else:
+            fd, t = tempfile.mkstemp(prefix="skani_b200.matrix.")
+            os.close(fd)
+            tmps.append(t)
+        tmps.append(tmp_beside(af_path))
+        eng.write_matrix(tmps[0], labels, "distance" if opt["distance"] else "ani")
+        eng.write_matrix(tmps[1], labels, "af")
+        if "out" in opt:
+            os.replace(tmps[0], opt["out"])
+        os.replace(tmps[1], af_path)
+        if "out" not in opt:
+            sys.stdout.flush()
+            with open(tmps[0], "rb") as f, open(sys.stdout.fileno(), "wb", closefd=False) as o:
+                shutil.copyfileobj(f, o, 1 << 24)
+    finally:
+        for t in tmps:
+            if os.path.exists(t):
+                os.unlink(t)
 
 
 def run_sketch(opt, engine_mod):
@@ -551,6 +611,13 @@ def _provenance(opt, sub, seconds):
                  "skani turns its learned ANI debias off in this mode, this engine keeps its debias substitute on -- the "
                  "difference is unpinned against skani\n"
                  % " ".join(f for f, k in (("-i", "per_seq"), ("--qi", "query_per_seq"), ("--ri", "ref_per_seq")) if opt[k]))
+    if opt.get("full_matrix"):
+        text += ("--full-matrix: the ANI and AF matrices as DESIGN.md section 3 defines them (every off-diagonal cell is "
+                 "the ANI / AF text of the -E row of that pair, 0.00 without one); their layout and the AF file's name "
+                 "are recalled, unpinned against skani's own matrices\n")
+    if opt.get("distance"):
+        text += ("--distance: every ANI cell is 100.00 minus its printed ANI, in hundredths (DESIGN.md section 3); "
+                 "unpinned against skani's own --distance\n")
     if opt.get("detailed"):
         text += ("--detailed: the 13 extra columns as DESIGN.md section 3 defines them; their names, order and definitions "
                  "are recalled, unpinned against skani's own --detailed output\n")

@@ -19,6 +19,7 @@
 #include "skb_best_n.cuh"
 #include "skb_common.cuh"
 #include "skb_index.cuh"
+#include "skb_matrix.cuh"
 #include "skb_sketch.cuh"
 
 using namespace skb;
@@ -111,6 +112,11 @@ struct skb_ctx {
     bool last_ci = false, last_detailed = false;       // that call ran with --ci / --detailed ...
     const skb_edge_detail *last_dev_detail = nullptr;  // ... and, with either, left the edges' details here
                                                        // (skb_last_edge_ci, skb_last_edge_detail)
+    uint64_t genome_set = 0;       // bumped by every call that adds, removes or clears genomes
+    int64_t whole_triangle = -1;   // genome_set of the whole skb_triangle that made last_dev_edges, else -1
+                                   // (skb_write_matrix with edges == NULL)
+    char *h_matrix[2] = {};        // pinned text of two row blocks (skb_write_matrix)
+    size_t h_matrix_cap[2] = {};
     std::vector<cudaEvent_t> anchor_ev;  // start/stop pairs around the anchor kernel launches of the current call
     int anchor_ev_used = 0;
     float last_ms_anchor = 0;
@@ -857,6 +863,7 @@ int edge_call(skb_ctx *c, double min_af_pct, skb_edge **edges, int64_t *n_edges,
         return fail(c, SKB_EINVAL, "the --ci interval and the --detailed columns are defined for the mean ANI estimator "
                                    "only (skb_set_ani_ci, skb_set_detailed, skb_set_ani_estimator)");
     const int64_t launches0 = c->launches;
+    c->whole_triangle = -1;
     cudaEvent_t *ev = call_events(c);
     CK(cudaEventRecord(ev[0], c->st));
     EdgePairs p;
@@ -1006,6 +1013,8 @@ void skb_destroy(skb_ctx *ctx) {
     if (ctx->t1) cudaEventDestroy(ctx->t1);
     for (cudaEvent_t e : ctx->call_ev)
         if (e) cudaEventDestroy(e);
+    for (char *p : ctx->h_matrix)
+        if (p) cudaFreeHost(p);
     if (ctx->st) {
         cudaStreamSynchronize(ctx->st);
         cudaStreamDestroy(ctx->st);
@@ -1031,6 +1040,7 @@ void skb_free(void *p) { std::free(p); }
 static int clear_impl(skb_ctx *ctx, bool keep_tables) {
     return guarded(ctx, [&]() -> int {
         CK(cudaStreamSynchronize(ctx->st));
+        ctx->genome_set++;
         ctx->db.clear();
         ctx->ix.clear();
         ctx->indexed = false;
@@ -1069,6 +1079,7 @@ int skb_timer_stop(skb_ctx *ctx, float *ms) {
 // skb_add_genomes (per_seq = false: one genome per packed file) and skb_add_sequences (per_seq: one per kept contig)
 static int add_impl(skb_ctx *ctx, int32_t n, const skb_packed *const *genomes, bool per_seq) {
     return guarded(ctx, [&]() -> int {
+        ctx->genome_set++;
         if (n < 0 || (n > 0 && !genomes)) return fail(ctx, SKB_EINVAL, "bad genome list");
         uint64_t n_new = per_seq ? 0 : (uint64_t)n;
         for (int32_t i = 0; i < n; i++) {
@@ -1457,6 +1468,7 @@ int skb_pop_last_add(skb_ctx *ctx) {
         const skb_ctx::AddCall a = c->add_calls.back();
         if (a.n_before < c->ix.n_inv_genomes) return fail(c, SKB_ESTATE, "cannot pop genomes that are part of the inverted index");
         CK(cudaStreamSynchronize(c->st));
+        c->genome_set++;
         c->add_calls.pop_back();
         c->db.truncate(a.n_before, a.mkeys_before);
         c->ix.truncate(c->db);
@@ -1567,8 +1579,10 @@ int skb_triangle(skb_ctx *ctx, double screen_pct, double min_af_pct, int32_t par
                  skb_edge **edges, int64_t *n_edges, skb_stats *stats) {
     return guarded(ctx, [&]() -> int {
         if (!n_edges) return fail(ctx, SKB_EINVAL, "bad arguments");
-        return edge_call(ctx, min_af_pct, edges, n_edges, stats,
-                         [&](EdgePairs &p) { return screen_triangle_impl(ctx, screen_pct, part, n_parts, p); });
+        const int rc = edge_call(ctx, min_af_pct, edges, n_edges, stats,
+                                 [&](EdgePairs &p) { return screen_triangle_impl(ctx, screen_pct, part, n_parts, p); });
+        if (rc == SKB_OK && n_parts == 1) ctx->whole_triangle = (int64_t)ctx->genome_set;
+        return rc;
     });
 }
 
@@ -1932,6 +1946,7 @@ int skb_db_load(skb_ctx *ctx, const char *dir) {
         skb_ctx *c = ctx;
         if (!dir) return fail(c, SKB_EINVAL, "no directory");
         if (c->n() != 0) return fail(c, SKB_ESTATE, "context already holds genomes");
+        c->genome_set++;
         const std::string path = std::string(dir) + "/sketches.skb";
         FILE *f = fopen(path.c_str(), "rb");
         if (!f) return fail(c, SKB_EIO, "cannot open " + path);
@@ -1982,19 +1997,9 @@ int skb_sketch_view_get(skb_ctx *ctx, skb_sketch_view *v) {
 
 // ---- binary hand-off to skDER's greedy selection -------------------------------------------------------------------
 // The value skDER's consumers see is the 2-decimal TEXT of an edge (`%.2f`, parsed back with stod): thresholds are
-// applied to that, not to the unrounded double.  round2() reproduces it exactly: x * 100 as an error-free product
-// (p + e), round-half-even on the exact value, one correctly rounded division.
-__device__ __forceinline__ double round2(double x) {
-    const double p = x * 100.0, e = fma(x, 100.0, -p);  // x * 100 == p + e exactly
-    double r = floor(p);
-    const double f = p - r;  // exact: p < 2^52
-    if (f > 0.5 || (f == 0.5 && (e > 0.0 || (e == 0.0 && fmod(r, 2.0) != 0.0)))) r += 1.0;
-    else if (f == 0.0 && e < 0.0) {
-        // p is an integer but the exact product lies just below it: the digits after the point are .99999..., which
-        // round back up to p -- nothing to do
-    }
-    return r / 100.0;
-}
+// applied to that, not to the unrounded double.  round2() reproduces it exactly: the printed hundredths
+// (skb_common.cuh), one correctly rounded division.
+__device__ __forceinline__ double round2(double x) { return hundredths(x) / 100.0; }
 // reference src/skDER/skDERsum.cpp:107-124: an edge (col0 = a, col1 = b, ANI, AF_a, AF_b) with ANI >= min_ani gives
 // genome a the member b if AF_b >= min_af, and genome b the member a if AF_a >= min_af
 __global__ void summary_keys_kernel(const skb_edge *__restrict__ edges, int64_t n, double min_ani, double min_af,
@@ -2039,6 +2044,7 @@ int skb_import_sketches(skb_ctx *ctx, int32_t n_genomes, const uint64_t *dev_see
         if (n_genomes < 0 || n_seeds < 0 || n_marker_keys < 0) return fail(c, SKB_EINVAL, "bad arguments");
         if (n_genomes == 0) return SKB_OK;
         if ((uint64_t)c->n() + (uint64_t)n_genomes >= GID_MASK) return fail(c, SKB_ELIMIT, "too many genomes");
+        c->genome_set++;
         const uint64_t cur = c->db.seed_off.back();
         c->add_calls.push_back({c->n(), c->db.n_mkeys});  // skb_pop_last_add undoes an import like an add
         c->d_seeds.reserve(cur + (uint64_t)n_seeds + 1, cur, c->st);
@@ -2129,6 +2135,146 @@ int skb_greedy_summary(skb_ctx *ctx, const skb_edge *edges, int64_t n_edges, int
         *member_off = off;
         *members = mem;
         return SKB_OK;
+    });
+}
+
+// ---- skani's triangle --full-matrix [--distance] (skb_matrix.cuh) ---------------------------------------------------
+int skb_write_matrix(skb_ctx *ctx, const char *path, int32_t kind, const skb_edge *edges, int64_t n_edges,
+                     int32_t n_genomes, const char *labels, const int64_t *label_off) {
+    return guarded(ctx, [&]() -> int {
+        skb_ctx *c = ctx;
+        if (!path || n_genomes < 0 || !label_off) return fail(c, SKB_EINVAL, "bad arguments");
+        if (kind != SKB_MATRIX_ANI && kind != SKB_MATRIX_DISTANCE && kind != SKB_MATRIX_AF)
+            return fail(c, SKB_EINVAL, "unknown matrix kind " + std::to_string(kind));
+        const int32_t n = n_genomes;
+        if (label_off[0] != 0) return fail(c, SKB_EINVAL, "label offsets must start at 0");
+        int64_t max_label = 0;
+        for (int32_t g = 0; g < n; g++) {
+            if (label_off[g + 1] < label_off[g]) return fail(c, SKB_EINVAL, "label offsets must not decrease");
+            max_label = std::max(max_label, label_off[g + 1] - label_off[g]);
+        }
+        if (label_off[n] && !labels) return fail(c, SKB_EINVAL, "no label bytes");
+        const skb_edge *d_edges = nullptr;
+        if (edges) {
+            if (n_edges < 0) return fail(c, SKB_EINVAL, "bad edge count");
+            for (int64_t i = 0; i < n_edges; i++) {
+                const skb_edge &e = edges[i];
+                if (!(e.a < e.b && e.b < (uint32_t)n)) return fail(c, SKB_EINVAL, "edge " + std::to_string(i) + ": ids out of range");
+                if (i && !(edges[i - 1].a < e.a || (edges[i - 1].a == e.a && edges[i - 1].b < e.b)))
+                    return fail(c, SKB_EINVAL, "edge " + std::to_string(i) + ": the list is not strictly increasing in (a, b)");
+                for (double x : {e.ani, e.af_a, e.af_b})
+                    if (!(x >= 0.0 && x <= 100.0)) return fail(c, SKB_EINVAL, "edge " + std::to_string(i) + ": a value outside [0, 100]");
+            }
+            if (n_edges >= (1ll << 31)) return fail(c, SKB_ELIMIT, "too many edges for the 32-bit cell map");
+            PoolRef<skb_edge> up(c->pool["matrix.edges"]);
+            up.reserve((size_t)std::max<int64_t>(n_edges, 1), 0, c->st);
+            if (n_edges) CK(cudaMemcpyAsync(up.p, edges, (size_t)n_edges * sizeof(skb_edge), cudaMemcpyHostToDevice, c->st));
+            d_edges = up.p;
+        } else {
+            if (c->whole_triangle < 0 || (uint64_t)c->whole_triangle != c->genome_set)
+                return fail(c, SKB_ESTATE, "no whole-triangle edge list: the last edge call was not a whole skb_triangle, or "
+                                           "genomes were added, removed or cleared since");
+            if (n != c->n()) return fail(c, SKB_EINVAL, "n_genomes differs from the context's genome count");
+            d_edges = c->last_dev_edges;
+            n_edges = c->last_n_edges;
+            if (n_edges >= (1ll << 31)) return fail(c, SKB_ELIMIT, "too many edges for the 32-bit cell map");
+        }
+        // rows per block: the cell map (4 bytes a cell), the row offsets and the text (at most 7 bytes a cell of values
+        // in [0, 100]) of R rows within the budget and within what the device has free
+        const char *mb = std::getenv("SKB_MATRIX_BLOCK_MB");
+        const uint64_t budget = (uint64_t)(mb && std::atoll(mb) > 0 ? std::atoll(mb) : 1024) << 20;
+        size_t free_b = 0, total_b = 0;
+        CK(cudaMemGetInfo(&free_b, &total_b));
+        const uint64_t per_row = 4ull * (uint64_t)n + 16 + (uint64_t)max_label + 1 + 7ull * (uint64_t)n;
+        const uint64_t room = free_b / 10 * 9;
+        if (n && per_row > room) return fail(c, SKB_ELIMIT, "one matrix row does not fit the device");
+        const int32_t R = n ? (int32_t)std::clamp<uint64_t>(std::min(budget, room) / per_row, 1, (uint64_t)n) : 0;
+
+        struct File {
+            FILE *f;
+            ~File() { if (f) fclose(f); }
+        } out{fopen(path, "wb")};
+        if (!out.f) return fail(c, SKB_EIO, std::string("cannot create ") + path);
+        const std::string first = std::to_string(n) + "\n";
+        if (!write_all(out.f, first.data(), first.size())) return fail(c, SKB_EIO, std::string("write failed: ") + path);
+        if (n == 0) {
+            FILE *f = out.f;
+            out.f = nullptr;
+            return fclose(f) == 0 ? SKB_OK : fail(c, SKB_EIO, std::string("write failed: ") + path);
+        }
+        PoolRef<char> d_labels(c->pool["matrix.labels"]), d_text(c->pool["matrix.text"]);
+        PoolRef<int64_t> d_label_off(c->pool["matrix.label_off"]);
+        PoolRef<int32_t> d_map(c->pool["matrix.map"]);
+        PoolRef<uint64_t> d_len(c->pool["matrix.row_len"]), d_off(c->pool["matrix.row_off"]);
+        d_labels.reserve((size_t)label_off[n] + 1, 0, c->st);
+        if (label_off[n]) CK(cudaMemcpyAsync(d_labels.p, labels, (size_t)label_off[n], cudaMemcpyHostToDevice, c->st));
+        d_label_off.reserve((size_t)n + 1, 0, c->st);
+        CK(cudaMemcpyAsync(d_label_off.p, label_off, ((size_t)n + 1) * 8, cudaMemcpyHostToDevice, c->st));
+        d_map.reserve((size_t)R * n, 0, c->st);
+        d_len.reserve((size_t)R + 1, 0, c->st);
+        d_off.reserve((size_t)R + 1, 0, c->st);
+        d_text.reserve((size_t)R * (per_row - 4ull * n - 16), 0, c->st);
+
+        struct Events {
+            cudaEvent_t rendered = nullptr, copied[2] = {};
+            ~Events() {
+                for (cudaEvent_t e : {rendered, copied[0], copied[1]})
+                    if (e) cudaEventDestroy(e);
+            }
+        } ev;
+        if (!c->st_copy) CK(cudaStreamCreateWithFlags(&c->st_copy, cudaStreamNonBlocking));
+        CK(cudaEventCreateWithFlags(&ev.rendered, cudaEventDisableTiming));
+        for (cudaEvent_t &e : ev.copied) CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+        // block k: the map, the row lengths and their scan, the block's size to the host; then its text is written on
+        // st and copied into pinned slot k % 2 on st_copy while the host writes block k - 1 to the file
+        uint64_t bytes[2] = {0, 0};
+        int64_t k = 0;
+        struct Drain {  // whatever else happens, no copy into a pinned slot is in flight when the call returns
+            cudaStream_t s;
+            ~Drain() { cudaStreamSynchronize(s); }
+        } drain{c->st_copy};
+        for (int32_t r0 = 0; r0 < n; r0 += R, k++) {
+            const int32_t rows = std::min(R, n - r0);
+            const int s = (int)(k & 1);
+            CK(cudaMemsetAsync(d_map.p, 0xff, (size_t)rows * n * 4, c->st));
+            if (n_edges)
+                launch(c, matrix_scatter_kernel, nblk((uint64_t)n_edges, 256), 256, 0, d_edges, n_edges, n, r0, rows, d_map.p);
+            launch(c, matrix_row_len_kernel, (unsigned)rows, MX_THREADS, 0, d_map.p, d_edges, d_label_off.p, n, r0, kind, d_len.p);
+            CK(cudaMemsetAsync(d_len.p + rows, 0, 8, c->st));
+            cub_run(c, 2, [&](void *tmp, size_t &b) {
+                return cub::DeviceScan::ExclusiveSum(tmp, b, d_len.p, d_off.p, rows + 1, c->st);
+            });
+            CK(cudaMemcpyAsync(&bytes[s], d_off.p + rows, 8, cudaMemcpyDeviceToHost, c->st));
+            CK(cudaStreamSynchronize(c->st));
+            if (bytes[s] > d_text.b.cap) {  // values outside [0, 100] print longer: the previous copy must be done
+                if (k) CK(cudaEventSynchronize(ev.copied[s ^ 1]));
+                d_text.reserve(bytes[s], 0, c->st);
+            }
+            if (bytes[s] > c->h_matrix_cap[s]) {  // slot s last held block k - 2, written to the file already
+                if (c->h_matrix[s]) CK(cudaFreeHost(c->h_matrix[s]));
+                c->h_matrix[s] = nullptr;
+                c->h_matrix_cap[s] = 0;
+                CK(cudaHostAlloc((void **)&c->h_matrix[s], bytes[s], cudaHostAllocDefault));
+                c->h_matrix_cap[s] = bytes[s];
+            }
+            if (k) CK(cudaStreamWaitEvent(c->st, ev.copied[s ^ 1], 0));  // d_text is free once block k - 1 is copied out
+            launch(c, matrix_write_kernel, (unsigned)rows, MX_THREADS, 0, d_map.p, d_edges, d_labels.p, d_label_off.p, n, r0,
+                   kind, d_off.p, d_text.p);
+            CK(cudaEventRecord(ev.rendered, c->st));
+            CK(cudaStreamWaitEvent(c->st_copy, ev.rendered, 0));
+            CK(cudaMemcpyAsync(c->h_matrix[s], d_text.p, bytes[s], cudaMemcpyDeviceToHost, c->st_copy));
+            CK(cudaEventRecord(ev.copied[s], c->st_copy));
+            if (k) {
+                CK(cudaEventSynchronize(ev.copied[s ^ 1]));
+                if (!write_all(out.f, c->h_matrix[s ^ 1], bytes[s ^ 1])) return fail(c, SKB_EIO, std::string("write failed: ") + path);
+            }
+        }
+        const int s = (int)((k - 1) & 1);
+        CK(cudaEventSynchronize(ev.copied[s]));
+        if (!write_all(out.f, c->h_matrix[s], bytes[s])) return fail(c, SKB_EIO, std::string("write failed: ") + path);
+        FILE *f = out.f;
+        out.f = nullptr;
+        return fclose(f) == 0 ? SKB_OK : fail(c, SKB_EIO, std::string("write failed: ") + path);
     });
 }
 

@@ -97,6 +97,21 @@ struct DbView {
     int64_t n_inv;
 };
 
+// The value a consumer of skani's text sees is `%.2f` of the double.  hundredths(x) is that text's value times 100 as
+// an integral double, exactly: x * 100 as an error-free product (p + e), rounded half to even on the exact value.  The
+// greedy summary's thresholds (skb_api.cu round2) and the matrix cells (skb_matrix.cuh) both read it from here.
+__device__ __forceinline__ double hundredths(double x) {
+    const double p = x * 100.0, e = fma(x, 100.0, -p);  // x * 100 == p + e exactly
+    double r = floor(p);
+    const double f = p - r;  // exact: p < 2^52
+    if (f > 0.5 || (f == 0.5 && (e > 0.0 || (e == 0.0 && fmod(r, 2.0) != 0.0)))) r += 1.0;
+    else if (f == 0.0 && e < 0.0) {
+        // p is an integer but the exact product lies just below it: the digits after the point are .99999..., which
+        // round back up to p -- nothing to do
+    }
+    return r;
+}
+
 struct PairOut {
     double ani, ani_raw, af_q, af_r;
     int64_t n_anchors, n_seeds, span_q, span_r;

@@ -366,6 +366,26 @@ class Engine:
                 self._L.skb_free(p)
         return c, o, m
 
+    MATRIX_KINDS = {"ani": 0, "distance": 1, "af": 2}  # SKB_MATRIX_ANI / _DISTANCE / _AF
+
+    def write_matrix(self, path, labels, kind="ani", edges=None):
+        """skani's --full-matrix files (DESIGN.md section 3), rendered on the device: "N\\n", then per genome its label
+        and one tab-separated `%.2f` cell per genome.  kind "ani": the edge's ANI, 100.00 on the diagonal, 0.00 for no
+        edge; "distance": 100.00 minus that cell's printed value; "af": the row genome's aligned fraction.  labels: one
+        str (or bytes) per genome, in id order.  edges: EDGE_DTYPE array sorted by (a, b), or None for the list the last
+        whole triangle() left on the device.  Writes `path` in place; the caller makes it atomic."""
+        enc = [lb if isinstance(lb, bytes) else lb.encode("utf-8", "surrogateescape") for lb in labels]
+        off = np.zeros(len(enc) + 1, np.int64)
+        off[1:] = np.cumsum([len(x) for x in enc])
+        if edges is not None:
+            edges = np.ascontiguousarray(edges, EDGE_DTYPE)
+        self._ck(
+            self._L.skb_write_matrix(self._h, os.fsencode(path), self.MATRIX_KINDS[kind],
+                                     edges.ctypes.data if edges is not None else None,
+                                     len(edges) if edges is not None else 0, len(enc), b"".join(enc), off.ctypes.data),
+            "skb_write_matrix",
+        )
+
     def device_edges(self):
         """(device pointer, count) of the last triangle/rect result; valid until the next call on this engine."""
         ptr, n = C.c_void_p(), C.c_int64()
