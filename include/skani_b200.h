@@ -121,6 +121,18 @@ int skb_marker_compression(const skb_ctx *ctx, int64_t *m);
  * context's m to the file's, so genomes added afterwards (a search's query) are sketched at the database's density. */
 int skb_db_save(skb_ctx *ctx, const char *dir);
 int skb_db_load(skb_ctx *ctx, const char *dir);
+/* What dir/sketches.skb holds, read from its header and host tables only (no seed or marker payload, no context, no
+ * device): its genome count, its marker compression m, and a 64-bit digest (FNV-1a) of every header and table byte --
+ * which changes whenever the file is rewritten with other genomes.  SKB_EIO for a missing or malformed file. */
+int skb_db_info(const char *dir, int32_t *n_genomes, int64_t *m, uint64_t *digest);
+/* Append the DB genomes ids[0 .. n) of dir/sketches.skb to the context, in that order, as one skb_add_genomes of the same
+ * FASTAs would: genome ids[r] becomes id n_before + r, with the seeds (repeat flags clear), contig tables and marker keys
+ * the add would have made, so seeds, markers and every edge are bit-identical.  Each genome's seeds are read from the
+ * file on their own; the marker keys are selected, re-tagged and grouped by the new id on the device.  Works on an empty
+ * or non-empty context before skb_index; one skb_pop_last_add undoes it.  An empty context takes the file's m (as
+ * skb_db_load); a non-empty one with another m: SKB_ESTATE.  An id out of range or repeated: SKB_EINVAL.  A missing or
+ * malformed file: SKB_EIO. */
+int skb_db_load_genomes(skb_ctx *ctx, const char *dir, const int32_t *ids, int32_t n);
 
 /* ---- pair results --------------------------------------------------------------------------- */
 typedef struct {

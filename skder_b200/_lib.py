@@ -111,7 +111,7 @@ SYMBOLS = [
     "skb_device_edges", "skb_set_owned", "skb_screen_triangle", "skb_pairs_edges", "skb_greedy_summary", "skb_index_seed_tables", "skb_clear_keep_tables",
     "skb_set_ani_estimator", "skb_set_ani_ci", "skb_last_edge_ci", "skb_set_detailed", "skb_last_edge_detail",
     "skb_genome_contig_stats", "skb_set_marker_compression", "skb_marker_compression", "skb_set_max_results",
-    "skb_add_sequences", "skb_write_matrix",
+    "skb_add_sequences", "skb_write_matrix", "skb_db_info", "skb_db_load_genomes",
 ]
 
 _lib = None
@@ -152,6 +152,8 @@ def lib():
     L.skb_get_markers.argtypes = [C.c_void_p, C.c_int32, C.c_void_p]
     L.skb_db_save.argtypes = [C.c_void_p, C.c_char_p]
     L.skb_db_load.argtypes = [C.c_void_p, C.c_char_p]
+    L.skb_db_info.argtypes = [C.c_char_p, C.POINTER(C.c_int32), C.POINTER(C.c_int64), C.POINTER(C.c_uint64)]
+    L.skb_db_load_genomes.argtypes = [C.c_void_p, C.c_char_p, C.c_void_p, C.c_int32]
     L.skb_triangle.argtypes = [
         C.c_void_p, C.c_double, C.c_double, C.c_int32, C.c_int32, C.POINTER(C.POINTER(Edge)), C.POINTER(C.c_int64),
         C.POINTER(Stats),

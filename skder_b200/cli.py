@@ -17,6 +17,14 @@ skani's own command forms work too (DESIGN.md section 3):
   skani dist     QUERY REF [REF ...] [-o OUT]
   skani search   QUERY ... [--ql LIST] -d DBDIR [-o OUT]
 
+`sketch -o DBDIR` also writes DBDIR/<basename>.sketch per input file (DESIGN.md section 3; recalled from skani, unpinned
+against it), and triangle and dist take such a file wherever they take a FASTA -- arguments, -q / -r values, -l / --ql /
+--rl entries -- as the genomes that input was sketched into: labelled by the path and names it records, loaded from the
+database (skb_db_load_genomes) instead of parsed and sketched again.  A label named both as a FASTA and by a sketch
+counts once and is loaded from the sketch.  Sketches carry their database's -m, which FASTA inputs of the same command
+are sketched at; another -m, databases of different m, a sketch whose database mode differs from its side's -i / --qi /
+--ri, or a stale descriptor (its database rewritten since) fail the command without output.  sketch refuses .sketch
+inputs; search does not take them.
 `-q` / `-r` (dist only) take every following argument up to the next one starting with '-'; each side is its values,
 then its list's entries, a path twice on one side counting once.  The positional dist form takes no -q, -r, --ql or
 --rl.  Without -o, triangle, dist and search write the TSV to stdout -- the bytes the -o file would hold, nothing on
@@ -127,6 +135,7 @@ def parse_args(argv):
         opt["threads"] = max(1, int(opt["threads"]))
     except ValueError as e:
         raise UsageError("bad numeric option: %s" % e)
+    opt["marker_c_given"] = "marker_c" in opt  # sketch inputs carry their database's m: -m may only repeat it
     if "marker_c" in opt:
         if sub == "search":
             raise UsageError("skani search takes no -m: the query is sketched at the database's marker compression")
@@ -212,25 +221,105 @@ def search_queries(opt):
     return qs
 
 
+def _entries(opt, values_key, list_key):
+    return opt.get(values_key, []) + (read_list(opt[list_key]) if list_key in opt else [])
+
+
 def inputs(sub, opt):
     """The FASTA paths a command names, as given, whatever form named them (DESIGN.md section 3):
     triangle: the FASTA arguments and the -l entries, deduplicated and sorted (the triangle's genome order);
-    sketch: the FASTA arguments in order, then the -l entries, nothing deduplicated;
+    sketch: the FASTA arguments in order, then the -l entries, nothing deduplicated (a .sketch among them: UsageError);
     dist: (refs, queries), each -r / -q's values followed by --rl / --ql's entries, or for `dist Q R1 [R2 ...]` the
     first argument as the query and the rest as references (a path twice on one side counts once, in run_dist);
-    search: search_queries()."""
-    def entries(values_key, list_key):
-        return opt.get(values_key, []) + (read_list(opt[list_key]) if list_key in opt else [])
-
+    search: search_queries().
+    In triangle and dist an entry ending in .sketch stands for the genomes its descriptor names (sketch_sources)."""
     if sub == "triangle":
-        return sorted(set(entries("positional", "list")))
+        return sorted(set(_entries(opt, "positional", "list")))
     if sub == "sketch":
-        return entries("positional", "list")
+        from .sketch_files import is_sketch
+
+        paths = _entries(opt, "positional", "list")
+        if any(is_sketch(p) for p in paths):
+            raise UsageError("skani sketch takes FASTA files, not sketches (%s)" % next(p for p in paths if is_sketch(p)))
+        return paths
     if sub == "dist":
         if opt["positional"]:
             return opt["positional"][1:], opt["positional"][:1]
-        return entries("r", "rl"), entries("q", "ql")
+        return _entries(opt, "r", "rl"), _entries(opt, "q", "ql")
     return search_queries(opt)
+
+
+def sketch_sources(entries, opt):
+    """{entry: sketch_files.Descriptor} of the .sketch entries among `entries`, each checked against its database, and
+    opt["marker_c"] set to their databases' m: the one m of the command, which its FASTA inputs are sketched at.  -m
+    giving another m, or sketches of databases of different m: UsageError."""
+    from . import sketch_files
+
+    descs = {e: sketch_files.Descriptor(e) for e in dict.fromkeys(entries) if sketch_files.is_sketch(e)}
+    ms = sorted({d.m for d in descs.values()})
+    if len(ms) > 1:
+        raise UsageError("sketches of databases made with different -m (%s) cannot be compared in one command"
+                         % ", ".join(map(str, ms)))
+    if ms and opt["marker_c_given"] and opt["marker_c"] != ms[0]:
+        raise UsageError("-m %d: the sketches given were made with -m %d" % (opt["marker_c"], ms[0]))
+    if ms:
+        opt["marker_c"] = ms[0]
+    opt["sketch_inputs"] = len(descs)
+    return descs
+
+
+def genome_unit(entry, split, descs, flag):
+    """((label, split), Descriptor or None) of one input entry on a side whose per-sequence flag is `split`: a FASTA is
+    its own label, a sketch is labelled by the path its descriptor records and must come from a database sketched in
+    the same mode"""
+    d = descs.get(entry)
+    if d is None:
+        return (entry, split), None
+    if d.per_sequence and not split:
+        raise UsageError("%s comes from a database sketched with -i (one genome per record): give %s" % (entry, flag))
+    if split and not d.per_sequence:
+        raise UsageError("%s comes from a database sketched without -i: it holds no record sketches for %s" % (entry, flag))
+    return (d.path, split), d
+
+
+def unit_sources(units):
+    """{(label, split): Descriptor or None} of `units` in first-appearance order: a label named both as a FASTA and by
+    a sketch is loaded from the sketch (the first one given)"""
+    src = {}
+    for k, d in units:
+        if k not in src or (src[k] is None and d is not None):
+            src[k] = d
+    return src
+
+
+def add_units(eng, engine_mod, src, threads, phases=None):
+    """The genomes of `src` ({(label, split): Descriptor or None}) added in its order: runs of FASTA labels through
+    stream_add (split: one genome per kept record), runs of sketched labels of one database through one
+    Engine.load_genomes.  Returns (paths, names, ids): every genome's file and name columns, in id order, and
+    {(label, split): its genome ids}."""
+    import itertools
+
+    ids, paths, names = {}, [], []
+    for (db, split), run in itertools.groupby(src.items(), key=lambda u: (u[1].db if u[1] else None, u[0][1])):
+        run = list(run)
+        if db is None:
+            files = [k[0] for k, _ in run]
+            if split:
+                gp, gn = stream_add(eng, engine_mod, files, threads, phases, per_sequence=True)
+            else:
+                gp, gn = files, stream_add(eng, engine_mod, files, threads, phases)
+        else:
+            t0 = time.time()
+            eng.load_genomes(db, [g for _, d in run for g in d.ids])
+            gp = [k[0] for k, d in run for _ in d.ids]
+            gn = [n for _, d in run for n in d.names]
+            if phases is not None:
+                phases["load_sketches_s"] = phases.get("load_sketches_s", 0.0) + time.time() - t0
+        for p in gp:
+            ids.setdefault((p, split), []).append(len(paths))
+            paths.append(p)
+        names += gn
+    return paths, names, ids
 
 
 def emit(opt, text):
@@ -343,9 +432,10 @@ def stream_add(eng, engine_mod, paths, threads, phases=None, per_sequence=False)
             del packed
             t_wait += t1 - t0
             t_add += time.time() - t1
-    if phases is not None:
-        phases["ingest_wait_s"] = t_wait  # time the device side waited for the parser (first batch + any shortfall)
-        phases["upload_sketch_s"] = t_add
+    if phases is not None:  # summed over the calls of one command
+        # time the device side waited for the parser (first batch + any shortfall)
+        phases["ingest_wait_s"] = phases.get("ingest_wait_s", 0.0) + t_wait
+        phases["upload_sketch_s"] = phases.get("upload_sketch_s", 0.0) + t_add
     return (gpaths, names) if per_sequence else names
 
 
@@ -356,15 +446,15 @@ def _phase_log(opt, phases):
 
 def run_triangle(opt, engine_mod):
     ph, t0 = {}, time.time()
-    paths = inputs("triangle", opt)
+    entries = _entries(opt, "positional", "list")
+    descs = sketch_sources(entries, opt)
+    src = unit_sources(genome_unit(e, opt["per_seq"], descs, "-i") for e in entries)
+    src = {k: src[k] for k in sorted(src)}  # the triangle's genome order: labels sorted (with -i each file's records)
     with engine_mod.Engine(_device()) as eng:
         ph["context_s"] = time.time() - t0
         apply_options(eng, opt)
         eng.set_marker_compression(opt["marker_c"])
-        if opt["per_seq"]:  # genomes: each file's kept records, files in sorted order
-            paths, names = stream_add(eng, engine_mod, paths, opt["threads"], ph, per_sequence=True)
-        else:
-            names = stream_add(eng, engine_mod, paths, opt["threads"], ph)
+        paths, names, _ = add_units(eng, engine_mod, src, opt["threads"], ph)
         t1 = time.time()
         eng.index()
         t2 = time.time()
@@ -378,7 +468,8 @@ def run_triangle(opt, engine_mod):
     if not opt["full_matrix"]:
         emit(opt, header(opt["ci"], opt["detailed"]) + "".join(triangle_rows(paths, names, edges, suffixes)))
     ph.update({"index_s": t2 - t1, "triangle_s": t3 - t2, "write_matrix_s" if opt["full_matrix"] else "write_tsv_s":
-               time.time() - t3, "total_s": time.time() - t0, "genomes": len(paths), "edges": int(st.n_edges)})
+               time.time() - t3, "total_s": time.time() - t0, "genomes": len(paths), "edges": int(st.n_edges),
+               "sketched_labels": sum(d is not None for d in src.values())})
     _phase_log(opt, ph)
     return st
 
@@ -420,7 +511,11 @@ def write_matrices(eng, opt, labels):
 
 
 def run_sketch(opt, engine_mod):
-    paths = inputs("sketch", opt)
+    """the database (sketches.skb, manifest.json) and one descriptor DBDIR/<basename>.sketch per input file, which
+    triangle and dist take in place of that FASTA (sketch_files)"""
+    from . import sketch_files
+
+    files = paths = inputs("sketch", opt)
     os.makedirs(opt["out"], exist_ok=True)
     from . import daemon
 
@@ -433,6 +528,7 @@ def run_sketch(opt, engine_mod):
             names = stream_add(eng, engine_mod, paths, opt["threads"])
         eng.save(opt["out"])
     write_atomic(os.path.join(opt["out"], "manifest.json"), json.dumps({"paths": paths, "names": names}))
+    sketch_files.write_all(opt["out"], files, paths, names, opt["per_seq"], write_atomic)
 
 
 def _daemon_search(opt, labels, dev, out):
@@ -554,32 +650,23 @@ def search_contig_stats(eng, db_stats=None):
 
 def run_dist(opt, engine_mod):
     """--ri / --qi split that side's files into records: a (file, split) pair is one unit of genomes, so a file split
-    on one side only is compared as records against itself as a whole, and one split on both sides shares its ids"""
-    import itertools
-
+    on one side only is compared as records against itself as a whole, and one split on both sides shares its ids.  A
+    sketch is the unit of the label its descriptor records."""
     refs, queries = inputs("dist", opt)
-    units = list(dict.fromkeys([(p, opt["ref_per_seq"]) for p in refs] + [(p, opt["query_per_seq"]) for p in queries]))
-    ids, paths, names = {}, [], []
+    descs = sketch_sources(refs + queries, opt)
+    refs = [genome_unit(e, opt["ref_per_seq"], descs, "--ri") for e in refs]
+    queries = [genome_unit(e, opt["query_per_seq"], descs, "--qi") for e in queries]
+    src = unit_sources(refs + queries)
     with engine_mod.Engine(_device()) as eng:
         apply_options(eng, opt)
         eng.set_marker_compression(opt["marker_c"])
-        for split, run in itertools.groupby(units, key=lambda u: u[1]):
-            run = [p for p, _ in run]
-            if split:
-                gp, gn = stream_add(eng, engine_mod, run, opt["threads"], per_sequence=True)
-            else:
-                gp, gn = run, stream_add(eng, engine_mod, run, opt["threads"])
-            for p in gp:
-                ids.setdefault((p, split), []).append(len(paths))
-                paths.append(p)
-            names += gn
+        paths, names, ids = add_units(eng, engine_mod, src, opt["threads"])
 
-        def genome_ids(side, split):
-            return [g for p in dict.fromkeys(side) for g in ids.get((p, split), [])]
+        def genome_ids(side):
+            return [g for k in dict.fromkeys(k for k, _ in side) for g in ids.get(k, [])]
 
         eng.index()
-        edges, st = eng.rect(genome_ids(refs, opt["ref_per_seq"]), genome_ids(queries, opt["query_per_seq"]),
-                             screen=opt["screen"], min_af=opt["min_af"])
+        edges, st = eng.rect(genome_ids(refs), genome_ids(queries), screen=opt["screen"], min_af=opt["min_af"])
         suffixes = row_suffixes(eng, opt, edges)
     emit(opt, header(opt["ci"], opt["detailed"]) + "".join(rect_rows(paths, names, edges, suffixes)))
     return st
@@ -618,6 +705,10 @@ def _provenance(opt, sub, seconds):
     if opt.get("distance"):
         text += ("--distance: every ANI cell is 100.00 minus its printed ANI, in hundredths (DESIGN.md section 3); "
                  "unpinned against skani's own --distance\n")
+    if opt.get("sketch_inputs"):
+        text += ("sketch files: %d .sketch input(s) named genomes loaded from `sketch -o` databases (DESIGN.md section "
+                 "3); the descriptor format and how skani itself treats such files are recalled, "
+                 "unpinned against skani\n" % opt["sketch_inputs"])
     if opt.get("detailed"):
         text += ("--detailed: the 13 extra columns as DESIGN.md section 3 defines them; their names, order and definitions "
                  "are recalled, unpinned against skani's own --detailed output\n")

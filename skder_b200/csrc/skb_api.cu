@@ -11,6 +11,7 @@
 #include <ctime>
 #include <cub/cub.cuh>
 #include <map>
+#include <memory>
 #include <string>
 #include <thread>
 #include <vector>
@@ -1941,6 +1942,41 @@ int skb_db_save(skb_ctx *ctx, const char *dir) {
     });
 }
 
+// The header and host tables of a sketches.skb (skb_db_load, skb_db_info, skb_db_load_genomes): read_db_head leaves the
+// file at the seed payload, whose marker keys follow it.
+struct DbHead {
+    uint64_t m = C_MARKER, n = 0, ns = 0, nm = 0, nc = 0;
+    std::vector<uint64_t> seed_off, total_len;
+    std::vector<uint32_t> ctg_off, ctg_len;
+    uint64_t digest = 1469598103934665603ull;  // FNV-1a 64 of every header and table byte, in file order
+    int64_t seeds_at = 0;                      // byte offset of the seed payload
+};
+
+// "" on success, else the error
+static std::string read_db_head(FILE *f, const std::string &path, DbHead &d) {
+    auto rd = [&](void *p, size_t bytes) {
+        if (!read_all(f, p, bytes)) return false;
+        for (size_t i = 0; i < bytes; i++) d.digest = (d.digest ^ ((const unsigned char *)p)[i]) * 1099511628211ull;
+        return true;
+    };
+    char magic[8];
+    bool ok = rd(magic, 8) && (std::memcmp(magic, kMagic, 8) == 0 || (std::memcmp(magic, kMagic2, 8) == 0 && rd(&d.m, 8))) &&
+              rd(&d.n, 8) && rd(&d.ns, 8) && rd(&d.nm, 8) && rd(&d.nc, 8);
+    if (!ok || d.n >= GID_MASK || d.m < 1 || d.m > (uint64_t)INT64_MAX || d.nc >= (1ull << 32))
+        return "not a sketch DB: " + path;
+    d.seed_off.resize(d.n + 1);
+    d.total_len.resize(d.n);
+    d.ctg_off.resize(d.n + 1);
+    d.ctg_len.resize(d.nc);
+    ok = rd(d.seed_off.data(), (d.n + 1) * 8) && rd(d.total_len.data(), d.n * 8) && rd(d.ctg_off.data(), (d.n + 1) * 4) &&
+         rd(d.ctg_len.data(), d.nc * 4);
+    if (!ok || d.seed_off[d.n] != d.ns || d.ctg_off[d.n] != d.nc) return "truncated sketch DB: " + path;
+    for (uint64_t g = 0; g < d.n; g++)
+        if (d.seed_off[g] > d.seed_off[g + 1] || d.ctg_off[g] > d.ctg_off[g + 1]) return "corrupt sketch DB tables: " + path;
+    d.seeds_at = (int64_t)ftello(f);
+    return "";
+}
+
 int skb_db_load(skb_ctx *ctx, const char *dir) {
     return guarded(ctx, [&]() -> int {
         skb_ctx *c = ctx;
@@ -1950,29 +1986,169 @@ int skb_db_load(skb_ctx *ctx, const char *dir) {
         const std::string path = std::string(dir) + "/sketches.skb";
         FILE *f = fopen(path.c_str(), "rb");
         if (!f) return fail(c, SKB_EIO, "cannot open " + path);
-        char magic[8];
-        uint64_t n = 0, ns = 0, nm = 0, nc = 0, m = C_MARKER;
-        bool ok = read_all(f, magic, 8) &&
-                  (std::memcmp(magic, kMagic, 8) == 0 || (std::memcmp(magic, kMagic2, 8) == 0 && read_all(f, &m, 8))) &&
-                  read_all(f, &n, 8) && read_all(f, &ns, 8) && read_all(f, &nm, 8) && read_all(f, &nc, 8);
-        if (!ok || n >= GID_MASK || m < 1 || m > (uint64_t)INT64_MAX) {
+        DbHead d;
+        const std::string err = read_db_head(f, path, d);
+        if (!err.empty()) {
             fclose(f);
-            return fail(c, SKB_EIO, "not a sketch DB: " + path);
+            return fail(c, SKB_EIO, err);
         }
-        std::vector<uint64_t> seed_off(n + 1), total_len(n), seeds(ns), mk(nm);
-        std::vector<uint32_t> ctg_off(n + 1), ctg_len(nc);
-        ok = read_all(f, seed_off.data(), (n + 1) * 8) && read_all(f, total_len.data(), n * 8) &&
-             read_all(f, ctg_off.data(), (n + 1) * 4) && read_all(f, ctg_len.data(), nc * 4) &&
-             read_all(f, seeds.data(), ns * 8) && read_all(f, mk.data(), nm * 8);
+        std::vector<uint64_t> seeds(d.ns), mk(d.nm);
+        const bool ok = read_all(f, seeds.data(), d.ns * 8) && read_all(f, mk.data(), d.nm * 8);
         fclose(f);
-        if (!ok || seed_off[n] != ns || ctg_off[n] != nc) return fail(c, SKB_EIO, "truncated sketch DB: " + path);
-        c->d_seeds.reserve(ns + 1, 0, c->st);
-        c->d_mkeys.reserve(nm + 1, 0, c->st);
-        if (ns) CK(cudaMemcpyAsync(c->d_seeds.p, seeds.data(), ns * 8, cudaMemcpyHostToDevice, c->st));
-        if (nm) CK(cudaMemcpyAsync(c->d_mkeys.p, mk.data(), nm * 8, cudaMemcpyHostToDevice, c->st));
+        if (!ok) return fail(c, SKB_EIO, "truncated sketch DB: " + path);
+        c->d_seeds.reserve(d.ns + 1, 0, c->st);
+        c->d_mkeys.reserve(d.nm + 1, 0, c->st);
+        if (d.ns) CK(cudaMemcpyAsync(c->d_seeds.p, seeds.data(), d.ns * 8, cudaMemcpyHostToDevice, c->st));
+        if (d.nm) CK(cudaMemcpyAsync(c->d_mkeys.p, mk.data(), d.nm * 8, cudaMemcpyHostToDevice, c->st));
         CK(cudaStreamSynchronize(c->st));
-        c->db = skb_ctx::SketchDb{std::move(seed_off), std::move(total_len), std::move(ctg_off), std::move(ctg_len), nm};
-        c->marker_c = m;  // genomes added later (a search's query) are sketched at the database's density
+        c->db = skb_ctx::SketchDb{std::move(d.seed_off), std::move(d.total_len), std::move(d.ctg_off), std::move(d.ctg_len),
+                                  d.nm};
+        c->marker_c = d.m;  // genomes added later (a search's query) are sketched at the database's density
+        c->indexed = false;
+        return SKB_OK;
+    });
+}
+
+int skb_db_info(const char *dir, int32_t *n_genomes, int64_t *m, uint64_t *digest) {
+    if (!dir) return SKB_EINVAL;
+    const std::string path = std::string(dir) + "/sketches.skb";
+    FILE *f = fopen(path.c_str(), "rb");
+    if (!f) return SKB_EIO;
+    DbHead d;
+    const bool ok = read_db_head(f, path, d).empty();
+    fclose(f);
+    if (!ok) return SKB_EIO;
+    if (n_genomes) *n_genomes = (int32_t)d.n;
+    if (m) *m = (int64_t)d.m;
+    if (digest) *digest = d.digest;
+    return SKB_OK;
+}
+
+// skb_db_load_genomes' marker keys.  The file's raw keys (marker << 22 | DB id) come genome by genome, ids ascending
+// (skb_db_save writes what skb_add_genomes appended), so each DB genome's keys are one run [start, end).
+__global__ void db_key_runs_kernel(const uint64_t *__restrict__ keys, uint64_t n, uint64_t n_db, uint32_t *__restrict__ start,
+                                   uint32_t *__restrict__ end, int *__restrict__ bad) {
+    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint64_t id = keys[i] & GID_MASK;
+    const uint64_t prev = i ? keys[i - 1] & GID_MASK : ~0ull, next = i + 1 < n ? keys[i + 1] & GID_MASK : ~0ull;
+    if (id >= n_db || (i && prev > id)) {  // not grouped by ascending id: the runs below would be wrong
+        *bad = 1;
+        return;
+    }
+    if (prev != id) start[id] = (uint32_t)i;
+    if (next != id) end[id] = (uint32_t)(i + 1);
+}
+// cnt[r] = key count of the r-th requested genome (ids[r]); cnt[n] = 0 closes the scan
+__global__ void db_key_counts_kernel(const int32_t *__restrict__ ids, int32_t n, const uint32_t *__restrict__ start,
+                                     const uint32_t *__restrict__ end, uint32_t *__restrict__ cnt) {
+    const int32_t r = blockIdx.x * blockDim.x + threadIdx.x;
+    if (r < n) cnt[r] = end[ids[r]] - start[ids[r]];
+    if (r == n) cnt[r] = 0;
+}
+// Keep the keys of the requested genomes, tagged with their new ids gid0 + rank, grouped by new id ascending with each
+// genome's keys in file order: a stable counting sort whose offsets `off` are the exclusive scan of the counts above.
+// (retag_keys_kernel shifts every id by one constant; here the shift differs per genome.)
+__global__ void db_select_keys_kernel(const uint64_t *__restrict__ keys, uint64_t n, const int32_t *__restrict__ rank,
+                                      const uint32_t *__restrict__ start, const uint32_t *__restrict__ off, uint64_t gid0,
+                                      uint64_t *__restrict__ out) {
+    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint64_t k = keys[i], id = k & GID_MASK;
+    const int32_t r = rank[id];
+    if (r >= 0) out[off[r] + (i - start[id])] = (k & ~GID_MASK) | (gid0 + (uint64_t)r);
+}
+
+int skb_db_load_genomes(skb_ctx *ctx, const char *dir, const int32_t *ids, int32_t n) {
+    return guarded(ctx, [&]() -> int {
+        skb_ctx *c = ctx;
+        if (!dir || n < 0 || (n > 0 && !ids)) return fail(c, SKB_EINVAL, "bad arguments");
+        const std::string path = std::string(dir) + "/sketches.skb";
+        std::unique_ptr<FILE, int (*)(FILE *)> f(fopen(path.c_str(), "rb"), fclose);
+        if (!f) return fail(c, SKB_EIO, "cannot open " + path);
+        DbHead d;
+        const std::string err = read_db_head(f.get(), path, d);
+        if (!err.empty()) return fail(c, SKB_EIO, err);
+        std::vector<int32_t> rank(std::max<uint64_t>(d.n, 1), -1);  // DB id -> position in ids, -1: not requested
+        uint64_t ns = 0;
+        for (int32_t r = 0; r < n; r++) {
+            const int32_t g = ids[r];
+            if (g < 0 || (uint64_t)g >= d.n)
+                return fail(c, SKB_EINVAL, "genome id " + std::to_string(g) + " out of range (" + std::to_string(d.n) + " in " + path + ")");
+            if (rank[g] >= 0) return fail(c, SKB_EINVAL, "genome id " + std::to_string(g) + " requested twice");
+            rank[g] = r;
+            ns += d.seed_off[g + 1] - d.seed_off[g];
+        }
+        if (c->n() > 0 && d.m != c->marker_c)
+            return fail(c, SKB_ESTATE, "the DB's marker compression " + std::to_string(d.m) + " differs from the context's " +
+                                           std::to_string(c->marker_c));
+        if ((uint64_t)c->n() + (uint64_t)n >= GID_MASK) return fail(c, SKB_ELIMIT, "too many genomes (22-bit ids)");
+        if (d.nm >= (1ull << 32)) return fail(c, SKB_ELIMIT, "too many marker keys");
+        // each genome's seeds on their own, a run of consecutive ids in one read
+        std::unique_ptr<uint64_t[]> seeds(new uint64_t[ns + 1]);
+        uint64_t w = 0;
+        for (int32_t r = 0; r < n;) {
+            int32_t r1 = r + 1;
+            while (r1 < n && ids[r1] == ids[r1 - 1] + 1) r1++;
+            const uint64_t a = d.seed_off[ids[r]], b = d.seed_off[ids[r1 - 1] + 1];
+            if (fseeko(f.get(), d.seeds_at + (int64_t)(a * 8), SEEK_SET) != 0 || !read_all(f.get(), seeds.get() + w, (b - a) * 8))
+                return fail(c, SKB_EIO, "truncated sketch DB: " + path);
+            w += b - a;
+            r = r1;
+        }
+        for (uint64_t i = 0; i < ns; i++) seeds[i] &= ~2ull;  // repeat flags are index state
+        std::unique_ptr<uint64_t[]> mk(new uint64_t[d.nm + 1]);
+        if (fseeko(f.get(), d.seeds_at + (int64_t)(d.ns * 8), SEEK_SET) != 0 || !read_all(f.get(), mk.get(), d.nm * 8))
+            return fail(c, SKB_EIO, "truncated sketch DB: " + path);
+        f.reset();
+
+        const int32_t g0 = c->n();
+        const uint64_t s0 = c->db.seed_off.back(), k0 = c->db.n_mkeys;
+        if (g0 == 0) c->marker_c = d.m;  // as skb_db_load: an empty context takes the DB's m
+        c->genome_set++;
+        c->add_calls.push_back({g0, k0});  // skb_pop_last_add undoes it like an add
+        c->d_seeds.reserve(s0 + ns + 1, s0, c->st);
+        if (ns) CK(cudaMemcpyAsync(c->d_seeds.p + s0, seeds.get(), ns * 8, cudaMemcpyHostToDevice, c->st));
+        uint32_t nk = 0;
+        if (d.nm && n) {
+            PoolRef<uint64_t> d_raw(c->pool["db_load_genomes.raw"]);
+            PoolRef<int32_t> d_rank(c->pool["db_load_genomes.rank"]), d_ids(c->pool["db_load_genomes.ids"]);
+            PoolRef<uint32_t> d_start(c->pool["db_load_genomes.start"]), d_end(c->pool["db_load_genomes.end"]),
+                d_cnt(c->pool["db_load_genomes.cnt"]), d_off(c->pool["db_load_genomes.off"]);
+            d_raw.reserve(d.nm, 0, c->st);
+            CK(cudaMemcpyAsync(d_raw.p, mk.get(), d.nm * 8, cudaMemcpyHostToDevice, c->st));
+            d_rank.upload(rank, c->st);
+            d_ids.upload(std::vector<int32_t>(ids, ids + n), c->st);
+            d_start.reserve(d.n, 0, c->st);
+            d_end.reserve(d.n, 0, c->st);
+            d_cnt.reserve((size_t)n + 1, 0, c->st);
+            d_off.reserve((size_t)n + 1, 0, c->st);
+            c->d_counter.reserve(1, 0, c->st);
+            CK(cudaMemsetAsync(d_start.p, 0, d.n * 4, c->st));
+            CK(cudaMemsetAsync(d_end.p, 0, d.n * 4, c->st));
+            CK(cudaMemsetAsync(c->d_counter.p, 0, sizeof(int), c->st));
+            launch(c, db_key_runs_kernel, nblk(d.nm, 256), 256, 0, d_raw.p, d.nm, d.n, d_start.p, d_end.p, c->d_counter.p);
+            launch(c, db_key_counts_kernel, nblk((uint64_t)n + 1, 256), 256, 0, d_ids.p, n, d_start.p, d_end.p, d_cnt.p);
+            exclusive_scan_u32(c, d_cnt.p, d_off.p, (size_t)n + 1);
+            int bad = 0;
+            CK(cudaMemcpyAsync(&nk, d_off.p + n, 4, cudaMemcpyDeviceToHost, c->st));
+            CK(cudaMemcpyAsync(&bad, c->d_counter.p, sizeof(int), cudaMemcpyDeviceToHost, c->st));
+            CK(cudaStreamSynchronize(c->st));
+            if (bad) {
+                c->add_calls.pop_back();
+                return fail(c, SKB_EIO, "marker keys not grouped by ascending genome id: " + path);
+            }
+            c->d_mkeys.reserve(k0 + nk + 1, k0, c->st);
+            launch(c, db_select_keys_kernel, nblk(d.nm, 256), 256, 0, d_raw.p, d.nm, d_rank.p, d_start.p, d_off.p,
+                   (uint64_t)g0, c->d_mkeys.p + k0);
+        }
+        CK(cudaStreamSynchronize(c->st));
+        for (int32_t r = 0; r < n; r++) {
+            const int32_t g = ids[r];
+            c->db.append(d.seed_off[g + 1] - d.seed_off[g], d.total_len[g], d.ctg_len.data() + d.ctg_off[g],
+                         d.ctg_off[g + 1] - d.ctg_off[g]);
+        }
+        c->db.n_mkeys = k0 + nk;
         c->indexed = false;
         return SKB_OK;
     });

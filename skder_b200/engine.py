@@ -107,6 +107,16 @@ def pack_contigs(seqs, min_contig_len=500):
     return PackedGenome(out)
 
 
+def db_info(directory):
+    """(genome count, marker compression m, 64-bit digest of the header and host tables) of directory/sketches.skb,
+    read without a context or a device (skb_db_info)"""
+    n, m, digest = C.c_int32(), C.c_int64(), C.c_uint64()
+    rc = _lib.lib().skb_db_info(os.fsencode(directory), C.byref(n), C.byref(m), C.byref(digest))
+    if rc != 0:
+        raise SkbError("cannot read the sketch DB in %s (code %d)" % (directory, rc))
+    return n.value, m.value, digest.value
+
+
 class Engine:
     def __init__(self, device=0, params=None):
         self._L = _lib.lib()
@@ -303,6 +313,15 @@ class Engine:
 
     def load(self, directory):
         self._ck(self._L.skb_db_load(self._h, os.fsencode(directory)), "skb_db_load")
+
+    db_info = staticmethod(db_info)
+
+    def load_genomes(self, directory, ids):
+        """Append the database genomes `ids` (in that order) of `directory` as new genomes, bit-identical to adding
+        their FASTAs (skb_db_load_genomes).  Before index(); one pop_last_add() undoes it."""
+        ids = np.ascontiguousarray(ids, np.int32)
+        self._ck(self._L.skb_db_load_genomes(self._h, os.fsencode(directory), ids.ctypes.data, len(ids)),
+                 "skb_db_load_genomes")
 
     # ---- pairs -----------------------------------------------------------------------------
     def _take_edges(self, ptr, n):
