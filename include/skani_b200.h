@@ -309,6 +309,16 @@ int skb_write_matrix(skb_ctx *ctx, const char *path, int32_t kind, const skb_edg
 
 void skb_free(void *p);
 
+/* Seed tables of the genomes a pair compares against (DESIGN.md section 2).  skb_index keeps every genome's table resident
+ * when they fit the table budget -- the density's budget of device memory, but at least half of the memory free, capped
+ * by SKB_TABLE_BUDGET_MB (MiB) -- and otherwise switches the context to on-demand tables: every edge call (skb_triangle,
+ * skb_rect, skb_pairs_edges, skb_pairs_detail) then builds the tables of the genomes that are the reference of a
+ * surviving pair, in blocks that fit the budget, and merges the blocks' results by each pair's position in the call's
+ * pair list, into the order one resident pass leaves; every result is the same.  A context with skb_set_owned keeps its
+ * tables resident.  *on_demand: 1 if the last skb_index chose on-demand tables; *blocks_last_call: the blocks the last
+ * edge call built (0 with resident tables).  Either pointer may be NULL. */
+int skb_table_blocks(const skb_ctx *ctx, int32_t *on_demand, int32_t *blocks_last_call);
+
 /* total kernels launched by this context so far (bench.py's gpu_launches) */
 int64_t skb_launch_count(const skb_ctx *ctx);
 /* device-side stopwatch: CUDA events recorded on the context's own stream */

@@ -111,7 +111,7 @@ SYMBOLS = [
     "skb_device_edges", "skb_set_owned", "skb_screen_triangle", "skb_pairs_edges", "skb_greedy_summary", "skb_index_seed_tables", "skb_clear_keep_tables",
     "skb_set_ani_estimator", "skb_set_ani_ci", "skb_last_edge_ci", "skb_set_detailed", "skb_last_edge_detail",
     "skb_genome_contig_stats", "skb_set_marker_compression", "skb_marker_compression", "skb_set_max_results",
-    "skb_add_sequences", "skb_write_matrix", "skb_db_info", "skb_db_load_genomes",
+    "skb_add_sequences", "skb_write_matrix", "skb_db_info", "skb_db_load_genomes", "skb_table_blocks",
 ]
 
 _lib = None
@@ -196,6 +196,7 @@ def lib():
     L.skb_timer_stop.argtypes = [C.c_void_p, C.POINTER(C.c_float)]
     L.skb_free.argtypes = [C.c_void_p]
     L.skb_free.restype = None
+    L.skb_table_blocks.argtypes = [C.c_void_p, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]
     L.skb_launch_count.argtypes = [C.c_void_p]
     L.skb_launch_count.restype = C.c_int64
     L.skb_stream.argtypes = [C.c_void_p]

@@ -8,7 +8,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "_lib")
 LIB = os.path.join(LIBDIR, "libskani_b200.so")
 SOURCES = ["skb_api.cu", "fasta_pack.cpp"]
-HEADERS = ["skb_common.cuh", "skb_sketch.cuh", "skb_index.cuh", "skb_probe.cuh", "skb_ani.cuh", "skb_best_n.cuh", "skb_matrix.cuh", "../../include/skani_b200.h"]
+HEADERS = ["skb_common.cuh", "skb_sketch.cuh", "skb_index.cuh", "skb_probe.cuh", "skb_ani.cuh", "skb_best_n.cuh", "skb_matrix.cuh", "skb_table_blocks.cuh", "../../include/skani_b200.h"]
 
 
 def _stale():

@@ -444,6 +444,13 @@ def _phase_log(opt, phases):
         write_atomic(opt["out"].rstrip("/") + ".skani_b200.phases.json", json.dumps(phases))
 
 
+def table_blocks(eng):
+    """the seed-table mode of the last index and the blocks of the last edge call (DESIGN.md section 2), for the phase
+    log and the daemon's ping"""
+    on, blocks = eng.table_blocks()
+    return {"on_demand": on, "blocks": blocks}
+
+
 def run_triangle(opt, engine_mod):
     ph, t0 = {}, time.time()
     entries = _entries(opt, "positional", "list")
@@ -459,6 +466,7 @@ def run_triangle(opt, engine_mod):
         eng.index()
         t2 = time.time()
         edges, st = eng.triangle(screen=opt["screen"], min_af=opt["min_af"], to_host=not opt["full_matrix"])
+        tb = table_blocks(eng)
         if opt["full_matrix"]:  # rendered from the device edge list, so while the context lives
             t3 = time.time()
             write_matrices(eng, opt, names if opt["per_seq"] else paths)
@@ -469,7 +477,7 @@ def run_triangle(opt, engine_mod):
         emit(opt, header(opt["ci"], opt["detailed"]) + "".join(triangle_rows(paths, names, edges, suffixes)))
     ph.update({"index_s": t2 - t1, "triangle_s": t3 - t2, "write_matrix_s" if opt["full_matrix"] else "write_tsv_s":
                time.time() - t3, "total_s": time.time() - t0, "genomes": len(paths), "edges": int(st.n_edges),
-               "sketched_labels": sum(d is not None for d in src.values())})
+               "sketched_labels": sum(d is not None for d in src.values()), "table_blocks": tb})
     _phase_log(opt, ph)
     return st
 
@@ -613,7 +621,9 @@ def run_search(opt, engine_mod):
         eng.load(opt["db"])
         eng.index()
         text, st = search_tsv(eng, engine_mod, paths, names, labels, labels, opt)
+        tb = table_blocks(eng)
     emit(opt, text)
+    _phase_log(opt, {"edges": int(st.n_edges), "table_blocks": tb})
     return st
 
 
@@ -668,7 +678,9 @@ def run_dist(opt, engine_mod):
         eng.index()
         edges, st = eng.rect(genome_ids(refs), genome_ids(queries), screen=opt["screen"], min_af=opt["min_af"])
         suffixes = row_suffixes(eng, opt, edges)
+        tb = table_blocks(eng)
     emit(opt, header(opt["ci"], opt["detailed"]) + "".join(rect_rows(paths, names, edges, suffixes)))
+    _phase_log(opt, {"edges": int(st.n_edges), "table_blocks": tb})
     return st
 
 

@@ -22,6 +22,7 @@
 #include "skb_index.cuh"
 #include "skb_matrix.cuh"
 #include "skb_sketch.cuh"
+#include "skb_table_blocks.cuh"
 
 using namespace skb;
 
@@ -192,6 +193,13 @@ struct skb_ctx {
     int tab_x2_forced = 0; // SKB_TAB_X2 (tests exercise the overflow chain with 1)
     int x2_decided = 0;    // density chosen from the free device memory the last time it was asked for ...
     uint64_t x2_decided_seeds = 0;  // ... and the owned seed count it was chosen for
+    double x2_budget = 0;           // ... and the table budget in bytes it was chosen under ...
+    double x2_room = 0;             // ... and the device memory free for the tables then (table_budget)
+    // on-demand seed tables (skb_index chose them: the tables of all genomes exceed the budget): d_tab holds the tables
+    // of one block of genomes at a time, built by the edge call that needs them (table_blocks)
+    bool on_demand = false;
+    int32_t blocks_last_call = 0;   // blocks the last edge call built (skb_table_blocks)
+    double block_budget = 0;        // bytes one block may take, once measured after skb_index (block_budget); 0: unknown
     DevBuf<uint64_t> d_seed_off, d_tab, d_tab_off, d_total_len, d_inv, d_markers, d_marker_off;
     DevBuf<uint32_t> d_tab_buckets;
     DevBuf<uint32_t> d_chunk_begin, d_chunk_start, d_chunk_len, d_chunk_off, d_ctg_pstart, d_ctg_len, d_ctg_off,
@@ -735,9 +743,10 @@ void run_ani(skb_ctx *c, const unsigned long long *d_pairs, int64_t n_pairs, Pai
 }
 
 // pairs on device -> ANI -> compacted edges on device (c->last_dev_edges, c->last_n_edges); sums: sum query seeds, sum
-// anchors
+// anchors.  pair_pos, edge_pos (on-demand tables: pairs_to_edges_blocks): a number per pair, copied for every edge
 void pairs_to_edges(skb_ctx *c, unsigned long long *d_pairs, int64_t n_pairs, double min_af_pct,
-                    unsigned long long sums[2], cudaEvent_t ev_mid, cudaEvent_t ev_end) {
+                    unsigned long long sums[2], cudaEvent_t ev_mid, cudaEvent_t ev_end, const uint32_t *pair_pos = nullptr,
+                    uint32_t *edge_pos = nullptr) {
     PoolRef<PairOut> d_out(c->pool["pairs_to_edges.d_out"]);
     PoolRef<skb_edge> d_edges(c->pool["pairs_to_edges.d_edges"]);
     PoolRef<unsigned long long> d_n(c->pool["pairs_to_edges.d_n"]);
@@ -770,6 +779,8 @@ void pairs_to_edges(skb_ctx *c, unsigned long long *d_pairs, int64_t n_pairs, do
         exclusive_scan_u32(c, d_ef.p, d_ep.p, (size_t)n_pairs);
         launch(c, edge_scatter_kernel, nblk((uint64_t)n_pairs, 256), 256, 0, d_pairs, d_out.p, n_pairs, d_ef.p, d_ep.p,
                d_edges.p, d_n.p);
+        if (edge_pos)
+            launch(c, edge_pos_kernel, nblk((uint64_t)n_pairs, 256), 256, 0, d_ef.p, d_ep.p, n_pairs, pair_pos, edge_pos);
         if (d_ci) {  // one record per edge serves both skb_last_edge_ci and skb_last_edge_detail
             PoolRef<skb_edge_detail> det_edges(c->pool["detail.edges"]);
             det_edges.reserve((size_t)n_pairs, 0, c->st);
@@ -839,6 +850,93 @@ void best_n_edges(skb_ctx *c, int64_t max_n) {
     c->last_n_edges = n_kept;
 }
 
+// ---- on-demand seed tables (skb_index chose them; DESIGN.md section 2) ------------------------------------------
+// Bytes the seed tables may take: table_density's budget, but at least half of the device memory free when it was set
+// (a device whose other tenants leave less than the 40 GiB table_density keeps for the rest still holds a small set's
+// tables resident), capped by SKB_TABLE_BUDGET_MB (MiB, fractions allowed; tests and benchmarks force on-demand tables
+// at small sizes with it)
+double table_budget(const skb_ctx *c) {
+    const double dev = std::max(c->x2_budget, c->x2_room / 2.0);
+    const char *e = std::getenv("SKB_TABLE_BUDGET_MB");
+    const double mb = e ? std::strtod(e, nullptr) : 0.0;
+    return mb > 0.0 ? std::min(dev, mb * (double)(1ull << 20)) : dev;
+}
+
+// Bytes one block of on-demand tables may take: the table budget, and the device memory free now (the scratch allocated
+// since the budget was set, such as skb_index's marker sort, is no longer free) less the 40 GiB table_density keeps for
+// the pair stage, but at least a tenth of it.  Measured once and kept until skb_index or skb_clear resets it:
+// cudaMemGetInfo stalls while a monitoring tool holds the driver lock (table_density), and a search serves many queries.
+double block_budget(skb_ctx *c) {
+    if (c->block_budget <= 0.0) {
+        size_t free_b = 0, total_b = 0;
+        CK(cudaMemGetInfo(&free_b, &total_b));
+        const double room = (double)free_b + (double)c->d_tab.cap * 8.0;
+        c->block_budget = std::min(table_budget(c), std::max(room - 40.0 * (double)(1ull << 30), room / 10.0));
+    }
+    return c->block_budget;
+}
+
+// Buckets of genome g's seed table at density tab_x2
+uint32_t table_buckets(const skb_ctx *c, int32_t g) {
+    const uint64_t ns = c->db.seed_off[g + 1] - c->db.seed_off[g];
+    return (uint32_t)std::max<uint64_t>(2, ns * (uint64_t)c->tab_x2 / 2 + 1);
+}
+
+// The genomes `ids` (ascending) packed in order into blocks under block_budget; a genome whose table alone exceeds it
+// gets a block of its own
+std::vector<std::vector<int32_t>> table_blocks(skb_ctx *c, const std::vector<int32_t> &ids) {
+    const double budget = block_budget(c);
+    std::vector<std::vector<int32_t>> blocks;
+    double bytes = 0;
+    for (const int32_t g : ids) {
+        const double b = (double)c->ix.tab_buckets[g] * BUCKET * 8.0;
+        if (blocks.empty() || bytes + b > budget) {
+            blocks.emplace_back();
+            bytes = 0;
+        }
+        blocks.back().push_back(g);
+        bytes += b;
+    }
+    return blocks;
+}
+
+// The seed tables and repeat flags of one block of genomes (ids ascending), laid out from slot 0 of d_tab; the per-genome
+// table offsets and bucket counts of the block's genomes point there (those of the other genomes are stale)
+void build_block_tables(skb_ctx *c, const std::vector<int32_t> &ids) {
+    const int k = (int)ids.size();
+    std::vector<uint32_t> gid(k), nb(k);
+    std::vector<uint64_t> loc(k), pref(k + 1, 0);
+    uint64_t words = 0;
+    for (int j = 0; j < k; j++) {
+        const int32_t g = ids[j];
+        gid[j] = (uint32_t)g;
+        nb[j] = c->ix.tab_buckets[g];
+        loc[j] = words;
+        words += (uint64_t)nb[j] * BUCKET;
+        pref[j + 1] = pref[j] + (c->db.seed_off[g + 1] - c->db.seed_off[g]);
+    }
+    PoolRef<uint32_t> d_gid(c->pool["table_blocks.gid"]), d_nb(c->pool["table_blocks.nb"]);
+    PoolRef<uint64_t> d_loc(c->pool["table_blocks.loc"]), d_pref(c->pool["table_blocks.pref"]);
+    d_gid.upload(gid, c->st);
+    d_nb.upload(nb, c->st);
+    d_loc.upload(loc, c->st);
+    d_pref.upload(pref, c->st);
+    launch(c, block_layout_kernel, nblk((uint64_t)k, 256), 256, 0, d_gid.p, d_loc.p, d_nb.p, k, c->d_tab_off.p,
+           c->d_tab_buckets.p);
+    if (words + BUCKET > c->d_tab.cap) {  // the previous block's tables are not needed: free them before growing
+        CK(cudaStreamSynchronize(c->st));
+        c->d_tab.release();
+    }
+    c->d_tab.reserve(words + BUCKET, 0, c->st);
+    CK(cudaMemsetAsync(c->d_tab.p, 0xFF, words * 8, c->st));
+    if (pref[k]) {
+        launch(c, block_tab_insert_kernel, nblk(pref[k], 256), 256, 0, c->d_seeds.p, c->d_seed_off.p, d_gid.p, d_pref.p, k,
+               c->d_tab.p, c->d_tab_off.p, c->d_tab_buckets.p);
+        launch(c, block_rep_flag_kernel, nblk(pref[k], 256), 256, 0, c->d_seeds.p, c->d_seed_off.p, d_gid.p, d_pref.p, k,
+               c->d_tab.p, c->d_tab_off.p, c->d_tab_buckets.p, c->prm.max_mult);
+    }
+}
+
 // The context's events around the stages of one screen or edge call: start, pairs ready, edges ready
 cudaEvent_t *call_events(skb_ctx *c) {
     for (cudaEvent_t &e : c->call_ev)
@@ -851,6 +949,110 @@ struct EdgePairs {
     unsigned long long *d_pairs = nullptr;
     int64_t n = 0, total = 0;
 };
+
+// pairs_to_edges with on-demand seed tables: the genomes that are the reference of a pair (ref_mark_kernel) are packed
+// into blocks under the table budget; per block its tables are built, its pairs selected in order
+// (pair_owned_flag_kernel over the block's id range, which holds no other reference) and evaluated, and its edges (and
+// --ci / --detailed records) appended with each edge's position in the pair list; the blocks' lists are then merged by
+// that position into the order one pass over the list leaves
+void pairs_to_edges_blocks(skb_ctx *c, unsigned long long *d_pairs, int64_t n_pairs, double min_af_pct,
+                           unsigned long long sums[2], cudaEvent_t ev_mid, cudaEvent_t ev_end) {
+    cudaEvent_t *ev = call_events(c);  // ev[3], ev[4] serve each block's pairs_to_edges (edge_call's -n stage comes after)
+    CK(cudaEventRecord(ev_mid, c->st));
+    const int32_t n = c->n();
+    std::vector<int32_t> refs;
+    if (n_pairs > 0) {
+        PoolRef<uint8_t> d_mark(c->pool["table_blocks.mark"]);
+        d_mark.reserve((size_t)n, 0, c->st);
+        CK(cudaMemsetAsync(d_mark.p, 0, (size_t)n, c->st));
+        launch(c, ref_mark_kernel, nblk((uint64_t)n_pairs, 256), 256, 0, c->d_seed_off.p, d_pairs, n_pairs, (uint32_t)n,
+               d_mark.p);
+        std::vector<uint8_t> mark((size_t)n);
+        CK(cudaMemcpyAsync(mark.data(), d_mark.p, (size_t)n, cudaMemcpyDeviceToHost, c->st));
+        CK(cudaStreamSynchronize(c->st));
+        for (int32_t g = 0; g < n; g++)
+            if (mark[(size_t)g]) refs.push_back(g);
+    }
+    const std::vector<std::vector<int32_t>> blocks = table_blocks(c, refs);
+    c->blocks_last_call = (int32_t)blocks.size();
+    if (blocks.size() <= 1) {  // every pair in one block: nothing to select or merge
+        if (!blocks.empty()) build_block_tables(c, blocks[0]);
+        pairs_to_edges(c, d_pairs, blocks.empty() ? 0 : n_pairs, min_af_pct, sums, ev[3], ev_end);
+        return;
+    }
+    if (n_pairs >= (1ll << 31)) throw CudaFail{"too many surviving pairs in one call"};  // as run_ani: 32-bit positions
+    const bool det = c->ci || c->detailed;  // pairs_to_edges leaves a detail record per edge
+    PoolRef<uint32_t> d_f(c->pool["table_blocks.flag"]), d_p(c->pool["table_blocks.pos"]);
+    PoolRef<unsigned long long> d_sel(c->pool["table_blocks.pairs"]);
+    PoolRef<uint32_t> d_sel_pos(c->pool["table_blocks.pair_pos"]), acc_pos(c->pool["table_blocks.edge_pos"]);
+    PoolRef<skb_edge> acc(c->pool["table_blocks.edges"]);
+    PoolRef<skb_edge_detail> acc_det(c->pool["table_blocks.detail"]);
+    d_f.reserve((size_t)n_pairs + 1, 0, c->st);
+    d_p.reserve((size_t)n_pairs + 1, 0, c->st);
+    d_sel.reserve((size_t)n_pairs, 0, c->st);
+    d_sel_pos.reserve((size_t)n_pairs, 0, c->st);
+    int64_t total = 0;
+    float ms_anchor = 0;
+    int anchor_launches = 0;
+    sums[0] = sums[1] = 0;
+    for (const std::vector<int32_t> &blk : blocks) {
+        build_block_tables(c, blk);
+        launch(c, pair_owned_flag_kernel, nblk((uint64_t)n_pairs, 256), 256, 0, c->d_seed_off.p, d_pairs, n_pairs,
+               (uint32_t)n, (uint32_t)blk.front(), (uint32_t)blk.back() + 1, d_f.p);
+        CK(cudaMemsetAsync(d_f.p + n_pairs, 0, 4, c->st));
+        exclusive_scan_u32(c, d_f.p, d_p.p, (size_t)n_pairs + 1);
+        launch(c, pair_keep_pos_kernel, nblk((uint64_t)n_pairs, 256), 256, 0, d_pairs, n_pairs, d_f.p, d_p.p, d_sel.p,
+               d_sel_pos.p);
+        uint32_t m = 0;
+        CK(cudaMemcpyAsync(&m, d_p.p + n_pairs, 4, cudaMemcpyDeviceToHost, c->st));
+        CK(cudaStreamSynchronize(c->st));
+        acc_pos.reserve((size_t)total + m, (size_t)total, c->st);  // the block's edges are at most its pairs
+        unsigned long long s[2];
+        pairs_to_edges(c, d_sel.p, m, min_af_pct, s, ev[3], ev[4], d_sel_pos.p, acc_pos.p + total);
+        sums[0] += s[0];
+        sums[1] += s[1];
+        ms_anchor += c->last_ms_anchor;
+        anchor_launches += c->last_anchor_launches;
+        const int64_t ne = c->last_n_edges;
+        if (ne) {
+            acc.reserve((size_t)(total + ne), (size_t)total, c->st);
+            CK(cudaMemcpyAsync(acc.p + total, c->last_dev_edges, (size_t)ne * sizeof(skb_edge), cudaMemcpyDeviceToDevice, c->st));
+            if (det) {
+                acc_det.reserve((size_t)(total + ne), (size_t)total, c->st);
+                CK(cudaMemcpyAsync(acc_det.p + total, c->last_dev_detail, (size_t)ne * sizeof(skb_edge_detail),
+                                   cudaMemcpyDeviceToDevice, c->st));
+            }
+        }
+        total += ne;
+    }
+    PoolRef<skb_edge> merged(c->pool["table_blocks.merged"]);
+    PoolRef<skb_edge_detail> merged_det(c->pool["table_blocks.merged_detail"]);
+    if (total) {
+        PoolRef<uint32_t> d_key_s(c->pool["table_blocks.pos_sorted"]);
+        PoolRef<uint32_t> d_idx(c->pool["table_blocks.idx"]), d_perm(c->pool["table_blocks.perm"]);
+        d_key_s.reserve((size_t)total, 0, c->st);
+        d_idx.reserve((size_t)total, 0, c->st);
+        d_perm.reserve((size_t)total, 0, c->st);
+        merged.reserve((size_t)total, 0, c->st);
+        launch(c, iota_u32_kernel, nblk((uint64_t)total, 256), 256, 0, total, d_idx.p);
+        int pos_bits = 1;  // positions < n_pairs
+        while (pos_bits < 32 && (1ll << pos_bits) < n_pairs) pos_bits++;
+        sort_pairs(c, acc_pos.p, d_key_s.p, d_idx.p, d_perm.p, (size_t)total, pos_bits);
+        launch(c, gather_kernel<skb_edge>, nblk((uint64_t)total, 256), 256, 0, acc.p, d_perm.p, total, merged.p);
+        if (det) {
+            merged_det.reserve((size_t)total, 0, c->st);
+            launch(c, gather_kernel<skb_edge_detail>, nblk((uint64_t)total, 256), 256, 0, acc_det.p, d_perm.p, total,
+                   merged_det.p);
+        }
+    }
+    CK(cudaEventRecord(ev_end, c->st));
+    CK(cudaEventSynchronize(ev_end));
+    c->last_dev_edges = merged.p;
+    c->last_dev_detail = det ? merged_det.p : nullptr;
+    c->last_n_edges = total;
+    c->last_ms_anchor = ms_anchor;
+    c->last_anchor_launches = anchor_launches;
+}
 
 // skb_triangle, skb_pairs_edges and skb_rect after their argument checks: `pairs(EdgePairs &)` checks the context's state
 // and leaves the pairs to evaluate (ms_screen), pairs_to_edges evaluates them (ms_ani), max_n > 0 cuts them to each
@@ -865,13 +1067,17 @@ int edge_call(skb_ctx *c, double min_af_pct, skb_edge **edges, int64_t *n_edges,
                                    "only (skb_set_ani_ci, skb_set_detailed, skb_set_ani_estimator)");
     const int64_t launches0 = c->launches;
     c->whole_triangle = -1;
+    c->blocks_last_call = 0;
     cudaEvent_t *ev = call_events(c);
     CK(cudaEventRecord(ev[0], c->st));
     EdgePairs p;
     const int rc = pairs(p);
     if (rc != SKB_OK) return rc;
     unsigned long long sums[2];
-    pairs_to_edges(c, p.d_pairs, p.n, min_af_pct, sums, ev[1], ev[2]);
+    if (c->on_demand)
+        pairs_to_edges_blocks(c, p.d_pairs, p.n, min_af_pct, sums, ev[1], ev[2]);
+    else
+        pairs_to_edges(c, p.d_pairs, p.n, min_af_pct, sums, ev[1], ev[2]);
     float ms_screen = 0, ms_ani = 0, ms_best_n = 0;
     CK(cudaEventElapsedTime(&ms_screen, ev[0], ev[1]));
     CK(cudaEventElapsedTime(&ms_ani, ev[1], ev[2]));
@@ -1035,6 +1241,12 @@ int skb_device_edges(skb_ctx *ctx, const skb_edge **dev_edges, int64_t *n_edges)
 }
 
 int64_t skb_launch_count(const skb_ctx *ctx) { return ctx ? ctx->launches : 0; }
+int skb_table_blocks(const skb_ctx *ctx, int32_t *on_demand, int32_t *blocks_last_call) {
+    if (!ctx) return SKB_EINVAL;
+    if (on_demand) *on_demand = ctx->on_demand ? 1 : 0;
+    if (blocks_last_call) *blocks_last_call = ctx->blocks_last_call;
+    return SKB_OK;
+}
 void *skb_stream(const skb_ctx *ctx) { return ctx ? (void *)ctx->st : nullptr; }
 void skb_free(void *p) { std::free(p); }
 
@@ -1048,6 +1260,8 @@ static int clear_impl(skb_ctx *ctx, bool keep_tables) {
         ctx->add_calls.clear();
         ctx->own_first = 0;
         ctx->own_count = -1;
+        ctx->on_demand = false;
+        ctx->block_budget = 0;
         if (!keep_tables) ctx->kept_n = 0;
         return SKB_OK;
     });
@@ -1192,22 +1406,24 @@ int skb_add_sequences(skb_ctx *ctx, int32_t n_files, const skb_packed *const *fi
 // The sparsest seed tables the device holds comfortably: a lookup is one sector read unless its bucket overflowed, and
 // at 0.5 records per bucket that is rare enough not to stall a warp (skb_probe.cuh).  SKB_TAB_X2 forces a density.
 static int table_density(skb_ctx *c, uint64_t own_seeds) {
-    if (c->tab_x2_forced) return c->tab_x2_forced;
     // decided once per sketch-DB size: cudaMemGetInfo takes a driver-wide lock and stalls for tens of ms whenever a
     // monitoring tool (nvidia-smi / NVML polling) holds it -- seen as 20-80 ms spikes of this call
-    if (c->x2_decided && c->x2_decided_seeds == own_seeds) return c->x2_decided;
-    size_t free_b = 0, total_b = 0;
-    CK(cudaMemGetInfo(&free_b, &total_b));
-    const double budget = std::min(0.35 * (double)total_b,
-                                   (double)free_b + (double)c->d_tab.cap * 8.0 - 40.0 * (double)(1ull << 30));
-    c->x2_decided = 1;
-    for (int x2 : {4, 2})
-        if (((double)own_seeds * x2 / 2 + (double)c->n()) * BUCKET * 8.0 <= budget) {
-            c->x2_decided = x2;
-            break;
-        }
-    c->x2_decided_seeds = own_seeds;
-    return c->x2_decided;
+    if (!c->x2_decided || c->x2_decided_seeds != own_seeds) {
+        size_t free_b = 0, total_b = 0;
+        CK(cudaMemGetInfo(&free_b, &total_b));
+        const double budget = std::min(0.35 * (double)total_b,
+                                       (double)free_b + (double)c->d_tab.cap * 8.0 - 40.0 * (double)(1ull << 30));
+        c->x2_decided = 1;
+        for (int x2 : {4, 2})
+            if (((double)own_seeds * x2 / 2 + (double)c->n()) * BUCKET * 8.0 <= budget) {
+                c->x2_decided = x2;
+                break;
+            }
+        c->x2_decided_seeds = own_seeds;
+        c->x2_budget = budget;
+        c->x2_room = (double)free_b + (double)c->d_tab.cap * 8.0;
+    }
+    return c->tab_x2_forced ? c->tab_x2_forced : c->x2_decided;
 }
 
 // Seed tables and repeat flags of the genomes [g0, n) at density tab_x2.  Only the genomes this context owns get a
@@ -1223,10 +1439,22 @@ static int build_seed_tables(skb_ctx *c, int32_t g0, bool reuse) {
     for (int32_t g = g0; g < n; g++) {
         const uint64_t ns = c->db.seed_off[g + 1] - c->db.seed_off[g];
         if (ns >= (1ull << 31)) return fail(c, SKB_ELIMIT, "genome has too many seeds");
-        buckets[g] = c->owns(g) ? (uint32_t)std::max<uint64_t>(2, ns * (uint64_t)c->tab_x2 / 2 + 1) : 0u;
+        buckets[g] = c->owns(g) ? table_buckets(c, g) : 0u;
         tab_off[g + 1] = tab_off[g] + (uint64_t)buckets[g] * BUCKET;
     }
     c->d_seed_off.upload(c->db.seed_off, g0, c->st);
+    if (c->on_demand) {
+        // the repeat flags of every genome (a query reads its own seeds' flags while only reference tables exist):
+        // the tables are built block by block for them and dropped; edge calls build the ones they need again
+        c->d_tab_off.reserve((size_t)n + 1, 0, c->st);
+        c->d_tab_buckets.reserve((size_t)n, 0, c->st);
+        std::vector<int32_t> ids(n - g0);
+        for (int32_t g = g0; g < n; g++) ids[g - g0] = g;
+        for (const std::vector<int32_t> &blk : table_blocks(c, ids)) build_block_tables(c, blk);
+        CK(cudaStreamSynchronize(c->st));
+        c->d_tab.release();  // the memory goes to the edge calls' blocks and their pair stage
+        return SKB_OK;
+    }
     c->d_tab_off.upload(tab_off, g0, c->st);
     c->d_tab_buckets.upload(buckets, g0, c->st);
     const uint64_t t0 = tab_off[g0], t1 = tab_off[n];
@@ -1339,6 +1567,11 @@ int skb_index(skb_ctx *ctx) {
         // tables of exactly the owned genomes are already in d_tab (built before the sketches were exchanged)
         const bool reuse = c->kept_n > 0 && c->kept_n == o1 - o0 && c->kept_seeds == own_seeds;
         c->tab_x2 = reuse ? c->kept_x2 : table_density(c, own_seeds);
+        // on-demand tables when the tables at that density, sized as table_density sizes them, exceed the budget; a
+        // context that owns part of the tables (skb_set_owned) keeps them resident
+        c->on_demand = !reuse && c->own_count < 0 &&
+                       ((double)own_seeds * c->tab_x2 / 2 + (double)n) * BUCKET * 8.0 > table_budget(c);
+        c->block_budget = 0;  // measured for the repeat flags' blocks now, and again by the first edge call (below)
         int rc = build_seed_tables(c, 0, reuse);
         if (rc != SKB_OK) return rc;
         c->kept_n = 0;
@@ -1385,6 +1618,7 @@ int skb_index(skb_ctx *ctx) {
         c->ix.n_indexed = n;
         c->ix.n_inv_genomes = n;
         c->ix.n_mkeys_indexed = nk;
+        c->block_budget = 0;  // the marker sort's scratch is allocated now
         c->indexed = true;
         return SKB_OK;
     });
@@ -1401,6 +1635,7 @@ int skb_index_seed_tables(skb_ctx *ctx) {
         const auto [o0, o1] = c->owned_in(0, n);
         const uint64_t own_seeds = c->db.seed_off[o1] - c->db.seed_off[o0];
         c->tab_x2 = table_density(c, own_seeds);
+        c->on_demand = false;
         const int rc = build_seed_tables(c, 0, false);
         if (rc != SKB_OK) return rc;
         CK(cudaStreamSynchronize(c->st));
@@ -1852,22 +2087,49 @@ int skb_pairs_detail(skb_ctx *ctx, const uint32_t *a, const uint32_t *b, int64_t
         if (!c->indexed || c->ix.n_indexed != c->n()) return fail(c, SKB_ESTATE, "call skb_index first");
         if (n == 0) return SKB_OK;
         std::vector<unsigned long long> hp((size_t)n);
+        std::vector<int32_t> ref((size_t)n);
         for (int64_t i = 0; i < n; i++) {
             if (a[i] >= (uint32_t)c->ix.n_indexed || b[i] >= (uint32_t)c->ix.n_indexed || a[i] == b[i])
                 return fail(c, SKB_EINVAL, "pair id out of range");
             hp[(size_t)i] = ((unsigned long long)a[i] << 32) | b[i];
             const uint64_t nsa = c->db.seed_off[a[i] + 1] - c->db.seed_off[a[i]], nsb = c->db.seed_off[b[i] + 1] - c->db.seed_off[b[i]];
-            if (!c->owns((int32_t)(nsb < nsa ? a[i] : b[i])))
+            ref[(size_t)i] = (int32_t)(nsb < nsa ? a[i] : b[i]);
+            if (!c->owns(ref[(size_t)i]))
                 return fail(c, SKB_ESTATE, "the reference genome of a pair is not owned by this context (skb_set_owned)");
         }
         PoolRef<unsigned long long> d_pairs(c->pool["skb_pairs_detail.d_pairs"]);
         PoolRef<PairOut> d_out(c->pool["skb_pairs_detail.d_out"]);
-        d_pairs.upload(hp, c->st);
-        d_out.reserve((size_t)n, 0, c->st);
-        run_ani(c, d_pairs.p, n, d_out.p);
         std::vector<PairOut> ho((size_t)n);
-        CK(cudaMemcpyAsync(ho.data(), d_out.p, (size_t)n * sizeof(PairOut), cudaMemcpyDeviceToHost, c->st));
-        CK(cudaStreamSynchronize(c->st));
+        // resident tables: every pair at once; on-demand tables: the pairs of one block of reference genomes at a time
+        // resident tables: every pair at once, in input order; on-demand tables: the pairs ordered by reference genome
+        // (ties in input order), one block of references -- a run of that order -- at a time
+        std::vector<int64_t> order((size_t)n);
+        for (int64_t i = 0; i < n; i++) order[(size_t)i] = i;
+        std::vector<std::vector<int32_t>> blocks{{}};
+        if (c->on_demand) {
+            std::stable_sort(order.begin(), order.end(), [&](int64_t x, int64_t y) { return ref[(size_t)x] < ref[(size_t)y]; });
+            std::vector<int32_t> refs;
+            for (const int64_t i : order)
+                if (refs.empty() || refs.back() != ref[(size_t)i]) refs.push_back(ref[(size_t)i]);
+            blocks = table_blocks(c, refs);
+        }
+        c->blocks_last_call = c->on_demand ? (int32_t)blocks.size() : 0;
+        size_t at0 = 0;
+        for (const std::vector<int32_t> &blk : blocks) {
+            size_t at1 = at0;  // the block's pairs: order[at0 .. at1)
+            while (at1 < order.size() && (!c->on_demand || ref[(size_t)order[at1]] <= blk.back())) at1++;
+            std::vector<unsigned long long> bp(at1 - at0);
+            for (size_t j = 0; j < bp.size(); j++) bp[j] = hp[(size_t)order[at0 + j]];
+            if (c->on_demand) build_block_tables(c, blk);
+            d_pairs.upload(bp, c->st);
+            d_out.reserve(bp.size(), 0, c->st);
+            run_ani(c, d_pairs.p, (int64_t)bp.size(), d_out.p);
+            std::vector<PairOut> bo(bp.size());
+            CK(cudaMemcpyAsync(bo.data(), d_out.p, bo.size() * sizeof(PairOut), cudaMemcpyDeviceToHost, c->st));
+            CK(cudaStreamSynchronize(c->st));
+            for (size_t j = 0; j < bo.size(); j++) ho[(size_t)order[at0 + j]] = bo[j];
+            at0 = at1;
+        }
         for (int64_t i = 0; i < n; i++) {
             const PairOut &o = ho[(size_t)i];
             skb_pair_detail &d = out[i];

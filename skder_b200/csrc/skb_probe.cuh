@@ -59,17 +59,8 @@ __device__ __forceinline__ int genome_of_warp(const uint64_t *__restrict__ off, 
     return g;
 }
 
-// one thread per seed record: insert into its genome's table (64-bit CAS; no deletions ever)
-__global__ void tab_insert_kernel(const uint64_t *__restrict__ seeds, uint64_t n_seeds,
-                                  const uint64_t *__restrict__ g_seed_off, int n_genomes, uint64_t *tab,
-                                  const uint64_t *__restrict__ g_tab_off, const uint32_t *__restrict__ g_tab_buckets,
-                                  uint64_t first /* records [first, n_seeds) are inserted */) {
-    uint64_t i = first + (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    const int g = genome_of_warp(g_seed_off, n_genomes, i < n_seeds ? i : n_seeds - 1);
-    if (i >= n_seeds) return;
-    const uint32_t nb = g_tab_buckets[g];
-    unsigned long long *T = reinterpret_cast<unsigned long long *>(tab + g_tab_off[g]);
-    const unsigned long long rec = seeds[i] | 2ull;  // both table flags clear (active low)
+// insert one table record into the table T of nb buckets (64-bit CAS; no deletions ever)
+__device__ __forceinline__ void tab_insert_rec(unsigned long long *T, uint32_t nb, unsigned long long rec) {
     uint32_t b = tab_home(seed_kmer(rec), nb);
     for (;;) {
         // occupancy from one 256-bit read (slots fill in order); .cg: other threads are inserting
@@ -86,6 +77,19 @@ __global__ void tab_insert_kernel(const uint64_t *__restrict__ seeds, uint64_t n
         if (a[BUCKET - 1] & 2ull) atomicAnd(&T[(size_t)b * BUCKET + BUCKET - 1], ~2ull);
         b = tab_next(b, nb);
     }
+}
+
+// one thread per seed record: insert into its genome's table
+__global__ void tab_insert_kernel(const uint64_t *__restrict__ seeds, uint64_t n_seeds,
+                                  const uint64_t *__restrict__ g_seed_off, int n_genomes, uint64_t *tab,
+                                  const uint64_t *__restrict__ g_tab_off, const uint32_t *__restrict__ g_tab_buckets,
+                                  uint64_t first /* records [first, n_seeds) are inserted */) {
+    uint64_t i = first + (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int g = genome_of_warp(g_seed_off, n_genomes, i < n_seeds ? i : n_seeds - 1);
+    if (i >= n_seeds) return;
+    const uint32_t nb = g_tab_buckets[g];
+    unsigned long long *T = reinterpret_cast<unsigned long long *>(tab + g_tab_off[g]);
+    tab_insert_rec(T, nb, seeds[i] | 2ull);  // both table flags clear (active low)
 }
 
 struct Bucket {
@@ -119,8 +123,23 @@ __device__ __forceinline__ int tab_count(const uint64_t *__restrict__ T, uint32_
     return c;
 }
 
-// flag seeds whose k-mer occurs more than max_mult times in their own genome (bit 1 of the seed record), and mark the
-// table records of every k-mer that occurs more than once (bit 1 of slots 0..2 of its home bucket, active low)
+// flag seed record i (s = seeds[i], km its k-mer) if its k-mer occurs more than max_mult times in its own genome (bit 1
+// of the seed record), and mark the table records of every k-mer that occurs more than once (bit 1 of slots 0..2 of its
+// home bucket, active low); T, nb: the genome's table
+__device__ __forceinline__ void rep_flag_seed(uint64_t *seeds, uint64_t i, uint64_t s, uint32_t km, uint64_t *T, uint32_t nb,
+                                              int max_mult) {
+    const int c = tab_count(T, nb, km, max_mult + 1);
+    if (c > max_mult) seeds[i] = s | 2ull;
+    if (c > 1) {  // rare.  Only bit 1 changes, which no concurrent tab_count looks at
+        unsigned long long *H = reinterpret_cast<unsigned long long *>(T) + (size_t)tab_home(km, nb) * BUCKET;
+        for (int k = 0; k < (int)BUCKET - 1; k++) {
+            const unsigned long long e = H[k];
+            if (e != TAB_EMPTY && seed_kmer(e) == km && (e & 2ull)) atomicAnd(&H[k], ~2ull);
+        }
+    }
+}
+
+// rep_flag_seed for every seed record [first, n_seeds)
 __global__ void rep_flag_kernel(uint64_t *seeds, uint64_t n_seeds, const uint64_t *__restrict__ g_seed_off,
                                 int n_genomes, uint64_t *tab,
                                 const uint64_t *__restrict__ g_tab_off, const uint32_t *__restrict__ g_tab_buckets,
@@ -131,15 +150,7 @@ __global__ void rep_flag_kernel(uint64_t *seeds, uint64_t n_seeds, const uint64_
     const uint64_t s = seeds[i];
     const uint32_t km = seed_kmer(s), nb = g_tab_buckets[g];
     uint64_t *T = tab + g_tab_off[g];
-    const int c = tab_count(T, nb, km, max_mult + 1);
-    if (c > max_mult) seeds[i] = s | 2ull;
-    if (c > 1) {  // rare.  Only bit 1 changes, which no concurrent tab_count looks at
-        unsigned long long *H = reinterpret_cast<unsigned long long *>(T) + (size_t)tab_home(km, nb) * BUCKET;
-        for (int k = 0; k < (int)BUCKET - 1; k++) {
-            const unsigned long long e = H[k];
-            if (e != TAB_EMPTY && seed_kmer(e) == km && (e & 2ull)) atomicAnd(&H[k], ~2ull);
-        }
-    }
+    rep_flag_seed(seeds, i, s, km, T, nb, max_mult);
 }
 
 // staged hit: (ref_pos << 1) | strand relation

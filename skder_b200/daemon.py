@@ -178,7 +178,7 @@ def serve(db_dir, device):
                         conn.send_bytes(json.dumps({"ok": False, "stale": True, "error": "database directory changed"}).encode())
                         stop = True
                     elif msg.get("op") == "ping":
-                        conn.send_bytes(json.dumps({"ok": True, "n": n_db}).encode())
+                        conn.send_bytes(json.dumps({"ok": True, "n": n_db, "table_blocks": cli.table_blocks(eng)}).encode())
                     elif msg.get("op") == "stop":
                         conn.send_bytes(json.dumps({"ok": True}).encode())
                         stop = True

@@ -285,6 +285,14 @@ class Engine:
     def launches(self):
         return self._L.skb_launch_count(self._h)
 
+    def table_blocks(self):
+        """(on_demand, blocks): whether the last index() chose on-demand seed tables -- the tables of all genomes exceed
+        the table budget (SKB_TABLE_BUDGET_MB caps it) -- and how many blocks of tables the last triangle / rect / search /
+        pairs_edges / pairs_detail call built (0 with resident tables).  DESIGN.md section 2."""
+        on, blocks = C.c_int32(), C.c_int32()
+        self._ck(self._L.skb_table_blocks(self._h, C.byref(on), C.byref(blocks)), "skb_table_blocks")
+        return bool(on.value), int(blocks.value)
+
     @property
     def stream(self):
         return self._L.skb_stream(self._h)
